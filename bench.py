@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the rl-rep update step on B200 (contract: see the task statement / DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one `agent.train(buffer, batch_size)` call = K_f feature iterations + critic + actor/alpha + Polyak.
 Default workload (BASELINE.json configs[1]): ctrlsac, HalfCheetah shapes (S=17, A=6), batch 256, feature_dim 2048,
@@ -20,6 +20,8 @@ The JSON line (rank 0):
   sharded      (state workloads) BASELINE configs[3]: ONE CTRL-SAC agent at global batch 16384 sharded by rows over all N
                ranks (N = 1 included, so the per-N lines form a strong-scaling curve) + `sharded_parity`, a small sharded
                update checked against the oracle on the global batch inside this run
+--dump-outputs DIR writes what the timed agent produced in its last timed update (see dump_outputs), so that two builds
+run with the same arguments, and hence the same inputs, can be compared output for output.
 N > 1 (torchrun): `value` is the population reading of the path -- independent agents, one per GPU, no collective in the
 data path; time = max over ranks, value = sum of updates / that time.
 `--impl reference` times the reference's own CPU implementation of the path (the oracle port with the as-written
@@ -37,6 +39,7 @@ import sys
 import tempfile
 import threading
 import time
+import zlib
 from pathlib import Path
 
 import numpy as np
@@ -180,6 +183,40 @@ def emit(line):
     out = _REAL_STDOUT or sys.stdout
     out.write(json.dumps(line) + "\n")
     out.flush()
+
+
+DUMP_BUDGET = 15_000_000  # float32 elements written by --dump-outputs: keeps a dump below 64 MB
+DUMP_WHOLE = 65_536  # tensors up to this many elements are always written whole
+
+
+def dump_outputs(out_dir, metrics, state):
+    """--dump-outputs: the metrics the last timed update returned (`metric.<name>.npy`, float64 scalars) and the agent's
+    parameters after it (`param.<name>.npy`, float32; float64 for log_alpha).
+
+    The dumped update is the last one of the last timed loop on the benched agent, which runs after the device-resident
+    loop that `value` times:
+      state agents   the end-to-end loop with noise_device="cuda" (torch's CUDA generator draws the noise; the
+                     device-resident loop uses host-drawn noise); the sharded agent: the end-to-end loop with host noise
+      pixel agents   the end-to-end loop with the frame stacks resident on the device
+    Every input of these loops is seeded, so runs with the same arguments dump the same update.
+
+    When the parameters exceed DUMP_BUDGET, each tensor larger than DUMP_WHOLE is reduced to a sample of its flattened
+    elements: the sorted distinct positions of draws from a generator seeded with the tensor's name, the same in every run
+    of the same workload."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for k, v in metrics.items():
+        np.save(out / f"metric.{k.replace('/', '.')}.npy", np.float64(v))
+    arrays = {k: v.detach().cpu().numpy() for k, v in state.items()}
+    small = sum(a.size for a in arrays.values() if a.size <= DUMP_WHOLE)
+    large = sum(a.size for a in arrays.values() if a.size > DUMP_WHOLE)
+    frac = min(1.0, max(0.0, DUMP_BUDGET - small) / max(large, 1))
+    for k, a in arrays.items():
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        if a.size > DUMP_WHOLE and frac < 1.0:
+            draws = np.random.default_rng(zlib.crc32(k.encode())).integers(0, a.size, int(a.size * frac))
+            a = a.reshape(-1)[np.unique(draws)]
+        np.save(out / f"param.{k.replace('/', '.')}.npy", a)
 
 
 def peaks():
@@ -440,6 +477,7 @@ def run_pixels(args, w, rank, world, local_rank):
         # (3) end to end with the frames already in HBM, as rlrep_b200.PixelReplayBuffer (the device-resident
         # EfficientReplayBuffer) hands them over: uint8 frame stacks are CUDA tensors, everything else stays on the host
         e2e_dev = []
+        last = info  # what the last timed update returned (--dump-outputs)
         if want_profile:
             is_u8 = lambda x: (isinstance(x, np.ndarray) and x.dtype == np.uint8) or \
                               (isinstance(x, torch.Tensor) and x.dtype == torch.uint8)
@@ -450,17 +488,19 @@ def run_pixels(args, w, rank, world, local_rank):
                 barrier()
                 t0 = time.perf_counter()
                 for i in range(args.steps):
-                    arm.step(dev_batches[i % 4], i)
+                    last = arm.step(dev_batches[i % 4], i)
                 barrier()
                 e2e_dev.append((time.perf_counter() - t0) * 1e3)
             del dev_batches
-        out = dict(dev_ms=median_of(dev), e2e_ms=median_of(e2e), dev_all=dev, e2e_all=e2e, clocks=clocks, info=info,
+        out = dict(dev_ms=median_of(dev), e2e_ms=median_of(e2e), dev_all=dev, e2e_all=e2e, clocks=clocks, info=info, last=last,
                    launches=getattr(agent, "gpu_launches_last_update", 0), arm=arm, batches=batches,
                    e2e_dev_ms=median_of(e2e_dev) if e2e_dev else None)
         return out
 
     res = measure(precision, True)
     arm, agent, D = res["arm"], res["arm"].agent, res["arm"].D
+    if args.dump_outputs and rank == 0:  # before the profiled updates below
+        dump_outputs(args.dump_outputs, res["last"], agent.state_dict())
     dev_ms, e2e_ms = res["dev_ms"], res["e2e_ms"]
     launches, clocks, info = res["launches"], res["clocks"], res["info"]
     e2e_dev_ms = res.get("e2e_dev_ms")
@@ -784,6 +824,7 @@ def time_state_agent(args, w, rank, world, local_rank, precision, barrier, repea
     # (3) the same end-to-end loop with the noise drawn by torch's CUDA generator (noise_device="cuda", the stream a
     # reference run on CUDA consumes): no host RNG, only the replay indices cross PCIe
     e2e_dn = []
+    last = info  # what the last timed train() call returned (--dump-outputs)
     if not sharded:
         agent.noise_device = "cuda"
         for _ in range(3):
@@ -792,12 +833,12 @@ def time_state_agent(args, w, rank, world, local_rank, precision, barrier, repea
             barrier()
             t0 = time.perf_counter()
             for _ in range(args.steps):
-                agent.train(buf, B)
+                last = agent.train(buf, B)
             barrier()
             e2e_dn.append((time.perf_counter() - t0) * 1e3)
         agent.noise_device = "cpu"
     return dict(agent=agent, buf=buf, dev_ms=median_of(dev), e2e_ms=median_of(e2e), dev_all=dev, e2e_all=e2e, clocks=clocks,
-                info=info, launches=agent.gpu_launches_last_train, sharded=sharded,
+                info=info, last=last, launches=agent.gpu_launches_last_train, sharded=sharded,
                 e2e_device_noise_ms=median_of(e2e_dn) if e2e_dn else None)
 
 
@@ -971,10 +1012,9 @@ def run_ours(args, w, rank, world, local_rank):
     sharded = bool(w.get("sharded"))
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
-    else:  # the sharded agent at N = 1 still goes through a (single-rank) process group and communicator
-        os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
-        os.environ.setdefault("MASTER_PORT", "29517")
-        dist.init_process_group("gloo", rank=0, world_size=1)
+    else:  # the sharded agent at N = 1 still goes through a (single-rank) process group and communicator; an in-process
+        #    store instead of a TCP one, so that runs sharing a host never compete for a port
+        dist.init_process_group("gloo", store=dist.HashStore(), rank=0, world_size=1)
     precision = args.precision or "tf32"
 
     def barrier():
@@ -991,6 +1031,8 @@ def run_ours(args, w, rank, world, local_rank):
         dev_ms, e2e_ms = t.tolist()
     h = res["agent"]._h
     ni, ne = h.n_idx, h.n_eps
+    if args.dump_outputs and rank == 0:  # before the profiled calls below, which train the agent further
+        dump_outputs(args.dump_outputs, res["last"], res["agent"].state_dict())
 
     roofline, top = None, []
     if sharded and rank != 0:  # the sharded update contains collectives: every rank has to take part in the profiled calls
@@ -1072,6 +1114,25 @@ def run_ours(args, w, rank, world, local_rank):
     dist.destroy_process_group()
 
 
+PIXEL_ALGS = ("drqv2", "mulvdrq", "ldiffsr")
+
+
+def default_counts(w, impl):
+    """(steps, warmup) of a run that does not give --steps / --warmup: 100 / 5, fewer steps where one step is slow.
+    An explicit --steps is always used as given, and so is an explicit --warmup, except that the CUDA paths warm up at
+    least 3 steps (eager call, graph capture, replay) and report the count they used."""
+    pixel = w["alg"] in PIXEL_ALGS
+    if impl == "reference":  # bounded samples of CPU work
+        if pixel:
+            return {"drqv2": 20, "mulvdrq": 8}.get(w["alg"], 3), 2
+        if w.get("sharded"):
+            return 2, 0  # ~17 TFLOP per update on the host cores
+        return (40 if w["alg"] == "ctrlsac" else 100), 5  # ctrlsac: ~0.5-2 s of CPU work per update
+    if w.get("population"):
+        return 20, 5
+    return (50 if pixel else 100), 5
+
+
 def main():
     # stdout carries the JSON line and nothing else: native libraries (NCCL's version banner ...) write to fd 1 directly,
     # so fd 1 is pointed at stderr for the duration of the run and the JSON line goes to the saved real stdout.
@@ -1081,8 +1142,9 @@ def main():
     os.dup2(2, 1)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
-    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps; default 100, fewer where one step is slow "
+                    "(see default_counts)")
+    ap.add_argument("--warmup", type=int, default=None, help="warm-up steps; default 5, at least 3 on the CUDA paths (see default_counts)")
     ap.add_argument("--repeats", type=int, default=5, help="the timed K-step loop is repeated this many times; the median is reported")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="ctrlsac_hc_b256", choices=list(WORKLOADS))
@@ -1091,27 +1153,34 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-alt-precision", action="store_true", help="skip the second (fp32 / tf32) figure")
     ap.add_argument("--no-sharded", action="store_true", help="skip the configs[3] section of the default workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the metrics of the last timed update and the parameters "
+                    "after it to DIR/<name>.npy (at most 64 MB; a fixed sample of larger parameter sets; which timed loop "
+                    "that is: see dump_outputs)")
     args = ap.parse_args()
     w = WORKLOADS[args.workload]
+    steps, warmup = default_counts(w, args.impl)
+    args.steps = steps if args.steps is None else args.steps
+    args.warmup = warmup if args.warmup is None else args.warmup
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs covers the CUDA implementation (--impl ours)")
+    if args.dump_outputs and w.get("population"):
+        # the members draw their noise from torch's one CPU generator from concurrent threads: which member receives which
+        # draws follows the thread schedule, so no two runs compute the same updates
+        ap.error("--dump-outputs: a population's updates differ from run to run, there is nothing to compare")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
-    if w["alg"] in ("drqv2", "mulvdrq", "ldiffsr"):
+    if w["alg"] in PIXEL_ALGS:
         if args.impl == "reference":
-            args.steps, args.warmup = min(args.steps, {"drqv2": 20, "mulvdrq": 8}.get(w["alg"], 3)), min(args.warmup, 2)
             run_pixel_reference(args, w, rank)
         elif w.get("population"):
-            args.steps = min(args.steps, 20)
             run_population(args, w, rank, world, local_rank)
         else:
-            args.steps = min(args.steps, 50)
             run_pixels(args, w, rank, world, local_rank)
         return
     if args.impl == "reference":
-        if w.get("sharded"):
-            args.steps, args.warmup = min(args.steps, 2), 0  # ~17 TFLOP per update on the host cores: a bounded sample
-        elif args.steps > 40 and w["alg"] == "ctrlsac":
-            args.steps = 40  # bounded sample: ~0.5-2 s of CPU work per update
         run_reference(args, w, rank, world)
         return
     run_ours(args, w, rank, world, local_rank)

@@ -10,6 +10,20 @@ import torch
 from oracle import rl_oracle as O
 
 GOLDEN = Path(__file__).resolve().parent / "golden"
+# Intra-op threads of the machine the fixtures were recorded on.  CPU kernels split their reductions by thread count, and
+# Adam's first step turns the last-bit differences of another split into +-lr moves (ldiffsr_b4 then misses its bar by up
+# to 2.8x at 1, 3 or 16 threads), so the oracle runs with the recording's thread count wherever the suite runs.
+GOLDEN_THREADS = 8
+
+
+@pytest.fixture(autouse=True)
+def golden_threads():
+    before = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(before)
+
+
 CASES = sorted(p.stem for p in GOLDEN.glob("*.npz") if not p.stem.startswith(("drqv2", "mulvdrq", "ldiffsr", "pixreplay")))
 DRQ_CASES = sorted(p.stem for p in GOLDEN.glob("drqv2*.npz"))
 MULV_CASES = sorted(p.stem for p in GOLDEN.glob("mulvdrq*.npz"))
