@@ -235,21 +235,13 @@ class GemmRunner {
   // inferred from the operands' addresses; the program is built on first use and cached by GEMM sequence).  A GEMM that
   // cannot join a chain (CUDA-core shapes) closes the chain recorded so far and runs on `s` in program order.  Callers
   // must not launch kernels that consume a recorded GEMM's output before end_chain().
-  bool chains_enabled() const { return prec_ == PREC_TF32 && chains_on_; }
+  bool chains_enabled() const { return prec_ == PREC_TF32; }
   void begin_chain(cudaStream_t s);
   void end_chain();
-  // Row operation (gemm.cuh RowOp) in program order with the recorded GEMMs: true when it was recorded into the open
-  // chain, false when no chain is being recorded -- the caller then launches the stand-alone kernel of the same operation.
-  bool row_op(const RowOp& op);
   bool recording() const { return recording_; }
 
  private:
   void flush_chain();
-  bool chains_on_ = true;
-  // RLREP_CHAIN_ROWOPS=1 lets row operations ride in the chain.  Off by default: measured on B200 (ctrlsac B = 256) one
-  // chain with gather + head levels is 0.809 ms/update against 0.787 ms with the two stand-alone kernels between two
-  // chains -- a level transition inside the chain costs more than a kernel boundary in a CUDA graph (DESIGN.md section 5)
-  bool row_ops_on_ = false;
   bool recording_ = false;
   cudaStream_t chain_stream_ = nullptr;
   std::vector<GemmArgs> pending_;
@@ -262,7 +254,6 @@ class GemmRunner {
   // shape -- the first call of every update path runs eagerly, so never inside a graph capture
   float* kg_ws_ = nullptr;
   size_t kg_ws_floats_ = 0;
-  bool kg_on_ = true;  // RLREP_GEMM_KGROUPS=0 disables
   std::unordered_map<std::string, TcGemmPlan> plans_;
 };
 

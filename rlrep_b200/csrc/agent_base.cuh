@@ -3,7 +3,6 @@
 // noise, metrics read-back, and the eager -> capture -> replay protocol of train().
 #pragma once
 #include "staging.cuh"
-#include <cstdlib>
 
 #include "agent.cuh"
 
@@ -325,7 +324,7 @@ class SacBase : public Agent {
   void actor_backward(Mat obs, const float* eps) {
     const Linear l0 = a0_.view(actor_g_), l1 = a1_.view(actor_g_), l2 = a2_.view(actor_g_);
     // dgrad chain on the main stream; weight / bias gradients trail it on an aux branch
-    cudaStream_t w = use_aux_ ? aux(1) : stream;
+    cudaStream_t w = aux(1);
     launch_actor_sample_bwd(head_, LDH_, B_, A_, eps, dsa_ + S_, LDSA_, dlogp_, dhead_, LDH_, stream);
     wait_for(w, mark(stream));
     linear_wgrad(gemm_, w, B_, Mat{dhead_, LDH_}, Mat{ah2_, AH_}, l2, Mat(), 0, false);
@@ -340,7 +339,7 @@ class SacBase : public Agent {
                               bias_job(B_, Mat{dah1_, AH_}, l0)};
       launch_colreduce_multi(jobs, 3, w);
     }
-    if (use_aux_) join_aux(1, stream);
+    join_aux(1, stream);
   }
   void actor_adam() {
     launch_adam_polyak(actor_g_.p, actor_g_.g, actor_g_.m, actor_g_.v, actor_g_.n, &ctl->actor, nullptr, 0, 0.f,
@@ -361,28 +360,15 @@ class SacBase : public Agent {
   int S_ = 0, A_ = 0, B_ = 0, AH_ = 0, R_ = 0, LDH_ = 0, LDSA_ = 0;
   cudaStream_t side_ = nullptr;
   cudaStream_t aux_[2] = {nullptr, nullptr};
-  double aux_share_ = [] {
-    const char* e = std::getenv("RLREP_AUX_SHARE");
-    return e ? std::atof(e) : 0.25;
-  }();
-  bool use_aux_ = [] {
-    const char* e = std::getenv("RLREP_USE_AUX");
-    return e ? std::atoi(e) != 0 : true;
-  }();
+  static constexpr double kAuxShare = 0.25;  // SM share the GEMMs on an aux stream plan for
   // Batches up to this size run their GEMM groups as chains (gemm_chain.cuh); larger batches are throughput- rather than
   // latency-bound and keep one kernel per GEMM.
-  int chain_max_batch_ = [] {
-    const char* e = std::getenv("RLREP_CHAIN_MAX_B");
-    return e ? std::atoi(e) : 512;
-  }();
-  bool chained() const { return gemm_.chains_enabled() && B_ <= chain_max_batch_; }
+  static constexpr int kChainMaxBatch = 512;
+  bool chained() const { return gemm_.chains_enabled() && B_ <= kChainMaxBatch; }
   std::vector<cudaEvent_t> events_;
   size_t ev_next_ = 0;
   bool serial_ = false;
-  double dual_share_ = [] {
-    const char* e = std::getenv("RLREP_DUAL_SHARE");
-    return e ? std::atof(e) : 0.5;
-  }();
+  double dual_share_ = 0.5;  // SM share inside fork() / join()
   DeviceArena arena_;
   GemmRunner gemm_;
   GraphReplay graph_;

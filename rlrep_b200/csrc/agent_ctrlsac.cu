@@ -179,8 +179,8 @@ class CtrlSacAgent final : public SacBase {
       gemm_.run(a, s0);
     }
     // the dgrad chain is the critical path; weight / bias gradients trail it on an aux stream
-    cudaStream_t w0 = use_aux_ ? aux(0) : s0, w1 = use_aux_ ? aux(1) : s1;
-    const double share = dual_share_, wshare = use_aux_ ? aux_share_ : dual_share_;
+    cudaStream_t w0 = aux(0), w1 = aux(1);
+    const double share = dual_share_, wshare = kAuxShare;
     wait_for(w0, mark(s0));
     gemm_.set_sm_share(wshare);
     linear_wgrad(gemm_, w0, B_, Mat{dzphi_, D_}, Mat{h2_, H_}, l3, Mat(), 0, false);
@@ -225,10 +225,8 @@ class CtrlSacAgent final : public SacBase {
                         bias_job(B_, Mat{dg1_, H_}, n1)};
       launch_colreduce_multi(jobs, 3, w1);
     }
-    if (use_aux_) {
-      join_aux(0, s0);
-      join_aux(1, s0);
-    }
+    join_aux(0, s0);
+    join_aux(1, s0);
     join();
     // ---- one fused Adam over phi | mu | theta, plus Polyak of phi_target (:242-244, :253-255)
     launch_adam_polyak(feat_g_.p, feat_g_.g, feat_g_.m, feat_g_.v, feat_g_.n, &ctl->feat[k],
@@ -240,25 +238,16 @@ class CtrlSacAgent final : public SacBase {
   // Same arithmetic, same kernels for everything that is not a GEMM; every group of GEMMs between two elementwise kernels
   // runs as ONE persistent chain kernel (gemm_chain.cuh) on the main stream instead of one launch per GEMM on up to four
   // streams: 57 launches per update instead of 149, and a dependent GEMM starts when its input tiles are complete.
-  // The replay gather, both towers, the logits, the contrastive head and the whole backward pass are ONE chain launch: the
-  // gather and the head ride in the chain as row operations (gemm.cuh RowOp) between the GEMMs they feed.
+  // The feature step is two chains: both towers and the logits, then the whole backward pass; the replay gather runs before
+  // the first and the contrastive head between the two as stand-alone kernels.
   void feature_step_chained(int k, Ring& ring) {  // ctrlsac_agent.py:213-251
     const Linear l1 = p1_.view(feat_g_), l2 = p2_.view(feat_g_), l3 = p3_.view(feat_g_);
     const Linear n1 = m1_.view(feat_g_), n2 = m2_.view(feat_g_), n3 = m3_.view(feat_g_);
     const Linear th = th_.view(feat_g_);
     const float inv_b = 1.f / (float)B_;
     cudaStream_t s0 = stream;
+    launch_gather(ring.data, R_ / 4, idx_dev_ + (size_t)k * B_, B_, batch_, s0);
     gemm_.begin_chain(s0);
-    {
-      RowOp op;
-      op.kind = ROWOP_GATHER;
-      op.rows = B_;
-      op.ring = ring.data;
-      op.idx = idx_dev_ + (size_t)k * B_;
-      op.out = batch_;
-      op.rec4 = R_ / 4;
-      if (!gemm_.row_op(op)) launch_gather(ring.data, R_ / 4, idx_dev_ + (size_t)k * B_, B_, batch_, s0);
-    }
     phi_forward(s0, sa(), Mat(), 0, zphi_, h1_, h2_);
     linear_fwd(gemm_, s0, B_, s2(), n1, ACT_ELU, g1_, H_);
     linear_fwd(gemm_, s0, B_, Mat{g1_, H_}, n2, ACT_ELU, g2_, H_);
@@ -271,25 +260,11 @@ class CtrlSacAgent final : public SacBase {
       a.C = logits_; a.ldc = B_;
       gemm_.run(a, s0);
     }
-    {  // row log-sum-exp / CE gradient (logits_ then holds dL/dlogits), reward head and the loss metrics
-      RowOp op;
-      op.kind = ROWOP_CTRL_HEAD;
-      op.rows = B_;
-      op.logits = logits_; op.ld = B_; op.cols = B_; op.diag_off = 0;
-      op.inv_batch = inv_b;
-      op.z = zphi_; op.ldz = D_; op.D = D_;
-      op.theta_w = th.W; op.theta_b = th.b;
-      op.reward = reward(); op.ld_r = R_;
-      op.loss_rows = loss_rows_; op.pred = rpred_; op.dpred = drp_;
-      op.metrics = metrics_dev_ + 0;
-      op.counter = head_ctr_;
-      if (!gemm_.row_op(op)) {
-        gemm_.end_chain();
-        launch_contrastive_head(logits_, B_, B_, B_, 0, inv_b, zphi_, D_, D_, th.W, th.b, reward(), R_, loss_rows_, rpred_,
-                                drp_, metrics_dev_ + 0, head_ctr_, s0);
-        gemm_.begin_chain(s0);
-      }
-    }
+    gemm_.end_chain();
+    // row log-sum-exp / CE gradient (logits_ then holds dL/dlogits), reward head and the loss metrics
+    launch_contrastive_head(logits_, B_, B_, B_, 0, inv_b, zphi_, D_, D_, th.W, th.b, reward(), R_, loss_rows_, rpred_, drp_,
+                            metrics_dev_ + 0, head_ctr_, s0);
+    gemm_.begin_chain(s0);
     {  // d z_phi = G mu + drp (x) theta.w
       GemmArgs a;
       a.M = B_; a.N = D_; a.K = B_;
@@ -421,15 +396,13 @@ class CtrlSacAgent final : public SacBase {
     const float* eps = eps_dev_;
     cudaStream_t s0 = stream, s1 = side();
     fork();
-    if (use_aux_) {
-      // Hoisted out of the actor step: a_pi ~ pi(s) and frozen_phi(s, a_pi) read only the actor, phi, the batch and the
-      // noise -- nothing the critic step writes -- so they run beside it on an aux branch; the actor step joins it
-      // before it evaluates the UPDATED critic on these features (reference order, ctrlsac_agent.py:299-305).
-      cudaStream_t a0 = aux(0);
-      wait_for(a0, mark(s0));
-      const Mat spi = actor_forward_cat(Mat{batch_, R_}, eps_dev_ + (size_t)B_ * A_, cat_pi_, logp_, a0, /*set=*/0);
-      phi_forward(a0, spi, Mat(), 0, zpi_, hc1_, hc2_);
-    }
+    // Hoisted out of the actor step: a_pi ~ pi(s) and frozen_phi(s, a_pi) read only the actor, phi, the batch and the
+    // noise -- nothing the critic step writes -- so they run beside it on an aux branch; the actor step joins it
+    // before it evaluates the UPDATED critic on these features (reference order, ctrlsac_agent.py:299-305).
+    cudaStream_t a0 = aux(0);
+    wait_for(a0, mark(s0));
+    const Mat spi = actor_forward_cat(Mat{batch_, R_}, eps_dev_ + (size_t)B_ * A_, cat_pi_, logp_, a0, /*set=*/0);
+    phi_forward(a0, spi, Mat(), 0, zpi_, hc1_, hc2_);
     // main stream: a' ~ pi(s'), frozen_phi_target(s', a'), target critic
     const Mat s2a = actor_forward_cat(s2(), eps, cat_next_, logp2_, s0, /*set=*/1);
     phi_forward(s0, s2a, Mat(), 0, zmu_, h1_, h2_);  // zmu_ is free after the feature loop
@@ -459,12 +432,7 @@ class CtrlSacAgent final : public SacBase {
   void actor_step() {  // ctrlsac_agent.py:295-325
     const float* eps = eps_dev_ + (size_t)B_ * A_;
     const Mat s{batch_, R_};
-    if (use_aux_) {
-      join_aux(0, stream);  // a_pi, log pi and frozen_phi(s, a_pi) were computed beside the critic step
-    } else {
-      const Mat spi = actor_forward_cat(s, eps, cat_pi_, logp_);
-      phi_forward(stream, spi, Mat(), 0, zpi_, hc1_, hc2_);  // frozen_phi(s, a_pi)
-    }
+    join_aux(0, stream);  // a_pi, log pi and frozen_phi(s, a_pi) were computed beside the critic step
     critic_forward(stream, zpi_, false, hid_, q1_, q2_);
     launch_actor_alpha_loss(q1_, q2_, logp_, B_, (float)(-A_), cfg.learn_alpha, ctl, dq1_, dq2_, dlogp_,
                             metrics_dev_ + 7, stream);

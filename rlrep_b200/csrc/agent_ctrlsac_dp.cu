@@ -17,16 +17,10 @@
 // Kernels are the single-GPU ones; b = 2048 rows per rank makes every GEMM throughput-bound, so the step runs eagerly
 // (no graph).
 //
-// Overlap (round 2).  One all-gather of mu_all (134 MB at 8 x 2048 rows) followed by one [b, Bg] logits GEMM leaves the
-// NVLink transfer exposed (nothing else can run: the logits need mu_all), and likewise the reduce-scatter behind the
-// d mu_all GEMM.  Both are pipelined in S ROW SLICES of the rank's batch: slice s of every rank's mu is gathered on a
-// communication stream while the logits columns of slice s-1 are being computed, and the d mu_all rows of slice s are
-// reduce-scattered while slice s+1 is computed.  The global column order of the logits becomes (slice, rank, row in
-// slice) instead of (rank, row) -- a permutation of the softmax axis, applied consistently to mu_all, G and d mu_all, so
-// every buffer stays contiguous, nothing is accumulated and the result is unchanged; only the column of a row's positive
-// moves (ce_rows: diag_blk / diag_stride).
-#include <algorithm>
-
+// Overlap.  The all-gather of mu runs on a communication stream while phi's forward runs on the main stream, and the
+// reduce-scatter of d mu_all while d z_phi and the phi backward are computed.  Pipelining the collectives in row slices
+// of the rank's batch was measured on 8 x B200 (DESIGN.md section 6): 1 slice 7.45 ms / update, 2 slices 7.61, 4 slices
+// 7.94 -- the smaller collectives lose more bandwidth, and take more SMs from the concurrent GEMMs, than the overlap wins.
 #include "agent_base.cuh"
 #include "comm.cuh"
 
@@ -44,15 +38,6 @@ class CtrlSacShardedAgent final : public SacBase {
     N_ = comm_->world;
     rank_ = comm_->rank;
     Bg_ = B_ * N_;
-    // row slices of the collectives' pipeline: slice rows must stay a multiple of 32 (MN-major GEMM operands)
-    // measured on 8 x B200 (DESIGN.md section 6): 1 slice 7.45 ms / update, 2 slices 7.61, 4 slices 7.94 -- the smaller
-    // collectives lose more bandwidth, and take more SMs from the concurrent GEMMs, than the overlap wins; the pipeline
-    // stays available (RLREP_DP_SLICES) but is off by default
-    int want_slices = 1;
-    if (const char* e = std::getenv("RLREP_DP_SLICES")) want_slices = std::max(1, std::atoi(e));
-    SL_ = 1;
-    for (int cand : {8, 4, 2})
-      if (cand <= want_slices && B_ % cand == 0 && (B_ / cand) % 32 == 0) { SL_ = cand; break; }
     cfg.use_graph = 0;
     dual_share_ = 1.0;  // throughput-bound GEMMs: plan each one for the whole GPU even when two branches overlap
     RLREP_CHECK(K_ >= 1 && K_ <= kMaxFeatureSteps, "extra_feature_steps out of range");
@@ -154,52 +139,45 @@ class CtrlSacShardedAgent final : public SacBase {
     const Linear th = th_.view(feat_g_);
     const float inv_bg = 1.f / (float)Bg_;
     cudaStream_t s = stream, s1 = side();
-    // mu on the side stream, phi on the main stream; the all-gather of mu runs slice by slice on the communication
-    // stream, and the logits columns of a slice are computed as soon as that slice has arrived.  Every rank issues the
-    // collectives in the same host order, which is all NCCL asks for.
+    // mu on the side stream, phi on the main stream; the all-gather of mu runs on the communication stream.  Every rank
+    // issues the collectives in the same host order, which is all NCCL asks for.
     cudaStream_t cs = aux(0);
-    const int bs = B_ / SL_;      // rows per slice on this rank
-    const int gs = Bg_ / SL_;     // columns (global rows) per slice
     fork();
     linear_fwd(gemm_, s1, B_, s2(), n1, ACT_ELU, g1_, H_);
     linear_fwd(gemm_, s1, B_, Mat{g1_, H_}, n2, ACT_ELU, g2_, H_);
     linear_fwd(gemm_, s1, B_, Mat{g2_, H_}, n3, ACT_TANH, zmu_, D_);
     wait_for(cs, mark(s1));
-    cudaEvent_t gathered[8];
-    for (int sl = 0; sl < SL_; ++sl) {  // slice sl of mu_all: rank r's rows [sl * bs, (sl + 1) * bs) at block offset r * bs
-      comm_->all_gather(zmu_ + (size_t)sl * bs * D_, zmu_all_ + (size_t)sl * gs * D_, (size_t)bs * D_, cs);
-      gathered[sl] = mark(cs);
-    }
+    comm_->all_gather(zmu_, zmu_all_, (size_t)B_ * D_, cs);  // rank r's rows at row offset r * b of mu_all
+    cudaEvent_t gathered = mark(cs);
     phi_forward(sa(), Mat(), 0, zphi_);
-    for (int sl = 0; sl < SL_; ++sl) {  // logits_local[i, sl * gs + j] = <phi_i, mu_all_slice_j>
-      wait_for(s, gathered[sl]);
+    wait_for(s, gathered);
+    {  // logits_local[i, j] = <phi_i, mu_all_j>
       GemmArgs a;
-      a.M = B_; a.N = gs; a.K = D_;
+      a.M = B_; a.N = Bg_; a.K = D_;
       a.A = zphi_; a.lda = D_;
-      a.B = zmu_all_ + (size_t)sl * gs * D_; a.ldb = D_;
-      a.C = logits_ + (size_t)sl * gs; a.ldc = Bg_;
+      a.B = zmu_all_; a.ldb = D_;
+      a.C = logits_; a.ldc = Bg_;
       gemm_.run(a, s);
     }
     join();
-    // positives: local row i = (slice, t) sits at column slice * gs + rank * bs + t
-    launch_ce_rows(logits_, Bg_, B_, Bg_, rank_ * bs, inv_bg, loss_rows_, s, bs, gs);
+    // positives: local row i sits at column rank * b + i
+    launch_ce_rows(logits_, Bg_, B_, Bg_, rank_ * B_, inv_bg, loss_rows_, s);
     launch_rowdot(zphi_, D_, B_, D_, th.W, th.b, rpred_, s);
     launch_feature_loss_finalize(loss_rows_, B_, rpred_, reward(), R_, inv_bg, drp_, metrics_dev_ + 0, s);
-    // every rank's contribution to d mu of ALL rows, slice by slice: G_local[:, slice]^T phi_local -> reduce-scatter of the
-    // slice on the communication stream while the next slice (and then d z_phi and the phi backward) is computed
-    cudaEvent_t scattered = nullptr;
-    for (int sl = 0; sl < SL_; ++sl) {
+    // every rank's contribution to d mu of ALL rows: G_local^T phi_local -> reduce-scatter on the communication stream
+    // while d z_phi and the phi backward are computed
+    {
       GemmArgs a;
-      a.M = gs; a.N = D_; a.K = B_;
-      a.A = logits_ + (size_t)sl * gs; a.lda = Bg_; a.a_mn = true;
+      a.M = Bg_; a.N = D_; a.K = B_;
+      a.A = logits_; a.lda = Bg_; a.a_mn = true;
       a.B = zphi_; a.ldb = D_; a.b_mn = true;
-      a.C = dmu_all_ + (size_t)sl * gs * D_; a.ldc = D_;
+      a.C = dmu_all_; a.ldc = D_;
       gemm_.run(a, s);
-      wait_for(cs, mark(s));
-      comm_->reduce_scatter(dmu_all_ + (size_t)sl * gs * D_, dzmu_ + (size_t)sl * bs * D_, (size_t)bs * D_, cs);
-      scattered = mark(cs);
     }
-    {  // d z_phi = G_local mu_all + drp (x) theta.w   (the same column permutation on both operands)
+    wait_for(cs, mark(s));
+    comm_->reduce_scatter(dmu_all_, dzmu_, (size_t)B_ * D_, cs);
+    cudaEvent_t scattered = mark(cs);
+    {  // d z_phi = G_local mu_all + drp (x) theta.w
       GemmArgs a;
       a.M = B_; a.N = D_; a.K = Bg_;
       a.A = logits_; a.lda = Bg_;
@@ -297,7 +275,7 @@ class CtrlSacShardedAgent final : public SacBase {
   }
 
   Comm* comm_ = nullptr;
-  int H_ = 0, D_ = 0, K_ = 0, N_ = 1, rank_ = 0, Bg_ = 0, SL_ = 1, off_r_ = 0, off_d_ = 0, off_s2_ = 0;
+  int H_ = 0, D_ = 0, K_ = 0, N_ = 1, rank_ = 0, Bg_ = 0, off_r_ = 0, off_d_ = 0, off_s2_ = 0;
   ParamGroup feat_g_, crit_g_;
   LinearSlot p1_, p2_, p3_, m1_, m2_, m3_, th_, c14_, c2_, c5_;
   float *h1_ = nullptr, *h2_ = nullptr, *g1_ = nullptr, *g2_ = nullptr, *zphi_ = nullptr, *zmu_ = nullptr;

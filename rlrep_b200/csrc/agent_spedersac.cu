@@ -145,14 +145,12 @@ class SpederSacAgent final : public SacBase {
     const float* eps = eps_dev_;
     cudaStream_t s0 = stream, s1 = side();
     fork();
-    if (use_aux_) {
-      // Hoisted out of the actor step (see agent_ctrlsac.cu): a_pi ~ pi(s) and phi(s, a_pi) read nothing the critic step
-      // writes, so they run beside it on an aux branch; the actor step joins before it evaluates the updated critic.
-      cudaStream_t a0 = aux(0);
-      wait_for(a0, mark(s0));
-      const Mat spi = actor_forward_cat(Mat{batch_, R_}, eps_dev_ + (size_t)B_ * A_, cat_pi_, logp_, a0, /*set=*/0);
-      trunk_forward(gemm_, a0, B_, phi_, feat_g_, false, spi, Mat(), 0, phi_acts_c_, zpi_, D_);
-    }
+    // Hoisted out of the actor step (see agent_ctrlsac.cu): a_pi ~ pi(s) and phi(s, a_pi) read nothing the critic step
+    // writes, so they run beside it on an aux branch; the actor step joins before it evaluates the updated critic.
+    cudaStream_t a0 = aux(0);
+    wait_for(a0, mark(s0));
+    const Mat spi = actor_forward_cat(Mat{batch_, R_}, eps_dev_ + (size_t)B_ * A_, cat_pi_, logp_, a0, /*set=*/0);
+    trunk_forward(gemm_, a0, B_, phi_, feat_g_, false, spi, Mat(), 0, phi_acts_c_, zpi_, D_);
     const Mat s2a = actor_forward_cat(s2(), eps, cat_next_, logp2_, s0, /*set=*/1);
     trunk_forward(gemm_, s0, B_, phi_, feat_g_, false, s2a, Mat(), 0, phi_acts_, zmu_, D_);
     critic_.forward(gemm_, s0, crit_g_, /*target=*/true, 0, zmu_);
@@ -169,12 +167,7 @@ class SpederSacAgent final : public SacBase {
   void actor_step() {  // spedersac_agent.py:259-289
     const float* eps = eps_dev_ + (size_t)B_ * A_;
     const Mat s{batch_, R_};
-    if (use_aux_) {
-      join_aux(0, stream);
-    } else {
-      const Mat spi = actor_forward_cat(s, eps, cat_pi_, logp_);
-      trunk_forward(gemm_, stream, B_, phi_, feat_g_, false, spi, Mat(), 0, phi_acts_c_, zpi_, D_);
-    }
+    join_aux(0, stream);
     critic_.forward(gemm_, stream, crit_g_, false, 0, zpi_);
     launch_actor_alpha_loss(critic_.q[0], critic_.q[0] + B_, logp_, B_, (float)(-A_), cfg.learn_alpha, ctl, dq_,
                             dq_ + B_, dlogp_, metrics_dev_ + 7, stream);

@@ -10,11 +10,10 @@
 //     own grid (the halo kernel, gemm_tc_kernel.cuh: one TMA box per tile, nine taps as shifted UMMA descriptors, valid
 //     rows stored compactly); data gradient = implicit full correlation on a zero-padded grid (conv_implicit.cu); weight
 //     gradient = a GEMM whose B operand reads the input map through a shifted 4-D TMA view (GemmArgs::conv_wgrad_hi).
-//   * strict-fp32 mode and RLREP_CONV_V1 / RLREP_CONV_WGRAD_V1: round 1's explicit im2col / folded-GEMM / col2im lowering.
+//   * strict-fp32 mode and batches that are not a multiple of 4: layers 2-4 run forward as explicit im2col + GEMM and their
+//     weight gradient as a folded GEMM over the column matrix; the data gradient is the implicit full correlation.
 #include "conv.cuh"
 #include "layout.cuh"
-
-#include <cstdlib>
 
 #include <algorithm>
 
@@ -81,33 +80,6 @@ __global__ void im2col_nhwc32_kernel(const float4* __restrict__ act, int B, int 
   }
 }
 
-// dX[b, iy, ix, c] = relu'(X) * sum over taps of dcol[(b, iy - ky, ix - kx), tap, c]   (gather form: deterministic)
-__global__ void col2im_nhwc32_kernel(const float4* __restrict__ dcol, const float4* __restrict__ x, int B, int H, int Ho,
-                                     float4* __restrict__ dx) {
-  const long long total = (long long)B * H * H * 8;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-    const int c4 = (int)(i & 7);
-    const long long pix = i >> 3;
-    const int ix = (int)(pix % H), iy = (int)((pix / H) % H), b = (int)(pix / ((long long)H * H));
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-    for (int ky = 0; ky < 3; ++ky) {
-      const int oy = iy - ky;
-      if (oy < 0 || oy >= Ho) continue;
-#pragma unroll
-      for (int kx = 0; kx < 3; ++kx) {
-        const int ox = ix - kx;
-        if (ox < 0 || ox >= Ho) continue;
-        const float4 g = dcol[(((long long)b * Ho + oy) * Ho + ox) * 72 + (ky * 3 + kx) * 8 + c4];
-        acc.x += g.x; acc.y += g.y; acc.z += g.z; acc.w += g.w;
-      }
-    }
-    const float4 xv = x[i];
-    dx[i] = make_float4(xv.x > 0.f ? acc.x : 0.f, xv.y > 0.f ? acc.y : 0.f, xv.z > 0.f ? acc.z : 0.f,
-                        xv.w > 0.f ? acc.w : 0.f);
-  }
-}
-
 // dW[o, k] = sum_p C[p*32 + o, p*ldk + k]: the diagonal blocks of the folded weight-gradient GEMM (see backward())
 __global__ void diag_block_sum_kernel(const float* __restrict__ C, int ldc, int P, int ldk, float* __restrict__ dW,
                                       int ld_dw) {
@@ -141,10 +113,7 @@ ConvEncoder::ConvEncoder(int batch, int in_channels, int height, Precision prec,
   for (int l = 1; l < 4; ++l) conv_[l] = add_linear(g_, "convnet." + std::to_string(2 * l), 32, 288);
   if (with_target) g_.n_target = g_.n;
   g_.want(arena_);
-  // RLREP_CONV_V1=1 keeps the explicit  dcol = dY W  +  col2im  data gradient (A/B runs); default: implicit
-  implicit_dgrad_ = !(std::getenv("RLREP_CONV_V1") && std::atoi(std::getenv("RLREP_CONV_V1")) != 0);
-  implicit_wgrad_ = implicit_dgrad_ && prec == PREC_TF32 && B_ % 4 == 0 &&
-                    !(std::getenv("RLREP_CONV_WGRAD_V1") && std::atoi(std::getenv("RLREP_CONV_WGRAD_V1")) != 0);
+  implicit_wgrad_ = prec == PREC_TF32 && B_ % 4 == 0;
   arena_.want(&col_[0], rows(0) * ldk1_);
   if (!implicit_wgrad_)  // 1.2 GB at B = 256 that the implicit path never allocates
     for (int l = 1; l < 4; ++l) arena_.want(&col_[l], rows(l) * 288);
@@ -153,8 +122,7 @@ ConvEncoder::ConvEncoder(int batch, int in_channels, int height, Precision prec,
     arena_.want(&act_[l], (rows(l) + 2 * hw_[l] + 8) * 32);
     arena_.want(&dact_[l], rows(l) * 32);
   }
-  if (implicit_dgrad_) corr_.want(arena_, B_, hw_[1]);
-  else arena_.want(&dcol_, rows(1) * 288);
+  corr_.want(arena_, B_, hw_[1]);
   arena_.want(&bias_partial_, kBiasChunks * 32);
   arena_.want(&wfold_, (size_t)32 * kFold * 288 * kFold);
   arena_.commit();
@@ -170,7 +138,7 @@ void ConvEncoder::forward(const unsigned char* obs_dev, const int* shifts_dev, f
   RLREP_LAUNCHED_W("im2col_u8_aug", s, (double)B_ * C_ * H_ * H_ + 4.0 * rows(0) * ldk1_, 0.0);
   linear_fwd(gemm_, s, (int)rows(0), Mat{col_[0], ldk1_}, conv_[0].view(g_, target), ACT_RELU, act_[0], 32);
   for (int l = 1; l < 4; ++l) {
-    if ((target || no_grad || implicit_wgrad_) && implicit_dgrad_) {
+    if (target || no_grad || implicit_wgrad_) {
       // no backward pass follows (target / no-grad evaluation), so no column matrix is needed: implicit convolution
       const Linear w = conv_[l].view(g_, target);
       valid_conv_3x3(gemm_, s, B_, hw_[l - 1], act_[l - 1], w.W, w.ld, w.b, ACT_RELU, act_[l], corr_);
@@ -218,17 +186,9 @@ void ConvEncoder::backward(const float* dfeat_dev, int ld_dfeat) {
     }
     if (!(l > 0 && implicit_wgrad_)) launch_colsum_tall(dy.p, 32, rows(l), 32, bias_partial_, kBiasChunks, w.db, s);
     if (l == 0) break;
-    if (implicit_dgrad_) {
-      // dX = full correlation of dY with W (x ReLU mask), the taps walked by the GEMM's TMA producer (conv_implicit.cu)
-      full_correlation_3x3(gemm_, s, B_, hw_[l], dact_[l], w.W, FC_CONV_DGRAD, nullptr, ACT_NONE, act_[l - 1],
-                           dact_[l - 1], corr_);
-      continue;
-    }
-    linear_dgrad(gemm_, s, (int)rows(l), dy, w, DACT_NONE, Mat(), dcol_, 288);
-    col2im_nhwc32_kernel<<<grid_for((long long)rows(l - 1) * 8, 256), 256, 0, s>>>(
-        reinterpret_cast<const float4*>(dcol_), reinterpret_cast<const float4*>(act_[l - 1]), B_, hw_[l - 1], hw_[l],
-        reinterpret_cast<float4*>(dact_[l - 1]));
-    RLREP_LAUNCHED_W("col2im_nhwc32", s, 4.0 * (rows(l) * 288 + 2.0 * rows(l - 1) * 32), 0.0);
+    // dX = full correlation of dY with W (x ReLU mask), the taps walked by the GEMM's TMA producer (conv_implicit.cu)
+    full_correlation_3x3(gemm_, s, B_, hw_[l], dact_[l], w.W, FC_CONV_DGRAD, nullptr, ACT_NONE, act_[l - 1], dact_[l - 1],
+                         corr_);
   }
 }
 

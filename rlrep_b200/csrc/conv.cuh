@@ -37,10 +37,8 @@ class ConvEncoder {
   float* col_[4] = {nullptr, nullptr, nullptr, nullptr};
   float* act_[4] = {nullptr, nullptr, nullptr, nullptr};
   float* dact_[4] = {nullptr, nullptr, nullptr, nullptr};
-  float* dcol_ = nullptr;
-  bool implicit_dgrad_ = true;
-  // layers 2-4 without column matrices at all (TF32 path): implicit forward convolution, implicit data gradient and the
-  // implicit weight gradient of GemmArgs::conv_wgrad_hi; RLREP_CONV_WGRAD_V1=1 keeps the explicit im2col + folded GEMM
+  // layers 2-4 without column matrices at all (TF32 path, B % 4 == 0): implicit forward convolution and the implicit
+  // weight gradient of GemmArgs::conv_wgrad_hi; otherwise explicit im2col + folded GEMM
   bool implicit_wgrad_ = false;
   FullCorrScratch corr_;
   static constexpr int kBiasChunks = 296;  // 2 x 148 SMs

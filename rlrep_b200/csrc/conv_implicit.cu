@@ -134,11 +134,7 @@ void conv3x3_wgrad_implicit(GemmRunner& g, cudaStream_t s, int B, int Hg, const 
   a.C = sc.wfold; a.ldc = 768;
   // nine or eighteen tiles x a split-K cluster of 8 leave half the GPU idle and every CTA with ~10 MB to stream: cut K
   // into groups with their own output matrices (summed by diag_tap_sum)
-  static const int want_groups = [] {
-    const char* e = std::getenv("RLREP_WGRAD_GROUPS");
-    return e ? std::max(1, std::min(kWgradGroupsMax, std::atoi(e))) : 4;  // measured at B = 256: 1 and 2 groups 131 us, 4 groups 117 us
-  }();
-  a.k_groups = want_groups;
+  a.k_groups = kWgradGroups;
   const int groups = (a.k_groups > 1 && ceil_div(a.K, 32) >= 64 * a.k_groups) ? a.k_groups : 1;  // make_tc_plan's rule
   g.run(a, s);
   diag_tap_sum_kernel<<<ceil_div(32 * 288, 256), 256, 0, s>>>(sc.wfold, groups, dW, ld_dw, transposed ? 1 : 0);

@@ -3,15 +3,14 @@
 // Conv2d(32, 3, kernel 2, padding 1): 35 -> 37 -> 39 -> 41 -> 83 -> 84, forward, L1 loss and backward.
 //
 // A transposed convolution is the data-gradient of a convolution, so it runs on the encoder's machinery with the roles
-// swapped (conv.cu): activations NHWC, forward  colT [B*Hi*Hi, 9*32] = X [B*Hi*Hi, 32] x Wd^T  (tcgen05 GEMM, K = 32)
-// followed by the gather-form col2im (+ bias + ReLU, stride 1 or 2);  backward  dcolT = im2col(dY) (stride 1 or 2),
-// dX = dcolT Wd (x ReLU mask),  dWd = dcolT^T X.  Wd[(ky*3 + kx)*32 + co, ci] = W_ref[ci, co, ky, kx] (permuted at the
+// swapped (conv.cu): activations NHWC.  Forward: the stride-1 layers are implicit full correlations (conv_implicit.cu); the
+// stride-2 layer runs as four parity classes on the halo kernel, or where that kernel does not apply as
+// colT [B*Hi*Hi, 9*32] = X [B*Hi*Hi, 32] x Wd^T  (tcgen05 GEMM, K = 32) followed by the gather-form col2im (+ bias + ReLU).
+// Backward  dcolT = im2col(dY) (stride 1 or 2),  dX = dcolT Wd (x ReLU mask),  dWd = dcolT^T X.  Wd[(ky*3 + kx)*32 + co, ci] = W_ref[ci, co, ky, kx] (permuted at the
 // API).  The 3-channel output layer is a direct CUDA-core kernel (384 FMAs per pixel) fused with nothing; its weight
 // gradient is a two-pass deterministic reduction.
 #include "deconv.cuh"
 #include "layout.cuh"
-
-#include <cstdlib>
 
 #include <algorithm>
 
@@ -417,11 +416,9 @@ ConvDecoder::ConvDecoder(int batch, Precision prec, cudaStream_t s, int out_kern
   arena_.want(&wg_partial_, (size_t)kWgBlocks * (96 * ks_ * ks_ + 4));
   arena_.want(&bias_partial_, kBiasChunks * 32);
   arena_.want(&wfold_, (size_t)288 * kFold * 32 * kFold);
-  implicit_fwd_ = !(std::getenv("RLREP_CONV_V1") && std::atoi(std::getenv("RLREP_CONV_V1")) != 0);
-  if (implicit_fwd_) corr_.want(arena_, B_, hw_[3]);  // grids up to (hw_[3] + 4)^2: the stride-2 layer's padded input
-  // the stride-1 layers' backward pass without column matrices (TF32 path); RLREP_CONV_WGRAD_V1=1 keeps im2col + folded GEMM
-  implicit_bwd_ = implicit_fwd_ && prec == PREC_TF32 && B_ % 4 == 0 &&
-                  !(std::getenv("RLREP_CONV_WGRAD_V1") && std::atoi(std::getenv("RLREP_CONV_WGRAD_V1")) != 0);
+  corr_.want(arena_, B_, hw_[3]);  // grids up to (hw_[3] + 4)^2: the stride-2 layer's padded input
+  // the stride-1 layers' backward pass without column matrices (TF32 path); otherwise im2col + folded GEMM
+  implicit_bwd_ = prec == PREC_TF32 && B_ % 4 == 0;
   arena_.commit();
   gemm_.init(prec, 0);
 }
@@ -443,20 +440,18 @@ void ConvDecoder::forward(const float* x_dev, int ld_x) {
   RLREP_LAUNCHED_W("nchw_to_nhwc", s, 8.0 * B_ * P0 * 32, 0.0);
   for (int l = 0; l < 4; ++l) {
     const int Hi = hw_[l], Ho = hw_[l + 1];
-    if (implicit_fwd_ && l < 3) {  // stride 1: a full correlation, the taps walked by the GEMM's TMA producer
+    if (l < 3) {  // stride 1: a full correlation, the taps walked by the GEMM's TMA producer
       full_correlation_3x3(gemm_, s, B_, Hi, act_[l], g_.p + w_off_[l], FC_DECONV_FWD, g_.p + b_off_[l], ACT_RELU, nullptr,
                            act_[l + 1], corr_);
       continue;
     }
-    if (implicit_fwd_ && l == 3 &&
-        deconv3x3_s2_forward(gemm_, s, B_, Hi, Ho, act_[l], g_.p + w_off_[l], g_.p + b_off_[l], act_[l + 1], corr_))
+    if (deconv3x3_s2_forward(gemm_, s, B_, Hi, Ho, act_[l], g_.p + w_off_[l], g_.p + b_off_[l], act_[l + 1], corr_))
       continue;  // stride 2: four parity classes on the halo kernel, no [rows, 288] matrix
     linear_fwd(gemm_, s, (int)rows(l), Mat{act_[l], 32}, layer(l), ACT_NONE, col_, 288);
     const float4* colT = reinterpret_cast<const float4*>(col_);
     const float4* bias = reinterpret_cast<const float4*>(g_.p + b_off_[l]);
     float4* y = reinterpret_cast<float4*>(act_[l + 1]);
-    if (l < 3) col2im_bias_relu_kernel<1><<<grid_for(rows(l + 1) * 8, 256), 256, 0, s>>>(colT, bias, B_, Hi, Ho, y);
-    else col2im_bias_relu_kernel<2><<<grid_for(rows(l + 1) * 8, 256), 256, 0, s>>>(colT, bias, B_, Hi, Ho, y);
+    col2im_bias_relu_kernel<2><<<grid_for(rows(l + 1) * 8, 256), 256, 0, s>>>(colT, bias, B_, Hi, Ho, y);
     RLREP_LAUNCHED_W("col2im_bias_relu", s, 4.0 * (rows(l) * 288 + rows(l + 1) * 32), 0.0);
   }
   if (ks_ == 2)

@@ -49,7 +49,6 @@ class ConvDecoder {
   static constexpr int kWgBlocks = 888, kWgBlocks2 = 592;
   static constexpr int kFold = 4;  // rows folded per GEMM row in the weight-gradient GEMMs (deconv.cu backward())
   float* wfold_ = nullptr;
-  bool implicit_fwd_ = true;
   bool implicit_bwd_ = false;
   FullCorrScratch corr_;
 };

@@ -17,36 +17,6 @@
 
 namespace rlrep {
 
-// Row operations that can ride in a GEMM chain (gemm_chain.cuh) between its GEMMs, executed by the chain kernel's
-// epilogue warps on (rows_per_item)-row items with the same dependency / publish protocol as a GEMM tile.  A GemmArgs
-// whose row.kind != ROWOP_NONE is such an operation, not a GEMM.
-enum RowOpKind : int { ROWOP_NONE = 0, ROWOP_CTRL_HEAD = 1, ROWOP_GATHER = 2 };
-struct RowOp {
-  int kind = ROWOP_NONE;
-  int rows = 0;
-  // ROWOP_CTRL_HEAD: contrastive_head_kernel (kernels.cuh) -- row log-sum-exp / CE gradient rewrite of `logits`, reward head
-  // pred = <z_row, theta_w> + theta_b, dpred = (pred - reward) * inv_batch, loss metrics by the last row to finish
-  float* logits = nullptr;
-  int ld = 0, cols = 0, diag_off = 0;
-  float inv_batch = 0.f;
-  const float* z = nullptr;
-  int ldz = 0, D = 0;
-  const float* theta_w = nullptr;
-  const float* theta_b = nullptr;
-  const float* reward = nullptr;
-  int ld_r = 0;
-  float* loss_rows = nullptr;
-  float* pred = nullptr;
-  float* dpred = nullptr;
-  float* metrics = nullptr;
-  unsigned* counter = nullptr;
-  // ROWOP_GATHER: gather_kernel -- out[b, :] = ring[idx[b], :], rows are rec4 float4 wide
-  const float* ring = nullptr;
-  const long long* idx = nullptr;
-  float* out = nullptr;
-  int rec4 = 0;
-};
-
 struct GemmArgs {
   int M = 0, N = 0, K = 0;
   const float* A = nullptr;
@@ -92,7 +62,6 @@ struct GemmArgs {
   float* C = nullptr;
   int ldc = 0;
   Epilogue epi;
-  RowOp row;  // row.kind != ROWOP_NONE: a row operation riding in a GEMM chain, the GEMM fields above are unused
 };
 
 // ---- tcgen05 path (TF32 inputs, FP32 accumulate in TMEM, TMA-fed) ----

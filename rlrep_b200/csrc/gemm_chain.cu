@@ -7,7 +7,6 @@
 #include "common.cuh"
 #include "gemm_chain.cuh"
 #include "ptx.cuh"
-#include "reduce.cuh"
 
 namespace rlrep {
 
@@ -29,7 +28,6 @@ constexpr int kSub = 4, kCtrStride = 32;
 constexpr int kDbgItems = 16, kDbgEvents = 10;  // debug timeline: items per CTA x events per item
 // events: 0 producer picks the item up, 1 dependencies satisfied, 2 last TMA of the item issued, 3 MMA sees the first
 // operands, 4 accumulator committed, 5 epilogue sees the accumulator, 6 split-K arrival counted, 7 tile published
-enum : int { kFlagNoTensormapFence = 1, kFlagNoProxyFence = 2, kFlagNoCooperative = 4 };
 constexpr int kSmemBytes = kStages * kStageBytes + 1024 + 256 + kTbufFloats * 4;
 static_assert(kSmemBytes <= 227 * 1024, "chain kernel shared memory");
 
@@ -186,143 +184,11 @@ __device__ __forceinline__ void chain_store_rows(const Epilogue& epi, const Chun
   }
 }
 
-// ------------------------------------------------------------------------------------------------ row operations
-// Executed by the 256 epilogue threads (et = 0..255) of a CTA.  Operands produced by other SMs of this launch are read with
-// ld.cg (never from this SM's L1).
-// One row of the CTRL contrastive head (contrastive_head_kernel in kernels.cu, same arithmetic up to summation order) by ONE
-// WARP: log-sum-exp of the logits row, in-place rewrite to (softmax - I) * inv_batch, reward-head prediction and its
-// gradient; the row that finishes last adds up the per-row terms in fixed order and writes the three loss metrics.  Rows of
-// up to 512 logits stay in registers between the three passes (one trip to L2 instead of three), and nothing synchronises
-// beyond the warp: an item's rows run on as many warps at once.
-__device__ __forceinline__ void row_op_ctrl_head(const RowOp& op, int row, int lane) {
-  float* l = op.logits + (size_t)row * op.ld;
-  const int cols = op.cols;
-  const int dj = op.diag_off + row;
-  float lse, diag;
-  const bool in_regs = cols <= 512 && (cols & 3) == 0 && (op.ld & 3) == 0 && (reinterpret_cast<uintptr_t>(op.logits) & 15) == 0;
-  if (in_regs) {
-    float4 v[4];
-    const float4* l4 = reinterpret_cast<const float4*>(l);
-    const int n4 = cols >> 2;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int j = lane + 32 * i;
-      v[i] = j < n4 ? __ldcg(l4 + j) : make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY);
-    }
-    float mx = -INFINITY;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) mx = fmaxf(mx, fmaxf(fmaxf(v[i].x, v[i].y), fmaxf(v[i].z, v[i].w)));
-    mx = warp_max(mx);
-    float sum = 0.f;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) sum += (expf(v[i].x - mx) + expf(v[i].y - mx)) + (expf(v[i].z - mx) + expf(v[i].w - mx));
-    sum = warp_sum(sum);
-    lse = mx + logf(sum);
-    // the diagonal logit: lane (dj / 4) % 32, register dj / 128, component dj % 4
-    float mine = 0.f;
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-      if (i == (dj >> 7)) mine = (dj & 3) == 0 ? v[i].x : (dj & 3) == 1 ? v[i].y : (dj & 3) == 2 ? v[i].z : v[i].w;
-    diag = __shfl_sync(0xffffffffu, mine, (dj >> 2) & 31);
-    float4* o4 = reinterpret_cast<float4*>(l);
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int j = lane + 32 * i;
-      if (j < n4) {
-        const int c = 4 * j;
-        float4 g;
-        g.x = (expf(v[i].x - lse) - (c == dj ? 1.f : 0.f)) * op.inv_batch;
-        g.y = (expf(v[i].y - lse) - (c + 1 == dj ? 1.f : 0.f)) * op.inv_batch;
-        g.z = (expf(v[i].z - lse) - (c + 2 == dj ? 1.f : 0.f)) * op.inv_batch;
-        g.w = (expf(v[i].w - lse) - (c + 3 == dj ? 1.f : 0.f)) * op.inv_batch;
-        o4[j] = g;
-      }
-    }
-  } else {
-    float mx = -INFINITY;
-    for (int j = lane; j < cols; j += 32) mx = fmaxf(mx, __ldcg(l + j));
-    mx = warp_max(mx);
-    float sum = 0.f;
-    for (int j = lane; j < cols; j += 32) sum += expf(__ldcg(l + j) - mx);
-    sum = warp_sum(sum);
-    lse = mx + logf(sum);
-    diag = __ldcg(l + dj);
-    __syncwarp();  // every lane has read l[dj] before it is rewritten
-    for (int j = lane; j < cols; j += 32) l[j] = (expf(__ldcg(l + j) - lse) - (j == dj ? 1.f : 0.f)) * op.inv_batch;
-  }
-  const float loss = lse - diag;
-  const float* x = op.z + (size_t)row * op.ldz;
-  float acc = 0.f;
-  if (((op.ldz | op.D) & 3) == 0 && ((reinterpret_cast<uintptr_t>(op.z) | reinterpret_cast<uintptr_t>(op.theta_w)) & 15) == 0) {
-    const float4* x4 = reinterpret_cast<const float4*>(x);
-    const float4* w4 = reinterpret_cast<const float4*>(op.theta_w);
-    float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-#pragma unroll 4
-    for (int j = lane; j < op.D / 4; j += 32) {
-      const float4 xv = __ldcg(x4 + j);
-      const float4 wv = __ldg(w4 + j);
-      a0 = fmaf(xv.x, wv.x, a0); a1 = fmaf(xv.y, wv.y, a1); a2 = fmaf(xv.z, wv.z, a2); a3 = fmaf(xv.w, wv.w, a3);
-    }
-    acc = (a0 + a1) + (a2 + a3);
-  } else {
-    for (int j = lane; j < op.D; j += 32) acc = fmaf(__ldcg(x + j), __ldg(op.theta_w + j), acc);
-  }
-  acc = warp_sum(acc);
-  unsigned last = 0;
-  if (lane == 0) {
-    const float p = acc + __ldg(op.theta_b);
-    op.loss_rows[row] = loss;
-    op.pred[row] = p;
-    op.dpred[row] = (p - __ldcg(op.reward + (size_t)row * op.ld_r)) * op.inv_batch;
-    last = atom_add_acq_rel(op.counter, 1u) == (unsigned)(op.rows - 1) ? 1u : 0u;
-  }
-  last = __shfl_sync(0xffffffffu, last, 0);
-  if (!last) return;
-  float ce = 0.f, se = 0.f;
-  for (int i = lane; i < op.rows; i += 32) {
-    ce += __ldcg(op.loss_rows + i);
-    const float d = __ldcg(op.pred + i) - __ldcg(op.reward + (size_t)i * op.ld_r);
-    se = fmaf(d, d, se);
-  }
-  ce = warp_sum(ce);
-  se = warp_sum(se);
-  if (lane == 0) {
-    const float model = ce * op.inv_batch;
-    const float r = 0.5f * (se * op.inv_batch);
-    op.metrics[0] = model + r;
-    op.metrics[1] = model;
-    op.metrics[2] = r;
-    *op.counter = 0;  // re-armed for the next launch
-  }
-}
-
-// Rows [row0, row0 + n) of the replay gather: out[b, :] = ring[idx[b], :] (gather_kernel in kernels.cu).
-__device__ __forceinline__ void row_op_gather(const RowOp& op, int row0, int n, int et) {
-  const float4* ring = reinterpret_cast<const float4*>(op.ring);
-  float4* out = reinterpret_cast<float4*>(op.out);
-  const int rec4 = op.rec4;
-  for (int i = et; i < n * rec4; i += 256) {
-    const int r = row0 + i / rec4, c = i % rec4;
-    out[(size_t)r * rec4 + c] = __ldg(ring + (size_t)__ldg(op.idx + r) * rec4 + c);
-  }
-}
-
-// Out of line: the row operations' registers must not weigh on the GEMM epilogue, which sits at the 168-register cap.
-__device__ __noinline__ void run_row_op(const ChainGemmDesc* g, int item, float* scratch, int et) {
-  const RowOp op = g->row;
-  const int rpi = g->rows_per_item, row0 = item * rpi, n = min(rpi, op.rows - row0);
-  if (op.kind == ROWOP_CTRL_HEAD) {
-    for (int r = et >> 5; r < n; r += kEpiWarps) row_op_ctrl_head(op, row0 + r, et & 31);
-  } else {
-    row_op_gather(op, row0, n, et);
-  }
-}
-
 // ------------------------------------------------------------------------------------------------ kernel
 __global__ void __launch_bounds__(kThreads, 1)
 gemm_chain_kernel(const ChainGemmDesc* __restrict__ gemms, const ChainTask* __restrict__ tasks,
                   const int* __restrict__ task_begin, unsigned* __restrict__ done, unsigned* __restrict__ exit_ctr,
-                  int n_gemms, int flags, unsigned long long* __restrict__ dbg) {
+                  int n_gemms, unsigned long long* __restrict__ dbg) {
   // Debug timeline (rlrep_gemm_chain_set_debug): %globaltimer stamps per (CTA, item, event); see kDbg* below.
   auto stamp = [&](int item, int ev) {
     if (dbg != nullptr && item < kDbgItems) {
@@ -373,7 +239,6 @@ gemm_chain_kernel(const ChainGemmDesc* __restrict__ gemms, const ChainTask* __re
       for (int t = t_begin; t < t_end; ++t) {
         const ChainTask tk = tasks[t];
         const ChainGemmDesc* g = gemms + tk.gemm;
-        const int kind = g->row.kind;
         // Everything that does not depend on the dependencies' DATA happens before the wait: the item's descriptor fields
         // go to registers and the tensor maps are made visible to the TMA unit, so that once the counters are reached only
         // the fences stand between this thread and the first operand load.
@@ -387,11 +252,9 @@ gemm_chain_kernel(const ChainGemmDesc* __restrict__ gemms, const ChainTask* __re
           dep_id[d] = d < n_deps ? g->dep[d] : 0;
           dep_tiles[d] = d < n_deps ? (int)g->dep_target[d] : 0;
         }
-        if (tk.gemm != last_gemm && kind == ROWOP_NONE) {
-          if (!(flags & kFlagNoTensormapFence)) {
-            fence_tensormap_acquire(&g->tmA);
-            fence_tensormap_acquire(&g->tmB);
-          }
+        if (tk.gemm != last_gemm) {
+          fence_tensormap_acquire(&g->tmA);
+          fence_tensormap_acquire(&g->tmB);
           last_gemm = tk.gemm;
         }
         stamp(t - t_begin, 0);
@@ -404,18 +267,9 @@ gemm_chain_kernel(const ChainGemmDesc* __restrict__ gemms, const ChainTask* __re
         if (n_deps > 0) {
           fence_acquire_gpu();
           // the tiles were written through the generic proxy by other SMs; TMA reads through the async proxy
-          if (!(flags & kFlagNoProxyFence)) fence_proxy_async_global();
+          fence_proxy_async_global();
         }
         stamp(t - t_begin, 1);
-        if (kind != ROWOP_NONE) {
-          // a row operation has no operands to stream: "dependencies met" travels to the MMA issuer through one (empty)
-          // pipeline stage, so that every barrier still sees each of its phases waited on in order
-          const int s = it % kStages;
-          ptx::mbar_wait(&empty_bar[s], ((it / kStages) & 1) ^ 1);
-          ptx::mbar_arrive(&full_bar[s]);
-          ++it;
-          continue;
-        }
         const uint32_t tx = kABytes + bn * kBK * 4;
         for (int kb = kb0; kb < kb1; ++kb, ++it) {
           const int s = it % kStages;
@@ -439,17 +293,6 @@ gemm_chain_kernel(const ChainGemmDesc* __restrict__ gemms, const ChainTask* __re
       for (int t = t_begin; t < t_end; ++t, ++tc) {
         const ChainTask tk = tasks[t];
         const ChainGemmDesc* g = gemms + tk.gemm;
-        if (g->row.kind != ROWOP_NONE) {
-          // row operation: nothing to multiply; hand the producer's "dependencies met" on to the epilogue warps through the
-          // accumulator slot this item stands in for
-          const int s = it % kStages, acc = tc & 1;
-          ptx::mbar_wait(&full_bar[s], (it / kStages) & 1);
-          ptx::mbar_arrive(&empty_bar[s]);
-          ++it;
-          ptx::mbar_wait(&acc_empty[acc], ((tc >> 1) & 1) ^ 1);
-          ptx::mbar_arrive(&acc_full[acc]);
-          continue;
-        }
         const int bn = g->bn, a_mn = g->a_mn, b_mn = g->b_mn;
         const int kb0 = tk.split * g->kb_per_split, kb1 = min(g->nkb, kb0 + g->kb_per_split);
         const uint32_t idesc = ptx::make_idesc_tf32(kBM, bn, a_mn != 0, b_mn != 0);
@@ -489,22 +332,6 @@ gemm_chain_kernel(const ChainGemmDesc* __restrict__ gemms, const ChainTask* __re
     for (int t = t_begin; t < t_end; ++t, ++tc) {
       const ChainTask tk = tasks[t];
       const ChainGemmDesc* g = gemms + tk.gemm;
-      if (g->row.kind != ROWOP_NONE) {
-        const int acc = tc & 1, et = threadIdx.x - 64;
-        ptx::mbar_wait(&acc_full[acc], (tc >> 1) & 1);
-        if (threadIdx.x == 64) stamp(t - t_begin, 5);
-        run_row_op(g, tk.tile, tbuf, et);
-        if (threadIdx.x == 64) stamp(t - t_begin, 9);
-        epilogue_bar();
-        if (threadIdx.x == 64) {
-          if (!(flags & kFlagNoProxyFence)) fence_proxy_async_global();
-          red_release_add(done + ((size_t)tk.gemm * kSub + (tk.tile % kSub)) * kCtrStride, 1u);
-          stamp(t - t_begin, 7);
-        }
-        __syncwarp();
-        if (lane == 0) ptx::mbar_arrive(&acc_empty[acc]);
-        continue;
-      }
       // everything this item needs from its descriptor, read ONCE into registers: a reference into global memory would be
       // re-read behind every store (the compiler must assume the stores alias it)
       const Epilogue epi = g->epi;
@@ -675,7 +502,7 @@ gemm_chain_kernel(const ChainGemmDesc* __restrict__ gemms, const ChainTask* __re
         if (threadIdx.x == 64) stamp(t - t_begin, 9);
         epilogue_bar();
         if (threadIdx.x == 64) {
-          if (!(flags & kFlagNoProxyFence)) fence_proxy_async_global();
+          fence_proxy_async_global();
           // a distributed reduction publishes once per (tile, split): each CTA's columns are final on their own
           const int pub = dist ? tk.tile * split_k + tk.split : tk.tile;
           red_release_add(done + ((size_t)tk.gemm * kSub + (pub % kSub)) * kCtrStride, 1u);
@@ -723,26 +550,6 @@ struct Footprint {
 };
 Footprint footprint(const GemmArgs& a) {
   Footprint f;
-  if (a.row.kind == ROWOP_CTRL_HEAD) {
-    const RowOp& o = a.row;
-    f.reads.push_back(range_of(o.logits, o.rows, o.ld, o.cols));
-    f.reads.push_back(range_of(o.z, o.rows, o.ldz, o.D));
-    f.reads.push_back(range_of(o.theta_w, 1, 0, o.D));
-    f.reads.push_back(range_of(o.theta_b, 1, 0, 1));
-    f.reads.push_back(range_of(o.reward, o.rows, o.ld_r, 1));
-    f.writes.push_back(range_of(o.logits, o.rows, o.ld, o.cols));
-    f.writes.push_back(range_of(o.loss_rows, 1, 0, o.rows));
-    f.writes.push_back(range_of(o.pred, 1, 0, o.rows));
-    f.writes.push_back(range_of(o.dpred, 1, 0, o.rows));
-    f.writes.push_back(range_of(o.metrics, 1, 0, 3));
-    return f;
-  }
-  if (a.row.kind == ROWOP_GATHER) {
-    const RowOp& o = a.row;
-    f.reads.push_back(range_of(reinterpret_cast<const float*>(o.idx), 1, 0, 2 * o.rows));
-    f.writes.push_back(range_of(o.out, o.rows, 4 * o.rec4, 4 * o.rec4));
-    return f;  // the ring itself is never written inside a chain
-  }
   f.reads.push_back(a.a_mn ? range_of(a.A, a.K, a.lda, a.M) : range_of(a.A, a.M, a.lda, a.K));
   f.reads.push_back(a.b_mn ? range_of(a.B, a.K, a.ldb, a.N) : range_of(a.B, a.N, a.ldb, a.K));
   f.reads.push_back(range_of(a.epi.bias, 1, 0, a.N));
@@ -803,7 +610,6 @@ double plan_cost(int tiles, int nkb, int bn, int split, int share, bool dist) {
 void set_chain_debug_buffer(unsigned long long* dev) { g_chain_dbg = dev; }
 
 bool chain_eligible(const GemmArgs& a) {
-  if (a.row.kind != ROWOP_NONE) return a.row.rows > 0;
   return tc_eligible(a) && a.conv_w == 0 && a.M >= 32 && a.N >= 32 && a.K >= 8;
 }
 
@@ -815,17 +621,6 @@ bool GemmChain::matches(const std::vector<GemmArgs>& seq) const {
   if (seq.size() != seq_.size()) return false;
   for (size_t i = 0; i < seq.size(); ++i) {
     const GemmArgs &x = seq[i], &y = seq_[i];
-    if (x.row.kind != y.row.kind) return false;
-    if (x.row.kind != ROWOP_NONE) {
-      const RowOp &p = x.row, &q = y.row;
-      if (p.rows != q.rows || p.logits != q.logits || p.ld != q.ld || p.cols != q.cols || p.diag_off != q.diag_off ||
-          p.inv_batch != q.inv_batch || p.z != q.z || p.ldz != q.ldz || p.D != q.D || p.theta_w != q.theta_w ||
-          p.theta_b != q.theta_b || p.reward != q.reward || p.ld_r != q.ld_r || p.loss_rows != q.loss_rows ||
-          p.pred != q.pred || p.dpred != q.dpred || p.metrics != q.metrics || p.counter != q.counter || p.ring != q.ring ||
-          p.idx != q.idx || p.out != q.out || p.rec4 != q.rec4)
-        return false;
-      continue;
-    }
     if (x.M != y.M || x.N != y.N || x.K != y.K || x.A != y.A || x.B != y.B || x.C != y.C || x.lda != y.lda ||
         x.ldb != y.ldb || x.ldc != y.ldc || x.a_mn != y.a_mn || x.b_mn != y.b_mn || x.epi.bias != y.epi.bias ||
         x.epi.r1_u != y.epi.r1_u || x.epi.r1_v != y.epi.r1_v || x.epi.aux != y.epi.aux || x.epi.pre_out != y.epi.pre_out ||
@@ -884,69 +679,31 @@ void GemmChain::build(const std::vector<GemmArgs>& seq, int force_bn, int force_
   }
   levels_ = 1 + *std::max_element(level.begin(), level.end());
 
-  // ---- per level: which GEMMs are on the critical path, SM share by work among those, tile width / K-split per GEMM.
-  // A GEMM whose output another GEMM of the chain reads is CRITICAL: the next level cannot start before its last tile, so
-  // the critical GEMMs of a level share all the SMs (K-split until they fill their share).  GEMMs nobody in the chain waits
-  // for (weight gradients) are FILLERS: no split, spread over all CTAs and queued behind the level's critical items, so
-  // they run in the gaps the dependency waits leave.  A level without critical members shares the SMs by work.
-  force_bn = force_bn ? force_bn : env_int("RLREP_CHAIN_BN", 0);
-  force_split = force_split ? force_split : env_int("RLREP_CHAIN_SPLIT", 0);
-  const bool use_fillers = env_int("RLREP_CHAIN_FILLERS", 0) != 0;  // measured: not worth it (DESIGN.md section 5)
-  std::vector<char> has_dependents(n, 0), filler(n, 0);
-  for (int j = 0; j < n; ++j)
-    for (int i : deps[j]) has_dependents[i] = 1;
-  std::vector<int> bn(n), split(n), share(n), first_cta(n), rpi(n, 0), dist(n, 0);
+  // ---- per level: SM share by work among the level's GEMMs, tile width / K-split per GEMM (K-split until it fills its share)
+  std::vector<int> bn(n), split(n), share(n), first_cta(n), dist(n, 0);
   const int dist_mode = env_int("RLREP_CHAIN_DIST", 1);  // 0: last-arriver reductions only, 1: cost model, 2: wherever possible
-  auto is_row = [&](int i) { return seq[i].row.kind != ROWOP_NONE; };
-  // a row operation counts as one k-block of work per 128 rows when it shares a level with GEMMs
   auto work_of = [&](int i) {
-    if (is_row(i)) return (double)ceil_div(seq[i].row.rows, kBM);
     return (double)ceil_div(seq[i].M, kBM) * ceil_div(seq[i].N, kMaxBn) * ceil_div(seq[i].K, kBK);
   };
   // items (= publishes on its completion counter) of chain member i
-  auto items_of = [&](int i) {
-    if (is_row(i)) return ceil_div(seq[i].row.rows, rpi[i]);
-    return ceil_div(seq[i].M, kBM) * ceil_div(seq[i].N, bn[i]) * (dist[i] ? split[i] : 1);
-  };
-  int filler_cursor = 0;
+  auto items_of = [&](int i) { return ceil_div(seq[i].M, kBM) * ceil_div(seq[i].N, bn[i]) * (dist[i] ? split[i] : 1); };
   for (int L = 0; L < levels_; ++L) {
     std::vector<int> members;
-    bool any_critical = false;
     for (int i = 0; i < n; ++i)
-      if (level[i] == L) {
-        members.push_back(i);
-        any_critical = any_critical || has_dependents[i];
-      }
+      if (level[i] == L) members.push_back(i);
     double total = 0.0;
-    for (int i : members) {
-      filler[i] = use_fillers && any_critical && !has_dependents[i];
-      if (!filler[i]) total += work_of(i);
-    }
-    int cursor = 0, n_sharing = 0, seen = 0;
-    for (int i : members) n_sharing += filler[i] ? 0 : 1;
+    for (int i : members) total += work_of(i);
+    int cursor = 0, seen = 0;
     for (int i : members) {
       const GemmArgs& a = seq[i];
       const int nkb = ceil_div(a.K, kBK);
-      int sh = n_cta;
-      if (filler[i]) {
-        first_cta[i] = filler_cursor % n_cta;
-      } else {
-        ++seen;
-        sh = std::max(4, (int)std::floor(n_cta * work_of(i) / total));
-        if (seen == n_sharing) sh = std::max(sh, n_cta - cursor);  // the last member takes what is left
-        sh = std::min(sh, n_cta);
-        first_cta[i] = cursor % n_cta;
-        cursor += sh;
-      }
+      ++seen;
+      int sh = std::max(4, (int)std::floor(n_cta * work_of(i) / total));
+      if (seen == (int)members.size()) sh = std::max(sh, n_cta - cursor);  // the last member takes what is left
+      sh = std::min(sh, n_cta);
+      first_cta[i] = cursor % n_cta;
+      cursor += sh;
       share[i] = sh;
-      if (is_row(i)) {
-        // rows spread evenly over the share, one item per CTA (a head row costs ~1.5 us of block reductions, far below
-        // what an extra dependency round trip would)
-        bn[i] = 32;
-        split[i] = 1;
-        rpi[i] = std::max(1, ceil_div(seq[i].row.rows, sh));
-        continue;
-      }
       double best = 1e300;
       for (int cbn : {32, 64, 128}) {
         if (force_bn && cbn != force_bn) continue;
@@ -954,7 +711,6 @@ void GemmChain::build(const std::vector<GemmArgs>& seq, int force_bn, int force_
         const int tiles = ceil_div(a.M, kBM) * ceil_div(a.N, cbn);
         for (int s : {1, 2, 4, 8, 16}) {
           if (force_split && s != force_split) continue;
-          if (filler[i] && !force_split && s > 1) continue;
           if (s > 1 && (s - 1) * ceil_div(nkb, s) >= nkb) continue;  // would leave an empty split
           for (int d = 0; d < 2; ++d) {
             if (d == 1 && (dist_mode == 0 || !dist_possible(cbn, s) || tiles * s > sh)) continue;  // the splits must share a wave
@@ -974,7 +730,6 @@ void GemmChain::build(const std::vector<GemmArgs>& seq, int force_bn, int force_
         split[i] = 1;
         dist[i] = 0;
       }
-      if (filler[i]) filler_cursor += ceil_div(a.M, kBM) * ceil_div(a.N, bn[i]);  // the next filler continues where this one ends
     }
   }
 
@@ -982,16 +737,14 @@ void GemmChain::build(const std::vector<GemmArgs>& seq, int force_bn, int force_
   std::vector<std::vector<ChainTask>> per_cta(n_cta);
   std::vector<int> order(n);
   for (int i = 0; i < n; ++i) order[i] = i;
-  std::stable_sort(order.begin(), order.end(), [&](int x, int y) {
-    return level[x] != level[y] ? level[x] < level[y] : filler[x] < filler[y];
-  });
+  std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return level[x] < level[y]; });
   size_t ws_floats = 0, ctr_count = 0;
   std::vector<size_t> ws_off(n, 0), ctr_off(n, 0);
   std::vector<ChainGemmDesc> descs(n);
   bytes_ = flops_ = 0.0;
   for (int i : order) {
     const GemmArgs& a = seq[i];
-    const int tiles_m = is_row(i) ? items_of(i) : ceil_div(a.M, kBM), tiles_n = is_row(i) ? 1 : ceil_div(a.N, bn[i]);
+    const int tiles_m = ceil_div(a.M, kBM), tiles_n = ceil_div(a.N, bn[i]);
     const int tiles = tiles_m * tiles_n;
     int item = 0;
     for (int t = 0; t < tiles; ++t)
@@ -999,12 +752,8 @@ void GemmChain::build(const std::vector<GemmArgs>& seq, int force_bn, int force_
         per_cta[(first_cta[i] + item % share[i]) % n_cta].push_back(ChainTask{i, t, s, 0});
     ChainGemmDesc& d = descs[i];
     std::memset(&d, 0, sizeof(d));
-    if (!is_row(i)) {
-      d.tmA = make_operand_map(a.A, a.a_mn, a.M, a.K, a.lda, kBM);
-      d.tmB = make_operand_map(a.B, a.b_mn, a.N, a.K, a.ldb, bn[i]);
-    }
-    d.row = a.row;
-    d.rows_per_item = rpi[i];
+    d.tmA = make_operand_map(a.A, a.a_mn, a.M, a.K, a.lda, kBM);
+    d.tmB = make_operand_map(a.B, a.b_mn, a.N, a.K, a.ldb, bn[i]);
     d.epi = a.epi;
     d.C = a.C;
     d.ldc = a.ldc; d.M = a.M; d.N = a.N; d.K = a.K;
@@ -1024,14 +773,8 @@ void GemmChain::build(const std::vector<GemmArgs>& seq, int force_bn, int force_
       ws_off[i] = ws_floats;
       ws_floats += (size_t)tiles * split[i] * kBM * bn[i];
     }
-    if (a.row.kind == ROWOP_CTRL_HEAD) {
-      bytes_ += 4.0 * ((double)a.row.rows * (2.0 * a.row.cols + a.row.D));
-    } else if (a.row.kind == ROWOP_GATHER) {
-      bytes_ += 2.0 * 16.0 * a.row.rows * a.row.rec4;
-    } else {
-      bytes_ += 4.0 * ((double)a.M * a.K + (double)a.N * a.K + (double)a.M * a.N);
-      flops_ += 2.0 * a.M * a.N * a.K;
-    }
+    bytes_ += 4.0 * ((double)a.M * a.K + (double)a.N * a.K + (double)a.M * a.N);
+    flops_ += 2.0 * a.M * a.N * a.K;
   }
   std::vector<ChainTask> tasks;
   std::vector<int> begin(n_cta + 1, 0);
@@ -1071,13 +814,9 @@ void GemmChain::build(const std::vector<GemmArgs>& seq, int force_bn, int force_
     std::fprintf(stderr, "rlrep chain: %d GEMMs, %d levels, %zu items, ws %.1f MB\n", n, levels_, tasks.size(),
                  ws_floats * 4 / 1e6);
     for (int i = 0; i < n; ++i)
-      if (is_row(i))
-        std::fprintf(stderr, "  [%d] L%d row op %d: rows=%d rows/item=%d share=%d deps=%d\n", i, level[i], seq[i].row.kind,
-                     seq[i].row.rows, rpi[i], share[i], (int)deps[i].size());
-      else
-        std::fprintf(stderr, "  [%d] L%d M=%d N=%d K=%d a_mn=%d b_mn=%d bn=%d split=%d%s share=%d deps=%d%s\n", i, level[i],
-                     seq[i].M, seq[i].N, seq[i].K, (int)seq[i].a_mn, (int)seq[i].b_mn, bn[i], split[i],
-                     dist[i] ? " (distributed)" : "", share[i], (int)deps[i].size(), filler[i] ? " filler" : "");
+      std::fprintf(stderr, "  [%d] L%d M=%d N=%d K=%d a_mn=%d b_mn=%d bn=%d split=%d%s share=%d deps=%d\n", i, level[i],
+                   seq[i].M, seq[i].N, seq[i].K, (int)seq[i].a_mn, (int)seq[i].b_mn, bn[i], split[i],
+                   dist[i] ? " (distributed)" : "", share[i], (int)deps[i].size());
   }
 }
 
@@ -1090,14 +829,13 @@ void GemmChain::launch(cudaStream_t stream) {
   cfg.stream = stream;
   // cooperative: all CTAs are co-scheduled or none is, so two chains launched on different streams can never hold part of
   // the GPU each while spinning on tiles of CTAs that are not resident
-  static const int flags = env_int("RLREP_CHAIN_FLAGS", 0);
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeCooperative;
   attr[0].val.cooperative = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = (flags & kFlagNoCooperative) ? 0 : 1;
+  cfg.numAttrs = 1;
   RLREP_CUDA(cudaLaunchKernelEx(&cfg, gemm_chain_kernel, (const ChainGemmDesc*)d_gemms_, (const ChainTask*)d_tasks_,
-                                (const int*)d_task_begin_, d_done_, d_exit_, (int)seq_.size(), flags, g_chain_dbg));
+                                (const int*)d_task_begin_, d_done_, d_exit_, (int)seq_.size(), g_chain_dbg));
   RLREP_LAUNCHED_W("gemm_chain", stream, bytes_, flops_);
 }
 

@@ -30,8 +30,6 @@ struct alignas(128) ChainGemmDesc {
   CUtensorMap tmA;  // 128 bytes each; TMA reads them from global memory
   CUtensorMap tmB;
   Epilogue epi;
-  RowOp row;           // row.kind != ROWOP_NONE: a row operation (items of rows_per_item rows), not a GEMM
-  int rows_per_item;
   int dist;            // split-K reduction distributed over the tile's split CTAs (each finalises bn / split_k columns)
   float* C;
   float* ws;           // split-K partial tiles [tile][split][bn / 4][128 rows][4]; nullptr when split_k == 1

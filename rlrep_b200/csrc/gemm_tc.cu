@@ -110,23 +110,13 @@ int max_clusters(int bn, bool a_mn, bool b_mn, int s, int stages, bool push) {
 
 // Ring depth.  A short K-slice is one burst of loads: a ring that fits twice into an SM (2 x ~113 KB) lets two CTAs
 // -- of this GEMM or of one running concurrently on another stream -- share the SM; long slices get the deepest ring.
-bool use_push(int bn, int s) {
-  static const int push_on = [] {
-    const char* e = std::getenv("RLREP_TC_PUSH");
-    return e ? std::atoi(e) : 1;
-  }();
-  return push_on && s > 1 && tc::push_possible(bn);
-}
+bool use_push(int bn, int s) { return s > 1 && tc::push_possible(bn); }
 
 int pick_stages(int bn, int kb_per, bool push) {
   if (push) return std::max(2, std::min(kb_per, tc::max_stages_push(bn)));
-  static const int shallow_on = [] {
-    const char* e = std::getenv("RLREP_TC_SHALLOW");
-    return e ? std::atoi(e) : 1;
-  }();
   const int deepest = tc::num_stages(bn), fewest = tc::min_stages(bn);
   const int shallow = (113 * 1024 - 1280) / tc::stage_bytes(bn);
-  if (!shallow_on || shallow < fewest || kb_per > 2 * shallow) return deepest;
+  if (shallow < fewest || kb_per > 2 * shallow) return deepest;
   return std::max(fewest, std::min(shallow, kb_per));
 }
 
@@ -145,14 +135,7 @@ double plan_cost(const GemmArgs& a, int nkb, int bn, int s, double sm_share, int
   const int clusters = ceil_div(a.M, BM) * ceil_div(a.N, bn) * groups;
   const double cap = std::max(1.0, max_clusters(bn, a.a_mn, a.b_mn, s, stages, push) * sm_share);
   const double waves = std::ceil(clusters / cap);
-  // When the GEMM shares the GPU with other branches the aggregate L2 -> SM operand traffic (not the per-CTA stream) is
-  // what saturates, so the load term is weighted up: plans with wider tiles (fewer re-reads of A) win there.
-  static const double l2_weight = [] {
-    const char* e = std::getenv("RLREP_L2_WEIGHT");
-    return e ? std::atof(e) : 1.0;
-  }();
-  const double contention = sm_share < 0.75 ? l2_weight : 1.0;
-  const double load = contention * (double)(BM + bn) * BK * 4 * kb_per / 48.0;
+  const double load = (double)(BM + bn) * BK * 4 * kb_per / 48.0;
   const double tile = (double)BM * bn * 4;
   // pull: every CTA reads its rows from all peers over DSMEM (dependent loads, ~16 B/clk); push: posted remote
   // stores overlapped with the TMEM drain (~2x cheaper end to end, measured)
@@ -234,30 +217,19 @@ TcGemmPlan make_tc_plan(const GemmArgs& a, int bn, int split_k, float* /*ws*/, s
     // L2-bandwidth bound; K=32, N=288 570 -> 309 us).  Wide tiles keep the one-tile-per-CTA kernel: two or three
     // co-resident CTAs overlap each other there, and the persistent epilogue (1.3 us per 128 x 32 chunk) would dominate
     // -- except for one- or two-k-block GEMMs (the stride-2 transposed conv's K = 32), where any tile width wins.
-    // RLREP_TC_PERSIST=0 disables it, =1 forces it for every GEMM with at least two waves of tiles.
-    static const int persist_mode = [] {
-      const char* e = std::getenv("RLREP_TC_PERSIST");
-      return e ? std::atoi(e) : -1;
-    }();
     const int tiles = ceil_div(a.M, BM) * ceil_div(a.N, p.bn);
-    if (persist_mode == 0) p.persistent = false;
-    else if (persist_mode > 0) p.persistent = p.split_k == 1 && tiles >= 2 * kNumSMs;
-    else p.persistent = p.split_k == 1 && tiles >= 4 * kNumSMs && ((p.bn <= 64 && nkb <= 16) || nkb <= 2);
+    p.persistent = p.split_k == 1 && tiles >= 4 * kNumSMs && ((p.bn <= 64 && nkb <= 16) || nkb <= 2);
   }
   // K-major operand: matrix [rows = M|N, cols = K]; MN-major: matrix [rows = K, cols = M|N].
   // implicit convolution: A is the [M, 32] pixel matrix itself (rows past M zero-fill), not an [M, 288] column matrix
   {
     // implicit convolution, many tiles, 32 output channels: the halo kernel (one A load per tile instead of nine)
-    static const int halo_on = [] {
-      const char* e = std::getenv("RLREP_CONV_HALO");
-      return e ? std::atoi(e) : 1;
-    }();
     const int rows = (128 + 2 * a.conv_w + 2 + 7) & ~7;
     // its epilogue is bias + activation + derivative mask (16-byte aligned, dense 32-column operands)
     const bool plain = a.epi.r1_u == nullptr && a.epi.pre_out == nullptr && !a.epi.accumulate &&
                        (a.epi.bias == nullptr || (reinterpret_cast<uintptr_t>(a.epi.bias) & 15) == 0) &&
                        (a.epi.dact == DACT_NONE || ((reinterpret_cast<uintptr_t>(a.epi.aux) & 15) == 0 && (a.epi.ld_aux & 3) == 0));
-    if (halo_on && plain && a.conv_w > 0 && p.persistent && p.bn == 32 && a.N <= 32 && rows <= 256) p.halo_rows = rows;
+    if (plain && a.conv_w > 0 && p.persistent && p.bn == 32 && a.N <= 32 && rows <= 256) p.halo_rows = rows;
   }
   // (a compacting GEMM whose plan has no halo is refused by GemmRunner::run_compact before anything is launched)
   p.tmA = a.a_mn ? make_map_mnmajor(a.A, a.K, a.M, a.lda, BM)

@@ -26,7 +26,6 @@
 // This header holds the device code and the per-variant launcher; it is included by the gemm_tc_inst_*.cu units (one
 // per (BN, A-major) pair so the 16 kernel variants compile in parallel) and by gemm_tc.cu for the tile constants.
 #pragma once
-#include <cstdlib>
 #include <algorithm>
 #include <cstdint>
 
@@ -301,11 +300,6 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   // `stages` is a launch parameter: short K-slices run with a shallow ring so that two CTAs (of this or of a
   // concurrent GEMM on another stream) fit on one SM; long ones get the deepest ring that fits.
   const int STAGES = stages;
-  // DRAFT (branch draft/pdl-gemm-chain, not verified on hardware): bit 1 of `push` marks a launch with programmatic
-  // stream serialization.  Such a CTA may start while the previous kernel of the stream is still running: it does its
-  // prologue (barrier init, TMEM allocation), lets ITS dependents start theirs (launch_dependents), and only then waits
-  // for the previous grid's memory (griddepcontrol.wait) before the first operand load.
-  const bool pdl = (push & 2) != 0;
   // bits 8..15: K groups - 1.  gridDim.z = groups x splits: every group of `splits` CTAs (one cluster) reduces its own K
   // range into its own output matrix, `group` matrices of ceil(M / 128) * 128 rows behind each other -- K-parallelism
   // beyond the 8 CTAs a cluster can hold, for the caller to sum (the implicit conv weight gradient: K ~ 1e5)
@@ -364,9 +358,8 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     else if (conv_w < 0) ptx::tma_load_4d(b_dst, &tmB, &full_bar[s], 0, k0, (n0 / 32) % 8, (n0 / 32) / 8);
     else ptx::tma_load_3d(b_dst, &tmB, &full_bar[s], 0, k0, n0 / 32);
   };
-  // one stage before the setup barrier (TMA issue itself is not free) -- except under PDL, where no global read may
-  // precede griddepcontrol.wait
-  const int first_round = pdl ? 0 : (nkb < 1 ? nkb : 1);
+  // one stage before the setup barrier (TMA issue itself is not free)
+  const int first_round = nkb < 1 ? nkb : 1;
   if (warp == 0 && lane == 0) {
     // The producer owns the barriers: it initialises them and immediately fills the ring (no empty-wait is needed
     // for the first round), so the first operands are in flight while the other warps allocate TMEM.
@@ -387,10 +380,6 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   ptx::tc_fence_after_sync();
   const uint32_t tmem_base = *tmem_slot;
   if (threadIdx.x == 0) trace(1);
-  if (pdl) {
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    asm volatile("griddepcontrol.wait;" ::: "memory");  // every thread: the epilogue reads aux / bias / C as well
-  }
 
   if (warp == 0) {
     // ------------------------------------------------------------ TMA producer
@@ -527,7 +516,7 @@ __device__ __forceinline__ void persist_store_rows(const Epilogue& epi, const fl
 // epilogue warps drain tile i (tcgen05.ld -> epilogue math -> 128-byte global stores, one output row per thread), the MMA
 // warp is already accumulating tile i + 1 into the other half of TMEM.
 //   warp 0: TMA producer | warp 1: MMA issuer (owns TMEM alloc / dealloc) | warps 2..5: epilogue (TMEM lane quarter w & 3)
-// Status: opt-in (RLREP_TC_PERSIST=1), see make_tc_plan -- functionally verified, not yet faster than one tile per CTA.
+// make_tc_plan picks it for conv-shaped GEMMs (thousands of narrow tiles with a handful of k-blocks each).
 constexpr int kPersistThreads = 192;
 
 template <int BN, bool A_MN, bool B_MN>
@@ -697,8 +686,7 @@ gemm_tf32_persistent_kernel(const __grid_constant__ CUtensorMap tmA, const __gri
 // [m0, m0 + 128 + 2 conv_w + 2) as one 128B-swizzled box -- and the nine taps are nine sets of MMAs whose A descriptors
 // start `shift` rows into that buffer.  Measured on B200: the 128-byte swizzle is a function of the ABSOLUTE shared-memory
 // address (bits 4-6 XOR bits 7-9), so a start address that is not 1024-byte aligned needs nothing else -- the descriptor's
-// base-offset field stays 0 (setting it to shift % 8 gives wrong products; RLREP_HALO_FLAGS=1 keeps that variant for the
-// record).  The 36 KB of weights are loaded once per CTA and stay resident.
+// base-offset field stays 0 (setting it to shift % 8 gives wrong products).  The 36 KB of weights are loaded once per CTA and stay resident.
 // N <= 32 (every convolution of the pixel agents has 32 output channels), A K-major.
 // Rows of a 32 x 16 accumulator chunk staged in tw[32][20]: lane = (row group of 8, 16-byte piece), four passes
 // Output mapping and tap list of a halo-kernel launch (GemmArgs::compact_* / conv_tap_*), by value
@@ -789,14 +777,10 @@ constexpr int kHaloBytes = kHaloMaxRows * 128;     // per stage
 constexpr int kHaloSmem = kHaloStages * kHaloBytes + 9 * 32 * BK * 4 + 1024 + 256 + 8 * 32 * 20 * 4;
 static_assert(kHaloSmem <= kMaxSmem, "halo kernel shared memory");
 
-__device__ __forceinline__ uint64_t smem_desc_sw128_rows(uint32_t addr, uint32_t base_offset) {
-  return ptx::make_smem_desc(addr, 16, 1024, 2) | (static_cast<uint64_t>(base_offset & 7u) << 49);
-}
-
 template <bool B_MN>
 __global__ void __launch_bounds__(kHaloThreads, 1)
 gemm_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                      float* __restrict__ C, int ldc, int M, int N, int halo_rows, int flags, const HaloGeom geo,
+                      float* __restrict__ C, int ldc, int M, int N, int halo_rows, const HaloGeom geo,
                       const Epilogue epi) {
   constexpr int BN = 32;
   constexpr int B_BYTES = BN * BK * 4;
@@ -878,10 +862,9 @@ gemm_conv_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
         for (int tap = 0; tap < 9; ++tap) {
           if (tap >= ntaps) break;
           const uint32_t a_addr = a_base + tap_a[tap], b_addr = b_base + tap_b[tap];
-          const uint32_t bo = (flags & 1) ? ((tap_a[tap] >> 7) & 7u) : 0u;
 #pragma unroll
           for (int k = 0; k < BK / UMMA_K; ++k) {
-            const uint64_t adesc = smem_desc_sw128_rows(a_addr + k * UMMA_K * 4, bo);
+            const uint64_t adesc = ptx::make_smem_desc(a_addr + k * UMMA_K * 4, 16, 1024, 2);
             const uint64_t bdesc = B_MN ? ptx::make_smem_desc(b_addr + k * 1024, 4096, 512, 1)
                                         : ptx::make_smem_desc(b_addr + k * UMMA_K * 4, 16, 1024, 2);
             ptx::mma_tf32_ss(d_tmem, adesc, bdesc, idesc, (tap > 0 || k > 0) ? 1u : 0u);
@@ -954,10 +937,6 @@ void launch_conv_halo(const TcGemmPlan& p, cudaStream_t stream) {
     RLREP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kHaloSmem));
     attr_set = true;
   }
-  static const int flags = [] {
-    const char* e = std::getenv("RLREP_HALO_FLAGS");
-    return e ? std::atoi(e) : 0;
-  }();
   const GemmArgs& a = p.args;
   const int tiles = ceil_div(a.M, BM);
   HaloGeom geo;
@@ -973,8 +952,8 @@ void launch_conv_halo(const TcGemmPlan& p, cudaStream_t stream) {
     RLREP_CHECK(t >= geo.ntaps || (geo.shift[t] >= 0 && geo.shift[t] + 128 <= p.halo_rows && geo.kb[t] >= 0 && geo.kb[t] < 9),
                 "halo convolution: tap outside the halo buffer");
   }
-  kern<<<std::min(tiles, kNumSMs), kHaloThreads, kHaloSmem, stream>>>(p.tmA, p.tmB, a.C, a.ldc, a.M, a.N, p.halo_rows, flags,
-                                                                       geo, a.epi);
+  kern<<<std::min(tiles, kNumSMs), kHaloThreads, kHaloSmem, stream>>>(p.tmA, p.tmB, a.C, a.ldc, a.M, a.N, p.halo_rows, geo,
+                                                                       a.epi);
   RLREP_LAUNCHED_W("gemm_conv_halo", stream, 4.0 * ((double)a.M * 32 + (double)a.N * a.K + (double)a.M * a.N),
                    2.0 * a.M * a.N * a.K);
 }
@@ -1005,15 +984,6 @@ void launch_variant_persistent(const TcGemmPlan& p, cudaStream_t stream) {
                    2.0 * a.M * a.N * a.K);
 }
 
-// DRAFT: RLREP_PDL=1 launches every one-tile GEMM with programmatic stream serialization (default off).
-inline bool pdl_enabled() {
-  static const bool on = [] {
-    const char* e = std::getenv("RLREP_PDL");
-    return e != nullptr && std::atoi(e) != 0;
-  }();
-  return on;
-}
-
 template <int BN, bool A_MN, bool B_MN>
 void fill_launch_config(cudaLaunchConfig_t& cfg, cudaLaunchAttribute* attr, dim3 grid, int split_k, int stages,
                         bool push, cudaStream_t stream) {
@@ -1034,11 +1004,6 @@ void fill_launch_config(cudaLaunchConfig_t& cfg, cudaLaunchAttribute* attr, dim3
   attr[0].val.clusterDim.z = split_k;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  if (pdl_enabled() && stream != nullptr) {
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.numAttrs = 2;
-  }
 }
 
 template <int BN, bool A_MN, bool B_MN>
@@ -1048,12 +1013,12 @@ void launch_variant(const TcGemmPlan& p, cudaStream_t stream) {
   RLREP_CHECK(p.stages >= (p.push ? 2 : min_stages(BN)) && p.stages <= num_stages(BN), "bad pipeline depth");
   RLREP_CHECK(!p.push || (p.split_k > 1 && smem_bytes(BN, p.stages, true) <= kMaxSmem), "bad push-mode plan");
   cudaLaunchConfig_t cfg;
-  cudaLaunchAttribute attr[2];
+  cudaLaunchAttribute attr[1];
   fill_launch_config<BN, A_MN, B_MN>(cfg, attr, dim3(ceil_div(a.N, BN), ceil_div(a.M, BM), p.split_k * p.k_groups),
                                      p.split_k, p.stages, p.push, stream);
   RLREP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tf32_kernel<BN, A_MN, B_MN>, p.tmA, p.tmB, a.C, a.ldc, a.M, a.N, a.K,
                                 p.kb_per_split, p.stages,
-                                (p.push ? 1 : 0) | (pdl_enabled() ? 2 : 0) | ((p.k_groups - 1) << 8),
+                                (p.push ? 1 : 0) | ((p.k_groups - 1) << 8),
                                 a.conv_wgrad_hi > 0 ? -1 : a.conv_w, a.epi));
   g_trace_reader = &read_trace_here;
   // implicit convolution: A is the [M, 32] pixel matrix, read once from HBM (the nine shifted re-reads hit L2)
@@ -1068,7 +1033,7 @@ void launch_variant(const TcGemmPlan& p, cudaStream_t stream) {
 template <int BN, bool A_MN, bool B_MN>
 int max_clusters_variant(int split_k, int stages, bool push) {
   cudaLaunchConfig_t cfg;
-  cudaLaunchAttribute attr[2];
+  cudaLaunchAttribute attr[1];
   fill_launch_config<BN, A_MN, B_MN>(cfg, attr, dim3(1, 1, split_k), split_k, stages, push, nullptr);
   int n = 0;
   if (cudaOccupancyMaxActiveClusters(&n, gemm_tf32_kernel<BN, A_MN, B_MN>, &cfg) != cudaSuccess || n <= 0) {

@@ -68,8 +68,7 @@ __global__ void ring_write_kernel(float4* __restrict__ ring, int rec4, long long
 // ------------------------------------------------------------------------------------------- contrastive CE
 // One CTA per row: online max/sum pass, then rewrite the row as the CE gradient.
 __global__ void __launch_bounds__(256) ce_rows_kernel(float* __restrict__ logits, int ld, int cols, int diag_off,
-                                                      float inv_batch, float* __restrict__ loss_rows, int diag_blk,
-                                                      int diag_stride) {
+                                                      float inv_batch, float* __restrict__ loss_rows) {
   __shared__ float scratch[33];
   const int row = blockIdx.x;
   float* l = logits + (size_t)row * ld;
@@ -80,9 +79,7 @@ __global__ void __launch_bounds__(256) ce_rows_kernel(float* __restrict__ logits
   for (int j = threadIdx.x; j < cols; j += 256) sum += expf(l[j] - mx);
   sum = block_sum<256>(sum, scratch);
   const float lse = mx + logf(sum);
-  // column of this row's positive: diag_off + row, or -- when the columns are laid out in slices of diag_blk rows per
-  // rank (the sharded update gathers mu in row slices) -- slice * diag_stride + diag_off + row % diag_blk
-  const int dj = diag_blk > 0 ? (row / diag_blk) * diag_stride + diag_off + row % diag_blk : diag_off + row;
+  const int dj = diag_off + row;  // column of this row's positive
   if (threadIdx.x == 0) loss_rows[row] = lse - l[dj];
   __syncthreads();
   for (int j = threadIdx.x; j < cols; j += 256) {
@@ -1068,8 +1065,8 @@ void launch_ring_write(float* ring, int rec4, long long capacity, long long star
 }
 
 void launch_ce_rows(float* logits, int ld, int rows, int cols, int diag_off, float inv_batch, float* loss_rows,
-                    cudaStream_t s, int diag_blk, int diag_stride) {
-  ce_rows_kernel<<<rows, 256, 0, s>>>(logits, ld, cols, diag_off, inv_batch, loss_rows, diag_blk, diag_stride);
+                    cudaStream_t s) {
+  ce_rows_kernel<<<rows, 256, 0, s>>>(logits, ld, cols, diag_off, inv_batch, loss_rows);
   RLREP_LAUNCHED_W("ce_rows", s, 3.0 * 4.0 * (double)rows * cols, 0.0);
 }
 

@@ -50,7 +50,7 @@ void launch_ring_write(float* ring, int rec4, long long capacity, long long star
 // Contrastive soft-label CE with identity labels (ctrlsac_agent.py:226-231):
 //   loss_i = logsumexp_j(l_ij) - l_{i, diag_off + i};  in place  l_ij <- (softmax_j(l_i)_j - [j == diag_off+i]) * inv_batch
 void launch_ce_rows(float* logits, int ld, int rows, int cols, int diag_off, float inv_batch, float* loss_rows,
-                    cudaStream_t s, int diag_blk = 0, int diag_stride = 0);
+                    cudaStream_t s);
 
 // y[i] = sum_j X[i,j] w[j] + b[0]  (N = 1 linear heads; one CTA per row)
 void launch_rowdot(const float* X, int ld, int rows, int D, const float* w, const float* b, float* y, cudaStream_t s);

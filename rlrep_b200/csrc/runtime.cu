@@ -1,7 +1,6 @@
 // Host runtime: replay ring, GEMM dispatch with cached TMA plans, linear-layer pass helpers, graph replay.
 #include <algorithm>
 #include <atomic>
-#include <cstdlib>
 
 #include "agent.cuh"
 
@@ -157,9 +156,6 @@ void Ring::gather_from_host_idx(const long long* idx_host, int B, float* out_dev
 // ================================================================================================ GemmRunner
 void GemmRunner::init(Precision prec, size_t ws_floats) {
   prec_ = prec;
-  if (const char* e = std::getenv("RLREP_CHAIN")) chains_on_ = std::atoi(e) != 0;
-  if (const char* e = std::getenv("RLREP_CHAIN_ROWOPS")) row_ops_on_ = std::atoi(e) != 0;
-  if (const char* e = std::getenv("RLREP_GEMM_KGROUPS")) kg_on_ = std::atoi(e) != 0;
   ws_floats_ = ws_floats;
   if (ws_floats_) RLREP_CUDA(cudaMalloc(&ws_, ws_floats_ * sizeof(float)));
 }
@@ -178,7 +174,7 @@ void GemmRunner::begin_chain(cudaStream_t s) {
 
 void GemmRunner::flush_chain() {
   if (pending_.empty()) return;
-  if (pending_.size() == 1 && pending_[0].row.kind == ROWOP_NONE) {  // nothing to chain: the one-GEMM kernels do this better
+  if (pending_.size() == 1) {  // nothing to chain: the one-GEMM kernels do this better
     const GemmArgs a = pending_[0];
     pending_.clear();
     const bool rec = recording_;
@@ -197,14 +193,6 @@ void GemmRunner::flush_chain() {
   }
   chain->launch(chain_stream_);
   pending_.clear();
-}
-
-bool GemmRunner::row_op(const RowOp& op) {
-  if (!recording_ || !row_ops_on_) return false;
-  GemmArgs a;
-  a.row = op;
-  pending_.push_back(a);
-  return true;
 }
 
 void GemmRunner::end_chain() {
@@ -250,14 +238,11 @@ void GemmRunner::run(const GemmArgs& a, cudaStream_t s) {
   // Deep and skinny (the pixel agents' 39,200-wide linears at batch 256: K = 39,200 and 2 x 1..4 tiles): a split-K cluster
   // holds 8 CTAs, so such a GEMM runs on 16-64 CTAs that stream ~5 MB each.  Cut K into groups (GemmArgs::k_groups: own
   // cluster and raw partial output each), then one elementwise pass adds the groups and applies the epilogue.
-  if (kg_on_ && a.k_groups == 1 && a.conv_w == 0 && a.conv_wgrad_hi == 0 && !recording_) {
+  if (a.k_groups == 1 && a.conv_w == 0 && a.conv_wgrad_hi == 0 && !recording_) {
     const int tiles = ceil_div(a.M, 128) * ceil_div(a.N, 128), nkb = ceil_div(a.K, 32);
     int groups = 1;
-    static const int cta_cap = [] {
-      const char* e = std::getenv("RLREP_GEMM_KGROUP_CTAS");
-      return e ? std::atoi(e) : 296;  // up to two waves of CTAs (measured on the muLV update: 148 -> 5.82 ms, 296 -> 5.77 ms)
-    }();
-    while (groups < 8 && tiles * 8 * groups * 2 <= cta_cap && nkb >= 256 * groups * 2) groups *= 2;
+    constexpr int kCtaCap = 296;  // up to two waves of CTAs (measured on the muLV update: 148 -> 5.82 ms, 296 -> 5.77 ms)
+    while (groups < 8 && tiles * 8 * groups * 2 <= kCtaCap && nkb >= 256 * groups * 2) groups *= 2;
     if (groups > 1 && nkb >= 1024) {
       const int ldw = (a.N + 3) & ~3, m_pad = ceil_div(a.M, 128) * 128;
       const size_t need = (size_t)groups * m_pad * ldw;

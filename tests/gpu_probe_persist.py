@@ -1,7 +1,7 @@
-"""Timeline of the persistent tcgen05 GEMM on conv-like shapes (many tiles, few k-blocks).  Run with RLREP_TC_PERSIST=1.
-Prints, for CTA 0's first 12 tiles, nanoseconds (relative to the first stamp) of: TMA issued, operands landed,
-accumulator committed, epilogue start, epilogue end; then the average time of the planned GEMM with and without it."""
-import os
+"""Timeline of the persistent tcgen05 GEMM on conv-like shapes (many tiles, few k-blocks), which make_tc_plan runs on the
+persistent kernel at bn = 32.  Prints, for CTA 0's first 12 tiles, nanoseconds (relative to the first stamp) of: TMA
+issued, operands landed, accumulator committed, epilogue start, epilogue end; then the average time of the GEMM planned
+at each tile width."""
 import sys
 from pathlib import Path
 
@@ -23,7 +23,7 @@ for (M, N, K) in [(430336, 288, 32), (430336, 32, 288)]:
     _lib.check(lib.rlrep_gemm_set_debug_buffer(None))
     t = dbg.cpu().reshape(5, 16)
     t0 = int(t[t > 0].min()) if (t > 0).any() else 0
-    print(f"M={M} N={N} K={K} persist={os.environ.get('RLREP_TC_PERSIST', '0')}")
+    print(f"M={M} N={N} K={K}")
     for i in range(12):
         print("  tile %2d: " % i + "  ".join(f"{(int(t[r, i]) - t0) if t[r, i] > 0 else -1:7d}" for r in range(5)))
     for bn in (32, 64, 128, 256):

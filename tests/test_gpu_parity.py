@@ -520,20 +520,3 @@ def test_device_noise_matches_oracle_on_the_same_stream(case):
     assert wi < BARS["fp32"], where_i
     assert wp < BARS["fp32"], where_p
     assert skipped < 2e-2
-
-
-def test_row_operations_inside_the_chain(monkeypatch):
-    """RLREP_CHAIN_ROWOPS=1: the replay gather and the contrastive head run as row-operation items of the feature step's
-    chain kernel (one launch per feature step) instead of stand-alone kernels between two chains -- same results."""
-    monkeypatch.setenv("RLREP_CHAIN_ROWOPS", "1")
-    alg, shp, kw, B = CASES["ctrlsac"]
-    agent, buf, oracle, oring = make_pair(alg, shp["S"], shp["A"], kw, rows=5000, precision="tf32",
-                                          oracle_kw=dict(as_written=False))
-    ci, oi = step_both(agent, buf, oracle, oring, B, 3)
-    wi, where_i = worst_info_error(ci, oi, atol=1e-5)
-    wp, where_p, _ = worst_param_error(agent, oracle)
-    print(f"row ops in chain: worst info rel {wi:.2e} at {where_i}; worst param rel-l2 {wp:.2e} at {where_p}; "
-          f"{agent.gpu_launches_last_train} launches")
-    assert wi < BARS["tf32"], where_i
-    assert wp < BARS["tf32"], where_p
-    assert agent.gpu_launches_last_train == 28  # 40 with the stand-alone gather / head kernels: 3 fewer per feature step
