@@ -293,8 +293,15 @@ RLREP_EXPORT int rlrep_drq_sync_targets(rlrep_drq* drq);
 RLREP_EXPORT int rlrep_drq_update(rlrep_drq* drq, const unsigned char* img, const float* action, const float* reward,
                                   const float* discount, const unsigned char* next_img, const int* shifts,
                                   const float* eps, float stddev, float* metrics_host);
-/* select_action (drqv2.py:74-82): obs uint8 [C, H, H]; eps_host == NULL -> dist.mean, else TruncatedNormal.sample(clip=None)
- * with eps[action_dim] ~ N(0, 1) and the schedule's stddev.  Not to be interleaved with rlrep_drq_update. */
+/* select_action (drqv2.py:74-82) on n observations: obs uint8 [n, C, H, H] in host memory or device memory (a CUDA
+ * tensor is copied device to device); eps_host == NULL -> dist.mean, else TruncatedNormal.sample(clip=None) with
+ * eps_host [n, action_dim] ~ N(0, 1) and the schedule's stddev; actions_host [n, action_dim].  Runs the small-batch policy
+ * (csrc/pixel_act.cu) in IEEE fp32 whatever the handle's precision, in chunks of 64 observations, on the handle's own
+ * buffers: it reads the current weights, touches no update buffer, and may be called between updates.  Each action is
+ * bit-identical to the n = 1 call on its observation.  n <= 0 or a null obs / actions pointer is an error.
+ * rlrep_drq_act is the n = 1 case. */
+RLREP_EXPORT int rlrep_drq_act_batch(rlrep_drq* drq, const unsigned char* obs, const float* eps_host, float stddev, int n,
+                                     float* actions_host);
 RLREP_EXPORT int rlrep_drq_act(rlrep_drq* drq, const unsigned char* obs_host, const float* eps_host, float stddev,
                                float* action_host);
 /* Benchmark aids on the batch uploaded by the last rlrep_drq_update: n_steps updates back to back with CUDA-event timing;
@@ -338,8 +345,12 @@ RLREP_EXPORT int rlrep_mulv_update(rlrep_mulv* h, const unsigned char* img, cons
                                    const float* discount, const unsigned char* next_img, const unsigned char* img_step1,
                                    const int* shifts, const float* eps_z, const float* eps_act, const float* noise,
                                    float stddev, float* metrics_host);
-/* act (drqv2.py:270-282): obs uint8 [C, 84, 84]; eps_host == NULL -> dist.mean (eval_mode), else
- * TruncatedNormal.sample(clip=None) with eps[action_dim] ~ N(0, 1).  Not to be interleaved with rlrep_mulv_update. */
+/* act (drqv2.py:270-282) on n observations, with the contract of rlrep_drq_act_batch: obs uint8 [n, C, 84, 84] host or
+ * device; eps_host == NULL -> dist.mean (eval_mode), else TruncatedNormal.sample(clip=None) with eps_host [n, action_dim]
+ * ~ N(0, 1); actions_host [n, action_dim].  The exploration phase's uniform actions are the caller's (rlrep_b200/pixel.py).
+ * rlrep_mulv_act is the n = 1 case. */
+RLREP_EXPORT int rlrep_mulv_act_batch(rlrep_mulv* h, const unsigned char* obs, const float* eps_host, float stddev, int n,
+                                      float* actions_host);
 RLREP_EXPORT int rlrep_mulv_act(rlrep_mulv* h, const unsigned char* obs_host, const float* eps_host, float stddev,
                                 float* action_host);
 RLREP_EXPORT int rlrep_mulv_update_resident(rlrep_mulv* h, int n_steps, float stddev, float* total_ms);

@@ -111,6 +111,7 @@ def _declare(lib: C.CDLL) -> None:
         "rlrep_drq_update": [vp, vp, vp, vp, vp, vp, vp, vp, C.c_float, vp],
         "rlrep_drq_last_launches": [vp, C.POINTER(i)],
         "rlrep_drq_act": [vp, vp, vp, C.c_float, vp],
+        "rlrep_drq_act_batch": [vp, vp, vp, C.c_float, i, vp],
         "rlrep_drq_update_resident": [vp, i, C.c_float, C.POINTER(C.c_float)],
         "rlrep_drq_profile_update": [vp, C.c_float, i, C.POINTER(C.c_char_p), C.POINTER(C.c_float), C.POINTER(C.c_double),
                                      C.POINTER(C.c_double), C.POINTER(i)],
@@ -137,6 +138,7 @@ def _declare(lib: C.CDLL) -> None:
         "rlrep_mulv_update": [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_float, vp],
         "rlrep_mulv_last_launches": [vp, C.POINTER(i)],
         "rlrep_mulv_act": [vp, vp, vp, C.c_float, vp],
+        "rlrep_mulv_act_batch": [vp, vp, vp, C.c_float, i, vp],
         "rlrep_mulv_update_resident": [vp, i, C.c_float, C.POINTER(C.c_float)],
         "rlrep_mulv_profile_update": [vp, C.c_float, i, C.POINTER(C.c_char_p), C.POINTER(C.c_float), C.POINTER(C.c_double),
                                       C.POINTER(C.c_double), C.POINTER(i)],

@@ -104,7 +104,7 @@ DrqV2::DrqV2(const DrqConfig& c, cudaStream_t s)
   const size_t img_bytes = (size_t)B_ * c.channels * c.height * c.height;
   stage_bytes_ = 2 * img_bytes + (size_t)4 * B_ * sizeof(int) + ((size_t)2 * B_ * A_ + (size_t)B_ * A_ + 2 * B_) * sizeof(float);
   RLREP_CUDA(cudaMallocHost(&stage_host_, stage_bytes_));
-  RLREP_CUDA(cudaMallocHost(&metrics_host_, (size_t)std::max(8, A_) * sizeof(float)));
+  RLREP_CUDA(cudaMallocHost(&metrics_host_, 8 * sizeof(float)));
   Control h;
   std::memset(&h, 0, sizeof(h));
   RLREP_CUDA(cudaMemcpyAsync(ctl_, &h, sizeof(h), cudaMemcpyHostToDevice, stream_));
@@ -183,28 +183,21 @@ void DrqV2::actor_forward(const float* latent, const float* eps, float stddev, i
   launch_trunc_normal_sample(raw_, LA_, B_, A_, eps, stddev, cfg_.stddev_clip, mu_, cat_[set] + bn_, LC_, stream_);
 }
 
-// select_action (drqv2.py:74-82): encoder (no augmentation) -> actor -> mu (deterministic) or
-// TruncatedNormal.sample(clip=None) with the caller's standard-normal draw.  Runs the batch-sized kernels with the
-// observation in row 0 (the other rows carry stale frames and are ignored), so it must not be interleaved with an
-// update -- the reference's agent is single-threaded as well.
-void DrqV2::act(const unsigned char* obs_host, const float* eps_host, float stddev, float* action_host) {
-  cudaStream_t s = stream_;
-  const size_t one = (size_t)cfg_.channels * cfg_.height * cfg_.height;
-  RLREP_CUDA(cudaStreamSynchronize(s));
-  std::memcpy(stage_host_, obs_host, one);
-  float* eps_stage = reinterpret_cast<float*>(stage_host_ + ((one + 15) & ~size_t(15)));
-  for (int j = 0; j < A_; ++j) eps_stage[j] = eps_host ? eps_host[j] : 0.f;
-  RLREP_CUDA(cudaMemcpyAsync(img_dev_, stage_host_, one, cudaMemcpyHostToDevice, s));
-  RLREP_CUDA(cudaMemcpyAsync(eps_dev_, eps_stage, A_ * sizeof(float), cudaMemcpyHostToDevice, s));
-  enc_->forward(img_dev_, nullptr, latent_, 0, false, /*no_grad=*/true);
-  const float saved_clip = cfg_.stddev_clip;
-  cfg_.stddev_clip = INFINITY;  // clip=None
-  actor_forward(latent_, eps_dev_, eps_host ? stddev : 0.f, 0, false);
-  cfg_.stddev_clip = saved_clip;
-  RLREP_CUDA(cudaMemcpy2DAsync(metrics_host_, A_ * sizeof(float), cat_[0] + bn_, LC_ * sizeof(float), A_ * sizeof(float), 1,
-                               cudaMemcpyDeviceToHost, s));
-  RLREP_CUDA(cudaStreamSynchronize(s));
-  std::memcpy(action_host, metrics_host_, A_ * sizeof(float));
+// select_action (drqv2.py:74-82) on n observations: the small-batch policy (pixel_act.cu) over this handle's
+// parameters, created on first use
+void DrqV2::act_batch(const unsigned char* obs, const float* eps_host, float stddev, int n, float* actions_host) {
+  if (!policy_) {
+    PixelPolicyWeights pw;
+    for (int l = 0; l < 4; ++l) pw.conv[l] = enc_->layer(l);
+    pw.trunk = at_.view(actor_g_);
+    pw.ln_w = actor_g_.p + aln_w_;
+    pw.ln_b = actor_g_.p + aln_b_;
+    pw.policy[0] = p0_.view(actor_g_);
+    pw.policy[1] = p1_.view(actor_g_);
+    pw.policy[2] = p2_.view(actor_g_);
+    policy_.reset(new PixelPolicy(cfg_.channels, cfg_.height, A_, pw, stream_));
+  }
+  policy_->act(obs, eps_host, stddev, n, actions_host);
 }
 
 float DrqV2::update_resident(int n_steps, float stddev) {

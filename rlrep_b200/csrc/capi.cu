@@ -523,9 +523,14 @@ int rlrep_drq_update(rlrep_drq* drq, const unsigned char* img, const float* acti
   RLREP_API_END
 }
 int rlrep_drq_act(rlrep_drq* drq, const unsigned char* obs_host, const float* eps_host, float stddev, float* action_host) {
+  return rlrep_drq_act_batch(drq, obs_host, eps_host, stddev, 1, action_host);
+}
+int rlrep_drq_act_batch(rlrep_drq* drq, const unsigned char* obs, const float* eps_host, float stddev, int n,
+                        float* actions_host) {
   RLREP_API_BEGIN_ON(drq)
-  RLREP_CHECK(drq && obs_host && action_host, "null argument");
-  drq->impl->act(obs_host, eps_host, stddev, action_host);
+  RLREP_CHECK(drq && obs && actions_host, "null argument");
+  RLREP_CHECK(n > 0, "n must be positive");
+  drq->impl->act_batch(obs, eps_host, stddev, n, actions_host);
   RLREP_API_END
 }
 int rlrep_drq_update_resident(rlrep_drq* drq, int n_steps, float stddev, float* total_ms) {
@@ -656,9 +661,14 @@ int rlrep_mulv_update(rlrep_mulv* h, const unsigned char* img, const float* acti
   RLREP_API_END
 }
 int rlrep_mulv_act(rlrep_mulv* h, const unsigned char* obs_host, const float* eps_host, float stddev, float* action_host) {
+  return rlrep_mulv_act_batch(h, obs_host, eps_host, stddev, 1, action_host);
+}
+int rlrep_mulv_act_batch(rlrep_mulv* h, const unsigned char* obs, const float* eps_host, float stddev, int n,
+                         float* actions_host) {
   RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && obs_host && action_host, "null argument");
-  h->impl->act(obs_host, eps_host, stddev, action_host);
+  RLREP_CHECK(h && obs && actions_host, "null argument");
+  RLREP_CHECK(n > 0, "n must be positive");
+  h->impl->act_batch(obs, eps_host, stddev, n, actions_host);
   RLREP_API_END
 }
 int rlrep_mulv_update_resident(rlrep_mulv* h, int n_steps, float stddev, float* total_ms) {

@@ -4,6 +4,7 @@
 
 #include "agent.cuh"
 #include "conv.cuh"
+#include "pixel_act.cuh"
 
 namespace rlrep {
 
@@ -31,8 +32,10 @@ class DrqV2 {
   // in milliseconds; one update with an event behind every launch.
   float update_resident(int n_steps, float stddev);
   std::vector<ProfileEntry> profile_update(float stddev);
-  // obs uint8 [C, H, H]; eps [A] standard normal or nullptr (deterministic: the mean); action [A]
-  void act(const unsigned char* obs_host, const float* eps_host, float stddev, float* action_host);
+  // select_action on n observations (PixelPolicy::act): obs uint8 [n, C, H, H] host or device; eps [n, A] standard normal
+  // or nullptr (deterministic: the mean); actions [n, A].  Reads the current weights and no update buffer.
+  // The policy's buffers are allocated by the first call: a handle that never acts allocates nothing for it.
+  void act_batch(const unsigned char* obs, const float* eps_host, float stddev, int n, float* actions_host);
   void sync_targets_from_params();
   std::vector<ParamGroup*> groups() { return {&enc_->group(), &actor_g_, &crit_g_}; }
   cudaStream_t stream() const { return stream_; }
@@ -68,6 +71,7 @@ class DrqV2 {
   float *dhid1_ = nullptr, *dhid0_ = nullptr, *dcat_ = nullptr, *dtpre_ = nullptr, *gb_ = nullptr, *gg_ = nullptr;
   float *draw_ = nullptr, *dap2_ = nullptr, *dap1_ = nullptr, *dth_ = nullptr, *metrics_host_ = nullptr;
   size_t stage_bytes_ = 0;
+  std::unique_ptr<PixelPolicy> policy_;
 };
 
 }  // namespace rlrep

@@ -5,6 +5,7 @@
 #include "agent.cuh"
 #include "conv.cuh"
 #include "deconv.cuh"
+#include "pixel_act.cuh"
 
 namespace rlrep {
 
@@ -42,9 +43,10 @@ class MulvDrq {
   void update(const unsigned char* img, const float* action, const float* reward, const float* discount,
               const unsigned char* next_img, const unsigned char* img_step1, const int* shifts, const float* eps_z,
               const float* eps_act, const float* noise, float stddev, float* metrics_out);
-  // act (drqv2.py:270-282): obs uint8 [C, H, H]; eps [A] standard normal or nullptr (eval_mode: the mean); action [A].
-  // Runs the batch-sized kernels with the observation in row 0; not to be interleaved with update().
-  void act(const unsigned char* obs_host, const float* eps_host, float stddev, float* action_host);
+  // act (drqv2.py:270-282) on n observations (PixelPolicy::act): obs uint8 [n, C, H, H] host or device; eps [n, A]
+  // standard normal or nullptr (eval_mode: the mean); actions [n, A].  Reads the current weights and no update buffer.
+  // The policy's buffers are allocated by the first call: a handle that never acts allocates nothing for it.
+  void act_batch(const unsigned char* obs, const float* eps_host, float stddev, int n, float* actions_host);
   float update_resident(int n_steps, float stddev);
   std::vector<ProfileEntry> profile_update(float stddev);
   void sync_targets_from_params();
@@ -95,6 +97,7 @@ class MulvDrq {
   float *dth_ = nullptr, *dtpre_ = nullptr;
   size_t stage_bytes_ = 0;
   static constexpr int kKlBlocks = 64;
+  std::unique_ptr<PixelPolicy> policy_;
 };
 
 }  // namespace rlrep

@@ -28,6 +28,36 @@ def _frames_arg(t):
     return a, a.ctypes.data
 
 
+def _obs_batch(obs, obs_shape):
+    """Observations [N, *obs_shape] uint8 -- numpy, a CPU tensor or a CUDA tensor -- as (keep-alive, pointer, N).  Wrong
+    dtypes and shapes raise ValueError here, before anything reaches the device."""
+    t = obs if isinstance(obs, torch.Tensor) else torch.as_tensor(np.asarray(obs))
+    if t.dtype != torch.uint8:
+        raise ValueError(f"observations must be uint8 frame stacks, got {t.dtype}")
+    if t.dim() != 1 + len(obs_shape) or tuple(t.shape[1:]) != tuple(obs_shape) or t.shape[0] == 0:
+        raise ValueError(f"observations must have shape [N, {', '.join(map(str, obs_shape))}] with N >= 1, "
+                         f"got {tuple(t.shape)}")
+    keep, ptr = _frames_arg(t)
+    _sync_if_cuda(keep)
+    return keep, ptr, int(t.shape[0])
+
+
+def _act_noise(n, action_dim, sample, explore=False):
+    """Host draws of n consecutive single acts, in their order.  Per observation: `torch.normal(zeros(1, A), ones(1, A))`
+    when sampling (TruncatedNormal.sample's _standard_normal), then, in muLV-Rep's exploration phase, the `uniform_(-1, 1)`
+    of [A] that replaces the action.  One [n, A] draw would consume the generator differently.
+    Returns (eps [n, A] float32 or None, uniform [n, A] float32 or None)."""
+    eps = np.empty((n, action_dim), dtype=np.float32) if sample else None
+    uni = np.empty((n, action_dim), dtype=np.float32) if explore else None
+    for i in range(n):
+        if sample:
+            z = torch.zeros(1, action_dim)
+            eps[i] = torch.normal(z, torch.ones_like(z)).numpy()[0]
+        if explore:
+            uni[i] = torch.empty(action_dim).uniform_(-1.0, 1.0).numpy()
+    return eps, uni
+
+
 def _host_f32(t):
     return np.ascontiguousarray(torch.as_tensor(t).detach().cpu().numpy(), dtype=np.float32).reshape(-1)
 
@@ -272,18 +302,21 @@ class DrQv2:
     def select_action(self, obs, step, deterministic=False):
         """drqv2.py:74-82.  `obs` is one uint8 frame stack [C, H, W]; the handle must exist (weights loaded after the
         first train_step, or call `prepare(batch_size)` first)."""
+        return self.select_actions(torch.as_tensor(obs).unsqueeze(0), step, deterministic)[0]
+
+    def select_actions(self, obs, step, deterministic=False):
+        """`select_action` on N observations at once: obs uint8 [N, C, H, W] (numpy, CPU or CUDA tensor) -> actions
+        [N, A].  Row i is bit-identical to `select_action(obs[i])`, and the generator advances exactly as N consecutive
+        select_action calls advance it."""
         if self._h is None:
             raise _lib.RlrepError("call prepare(batch_size) or train_step once before select_action")
-        o = np.ascontiguousarray(torch.as_tensor(obs).cpu().numpy())
-        assert o.dtype == np.uint8 and tuple(o.shape) == self.obs_dim
+        keep, ptr, n = _obs_batch(obs, self.obs_dim)
         stddev = float(self.stddev_schedule(step))
-        eps = None
-        if not deterministic:  # TruncatedNormal.sample(clip=None): one _standard_normal([1, A]) draw
-            z = torch.zeros(1, self.action_dim)
-            eps = np.ascontiguousarray(torch.normal(z, torch.ones_like(z)).numpy().reshape(-1))
-        out = np.empty(self.action_dim, dtype=np.float32)
-        _lib.check(self.lib.rlrep_drq_act(self._h, o.ctypes.data, eps.ctypes.data if eps is not None else None, stddev,
-                                          out.ctypes.data))
+        eps, _ = _act_noise(n, self.action_dim, sample=not deterministic)
+        out = np.empty((n, self.action_dim), dtype=np.float32)
+        _lib.check(self.lib.rlrep_drq_act_batch(self._h, ptr, eps.ctypes.data if eps is not None else None, stddev, n,
+                                                out.ctypes.data))
+        del keep
         return out
 
     def prepare(self, batch_size):
@@ -486,21 +519,22 @@ class MuLVDrQv2:
         """drqv2.py:270-282.  `obs` is one uint8 frame stack [C, H, W]; the handle must exist (`prepare(batch_size)` or one
         `update`).  Exploration (`step < num_expl_steps`, not eval_mode) replaces the sample by U(-1, 1) after drawing it,
         like the reference."""
+        return self.act_batch(torch.as_tensor(obs).unsqueeze(0), step, eval_mode)[0]
+
+    def act_batch(self, obs, step, eval_mode):
+        """`act` on N observations at once: obs uint8 [N, C, H, W] (numpy, CPU or CUDA tensor) -> actions [N, A].  Row i
+        is bit-identical to `act(obs[i])`, and the generator advances exactly as N consecutive act calls advance it."""
         if self._h is None:
             raise _lib.RlrepError("call prepare(batch_size) or update once before act")
-        o = np.ascontiguousarray(torch.as_tensor(obs).cpu().numpy())
-        assert o.dtype == np.uint8 and tuple(o.shape) == self.obs_shape
+        keep, ptr, n = _obs_batch(obs, self.obs_shape)
         stddev = float(self.stddev_schedule(step))
-        eps = None
-        if not eval_mode:  # TruncatedNormal.sample(clip=None): one _standard_normal([1, A]) draw
-            z = torch.zeros(1, self.action_dim)
-            eps = np.ascontiguousarray(torch.normal(z, torch.ones_like(z)).numpy().reshape(-1))
-        out = np.empty(self.action_dim, dtype=np.float32)
-        _lib.check(self.lib.rlrep_mulv_act(self._h, o.ctypes.data, eps.ctypes.data if eps is not None else None, stddev,
-                                           out.ctypes.data))
-        if not eval_mode and step < int(_cfg_get(self.cfg, "num_expl_steps", 2000)):
-            out = torch.empty(self.action_dim).uniform_(-1.0, 1.0).numpy()
-        return out
+        explore = not eval_mode and step < int(_cfg_get(self.cfg, "num_expl_steps", 2000))
+        eps, uni = _act_noise(n, self.action_dim, sample=not eval_mode, explore=explore)
+        out = np.empty((n, self.action_dim), dtype=np.float32)
+        _lib.check(self.lib.rlrep_mulv_act_batch(self._h, ptr, eps.ctypes.data if eps is not None else None, stddev, n,
+                                                 out.ctypes.data))
+        del keep
+        return uni if explore else out
 
     def update(self, replay_iter, step):
         if step % self.up_every != 0:
