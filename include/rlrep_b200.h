@@ -266,6 +266,36 @@ RLREP_EXPORT int rlrep_conv_encoder_backward(rlrep_conv_encoder* enc, const floa
 RLREP_EXPORT int rlrep_conv_encoder_feature_dim(rlrep_conv_encoder* enc, int* dim);
 
 /* ------------------------------------------------------------------------------------------------
+ * Pixel decoder on its own -- the 3 x ConvTranspose2d(s1) + ConvTranspose2d(s2) + Conv2d stack of muLV-Rep
+ * (agent/mulvdrq/drqv2.py:98-117, out_kernel 2) and of the latent Diff-SR VAE (vae_1d.Decoder, out_kernel 3, stride-2
+ * layer with output_padding 1), as the agents run it, for kernel-level tests.  Layer l = 0..3 is `deconvnet.{2l}`
+ * (weights [ci, co, 3, 3] / [32]), layer 4 the output conv `deconvnet.8` ([3, 32, k, k] / [3]).
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct rlrep_conv_decoder rlrep_conv_decoder;
+RLREP_EXPORT int rlrep_conv_decoder_create(int batch, int out_kernel, int precision, void* stream,
+                                           rlrep_conv_decoder** out);
+RLREP_EXPORT int rlrep_conv_decoder_destroy(rlrep_conv_decoder* dec);
+/* what: 0 = weight, 1 = bias, 2 = weight gradient, 3 = bias gradient (host buffers, reference layout); write takes 0 / 1 */
+RLREP_EXPORT int rlrep_conv_decoder_read(rlrep_conv_decoder* dec, int layer, int what, float* out_host);
+RLREP_EXPORT int rlrep_conv_decoder_write(rlrep_conv_decoder* dec, int layer, int what, const float* in_host);
+/* x_dev fp32 [B, 32*35*35] in the reference's (channel, row, column) order with row pitch ld_x (0 = dense); the
+ * prediction [B, 3, 84, 84] stays in the handle. */
+RLREP_EXPORT int rlrep_conv_decoder_forward(rlrep_conv_decoder* dec, const float* x_dev, int ld_x);
+/* loss_dev[0] = 10 * mean |pred - (target / 255 - 0.5)|; target uint8 [B, 3, 84, 84]; keeps grad_scale * d loss / d pred */
+RLREP_EXPORT int rlrep_conv_decoder_l1_loss(rlrep_conv_decoder* dec, const unsigned char* target_dev, float grad_scale,
+                                            float* loss_dev);
+/* loss_dev[0] = sum (pred - (shifted target / 255 - 0.5))^2 / B; shifts_dev int32 [B, 2] = (x, y) in [0, 8] or NULL */
+RLREP_EXPORT int rlrep_conv_decoder_mse_sum_loss(rlrep_conv_decoder* dec, const unsigned char* target_dev,
+                                                 const int* shifts_dev, float grad_scale, float* loss_dev);
+/* parameter gradients of the five layers (readable with _read) and dx_dev [B, 32*35*35] with row pitch ld_dx (0 = dense;
+ * the columns past 32*35*35 are not written) */
+RLREP_EXPORT int rlrep_conv_decoder_backward(rlrep_conv_decoder* dec, float* dx_dev, int ld_dx);
+/* Copies an internal map of the last forward / loss / backward to out_dev in NCHW: which 0 = the input of layer i
+ * (i = 0..4, [B, 32, h_i, h_i]), 1 = the gradient with respect to it (ReLU mask applied for i > 0), 2 = pred,
+ * 3 = grad_scale * d loss / d pred (both [B, 3, 84, 84]; i is ignored). */
+RLREP_EXPORT int rlrep_conv_decoder_read_map(rlrep_conv_decoder* dec, int which, int i, float* out_dev);
+
+/* ------------------------------------------------------------------------------------------------
  * Plain DrQ-v2 pixel agent -- replaces `DrQv2(obs_space, action_space, args)` and the updating half of
  * `DrQv2.train_step(replay_iter, step)` (agent/diffsrdrq/drqv2.py:12-148).  The caller keeps `_step` / `update_every`,
  * evaluates the std-dev schedule and draws the randomness in the reference's order on the CPU generator:

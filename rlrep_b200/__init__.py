@@ -15,7 +15,7 @@ def __getattr__(name):  # lazy: importing the package must not require torch.cud
                 "AGENTS"):
         from . import agents
         return getattr(agents, name)
-    if name in ("ConvEncoder", "DrQv2", "MuLVDrQv2", "LatentDiffSRDrQv2"):
+    if name in ("ConvEncoder", "ConvDecoder", "DrQv2", "MuLVDrQv2", "LatentDiffSRDrQv2"):
         from . import pixel
         return getattr(pixel, name)
     if name == "PixelReplayBuffer":

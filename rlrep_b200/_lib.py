@@ -101,6 +101,15 @@ def _declare(lib: C.CDLL) -> None:
         "rlrep_conv_encoder_forward": [vp, vp, vp, vp],
         "rlrep_conv_encoder_backward": [vp, vp],
         "rlrep_conv_encoder_feature_dim": [vp, C.POINTER(i)],
+        "rlrep_conv_decoder_create": [i, i, i, vp, C.POINTER(vp)],
+        "rlrep_conv_decoder_destroy": [vp],
+        "rlrep_conv_decoder_read": [vp, i, i, vp],
+        "rlrep_conv_decoder_write": [vp, i, i, vp],
+        "rlrep_conv_decoder_forward": [vp, vp, i],
+        "rlrep_conv_decoder_l1_loss": [vp, vp, f, vp],
+        "rlrep_conv_decoder_mse_sum_loss": [vp, vp, vp, f, vp],
+        "rlrep_conv_decoder_backward": [vp, vp, i],
+        "rlrep_conv_decoder_read_map": [vp, i, i, vp],
         "rlrep_drq_create": [vp, vp, C.POINTER(vp)],
         "rlrep_drq_destroy": [vp],
         "rlrep_drq_num_tensors": [vp, C.POINTER(i)],

@@ -10,7 +10,9 @@
 #include "comm.cuh"
 #include "common.cuh"
 #include "conv.cuh"
+#include "deconv.cuh"
 #include "drq.cuh"
+#include "layout.cuh"
 #include "mulv.cuh"
 #include "pixel_replay.cuh"
 #include "ldiffsr.cuh"
@@ -424,6 +426,125 @@ int rlrep_conv_encoder_feature_dim(rlrep_conv_encoder* enc, int* dim) {
   RLREP_API_BEGIN_ON(enc)
   RLREP_CHECK(enc && dim, "null argument");
   *dim = enc->impl->feature_dim();
+  RLREP_API_END
+}
+
+// ------------------------------------------------------------------------------------------------ pixel decoder
+struct rlrep_conv_decoder {
+  int device = current_device();
+  std::unique_ptr<ConvDecoder> impl;
+  cudaStream_t owned_stream = nullptr;
+};
+
+// Reference layout [ci, co, 3, 3] of a transposed layer (0-3) <-> stored [(ky, kx, co), ci]; the output conv (layer 4) is
+// stored in the reference's [3, 32, k, k] as is.
+static void deconv_layout(int layer, size_t n, bool to_stored, const float* in, float* out) {
+  if (layer == 4) {
+    std::copy(in, in + n, out);
+    return;
+  }
+  for (int ci = 0; ci < 32; ++ci)
+    for (int co = 0; co < 32; ++co)
+      for (int t = 0; t < 9; ++t) {
+        const size_t ref = ((size_t)ci * 32 + co) * 9 + t, st = ((size_t)t * 32 + co) * 32 + ci;
+        if (to_stored) out[st] = in[ref];
+        else out[ref] = in[st];
+      }
+}
+static size_t deconv_param_size(const ConvDecoder& d, int layer, bool bias) {
+  if (layer == 4) return bias ? 3 : (size_t)3 * 32 * d.out_kernel() * d.out_kernel();
+  return bias ? 32 : 288 * 32;
+}
+
+int rlrep_conv_decoder_create(int batch, int out_kernel, int precision, void* stream, rlrep_conv_decoder** out) {
+  RLREP_API_BEGIN
+  RLREP_CHECK(out != nullptr, "null out pointer");
+  std::unique_ptr<rlrep_conv_decoder> h(new rlrep_conv_decoder);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (st == nullptr) {
+    RLREP_CUDA(cudaStreamCreateWithFlags(&h->owned_stream, cudaStreamNonBlocking));
+    st = h->owned_stream;
+  }
+  h->impl.reset(new ConvDecoder(batch, static_cast<Precision>(precision), st, out_kernel));
+  *out = h.release();
+  RLREP_API_END
+}
+int rlrep_conv_decoder_destroy(rlrep_conv_decoder* dec) {
+  RLREP_API_BEGIN_ON(dec)
+  if (dec) {
+    if (dec->impl) cudaStreamSynchronize(dec->impl->stream());
+    dec->impl.reset();
+    if (dec->owned_stream) cudaStreamDestroy(dec->owned_stream);
+  }
+  delete dec;
+  RLREP_API_END
+}
+int rlrep_conv_decoder_read(rlrep_conv_decoder* dec, int layer, int what, float* out_host) {
+  RLREP_API_BEGIN_ON(dec)
+  RLREP_CHECK(dec && out_host && layer >= 0 && layer < 5 && what >= 0 && what < 4, "bad argument");
+  ConvDecoder& d = *dec->impl;
+  const bool bias = what == 1 || what == 3;
+  const size_t n = deconv_param_size(d, layer, bias);
+  const float* src = (what < 2 ? d.group().p : d.group().g) + (bias ? d.bias_offset(layer) : d.weight_offset(layer));
+  std::vector<float> tmp(n);
+  cudaStream_t st = d.stream();
+  RLREP_CUDA(cudaMemcpyAsync(tmp.data(), src, n * sizeof(float), cudaMemcpyDeviceToHost, st));
+  RLREP_CUDA(cudaStreamSynchronize(st));
+  if (bias) std::copy(tmp.begin(), tmp.end(), out_host);
+  else deconv_layout(layer, n, false, tmp.data(), out_host);
+  RLREP_API_END
+}
+int rlrep_conv_decoder_write(rlrep_conv_decoder* dec, int layer, int what, const float* in_host) {
+  RLREP_API_BEGIN_ON(dec)
+  RLREP_CHECK(dec && in_host && layer >= 0 && layer < 5 && (what == 0 || what == 1), "bad argument");
+  ConvDecoder& d = *dec->impl;
+  const bool bias = what == 1;
+  const size_t n = deconv_param_size(d, layer, bias);
+  std::vector<float> tmp(in_host, in_host + n);
+  if (!bias) deconv_layout(layer, n, true, in_host, tmp.data());
+  cudaStream_t st = d.stream();
+  RLREP_CUDA(cudaMemcpyAsync(d.group().p + (bias ? d.bias_offset(layer) : d.weight_offset(layer)), tmp.data(),
+                             n * sizeof(float), cudaMemcpyHostToDevice, st));
+  RLREP_CUDA(cudaStreamSynchronize(st));
+  RLREP_API_END
+}
+int rlrep_conv_decoder_forward(rlrep_conv_decoder* dec, const float* x_dev, int ld_x) {
+  RLREP_API_BEGIN_ON(dec)
+  RLREP_CHECK(dec && x_dev && ld_x >= 0, "bad argument");
+  dec->impl->forward(x_dev, ld_x);
+  RLREP_API_END
+}
+int rlrep_conv_decoder_l1_loss(rlrep_conv_decoder* dec, const unsigned char* target_dev, float grad_scale,
+                               float* loss_dev) {
+  RLREP_API_BEGIN_ON(dec)
+  RLREP_CHECK(dec && target_dev && loss_dev, "null argument");
+  dec->impl->l1_loss(target_dev, grad_scale, loss_dev);
+  RLREP_API_END
+}
+int rlrep_conv_decoder_mse_sum_loss(rlrep_conv_decoder* dec, const unsigned char* target_dev, const int* shifts_dev,
+                                    float grad_scale, float* loss_dev) {
+  RLREP_API_BEGIN_ON(dec)
+  RLREP_CHECK(dec && target_dev && loss_dev, "null argument");
+  dec->impl->mse_sum_loss(target_dev, shifts_dev, grad_scale, loss_dev);
+  RLREP_API_END
+}
+int rlrep_conv_decoder_backward(rlrep_conv_decoder* dec, float* dx_dev, int ld_dx) {
+  RLREP_API_BEGIN_ON(dec)
+  RLREP_CHECK(dec && dx_dev && ld_dx >= 0, "bad argument");
+  dec->impl->backward(dx_dev, ld_dx);
+  RLREP_API_END
+}
+int rlrep_conv_decoder_read_map(rlrep_conv_decoder* dec, int which, int i, float* out_dev) {
+  RLREP_API_BEGIN_ON(dec)
+  RLREP_CHECK(dec && out_dev && which >= 0 && which < 4 && (which >= 2 || (i >= 0 && i < 5)), "bad argument");
+  ConvDecoder& d = *dec->impl;
+  if (which >= 2) {
+    d.copy_pred(out_dev, which == 3);
+  } else {
+    const int P = d.hw(i) * d.hw(i);
+    launch_nhwc_to_cp(which == 0 ? d.act(i) : d.dact(i), d.batch(), P, out_dev, (long long)P * 32, d.stream());
+    RLREP_LAUNCHED("nhwc_to_nchw", d.stream());
+  }
   RLREP_API_END
 }
 

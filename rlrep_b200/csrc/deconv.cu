@@ -547,10 +547,10 @@ void ConvDecoder::backward(float* dx_dev, int ld_dx) {
   RLREP_LAUNCHED_W("nhwc_to_nchw", s, 8.0 * B_ * P0 * 32, 0.0);
 }
 
-void ConvDecoder::copy_pred(float* pred_nchw_dev) {
+void ConvDecoder::copy_pred(float* pred_nchw_dev, bool grad) {
   const long long P = (long long)hw_[5] * hw_[5];
-  pred_to_nchw_kernel<<<grid_for((long long)B_ * P, 256), 256, 0, stream_>>>(reinterpret_cast<const float4*>(pred_), B_, P,
-                                                                            pred_nchw_dev);
+  pred_to_nchw_kernel<<<grid_for((long long)B_ * P, 256), 256, 0, stream_>>>(
+      reinterpret_cast<const float4*>(grad ? dpred_ : pred_), B_, P, pred_nchw_dev);
   RLREP_LAUNCHED("pred_to_nchw", stream_);
 }
 

@@ -21,11 +21,21 @@ class ConvDecoder {
   void mse_sum_loss(const unsigned char* target_dev, const int* shifts_dev, float grad_scale, float* loss_out_dev);
   // parameter gradients of the five layers and dx [B, 32 * 35 * 35] (row pitch ld_dx)
   void backward(float* dx_dev, int ld_dx);
-  void copy_pred(float* pred_nchw_dev);  // [B, 3, 84, 84]
+  void copy_pred(float* pred_nchw_dev, bool grad = false);  // [B, 3, 84, 84]; grad: d loss / d pred * grad_scale instead
 
   ParamGroup& group() { return g_; }
   int batch() const { return B_; }
+  int out_kernel() const { return ks_; }
   cudaStream_t stream() const { return stream_; }
+
+  // Read-only views of the internal maps, for kernel-level tests: act(i) [B, hw(i), hw(i), 32] is layer i's input
+  // (i = 0: the decoder input); dact(i) the gradient with respect to it, ReLU mask applied for i > 0.  Weight / bias
+  // offsets l = 0..4 index group().p and group().g.
+  int hw(int i) const { return hw_[i]; }
+  const float* act(int i) const { return act_[i]; }
+  const float* dact(int i) const { return dact_[i]; }
+  size_t weight_offset(int l) const { return w_off_[l]; }
+  size_t bias_offset(int l) const { return b_off_[l]; }
 
  private:
   long long rows(int i) const { return (long long)B_ * hw_[i] * hw_[i]; }

@@ -152,6 +152,116 @@ class ConvEncoder:
         self._keep_d = dfeat
 
 
+class ConvDecoder:
+    """The pixel decoder on its own (`rlrep_conv_decoder_*`): muLV-Rep's `Decoder` (agent/mulvdrq/drqv2.py:98-117,
+    out_kernel=2) or the latent Diff-SR VAE decoder's convolutions (out_kernel=3), x [B, 32*35*35] -> pred [B, 3, 84, 84],
+    its two losses and the backward pass, with the handle's internal maps readable for kernel-level tests."""
+    LAYERS = ("deconvnet.0", "deconvnet.2", "deconvnet.4", "deconvnet.6", "deconvnet.8")
+    MAPS = {"act": 0, "dact": 1, "pred": 2, "dpred": 3}
+    IN_DIM = 32 * 35 * 35
+
+    def __init__(self, batch=256, out_kernel=2, precision="tf32"):
+        if not torch.cuda.is_available():
+            raise _lib.RlrepError("rlrep_b200.ConvDecoder needs a CUDA device (there is no CPU fallback)")
+        self.lib = _lib.load()
+        self.batch, self.out_kernel = int(batch), int(out_kernel)
+        self.hw = (35, 37, 39, 41, 83 if self.out_kernel == 2 else 84)
+        self._stream = torch.cuda.Stream()
+        self._h = C.c_void_p()
+        _lib.check(self.lib.rlrep_conv_decoder_create(self.batch, self.out_kernel, _lib.PRECISION[precision],
+                                                      self._stream.cuda_stream, C.byref(self._h)))
+        self._loss = torch.zeros(1, device="cuda")
+
+    def close(self):
+        h, self._h = self._h, None
+        if h:
+            self.lib.rlrep_conv_decoder_destroy(h)
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _shape(self, layer, bias):
+        if layer == 4:
+            return (3,) if bias else (3, 32, self.out_kernel, self.out_kernel)
+        return (32,) if bias else (32, 32, 3, 3)
+
+    def _read(self, layer, what):
+        out = np.empty(self._shape(layer, what in (1, 3)), dtype=np.float32)
+        _lib.check(self.lib.rlrep_conv_decoder_read(self._h, layer, what, out.ctypes.data))
+        return torch.from_numpy(out)
+
+    def state_dict(self):
+        return {f"{n}.{k}": self._read(i, w) for i, n in enumerate(self.LAYERS) for w, k in ((0, "weight"), (1, "bias"))}
+
+    def grads(self):
+        return {f"{n}.{k}": self._read(i, w) for i, n in enumerate(self.LAYERS) for w, k in ((2, "weight"), (3, "bias"))}
+
+    def load_state_dict(self, sd):
+        for i, name in enumerate(self.LAYERS):
+            for what, key in ((0, ".weight"), (1, ".bias")):
+                arr = np.ascontiguousarray(torch.as_tensor(sd[name + key]).detach().cpu().float().numpy())
+                if arr.shape != self._shape(i, what == 1):
+                    raise ValueError(f"{name + key}: expected {self._shape(i, what == 1)}, got {arr.shape}")
+                _lib.check(self.lib.rlrep_conv_decoder_write(self._h, i, what, arr.ctypes.data))
+
+    def _call(self, fn, *args, keep=()):
+        cur = torch.cuda.current_stream()
+        self._stream.wait_stream(cur)
+        _lib.check(fn(self._h, *args))
+        cur.wait_stream(self._stream)
+        self._keep = keep
+
+    def _rows(self, t, name):
+        """[B, >= 32*35*35] fp32 CUDA rows with unit column stride (the row pitch is passed on, as the agents do)."""
+        if not (t.is_cuda and t.dtype == torch.float32 and t.dim() == 2 and t.shape[0] == self.batch
+                and t.shape[1] == self.IN_DIM and t.stride(1) == 1 and t.stride(0) >= self.IN_DIM):
+            raise ValueError(f"{name} must be fp32 CUDA rows [{self.batch}, {self.IN_DIM}] with unit column stride")
+        return t.stride(0)
+
+    def forward(self, x: torch.Tensor) -> None:
+        """x [B, 32*35*35] (a view with a wider row pitch is read in place)."""
+        ld = self._rows(x, "x")
+        self._call(self.lib.rlrep_conv_decoder_forward, x.data_ptr(), ld, keep=(x,))
+
+    def l1_loss(self, target: torch.Tensor, grad_scale=1.0) -> float:
+        assert target.is_cuda and target.dtype == torch.uint8 and tuple(target.shape) == (self.batch, 3, 84, 84)
+        target = target.contiguous()
+        self._call(self.lib.rlrep_conv_decoder_l1_loss, target.data_ptr(), float(grad_scale), self._loss.data_ptr(),
+                   keep=(target,))
+        return self._loss.item()
+
+    def mse_sum_loss(self, target: torch.Tensor, shifts: torch.Tensor | None = None, grad_scale=1.0) -> float:
+        """shifts int32 [B, 2] = (x, y) in [0, 8] (RandomShiftsAug's draw) or None."""
+        assert target.is_cuda and target.dtype == torch.uint8 and tuple(target.shape) == (self.batch, 3, 84, 84)
+        target = target.contiguous()
+        if shifts is not None:
+            shifts = shifts.to(device=target.device, dtype=torch.int32).reshape(self.batch, 2).contiguous()
+        self._call(self.lib.rlrep_conv_decoder_mse_sum_loss, target.data_ptr(),
+                   shifts.data_ptr() if shifts is not None else None, float(grad_scale), self._loss.data_ptr(),
+                   keep=(target, shifts))
+        return self._loss.item()
+
+    def backward(self, dx: torch.Tensor | None = None) -> torch.Tensor:
+        """Fills the parameter gradients and dx [B, 32*35*35] (allocated when None; a view with a wider row pitch is
+        written in place, its padding columns untouched)."""
+        if dx is None:
+            dx = torch.empty(self.batch, self.IN_DIM, device="cuda")
+        ld = self._rows(dx, "dx")
+        self._call(self.lib.rlrep_conv_decoder_backward, dx.data_ptr(), ld, keep=(dx,))
+        return dx
+
+    def read_map(self, which: str, i: int = 0) -> torch.Tensor:
+        """'act' / 'dact' i = 0..4 -> [B, 32, h_i, h_i]; 'pred' / 'dpred' -> [B, 3, 84, 84] (NCHW copies)."""
+        w = self.MAPS[which]
+        shape = (self.batch, 32, self.hw[i], self.hw[i]) if w < 2 else (self.batch, 3, 84, 84)
+        out = torch.empty(shape, device="cuda")
+        self._call(self.lib.rlrep_conv_decoder_read_map, w, int(i), out.data_ptr(), keep=(out,))
+        return out
+
+
 class DrqConfig(C.Structure):
     """Mirror of `rlrep_drq_config` (include/rlrep_b200.h)."""
     _fields_ = [("batch_size", C.c_int), ("channels", C.c_int), ("height", C.c_int), ("action_dim", C.c_int),
