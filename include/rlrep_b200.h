@@ -441,6 +441,9 @@ RLREP_EXPORT int rlrep_ldiff_last_launches(rlrep_ldiff* h, int* launches);
 RLREP_EXPORT int rlrep_agent_act_batch(rlrep_agent* agent, const float* states_host, const float* eps_host, int rows,
                                        float* actions_host);
 RLREP_EXPORT int rlrep_agent_last_launches(rlrep_agent* agent, int* launches);
+/* The captured train() graph: its kernel nodes, and how many of its edges are programmatic (a kernel that may start
+ * while the kernel before it is still running, programmatic dependent launch).  Fails before the graph exists. */
+RLREP_EXPORT int rlrep_agent_graph_stats(rlrep_agent* agent, int* kernel_nodes, int* programmatic_edges);
 
 #ifdef __cplusplus
 }

@@ -176,6 +176,7 @@ def _declare(lib: C.CDLL) -> None:
         "rlrep_pixring_gather": [vp, vp, i, vp, C.c_float, vp, vp, vp, vp, vp, vp],
         "rlrep_agent_act_batch": [vp, vp, vp, i, vp],
         "rlrep_agent_last_launches": [vp, C.POINTER(i)],
+        "rlrep_agent_graph_stats": [vp, C.POINTER(i), C.POINTER(i)],
         "rlrep_agent_train_resident": [vp, vp, vp, vp, i, C.POINTER(C.c_float)],
         "rlrep_agent_profile_train": [vp, vp, vp, vp, i, C.POINTER(C.c_char_p), C.POINTER(C.c_float),
                                       C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(i)],

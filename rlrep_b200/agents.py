@@ -145,6 +145,13 @@ class _Handle:
         _lib.check(self.lib.rlrep_agent_last_launches(self.h, C.byref(v)))
         return v.value
 
+    @property
+    def graph_stats(self) -> tuple[int, int]:
+        """(kernel nodes, programmatic edges) of the captured train() graph."""
+        k, p = C.c_int(), C.c_int()
+        _lib.check(self.lib.rlrep_agent_graph_stats(self.h, C.byref(k), C.byref(p)))
+        return k.value, p.value
+
 
 class SACAgent:
     """Drop-in for agent.sac.sac_agent.SACAgent (sac_agent.py:16-188)."""

@@ -287,6 +287,8 @@ class GraphReplay {
   // graph; later calls replay.  `enabled = false` always runs eagerly.
   void run(cudaStream_t s, bool enabled, const std::function<void()>& body);
   bool captured() const { return exec_ != nullptr; }
+  // Kernel nodes of the captured graph and its edges of type programmatic (PDL); false while nothing is captured.
+  bool stats(int* kernel_nodes, int* programmatic_edges) const;
 
  private:
   int calls_ = 0;
@@ -331,6 +333,8 @@ class Agent {
   // `rows` observations [rows, S] (and noise [rows, A] or nullptr) -> actions [rows, A]: batched policy evaluation
   virtual void act_batch(const float* states_host, const float* eps_host, int rows, float* actions_host) = 0;
   virtual void sync_targets_from_params() = 0;  // target <- param copies (after loading weights)
+  // Shape of the captured train() graph (GraphReplay::stats); false before the graph has been captured.
+  virtual bool graph_stats(int* kernel_nodes, int* programmatic_edges) const = 0;
 
   AgentConfig cfg;
   cudaStream_t stream = nullptr;

@@ -115,6 +115,10 @@ class SacBase : public Agent {
   // action range is done by the caller (the range belongs to the environment, not to this handle).  `rows` observations
   // are evaluated by ONE kernel launch per chunk of kActRows; the kernel reads them from, and writes the actions to, mapped
   // pinned host memory, so a call is: memcpy into the staging buffer, one launch, one stream synchronise.
+  bool graph_stats(int* kernel_nodes, int* programmatic_edges) const override {
+    return graph_.stats(kernel_nodes, programmatic_edges);
+  }
+
   void act(const float* state_host, const float* eps_host, float* action_host) override {
     act_batch(state_host, eps_host, 1, action_host);
   }
@@ -285,9 +289,12 @@ class SacBase : public Agent {
     linear_fwd(gemm_, s, B_, Mat{h1, AH_}, l1, ACT_ELU, h2, AH_);
     linear_fwd(gemm_, s, B_, Mat{h2, AH_}, l2, ACT_NONE, hd, LDH_);
   }
-  Mat actor_sample_cat(Mat obs, const float* eps, float* cat_buf, float* logp_out, int set, cudaStream_t s) {
-    launch_actor_sample(set == 0 ? head_ : bhead_, LDH_, B_, A_, eps, cat_buf + S_, LDSA_, logp_out, s, obs.p, obs.ld, S_);
-    return Mat{cat_buf, LDSA_};
+  // Both samples after actor_trunk(next_obs, 1) and actor_trunk(obs, 0), in one launch: cat(s', a') into cat_next_ with
+  // log pi(a'|s') into logp_next, and cat(s, a_pi) into cat_pi_ with log pi(a_pi|s) into logp_.
+  void actor_sample_cat_pair(Mat next_obs, const float* eps_next, float* logp_next, Mat obs, const float* eps_pi,
+                             cudaStream_t s) {
+    launch_actor_sample_pair(ActorSampleJob{bhead_, eps_next, cat_next_ + S_, logp_next, next_obs.p, next_obs.ld},
+                             ActorSampleJob{head_, eps_pi, cat_pi_ + S_, logp_, obs.p, obs.ld}, LDH_, B_, A_, LDSA_, S_, s);
   }
   // actor_backward with the five GEMMs as one chain on the main stream (no aux branches)
   void actor_backward_chained(Mat obs, const float* eps) {

@@ -237,7 +237,8 @@ class CtrlSacAgent final : public SacBase {
   // ---------------------------------------------------------------------------------------------- chained variants
   // Same arithmetic, same kernels for everything that is not a GEMM; every group of GEMMs between two elementwise kernels
   // runs as ONE persistent chain kernel (gemm_chain.cuh) on the main stream instead of one launch per GEMM on up to four
-  // streams: 57 launches per update instead of 149, and a dependent GEMM starts when its input tiles are complete.
+  // streams: 38 launches per update instead of 149, and a dependent GEMM starts when its input tiles are complete.  Every
+  // kernel of this path is a programmatic dependent launch (launch_pdl): its CTAs start while the kernel before it finishes.
   // The feature step is two chains: both towers and the logits, then the whole backward pass; the replay gather runs before
   // the first and the contrastive head between the two as stand-alone kernels.
   void feature_step_chained(int k, Ring& ring) {  // ctrlsac_agent.py:213-251
@@ -259,6 +260,13 @@ class CtrlSacAgent final : public SacBase {
       a.B = zmu_; a.ldb = D_;
       a.C = logits_; a.ldc = B_;
       gemm_.run(a, s0);
+    }
+    if (k == K_ - 1) {
+      // The critic step's actor trunks, a' ~ pi(s') and a_pi ~ pi(s): they read only the actor, which the feature loop
+      // does not touch, and this last batch, so they share this chain's levels with phi and mu instead of running as a
+      // chain of their own on the critical path.
+      actor_trunk(s2(), /*set=*/1, s0);
+      actor_trunk(Mat{batch_, R_}, /*set=*/0, s0);
     }
     gemm_.end_chain();
     // row log-sum-exp / CE gradient (logits_ then holds dL/dlogits), reward head and the loss metrics
@@ -313,13 +321,10 @@ class CtrlSacAgent final : public SacBase {
     const float* eps_pi = eps_dev_ + (size_t)B_ * A_;
     const Linear l14t = c14_.view(crit_g_, true), l14 = c14_.view(crit_g_), l2 = c2_.view(crit_g_), l5 = c5_.view(crit_g_);
     const Linear l2t = c2_.view(crit_g_, true), l5t = c5_.view(crit_g_, true);
-    // a' ~ pi(s') for the TD target and a_pi ~ pi(s) for the actor step (reads nothing the critic step writes)
-    gemm_.begin_chain(s0);
-    actor_trunk(s2(), /*set=*/1, s0);
-    actor_trunk(Mat{batch_, R_}, /*set=*/0, s0);
-    gemm_.end_chain();
-    const Mat s2a = actor_sample_cat(s2(), eps_next, cat_next_, logp2_, 1, s0);
-    const Mat spi = actor_sample_cat(Mat{batch_, R_}, eps_pi, cat_pi_, logp_, 0, s0);
+    // a' ~ pi(s') for the TD target and a_pi ~ pi(s) for the actor step; their trunks ran in the last feature step's
+    // forward chain
+    actor_sample_cat_pair(s2(), eps_next, logp2_, Mat{batch_, R_}, eps_pi, s0);
+    const Mat s2a{cat_next_, LDSA_}, spi{cat_pi_, LDSA_};
     gemm_.begin_chain(s0);
     phi_forward(s0, s2a, Mat(), 0, zmu_, h1_, h2_);  // frozen_phi_target(s', a'); zmu_ is free after the feature loop
     linear_fwd(gemm_, s0, B_, Mat{zmu_, D_}, l14t, ACT_ELU, hid_t_, 2 * H_);

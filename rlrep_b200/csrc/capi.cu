@@ -1232,6 +1232,13 @@ int rlrep_agent_last_launches(rlrep_agent* agent, int* launches) {
   *launches = agent->impl->last_launches;
   RLREP_API_END
 }
+int rlrep_agent_graph_stats(rlrep_agent* agent, int* kernel_nodes, int* programmatic_edges) {
+  RLREP_API_BEGIN_ON(agent)
+  RLREP_CHECK(agent && kernel_nodes && programmatic_edges, "null argument");
+  RLREP_CHECK(agent->impl->graph_stats(kernel_nodes, programmatic_edges),
+              "no captured graph yet (train() captures it on its second call, with use_graph on)");
+  RLREP_API_END
+}
 int rlrep_agent_train_resident(rlrep_agent* agent, rlrep_ring* ring, const int64_t* idx_host, const float* eps_host,
                                int n_steps, float* total_ms) {
   RLREP_API_BEGIN_ON(agent)

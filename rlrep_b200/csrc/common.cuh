@@ -6,6 +6,7 @@
 #include <cstdio>
 #include <stdexcept>
 #include <string>
+#include <utility>
 #include <vector>
 
 namespace rlrep {
@@ -52,6 +53,28 @@ long long launch_count();
     RLREP_CUDA(cudaGetLastError());                             \
     ::rlrep::note_launch(name, stream, (bytes), (flops));       \
   } while (0)
+
+// Programmatic dependent launch: the kernel may be scheduled while the previous kernel in `stream` is still running
+// and must call ptx::pdl_wait() before it touches memory that kernel may read or write (ptx.cuh).  In a captured graph
+// the edge from the previous kernel becomes a programmatic edge.
+inline cudaLaunchAttribute pdl_attribute() {
+  cudaLaunchAttribute a = {};
+  a.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  a.val.programmaticStreamSerializationAllowed = 1;
+  return a;
+}
+template <typename... KernelArgs, typename... Args>
+void launch_pdl(void (*kernel)(KernelArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args&&... args) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = grid;
+  cfg.blockDim = block;
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = stream;
+  cudaLaunchAttribute attr[1] = {pdl_attribute()};
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  RLREP_CUDA(cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...));
+}
 
 // Per-kernel timing of an eager (non-graph) launch sequence: begin, run the launches, end -> (name, ms) per launch.
 void profile_begin(cudaStream_t stream);

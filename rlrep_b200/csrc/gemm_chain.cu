@@ -231,6 +231,9 @@ gemm_chain_kernel(const ChainGemmDesc* __restrict__ gemms, const ChainTask* __re
   __syncthreads();
   ptx::tc_fence_after_sync();
   const uint32_t tmem_base = *tmem_slot;
+  // Everything above reads build-time data only (task lists); the completion counters, operands and outputs belong to the
+  // previous kernel until it has completed.
+  ptx::pdl_wait();
 
   if (warp == 0) {
     // ------------------------------------------------------------ TMA producer
@@ -518,6 +521,8 @@ gemm_chain_kernel(const ChainGemmDesc* __restrict__ gemms, const ChainTask* __re
       if (lane == 0) ptx::mbar_arrive(&acc_empty[acc]);
     }
   }
+  // This thread's role is done: the tail below (TMEM release, exit counter, counter re-arm) overlaps the next kernel's start.
+  ptx::pdl_launch_dependents();
   ptx::tc_fence_before_sync();
   __syncthreads();
   if (warp == 1) ptx::tmem_dealloc(tmem_base, 2 * kMaxBn);
@@ -829,11 +834,12 @@ void GemmChain::launch(cudaStream_t stream) {
   cfg.stream = stream;
   // cooperative: all CTAs are co-scheduled or none is, so two chains launched on different streams can never hold part of
   // the GPU each while spinning on tiles of CTAs that are not resident
-  cudaLaunchAttribute attr[1];
+  cudaLaunchAttribute attr[2];
   attr[0].id = cudaLaunchAttributeCooperative;
   attr[0].val.cooperative = 1;
+  attr[1] = pdl_attribute();
   cfg.attrs = attr;
-  cfg.numAttrs = 1;
+  cfg.numAttrs = 2;
   RLREP_CUDA(cudaLaunchKernelEx(&cfg, gemm_chain_kernel, (const ChainGemmDesc*)d_gemms_, (const ChainTask*)d_tasks_,
                                 (const int*)d_task_begin_, d_done_, d_exit_, (int)seq_.size(), g_chain_dbg));
   RLREP_LAUNCHED_W("gemm_chain", stream, bytes_, flops_);

@@ -369,12 +369,15 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     }
     ptx::mbar_init(accum_bar, 1);
     ptx::fence_mbar_init();
-    for (int it = 0; it < first_round; ++it) produce(it);
   }
   if (warp == 2) {
     ptx::tmem_alloc(tmem_slot, TMEM_COLS);
     ptx::tmem_relinquish();
   }
+  // the operands and C may still be in use by the previous kernel (launch_variant launches with PDL)
+  ptx::pdl_wait();
+  if (warp == 0 && lane == 0)
+    for (int it = 0; it < first_round; ++it) produce(it);
   ptx::tc_fence_before_sync();
   __syncthreads();
   ptx::tc_fence_after_sync();
@@ -462,6 +465,7 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   if (splits > 1) ptx::cluster_sync(); else __syncthreads();
   if (threadIdx.x == 0) trace(6);
   if (warp == 2) ptx::tmem_dealloc(tmem_base, TMEM_COLS);  // every tcgen05.ld has completed: the tile is in shared memory
+  ptx::pdl_launch_dependents();  // only the reduction and the stores remain
 
   // ---------------------------------------------------------------- reduce + epilogue + coalesced store (all warps)
   {
@@ -1013,9 +1017,11 @@ void launch_variant(const TcGemmPlan& p, cudaStream_t stream) {
   RLREP_CHECK(p.stages >= (p.push ? 2 : min_stages(BN)) && p.stages <= num_stages(BN), "bad pipeline depth");
   RLREP_CHECK(!p.push || (p.split_k > 1 && smem_bytes(BN, p.stages, true) <= kMaxSmem), "bad push-mode plan");
   cudaLaunchConfig_t cfg;
-  cudaLaunchAttribute attr[1];
+  cudaLaunchAttribute attr[2];
   fill_launch_config<BN, A_MN, B_MN>(cfg, attr, dim3(ceil_div(a.N, BN), ceil_div(a.M, BM), p.split_k * p.k_groups),
                                      p.split_k, p.stages, p.push, stream);
+  attr[1] = pdl_attribute();
+  cfg.numAttrs = 2;
   RLREP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tf32_kernel<BN, A_MN, B_MN>, p.tmA, p.tmB, a.C, a.ldc, a.M, a.N, a.K,
                                 p.kb_per_split, p.stages,
                                 (p.push ? 1 : 0) | ((p.k_groups - 1) << 8),

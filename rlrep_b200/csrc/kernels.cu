@@ -4,6 +4,7 @@
 #include "common.cuh"
 #include "epilogue.cuh"
 #include "kernels.cuh"
+#include "ptx.cuh"
 #include "reduce.cuh"
 
 namespace rlrep {
@@ -24,6 +25,8 @@ __device__ __forceinline__ AdamHyper adam_hyper(double lr, long long t) {
 __global__ void tick_kernel(Control* c, const TickParams p) {
   // One warp: every lane reads the counters, then each of the (k_feat + 5) independent results -- two double-precision
   // pow() each -- is computed by its own lane instead of one after the other (7.5 us -> ~2 us at the head of every update).
+  ptx::pdl_wait();
+  ptx::pdl_launch_dependents();
   const int lane = threadIdx.x;
   if (blockIdx.x != 0 || lane >= 32) return;
   const long long t_feat = c->t_feat, t_critic = c->t_critic, t_actor = c->t_actor, t_alpha = c->t_alpha;
@@ -50,6 +53,8 @@ __global__ void tick_kernel(Control* c, const TickParams p) {
 // ------------------------------------------------------------------------------------------- ring
 __global__ void gather_kernel(const float4* __restrict__ ring, int rec4, const long long* __restrict__ idx, int B,
                               float4* __restrict__ out) {
+  ptx::pdl_wait();
+  ptx::pdl_launch_dependents();
   const int total = B * rec4;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
     const int b = i / rec4, c = i - b * rec4;
@@ -235,6 +240,8 @@ struct ColJobs {
 // memory round trip for the whole reduction instead of 32 dependent-latency steps), then a fixed-order smem tree.
 __global__ void __launch_bounds__(1024) colreduce_multi_kernel(const ColJobs jobs) {
   __shared__ float part[32][33];
+  ptx::pdl_wait();
+  ptx::pdl_launch_dependents();
   const ColJob& jb = jobs.j[blockIdx.y];
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
   const int j = blockIdx.x * 32 + tx;
@@ -322,6 +329,8 @@ __global__ void __launch_bounds__(256) contrastive_head_kernel(float* __restrict
                                                                unsigned* __restrict__ counter, int rows) {
   __shared__ float scratch[33];
   __shared__ bool last;
+  ptx::pdl_wait();
+  ptx::pdl_launch_dependents();
   const int row = blockIdx.x;
   float* l = logits + (size_t)row * ld;
   float mx = -INFINITY;
@@ -389,10 +398,20 @@ constexpr float kLogStdMin = -5.f, kLogStdMax = 2.f;  // sac_agent.py:64
 
 // One warp per row: lane j handles action dimension j (+32, ...), the log-prob terms are warp-reduced, and -- when
 // `obs` is given -- all lanes copy the S observation columns in front of the action so that `action - S` becomes the
-// contiguous cat(obs, action) row the next network's first layer reads (row pitch lda).
-__global__ void actor_sample_kernel(const float* __restrict__ head, int ld_head, int B, int A,
-                                    const float* __restrict__ eps, float* __restrict__ action, int lda,
-                                    float* __restrict__ logp, const float* __restrict__ obs, int ld_obs, int S) {
+// contiguous cat(obs, action) row the next network's first layer reads (row pitch lda).  blockIdx.y selects the job.
+struct ActorSampleJobs {
+  ActorSampleJob j[2];
+};
+__global__ void actor_sample_kernel(const ActorSampleJobs jobs, int ld_head, int B, int A, int lda, int S) {
+  ptx::pdl_wait();
+  ptx::pdl_launch_dependents();
+  const ActorSampleJob& jb = jobs.j[blockIdx.y];
+  const float* __restrict__ head = jb.head;
+  const float* __restrict__ eps = jb.eps;
+  float* __restrict__ action = jb.action;
+  float* __restrict__ logp = jb.logp;
+  const float* __restrict__ obs = jb.obs;
+  const int ld_obs = jb.ld_obs;
   const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (b >= B) return;
   const float* h = head + (size_t)b * ld_head;
@@ -471,6 +490,8 @@ __global__ void __launch_bounds__(256) actor_act_kernel(const float* __restrict_
 __global__ void actor_sample_bwd_kernel(const float* __restrict__ head, int ld_head, int B, int A,
                                         const float* __restrict__ eps, const float* __restrict__ d_action, int ldd,
                                         const float* __restrict__ dlogp_scalar, float* __restrict__ dhead, int ld_dh) {
+  ptx::pdl_wait();
+  ptx::pdl_launch_dependents();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B * A) return;
   const int b = i / A, j = i - b * A;
@@ -605,6 +626,8 @@ __global__ void __launch_bounds__(256) critic_td_head_kernel(const CriticHeadArg
   __shared__ float scratch[33];
   __shared__ float bc[2];
   __shared__ bool last;
+  ptx::pdl_wait();
+  ptx::pdl_launch_dependents();
   const int row = blockIdx.x, tid = threadIdx.x, H = a.H;
   const float* ht = a.hid_t + (size_t)row * a.ldh;
   const float* h = a.hid + (size_t)row * a.ldh;
@@ -663,6 +686,8 @@ __global__ void __launch_bounds__(256) actor_head_kernel(const ActorHeadArgs a) 
   __shared__ float scratch[33];
   __shared__ float bc[2];
   __shared__ bool last;
+  ptx::pdl_wait();
+  ptx::pdl_launch_dependents();
   const int row = blockIdx.x, tid = threadIdx.x, H = a.H;
   const float* h = a.hid + (size_t)row * a.ldh;
   float q1 = block_sum<256>(head_dot(h, a.w2, H, tid), scratch);
@@ -780,6 +805,8 @@ __global__ void __launch_bounds__(256) adam_polyak_kernel(float4* __restrict__ p
                                                           const AdamHyper* __restrict__ hyper,
                                                           float4* __restrict__ target, size_t n4_polyak, float tau,
                                                           const int* __restrict__ polyak_flag) {
+  ptx::pdl_wait();
+  ptx::pdl_launch_dependents();
   const float ss = hyper->step_size, bc2s = hyper->bc2_sqrt;
   const bool do_polyak = target != nullptr && (polyak_flag == nullptr || *polyak_flag != 0);
   const float omt = 1.f - tau;
@@ -1046,13 +1073,13 @@ int grid_for(size_t work_items, int threads, int per_sm = 8) {
 
 void launch_tick(Control* c, const TickParams& p, cudaStream_t s) {
   RLREP_CHECK(p.k_feat <= kMaxFeatureSteps, "too many feature steps per update");
-  tick_kernel<<<1, 32, 0, s>>>(c, p);
+  launch_pdl(tick_kernel, 1, 32, 0, s, c, p);
   RLREP_LAUNCHED("tick", s);
 }
 
 void launch_gather(const float* ring, int rec4, const long long* idx, int B, float* out, cudaStream_t s) {
-  gather_kernel<<<grid_for((size_t)B * rec4, 256), 256, 0, s>>>(reinterpret_cast<const float4*>(ring), rec4, idx, B,
-                                                               reinterpret_cast<float4*>(out));
+  launch_pdl(gather_kernel, grid_for((size_t)B * rec4, 256), 256, 0, s, reinterpret_cast<const float4*>(ring), rec4, idx, B,
+             reinterpret_cast<float4*>(out));
   RLREP_LAUNCHED_W("gather", s, 2.0 * 16.0 * (double)B * rec4, 0.0);
 }
 
@@ -1123,7 +1150,7 @@ void launch_colreduce_multi(const ColJob* jobs, int n_jobs, cudaStream_t s) {
     js.j[i] = jobs[i];
     if (jobs[i].cols > max_cols) max_cols = jobs[i].cols;
   }
-  colreduce_multi_kernel<<<dim3(ceil_div(max_cols, 32), n_jobs), 1024, 0, s>>>(js);
+  launch_pdl(colreduce_multi_kernel, dim3(ceil_div(max_cols, 32), n_jobs), 1024, 0, s, js);
   RLREP_LAUNCHED("colreduce_multi", s);
 }
 
@@ -1144,23 +1171,34 @@ void launch_contrastive_head(float* logits, int ld, int rows, int cols, int diag
                              int D, const float* theta_w, const float* theta_b, const float* reward, int ld_r,
                              float* loss_rows, float* pred, float* dpred, float* metrics, unsigned* counter,
                              cudaStream_t s) {
-  contrastive_head_kernel<<<rows, 256, 0, s>>>(logits, ld, cols, diag_off, inv_batch, z, ldz, D, theta_w, theta_b, reward, ld_r,
-                                               loss_rows, pred, dpred, metrics, counter, rows);
+  launch_pdl(contrastive_head_kernel, rows, 256, 0, s, logits, ld, cols, diag_off, inv_batch, z, ldz, D, theta_w, theta_b,
+             reward, ld_r, loss_rows, pred, dpred, metrics, counter, rows);
   RLREP_LAUNCHED_W("contrastive_head", s, 3.0 * 4.0 * (double)rows * cols + 4.0 * (double)rows * D, 0.0);
 }
 
 void launch_critic_td_head(const CriticHeadArgs& a, cudaStream_t s) {
-  critic_td_head_kernel<<<a.B, 256, 0, s>>>(a);
+  launch_pdl(critic_td_head_kernel, a.B, 256, 0, s, a);
   RLREP_LAUNCHED_W("critic_td_head", s, 4.0 * a.B * (4.0 * a.H + 2.0 * a.H), 0.0);
 }
 void launch_actor_head(const ActorHeadArgs& a, cudaStream_t s) {
-  actor_head_kernel<<<a.B, 256, 0, s>>>(a);
+  launch_pdl(actor_head_kernel, a.B, 256, 0, s, a);
   RLREP_LAUNCHED_W("actor_head", s, 4.0 * a.B * (4.0 * a.H), 0.0);
 }
 
 void launch_actor_sample(const float* head, int ld_head, int B, int A, const float* eps, float* action, int lda,
                          float* logp, cudaStream_t s, const float* obs, int ld_obs, int S) {
-  actor_sample_kernel<<<ceil_div(B * 32, 128), 128, 0, s>>>(head, ld_head, B, A, eps, action, lda, logp, obs, ld_obs, S);
+  ActorSampleJobs js;
+  js.j[0] = ActorSampleJob{head, eps, action, logp, obs, ld_obs};
+  js.j[1] = js.j[0];
+  launch_pdl(actor_sample_kernel, dim3(ceil_div(B * 32, 128), 1), 128, 0, s, js, ld_head, B, A, lda, S);
+  RLREP_LAUNCHED("actor_sample", s);
+}
+void launch_actor_sample_pair(const ActorSampleJob& j0, const ActorSampleJob& j1, int ld_head, int B, int A, int lda, int S,
+                              cudaStream_t s) {
+  ActorSampleJobs js;
+  js.j[0] = j0;
+  js.j[1] = j1;
+  launch_pdl(actor_sample_kernel, dim3(ceil_div(B * 32, 128), 2), 128, 0, s, js, ld_head, B, A, lda, S);
   RLREP_LAUNCHED("actor_sample", s);
 }
 
@@ -1175,8 +1213,8 @@ void launch_actor_act(const float* in, int rows, int S, int A, int H, const floa
 
 void launch_actor_sample_bwd(const float* head, int ld_head, int B, int A, const float* eps, const float* d_action,
                              int ldd, const float* dlogp_scalar, float* dhead, int ld_dhead, cudaStream_t s) {
-  actor_sample_bwd_kernel<<<ceil_div(B * A, 128), 128, 0, s>>>(head, ld_head, B, A, eps, d_action, ldd, dlogp_scalar,
-                                                               dhead, ld_dhead);
+  launch_pdl(actor_sample_bwd_kernel, ceil_div(B * A, 128), 128, 0, s, head, ld_head, B, A, eps, d_action, ldd, dlogp_scalar,
+             dhead, ld_dhead);
   RLREP_LAUNCHED("actor_sample_bwd", s);
 }
 
@@ -1270,9 +1308,9 @@ void launch_adam_polyak(float* p, const float* g, float* m, float* v, size_t n, 
                         size_t n_polyak, float tau, const int* polyak_flag, cudaStream_t s) {
   RLREP_CHECK(n % 4 == 0 && n_polyak % 4 == 0, "optimizer arenas are padded to float4");
   const size_t n4 = n / 4;
-  adam_polyak_kernel<<<grid_for(n4, 256, 16), 256, 0, s>>>(
-      reinterpret_cast<float4*>(p), reinterpret_cast<const float4*>(g), reinterpret_cast<float4*>(m),
-      reinterpret_cast<float4*>(v), n4, hyper, reinterpret_cast<float4*>(target), n_polyak / 4, tau, polyak_flag);
+  launch_pdl(adam_polyak_kernel, grid_for(n4, 256, 16), 256, 0, s, reinterpret_cast<float4*>(p),
+             reinterpret_cast<const float4*>(g), reinterpret_cast<float4*>(m), reinterpret_cast<float4*>(v), n4, hyper,
+             reinterpret_cast<float4*>(target), n_polyak / 4, tau, polyak_flag);
   // 28 B/param (p, g, m, v read; p, m, v written) + 12 B/param of Polyak (p is already in registers: target read +
   // written = 8 B; counted as 12 like SURVEY.md 8d counts a stand-alone Polyak) -- a gated Polyak fires every 2nd step
   const double polyak = target ? 12.0 * (double)n_polyak * (polyak_flag ? 0.5 : 1.0) : 0.0;

@@ -99,6 +99,17 @@ void launch_feature_loss_finalize(const float* loss_rows, int rows, const float*
 // obs != nullptr: also copy obs[b, 0:S] to action[b, -S:0], i.e. build the contiguous cat(obs, action) row.
 void launch_actor_sample(const float* head, int ld_head, int B, int A, const float* eps, float* action, int lda,
                          float* logp, cudaStream_t s, const float* obs = nullptr, int ld_obs = 0, int S = 0);
+// Two independent launch_actor_sample calls with the same shapes (ld_head, B, A, lda, S) as one launch.
+struct ActorSampleJob {
+  const float* head;
+  const float* eps;
+  float* action;
+  float* logp;
+  const float* obs;
+  int ld_obs;
+};
+void launch_actor_sample_pair(const ActorSampleJob& j0, const ActorSampleJob& j1, int ld_head, int B, int A, int lda, int S,
+                              cudaStream_t s);
 // Backward of the above: dhead [B, ld_dhead >= 2A] from d_action [B, ldd] and the per-row d_logp scalar.
 // launch_ce_rows + launch_rowdot (reward head theta) + launch_feature_loss_finalize as one launch; `counter` is a
 // zero-initialised device word owned by the caller (arrival counter of the row CTAs, re-armed by the kernel).

@@ -26,6 +26,17 @@ __device__ __forceinline__ bool elect_one() {
   return pred != 0;
 }
 
+// ---------------------------------------------------------------- programmatic dependent launch
+// A kernel launched with the programmatic-serialization attribute (launch_pdl, common.cuh) may start while the kernel
+// before it in the stream is still running.  pdl_wait() blocks until that kernel has completed and its writes are
+// visible; before it a kernel may only touch shared memory, TMEM and data written at build time.  Every CTA must wait,
+// also one with nothing to do: the next kernel's wait covers this kernel's predecessor only through this kernel's wait.
+// In a kernel launched without the attribute both instructions do nothing.
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+// Lets the next kernel in the stream start its CTAs (they stop at their own pdl_wait()).  Once every CTA of this grid
+// has issued it or exited, the dependent grid may be scheduled.
+__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
 // ---------------------------------------------------------------- mbarrier
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");

@@ -386,4 +386,29 @@ void GraphReplay::run(cudaStream_t s, bool enabled, const std::function<void()>&
   RLREP_CUDA(cudaGraphLaunch(exec_, s));
 }
 
+bool GraphReplay::stats(int* kernel_nodes, int* programmatic_edges) const {
+  if (exec_ == nullptr) return false;
+  size_t n_nodes = 0;
+  RLREP_CUDA(cudaGraphGetNodes(graph_, nullptr, &n_nodes));
+  std::vector<cudaGraphNode_t> nodes(n_nodes);
+  RLREP_CUDA(cudaGraphGetNodes(graph_, nodes.data(), &n_nodes));
+  int kernels = 0;
+  for (cudaGraphNode_t n : nodes) {
+    cudaGraphNodeType t;
+    RLREP_CUDA(cudaGraphNodeGetType(n, &t));
+    if (t == cudaGraphNodeTypeKernel) ++kernels;
+  }
+  size_t n_edges = 0;
+  RLREP_CUDA(cudaGraphGetEdges_v2(graph_, nullptr, nullptr, nullptr, &n_edges));
+  std::vector<cudaGraphNode_t> from(n_edges), to(n_edges);
+  std::vector<cudaGraphEdgeData> data(n_edges);
+  RLREP_CUDA(cudaGraphGetEdges_v2(graph_, from.data(), to.data(), data.data(), &n_edges));
+  int programmatic = 0;
+  for (size_t i = 0; i < n_edges; ++i)
+    if (data[i].type == cudaGraphDependencyTypeProgrammatic) ++programmatic;
+  *kernel_nodes = kernels;
+  *programmatic_edges = programmatic;
+  return true;
+}
+
 }  // namespace rlrep
