@@ -258,12 +258,23 @@ RLREP_EXPORT int rlrep_conv_encoder_destroy(rlrep_conv_encoder* enc);
 /* what: 0 = weight, 1 = bias, 2 = weight gradient, 3 = bias gradient (host buffers, reference layout) */
 RLREP_EXPORT int rlrep_conv_encoder_read(rlrep_conv_encoder* enc, int layer, int what, float* out_host);
 RLREP_EXPORT int rlrep_conv_encoder_write(rlrep_conv_encoder* enc, int layer, int what, const float* in_host);
-/* obs_dev uint8 [B, C, H, H]; shifts_dev int32 [B, 2] = (x, y) shift in [0, 8] or NULL; feat_dev fp32 [B, 32*35*35] in
- * the reference's flatten order.  backward consumes d(feat) of the same shape and leaves dW / db readable. */
+/* obs_dev uint8 [B, C, H, H]; shifts_dev int32 [B, 2] = (x, y) shift in [0, 8] or NULL; feat_dev fp32 [B, 32*h*h]
+ * (h = 35 for 84-pixel frames) in the reference's flatten order.  backward consumes d(feat) of the same shape and
+ * leaves dW / db readable. */
 RLREP_EXPORT int rlrep_conv_encoder_forward(rlrep_conv_encoder* enc, const unsigned char* obs_dev, const int* shifts_dev,
                                             float* feat_dev);
 RLREP_EXPORT int rlrep_conv_encoder_backward(rlrep_conv_encoder* enc, const float* dfeat_dev);
 RLREP_EXPORT int rlrep_conv_encoder_feature_dim(rlrep_conv_encoder* enc, int* dim);
+/* The same with a row pitch: ld_feat / ld_dfeat floats between rows (0 = dense; the columns past the feature dimension
+ * are neither read nor written).  no_grad != 0 promises that no backward follows (layers 1-3 then run without column
+ * matrices); backward after a no_grad forward fails.  forward / backward are the (0, 0) / 0 cases. */
+RLREP_EXPORT int rlrep_conv_encoder_forward_pitched(rlrep_conv_encoder* enc, const unsigned char* obs_dev,
+                                                    const int* shifts_dev, float* feat_dev, int ld_feat, int no_grad);
+RLREP_EXPORT int rlrep_conv_encoder_backward_pitched(rlrep_conv_encoder* enc, const float* dfeat_dev, int ld_dfeat);
+/* Copies an internal map to out_dev in NCHW, [B, 32, h_l, h_l] for layer l = 0..3 (h_l = 41, 39, 37, 35 for 84-pixel
+ * frames): which 0 = the post-ReLU output of layer l (last forward), 1 = the gradient with respect to its
+ * pre-activation, ReLU mask applied (last backward). */
+RLREP_EXPORT int rlrep_conv_encoder_read_map(rlrep_conv_encoder* enc, int which, int layer, float* out_dev);
 
 /* ------------------------------------------------------------------------------------------------
  * Pixel decoder on its own -- the 3 x ConvTranspose2d(s1) + ConvTranspose2d(s2) + Conv2d stack of muLV-Rep

@@ -101,6 +101,9 @@ def _declare(lib: C.CDLL) -> None:
         "rlrep_conv_encoder_forward": [vp, vp, vp, vp],
         "rlrep_conv_encoder_backward": [vp, vp],
         "rlrep_conv_encoder_feature_dim": [vp, C.POINTER(i)],
+        "rlrep_conv_encoder_forward_pitched": [vp, vp, vp, vp, i, i],
+        "rlrep_conv_encoder_backward_pitched": [vp, vp, i],
+        "rlrep_conv_encoder_read_map": [vp, i, i, vp],
         "rlrep_conv_decoder_create": [i, i, i, vp, C.POINTER(vp)],
         "rlrep_conv_decoder_destroy": [vp],
         "rlrep_conv_decoder_read": [vp, i, i, vp],

@@ -409,17 +409,35 @@ int rlrep_conv_encoder_write(rlrep_conv_encoder* enc, int layer, int what, const
   RLREP_CUDA(cudaStreamSynchronize(st));
   RLREP_API_END
 }
-int rlrep_conv_encoder_forward(rlrep_conv_encoder* enc, const unsigned char* obs_dev, const int* shifts_dev,
-                               float* feat_dev) {
+int rlrep_conv_encoder_forward_pitched(rlrep_conv_encoder* enc, const unsigned char* obs_dev, const int* shifts_dev,
+                                       float* feat_dev, int ld_feat, int no_grad) {
   RLREP_API_BEGIN_ON(enc)
   RLREP_CHECK(enc && obs_dev && feat_dev, "null argument");
-  enc->impl->forward(obs_dev, shifts_dev, feat_dev);
+  RLREP_CHECK(ld_feat == 0 || ld_feat >= enc->impl->feature_dim(), "feature row pitch narrower than a feature row");
+  enc->impl->forward(obs_dev, shifts_dev, feat_dev, ld_feat, /*target=*/false, no_grad != 0);
+  RLREP_API_END
+}
+int rlrep_conv_encoder_forward(rlrep_conv_encoder* enc, const unsigned char* obs_dev, const int* shifts_dev,
+                               float* feat_dev) {
+  return rlrep_conv_encoder_forward_pitched(enc, obs_dev, shifts_dev, feat_dev, 0, 0);
+}
+int rlrep_conv_encoder_backward_pitched(rlrep_conv_encoder* enc, const float* dfeat_dev, int ld_dfeat) {
+  RLREP_API_BEGIN_ON(enc)
+  RLREP_CHECK(enc && dfeat_dev, "null argument");
+  RLREP_CHECK(ld_dfeat == 0 || ld_dfeat >= enc->impl->feature_dim(), "gradient row pitch narrower than a feature row");
+  enc->impl->backward(dfeat_dev, ld_dfeat);
   RLREP_API_END
 }
 int rlrep_conv_encoder_backward(rlrep_conv_encoder* enc, const float* dfeat_dev) {
+  return rlrep_conv_encoder_backward_pitched(enc, dfeat_dev, 0);
+}
+int rlrep_conv_encoder_read_map(rlrep_conv_encoder* enc, int which, int layer, float* out_dev) {
   RLREP_API_BEGIN_ON(enc)
-  RLREP_CHECK(enc && dfeat_dev, "null argument");
-  enc->impl->backward(dfeat_dev);
+  RLREP_CHECK(enc && out_dev && (which == 0 || which == 1) && layer >= 0 && layer < 4, "bad argument");
+  ConvEncoder& e = *enc->impl;
+  const int P = e.hw(layer) * e.hw(layer);
+  launch_nhwc_to_cp(which == 0 ? e.act(layer) : e.dact(layer), e.batch(), P, out_dev, (long long)P * 32, e.stream());
+  RLREP_LAUNCHED("nhwc_to_nchw", e.stream());
   RLREP_API_END
 }
 int rlrep_conv_encoder_feature_dim(rlrep_conv_encoder* enc, int* dim) {

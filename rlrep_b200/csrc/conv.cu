@@ -133,6 +133,7 @@ void ConvEncoder::forward(const unsigned char* obs_dev, const int* shifts_dev, f
                           bool no_grad) {
   cudaStream_t s = stream_;
   RLREP_CHECK(!target || g_.n_target == g_.n, "this encoder has no target copy");
+  backward_ready_ = !target && !no_grad;
   im2col_u8_aug_kernel<<<grid_for((long long)rows(0) * (ldk1_ / 4), 256), 256, 0, s>>>(
       obs_dev, shifts_dev, B_, C_, H_, hw_[0], reinterpret_cast<float4*>(col_[0]), ldk1_);
   RLREP_LAUNCHED_W("im2col_u8_aug", s, (double)B_ * C_ * H_ * H_ + 4.0 * rows(0) * ldk1_, 0.0);
@@ -155,6 +156,8 @@ void ConvEncoder::forward(const unsigned char* obs_dev, const int* shifts_dev, f
 }
 
 void ConvEncoder::backward(const float* dfeat_dev, int ld_dfeat) {
+  RLREP_CHECK(backward_ready_, "encoder backward() needs the last forward to have run with gradients: after a target "
+                               "or no_grad forward (or none) the maps it differentiates belong to no such input");
   cudaStream_t s = stream_;
   const int P = hw_[3] * hw_[3];
   launch_cp_to_nhwc(dfeat_dev, ld_dfeat > 0 ? ld_dfeat : (long long)P * 32, B_, P, /*mask=*/act_[3], dact_[3], s);

@@ -15,8 +15,15 @@ class ConvEncoder {
   // forward (layers 2-4 then run as implicit convolutions, without column matrices)
   void forward(const unsigned char* obs_dev, const int* shifts_dev, float* feat_dev, int ld_feat = 0, bool target = false,
                bool no_grad = false);
-  // dfeat [B, 32 * 35 * 35] (row pitch ld_dfeat) -> dW / db of the four layers (activations of the last forward are reused)
+  // dfeat [B, 32 * 35 * 35] (row pitch ld_dfeat) -> dW / db of the four layers (activations of the last forward are
+  // reused, so that forward must have run with target = false and no_grad = false; anything else is refused)
   void backward(const float* dfeat_dev, int ld_dfeat = 0);
+
+  // Read-only views of the internal maps, for kernel-level tests: act(l) [B, hw(l), hw(l), 32] is the post-ReLU output
+  // of layer l (last forward), dact(l) the gradient with respect to its pre-activation, ReLU mask applied (last backward).
+  int hw(int l) const { return hw_[l]; }
+  const float* act(int l) const { return act_[l]; }
+  const float* dact(int l) const { return dact_[l]; }
 
   int batch() const { return B_; }
   int feature_dim() const { return 32 * hw_[3] * hw_[3]; }
@@ -40,6 +47,9 @@ class ConvEncoder {
   // layers 2-4 without column matrices at all (TF32 path, B % 4 == 0): implicit forward convolution and the implicit
   // weight gradient of GemmArgs::conv_wgrad_hi; otherwise explicit im2col + folded GEMM
   bool implicit_wgrad_ = false;
+  // the last forward ran the online weights with gradients: act_ (and on the explicit path every col_) hold the maps of
+  // the input backward() differentiates.  A target / no_grad forward overwrites them with another input's.
+  bool backward_ready_ = false;
   FullCorrScratch corr_;
   static constexpr int kBiasChunks = 296;  // 2 x 148 SMs
   float* bias_partial_ = nullptr;

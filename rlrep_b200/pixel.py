@@ -126,30 +126,65 @@ class ConvEncoder:
                     raise ValueError(f"{name + key}: expected {self._shape(i, what == 1)}, got {arr.shape}")
                 _lib.check(self.lib.rlrep_conv_encoder_write(self._h, i, what, arr.ctypes.data))
 
-    def forward(self, obs: torch.Tensor, shifts: torch.Tensor | None = None) -> torch.Tensor:
+    def _pitch(self, t, name):
+        """Row pitch of fp32 CUDA rows [B, repr_dim] with unit column stride (a view with a wider pitch is used in place,
+        as the agents pass their wider feature buffers)."""
+        if not (t.is_cuda and t.dtype == torch.float32 and t.dim() == 2 and tuple(t.shape) == (self.batch, self.repr_dim)
+                and t.stride(1) == 1 and t.stride(0) >= self.repr_dim):
+            raise ValueError(f"{name} must be fp32 CUDA rows [{self.batch}, {self.repr_dim}] with unit column stride")
+        return t.stride(0)
+
+    def forward(self, obs: torch.Tensor, shifts: torch.Tensor | None = None, out: torch.Tensor | None = None,
+                no_grad: bool = False) -> torch.Tensor:
         """obs uint8 [B, C, H, W] on the GPU; shifts int32 [B, 2] = (x, y) in [0, 8] as drawn by RandomShiftsAug's
-        `torch.randint(0, 2 * pad + 1, (n, 1, 1, 2))` (drqv2.py:43-47), or None for no augmentation."""
+        `torch.randint(0, 2 * pad + 1, (n, 1, 1, 2))` (drqv2.py:43-47), or None for no augmentation.  The features go
+        to `out` [B, repr_dim] (allocated when None; a view with a wider row pitch is written in place, its padding
+        columns untouched).  no_grad=True runs the evaluation-only path; backward() must not follow it."""
         assert obs.is_cuda and obs.dtype == torch.uint8 and tuple(obs.shape) == (self.batch, *self.obs_shape)
         obs = obs.contiguous()
         if shifts is not None:
             shifts = shifts.to(device=obs.device, dtype=torch.int32).reshape(self.batch, 2).contiguous()
-        feat = torch.empty(self.batch, self.repr_dim, device=obs.device, dtype=torch.float32)
+        if out is None:
+            out = torch.empty(self.batch, self.repr_dim, device=obs.device, dtype=torch.float32)
+        ld = self._pitch(out, "out")
         cur = torch.cuda.current_stream()
         self._stream.wait_stream(cur)
-        _lib.check(self.lib.rlrep_conv_encoder_forward(self._h, obs.data_ptr(),
-                                                       shifts.data_ptr() if shifts is not None else None, feat.data_ptr()))
+        _lib.check(self.lib.rlrep_conv_encoder_forward_pitched(
+            self._h, obs.data_ptr(), shifts.data_ptr() if shifts is not None else None, out.data_ptr(), ld, int(no_grad)))
         cur.wait_stream(self._stream)
-        self._keep = (obs, shifts)
-        return feat
+        self._keep = (obs, shifts, out)
+        return out
 
     def backward(self, dfeat: torch.Tensor) -> None:
+        """dfeat [B, repr_dim] (a view with a wider row pitch is read in place).  Raises RlrepError unless the last
+        forward ran with gradients."""
         assert dfeat.is_cuda and dfeat.dtype == torch.float32 and tuple(dfeat.shape) == (self.batch, self.repr_dim)
-        dfeat = dfeat.contiguous()
+        if dfeat.stride(1) != 1 or dfeat.stride(0) < self.repr_dim:
+            dfeat = dfeat.contiguous()
+        ld = self._pitch(dfeat, "dfeat")
         cur = torch.cuda.current_stream()
         self._stream.wait_stream(cur)
-        _lib.check(self.lib.rlrep_conv_encoder_backward(self._h, dfeat.data_ptr()))
+        _lib.check(self.lib.rlrep_conv_encoder_backward_pitched(self._h, dfeat.data_ptr(), ld))
         cur.wait_stream(self._stream)
         self._keep_d = dfeat
+
+    def hw(self, layer: int) -> int:
+        """Side of layer `layer`'s output map (41, 39, 37, 35 for 84-pixel frames)."""
+        h = (self.obs_shape[1] - 3) // 2 + 1
+        return h - 2 * int(layer)
+
+    def read_map(self, which: str, layer: int) -> torch.Tensor:
+        """NCHW copy [B, 32, h, h] of an internal map: 'act' = layer `layer`'s post-ReLU output (last forward), 'dact' =
+        the gradient with respect to its pre-activation, ReLU mask applied (last backward)."""
+        w = {"act": 0, "dact": 1}[which]
+        h = self.hw(layer)
+        out = torch.empty(self.batch, 32, h, h, device="cuda")
+        cur = torch.cuda.current_stream()
+        self._stream.wait_stream(cur)
+        _lib.check(self.lib.rlrep_conv_encoder_read_map(self._h, w, int(layer), out.data_ptr()))
+        cur.wait_stream(self._stream)
+        self._keep_m = out
+        return out
 
 
 class ConvDecoder:
