@@ -400,7 +400,7 @@ RLREP_EXPORT int rlrep_mulv_profile_update(rlrep_mulv* h, float stddev, int max_
 RLREP_EXPORT int rlrep_mulv_last_launches(rlrep_mulv* h, int* launches);
 
 /* ------------------------------------------------------------------------------------------------
- * DRAFT (branch draft/ldiffsr-agent, not verified on hardware): latent Diff-SR DrQ-v2 pixel agent -- replaces
+ * Latent Diff-SR DrQ-v2 pixel agent -- replaces
  * `LatentDiffSRDrQv2(obs_space, action_space, args)` and the updating half of `train_step(replay_iter, step)`
  * (agent/diffsrdrq/latent_diff_sr.py:13-139, :306-390) on configs/latent_diff_sr.yaml's path.  The caller keeps `_step` /
  * `update_every`, evaluates the std-dev schedule and draws ALL randomness in the reference's order on the CPU generator

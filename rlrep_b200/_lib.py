@@ -114,46 +114,16 @@ def _declare(lib: C.CDLL) -> None:
         "rlrep_conv_decoder_backward": [vp, vp, i],
         "rlrep_conv_decoder_read_map": [vp, i, i, vp],
         "rlrep_drq_create": [vp, vp, C.POINTER(vp)],
-        "rlrep_drq_destroy": [vp],
-        "rlrep_drq_num_tensors": [vp, C.POINTER(i)],
-        "rlrep_drq_tensor_info": [vp, i, C.POINTER(C.c_char_p), C.POINTER(vp), C.POINTER(i), C.POINTER(i)],
-        "rlrep_drq_tensor_read": [vp, i, vp],
-        "rlrep_drq_tensor_write": [vp, i, vp],
-        "rlrep_drq_sync_targets": [vp],
         "rlrep_drq_update": [vp, vp, vp, vp, vp, vp, vp, vp, C.c_float, vp],
-        "rlrep_drq_last_launches": [vp, C.POINTER(i)],
         "rlrep_drq_act": [vp, vp, vp, C.c_float, vp],
         "rlrep_drq_act_batch": [vp, vp, vp, C.c_float, i, vp],
-        "rlrep_drq_update_resident": [vp, i, C.c_float, C.POINTER(C.c_float)],
-        "rlrep_drq_profile_update": [vp, C.c_float, i, C.POINTER(C.c_char_p), C.POINTER(C.c_float), C.POINTER(C.c_double),
-                                     C.POINTER(C.c_double), C.POINTER(i)],
         "rlrep_gemm_set_debug_buffer": [vp],
         "rlrep_ldiff_create": [vp, vp, C.POINTER(vp)],
-        "rlrep_ldiff_destroy": [vp],
-        "rlrep_ldiff_num_tensors": [vp, C.POINTER(i)],
-        "rlrep_ldiff_tensor_info": [vp, i, C.POINTER(C.c_char_p), C.POINTER(vp), C.POINTER(i), C.POINTER(i)],
-        "rlrep_ldiff_tensor_read": [vp, i, vp],
-        "rlrep_ldiff_tensor_write": [vp, i, vp],
-        "rlrep_ldiff_sync_targets": [vp],
         "rlrep_ldiff_update": [vp, vp, vp],
-        "rlrep_ldiff_update_resident": [vp, i, C.c_float, C.POINTER(C.c_float)],
-        "rlrep_ldiff_profile_update": [vp, C.c_float, i, C.POINTER(C.c_char_p), C.POINTER(C.c_float),
-                                       C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(i)],
-        "rlrep_ldiff_last_launches": [vp, C.POINTER(i)],
         "rlrep_mulv_create": [vp, vp, C.POINTER(vp)],
-        "rlrep_mulv_destroy": [vp],
-        "rlrep_mulv_num_tensors": [vp, C.POINTER(i)],
-        "rlrep_mulv_tensor_info": [vp, i, C.POINTER(C.c_char_p), C.POINTER(vp), C.POINTER(i), C.POINTER(i)],
-        "rlrep_mulv_tensor_read": [vp, i, vp],
-        "rlrep_mulv_tensor_write": [vp, i, vp],
-        "rlrep_mulv_sync_targets": [vp],
         "rlrep_mulv_update": [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_float, vp],
-        "rlrep_mulv_last_launches": [vp, C.POINTER(i)],
         "rlrep_mulv_act": [vp, vp, vp, C.c_float, vp],
         "rlrep_mulv_act_batch": [vp, vp, vp, C.c_float, i, vp],
-        "rlrep_mulv_update_resident": [vp, i, C.c_float, C.POINTER(C.c_float)],
-        "rlrep_mulv_profile_update": [vp, C.c_float, i, C.POINTER(C.c_char_p), C.POINTER(C.c_float), C.POINTER(C.c_double),
-                                      C.POINTER(C.c_double), C.POINTER(i)],
         "rlrep_comm_unique_id": [vp],
         "rlrep_comm_create": [vp, i, i, C.POINTER(vp)],
         "rlrep_comm_destroy": [vp],
@@ -184,6 +154,20 @@ def _declare(lib: C.CDLL) -> None:
         "rlrep_agent_profile_train": [vp, vp, vp, vp, i, C.POINTER(C.c_char_p), C.POINTER(C.c_float),
                                       C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(i)],
     }
+    # the pixel agents' handle entry points, the same for each agent (rlrep_drq_*, rlrep_mulv_*, rlrep_ldiff_*)
+    for prefix in ("drq", "mulv", "ldiff"):
+        sigs.update({
+            f"rlrep_{prefix}_destroy": [vp],
+            f"rlrep_{prefix}_num_tensors": [vp, C.POINTER(i)],
+            f"rlrep_{prefix}_tensor_info": [vp, i, C.POINTER(C.c_char_p), C.POINTER(vp), C.POINTER(i), C.POINTER(i)],
+            f"rlrep_{prefix}_tensor_read": [vp, i, vp],
+            f"rlrep_{prefix}_tensor_write": [vp, i, vp],
+            f"rlrep_{prefix}_sync_targets": [vp],
+            f"rlrep_{prefix}_update_resident": [vp, i, C.c_float, C.POINTER(C.c_float)],
+            f"rlrep_{prefix}_profile_update": [vp, C.c_float, i, C.POINTER(C.c_char_p), C.POINTER(C.c_float),
+                                               C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(i)],
+            f"rlrep_{prefix}_last_launches": [vp, C.POINTER(i)],
+        })
     lib.rlrep_agent_metric_name.argtypes = [vp, i]
     lib.rlrep_agent_metric_name.restype = C.c_char_p
     for name, argtypes in sigs.items():

@@ -20,7 +20,7 @@
 namespace rlrep {
 
 DrqV2::DrqV2(const DrqConfig& c, cudaStream_t s)
-    : cfg_(c), stream_(s), B_(c.batch), A_(c.action_dim), bn_(c.bn_dim), H_(c.hidden_dim) {
+    : PixelAgent(s), cfg_(c), B_(c.batch), A_(c.action_dim), bn_(c.bn_dim), H_(c.hidden_dim) {
   RLREP_CHECK(B_ > 0 && A_ > 0 && bn_ > 0 && H_ % 32 == 0, "bad DrQ-v2 dimensions (hidden_dim must be a multiple of 32)");
   enc_.reset(new ConvEncoder(B_, c.channels, c.height, static_cast<Precision>(c.precision), s));
   F_ = enc_->feature_dim();
@@ -102,22 +102,10 @@ DrqV2::DrqV2(const DrqConfig& c, cudaStream_t s)
   arena_.commit();
   gemm_.init(static_cast<Precision>(c.precision), 0);
   const size_t img_bytes = (size_t)B_ * c.channels * c.height * c.height;
-  stage_bytes_ = 2 * img_bytes + (size_t)4 * B_ * sizeof(int) + ((size_t)2 * B_ * A_ + (size_t)B_ * A_ + 2 * B_) * sizeof(float);
-  RLREP_CUDA(cudaMallocHost(&stage_host_, stage_bytes_));
-  RLREP_CUDA(cudaMallocHost(&metrics_host_, 8 * sizeof(float)));
+  alloc_host(2 * img_bytes + (size_t)4 * B_ * sizeof(int) + ((size_t)2 * B_ * A_ + (size_t)B_ * A_ + 2 * B_) * sizeof(float));
   Control h;
   std::memset(&h, 0, sizeof(h));
   RLREP_CUDA(cudaMemcpyAsync(ctl_, &h, sizeof(h), cudaMemcpyHostToDevice, stream_));
-  RLREP_CUDA(cudaStreamSynchronize(stream_));
-}
-
-DrqV2::~DrqV2() {
-  if (stage_host_) cudaFreeHost(stage_host_);
-  if (metrics_host_) cudaFreeHost(metrics_host_);
-}
-
-void DrqV2::sync_targets_from_params() {
-  RLREP_CUDA(cudaMemcpyAsync(crit_g_.target, crit_g_.p, crit_g_.n_target * 4, cudaMemcpyDeviceToDevice, stream_));
   RLREP_CUDA(cudaStreamSynchronize(stream_));
 }
 
@@ -186,42 +174,10 @@ void DrqV2::actor_forward(const float* latent, const float* eps, float stddev, i
 // select_action (drqv2.py:74-82) on n observations: the small-batch policy (pixel_act.cu) over this handle's
 // parameters, created on first use
 void DrqV2::act_batch(const unsigned char* obs, const float* eps_host, float stddev, int n, float* actions_host) {
-  if (!policy_) {
-    PixelPolicyWeights pw;
-    for (int l = 0; l < 4; ++l) pw.conv[l] = enc_->layer(l);
-    pw.trunk = at_.view(actor_g_);
-    pw.ln_w = actor_g_.p + aln_w_;
-    pw.ln_b = actor_g_.p + aln_b_;
-    pw.policy[0] = p0_.view(actor_g_);
-    pw.policy[1] = p1_.view(actor_g_);
-    pw.policy[2] = p2_.view(actor_g_);
-    policy_.reset(new PixelPolicy(cfg_.channels, cfg_.height, A_, pw, stream_));
-  }
+  if (!policy_)
+    policy_.reset(new PixelPolicy(cfg_.channels, cfg_.height, A_,
+                                  actor_policy_weights(*enc_, actor_g_, at_, aln_w_, aln_b_, p0_, p1_, p2_), stream_));
   policy_->act(obs, eps_host, stddev, n, actions_host);
-}
-
-float DrqV2::update_resident(int n_steps, float stddev) {
-  RLREP_CHECK(n_steps > 0, "bad step count");
-  cudaEvent_t e0, e1;
-  RLREP_CUDA(cudaEventCreate(&e0));
-  RLREP_CUDA(cudaEventCreate(&e1));
-  RLREP_CUDA(cudaStreamSynchronize(stream_));
-  RLREP_CUDA(cudaEventRecord(e0, stream_));
-  for (int i = 0; i < n_steps; ++i) launch_update(stddev);
-  RLREP_CUDA(cudaEventRecord(e1, stream_));
-  RLREP_CUDA(cudaEventSynchronize(e1));
-  float ms = 0.f;
-  RLREP_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
-  return ms;
-}
-
-std::vector<ProfileEntry> DrqV2::profile_update(float stddev) {
-  RLREP_CUDA(cudaStreamSynchronize(stream_));
-  profile_begin(stream_);
-  launch_update(stddev);
-  return profile_end(stream_);
 }
 
 void DrqV2::update(const unsigned char* img, const float* action, const float* reward, const float* discount,
@@ -239,12 +195,7 @@ void DrqV2::update(const unsigned char* img, const float* action, const float* r
   put(action_dev_, action, (size_t)B_ * A_ * sizeof(float));
   put(reward_dev_, reward, B_ * sizeof(float));
   put(discount_dev_, discount, B_ * sizeof(float));
-  const long long before = launch_count();
-  launch_update(stddev);
-  last_launches = (int)(launch_count() - before);
-  RLREP_CUDA(cudaMemcpyAsync(metrics_host_, metrics_dev_, 8 * sizeof(float), cudaMemcpyDeviceToHost, s));
-  RLREP_CUDA(cudaStreamSynchronize(s));
-  std::memcpy(metrics_out, metrics_host_, 5 * sizeof(float));
+  finish_update(stddev, metrics_out, 5);
 }
 
 // Every launch of one update on the batch currently resident in the device buffers.

@@ -1,5 +1,3 @@
-// DRAFT (branch draft/ldiffsr-agent; written after the round's GPU budget was spent -- compiles, NOT verified on hardware).
-//
 // Latent Diff-SR DrQ-v2 pixel update (reference: agent/diffsrdrq/latent_diff_sr.py:306-390 `train_step` with `ae_step`
 // :234-259, `score_step` :275-304, `critic_step` :355-379, `actor_step` :381-390, `update_target` :135-139) on
 // configs/latent_diff_sr.yaml's path: use_repr_target, back_critic_grad, critic_loss mse, reg_coef 0, grad_norm null,
@@ -59,7 +57,7 @@ ResNetSlots LatentDiffSR::add_resnet(const std::string& prefix, int depth, int i
 }
 
 LatentDiffSR::LatentDiffSR(const LdiffConfig& c, cudaStream_t s)
-    : cfg_(c), stream_(s), B_(c.batch), N_(4 * c.batch), A_(c.action_dim), L_(c.latent), feat_(c.feat), bn_(c.bn),
+    : PixelAgent(s), cfg_(c), B_(c.batch), N_(4 * c.batch), A_(c.action_dim), L_(c.latent), feat_(c.feat), bn_(c.bn),
       H_(c.hidden) {
   RLREP_CHECK(B_ > 0 && A_ > 0 && L_ % 64 == 0 && feat_ % 32 == 0 && bn_ % 32 == 0 && H_ % 32 == 0,
               "bad latent Diff-SR dimensions (latent % 64, feature / bn / hidden % 32)");
@@ -67,10 +65,12 @@ LatentDiffSR::LatentDiffSR(const LdiffConfig& c, cudaStream_t s)
   const Precision prec = static_cast<Precision>(c.precision);
   enc_.reset(new ConvEncoder(N_, 3, 84, prec, s, /*with_target=*/true));
   enc_->group().name = "vae.encoder";
-  enc_->group().target_prefix_to = "vae_target.encoder.";
+  enc_->group().target_prefix_from = "vae.";
+  enc_->group().target_prefix_to = "vae_target.";
   dec_.reset(new ConvDecoder(N_, prec, s, /*out_kernel=*/3, /*with_target=*/true));
   dec_->group().name = "vae.decoder";
-  dec_->group().target_prefix_to = "vae_target.decoder.";
+  dec_->group().target_prefix_from = "vae.";
+  dec_->group().target_prefix_to = "vae_target.";
   F_ = enc_->feature_dim();
   LA_ = round_up32(A_);
   T_ = L_ / 2;
@@ -175,25 +175,12 @@ LatentDiffSR::LatentDiffSR(const LdiffConfig& c, cudaStream_t s)
   arena_.commit();
   gemm_.init(prec, 0);
 
-  stage_bytes_ = 2 * N_ * frame + (size_t)4 * N_ * sizeof(int) +
-                 ((size_t)B_ * A_ + 2 * B_ + NL + B_ + (size_t)B_ * T_ + (size_t)B_ * L_ + (size_t)c.psi_d * B2 * c.psi_h +
-                  (size_t)c.zeta_d * B_ * c.zeta_h + (size_t)2 * B_ * A_) * sizeof(float);
-  RLREP_CUDA(cudaMallocHost(&stage_host_, stage_bytes_));
-  RLREP_CUDA(cudaMallocHost(&metrics_host_, 8 * sizeof(float)));
+  alloc_host(2 * N_ * frame + (size_t)4 * N_ * sizeof(int) +
+             ((size_t)B_ * A_ + 2 * B_ + NL + B_ + (size_t)B_ * T_ + (size_t)B_ * L_ + (size_t)c.psi_d * B2 * c.psi_h +
+              (size_t)c.zeta_d * B_ * c.zeta_h + (size_t)2 * B_ * A_) * sizeof(float));
   Control h;
   std::memset(&h, 0, sizeof(h));
   RLREP_CUDA(cudaMemcpyAsync(ctl_, &h, sizeof(h), cudaMemcpyHostToDevice, stream_));
-  RLREP_CUDA(cudaStreamSynchronize(stream_));
-}
-
-LatentDiffSR::~LatentDiffSR() {
-  if (stage_host_) cudaFreeHost(stage_host_);
-  if (metrics_host_) cudaFreeHost(metrics_host_);
-}
-
-void LatentDiffSR::sync_targets_from_params() {
-  for (ParamGroup* g : groups())
-    if (g->n_target) RLREP_CUDA(cudaMemcpyAsync(g->target, g->p, g->n_target * 4, cudaMemcpyDeviceToDevice, stream_));
   RLREP_CUDA(cudaStreamSynchronize(stream_));
 }
 
@@ -374,36 +361,7 @@ void LatentDiffSR::update(const Inputs& in, float* metrics_out) {
   put(psi_masks_dev_, in.psi_masks, (size_t)cfg_.psi_d * B2 * cfg_.psi_h * 4);
   put(zeta_masks_dev_, in.zeta_masks, (size_t)cfg_.zeta_d * B_ * cfg_.zeta_h * 4);
   put(eps_act_dev_, in.eps_act, (size_t)2 * B_ * A_ * 4);
-  const long long before = launch_count();
-  launch_update(in.stddev);
-  last_launches = (int)(launch_count() - before);
-  RLREP_CUDA(cudaMemcpyAsync(metrics_host_, metrics_dev_, 8 * sizeof(float), cudaMemcpyDeviceToHost, s));
-  RLREP_CUDA(cudaStreamSynchronize(s));
-  std::memcpy(metrics_out, metrics_host_, 8 * sizeof(float));
-}
-
-float LatentDiffSR::update_resident(int n_steps, float stddev) {
-  RLREP_CHECK(n_steps > 0, "bad step count");
-  cudaEvent_t e0, e1;
-  RLREP_CUDA(cudaEventCreate(&e0));
-  RLREP_CUDA(cudaEventCreate(&e1));
-  RLREP_CUDA(cudaStreamSynchronize(stream_));
-  RLREP_CUDA(cudaEventRecord(e0, stream_));
-  for (int i = 0; i < n_steps; ++i) launch_update(stddev);
-  RLREP_CUDA(cudaEventRecord(e1, stream_));
-  RLREP_CUDA(cudaEventSynchronize(e1));
-  float ms = 0.f;
-  RLREP_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
-  return ms;
-}
-
-std::vector<ProfileEntry> LatentDiffSR::profile_update(float stddev) {
-  RLREP_CUDA(cudaStreamSynchronize(stream_));
-  profile_begin(stream_);
-  launch_update(stddev);
-  return profile_end(stream_);
+  finish_update(in.stddev, metrics_out, 8);
 }
 
 void LatentDiffSR::launch_update(float stddev) {

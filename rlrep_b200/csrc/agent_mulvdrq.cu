@@ -58,13 +58,14 @@ void want_gauss(DeviceArena& a, GaussActs& g, int B, int LF) {
 }  // namespace
 
 MulvDrq::MulvDrq(const MulvConfig& c, cudaStream_t s)
-    : cfg_(c), stream_(s), B_(c.batch), A_(c.action_dim), D_(c.feat_dim), H_(c.hidden_dim), NN_(c.num_noise) {
+    : PixelAgent(s), cfg_(c), B_(c.batch), A_(c.action_dim), D_(c.feat_dim), H_(c.hidden_dim), NN_(c.num_noise) {
   RLREP_CHECK(B_ > 0 && A_ > 0 && D_ > 0 && NN_ > 0 && H_ % 32 == 0,
               "bad muLV-DrQ dimensions (hidden_dim must be a multiple of 32)");
   RLREP_CHECK(c.height == 84, "the pixel decoder is built for 84 x 84 frames (35 -> 37 -> 39 -> 41 -> 83 -> 84)");
   const Precision prec = static_cast<Precision>(c.precision);
   enc_.reset(new ConvEncoder(B_, c.channels, c.height, prec, s, /*with_target=*/true));
   enc_->group().name = "encoder";
+  enc_->group().target_prefix_from = "encoder.";
   enc_->group().target_prefix_to = "encoder_target.";
   penc_.reset(new ConvEncoder(B_, 3, c.height, prec, s));
   penc_->group().name = "predict_encoder";
@@ -170,25 +171,11 @@ MulvDrq::MulvDrq(const MulvConfig& c, cudaStream_t s)
   arena_.commit();
   gemm_.init(prec, 0);
 
-  stage_bytes_ = 2 * img_bytes + step1_bytes + (size_t)4 * B_ * sizeof(int) +
-                 ((size_t)B_ * D_ + (size_t)2 * B_ * A_ + (size_t)3 * NN_ * D_ + (size_t)B_ * A_ + 2 * B_) * sizeof(float);
-  RLREP_CUDA(cudaMallocHost(&stage_host_, stage_bytes_));
-  RLREP_CUDA(cudaMallocHost(&metrics_host_, 8 * sizeof(float)));
+  alloc_host(2 * img_bytes + step1_bytes + (size_t)4 * B_ * sizeof(int) +
+             ((size_t)B_ * D_ + (size_t)2 * B_ * A_ + (size_t)3 * NN_ * D_ + (size_t)B_ * A_ + 2 * B_) * sizeof(float));
   Control h;
   std::memset(&h, 0, sizeof(h));
   RLREP_CUDA(cudaMemcpyAsync(ctl_, &h, sizeof(h), cudaMemcpyHostToDevice, stream_));
-  RLREP_CUDA(cudaStreamSynchronize(stream_));
-}
-
-MulvDrq::~MulvDrq() {
-  if (stage_host_) cudaFreeHost(stage_host_);
-  if (metrics_host_) cudaFreeHost(metrics_host_);
-}
-
-void MulvDrq::sync_targets_from_params() {
-  ParamGroup* gs[3] = {&enc_->group(), &crit_g_, &ff_g_};
-  for (ParamGroup* g : gs)
-    RLREP_CUDA(cudaMemcpyAsync(g->target, g->p, g->n_target * 4, cudaMemcpyDeviceToDevice, stream_));
   RLREP_CUDA(cudaStreamSynchronize(stream_));
 }
 
@@ -289,42 +276,10 @@ void MulvDrq::actor_forward(const float* latent, int ld_latent, const float* eps
 // act (drqv2.py:270-282) on n observations: the small-batch policy (pixel_act.cu) over this handle's parameters,
 // created on first use
 void MulvDrq::act_batch(const unsigned char* obs, const float* eps_host, float stddev, int n, float* actions_host) {
-  if (!policy_) {
-    PixelPolicyWeights pw;
-    for (int l = 0; l < 4; ++l) pw.conv[l] = enc_->layer(l);
-    pw.trunk = at_.view(actor_g_);
-    pw.ln_w = actor_g_.p + aln_w_;
-    pw.ln_b = actor_g_.p + aln_b_;
-    pw.policy[0] = p0_.view(actor_g_);
-    pw.policy[1] = p1_.view(actor_g_);
-    pw.policy[2] = p2_.view(actor_g_);
-    policy_.reset(new PixelPolicy(cfg_.channels, cfg_.height, A_, pw, stream_));
-  }
+  if (!policy_)
+    policy_.reset(new PixelPolicy(cfg_.channels, cfg_.height, A_,
+                                  actor_policy_weights(*enc_, actor_g_, at_, aln_w_, aln_b_, p0_, p1_, p2_), stream_));
   policy_->act(obs, eps_host, stddev, n, actions_host);
-}
-
-float MulvDrq::update_resident(int n_steps, float stddev) {
-  RLREP_CHECK(n_steps > 0, "bad step count");
-  cudaEvent_t e0, e1;
-  RLREP_CUDA(cudaEventCreate(&e0));
-  RLREP_CUDA(cudaEventCreate(&e1));
-  RLREP_CUDA(cudaStreamSynchronize(stream_));
-  RLREP_CUDA(cudaEventRecord(e0, stream_));
-  for (int i = 0; i < n_steps; ++i) launch_update(stddev);
-  RLREP_CUDA(cudaEventRecord(e1, stream_));
-  RLREP_CUDA(cudaEventSynchronize(e1));
-  float ms = 0.f;
-  RLREP_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
-  return ms;
-}
-
-std::vector<ProfileEntry> MulvDrq::profile_update(float stddev) {
-  RLREP_CUDA(cudaStreamSynchronize(stream_));
-  profile_begin(stream_);
-  launch_update(stddev);
-  return profile_end(stream_);
 }
 
 void MulvDrq::update(const unsigned char* img, const float* action, const float* reward, const float* discount,
@@ -346,12 +301,7 @@ void MulvDrq::update(const unsigned char* img, const float* action, const float*
   put(action_dev_, action, (size_t)B_ * A_ * sizeof(float));
   put(reward_dev_, reward, B_ * sizeof(float));
   put(discount_dev_, discount, B_ * sizeof(float));
-  const long long before = launch_count();
-  launch_update(stddev);
-  last_launches = (int)(launch_count() - before);
-  RLREP_CUDA(cudaMemcpyAsync(metrics_host_, metrics_dev_, 8 * sizeof(float), cudaMemcpyDeviceToHost, s));
-  RLREP_CUDA(cudaStreamSynchronize(s));
-  std::memcpy(metrics_out, metrics_host_, 8 * sizeof(float));
+  finish_update(stddev, metrics_out, 8);
 }
 
 // Every launch of one update on the batch currently resident in the device buffers.

@@ -94,6 +94,35 @@ struct TensorRef {
   int rows, cols, ld;
 };
 
+// The tensor index of a handle: entry i by index, its description, and synchronous copies between its [rows, cols]
+// (row pitch ld) and a dense host array.
+static const TensorRef& tensor_at(const std::vector<TensorRef>& ts, int i) {
+  RLREP_CHECK(i >= 0 && i < (int)ts.size(), "tensor index out of range");
+  return ts[i];
+}
+static void tensor_info(const std::vector<TensorRef>& ts, int i, const char** name, float** ptr_dev, int* rows,
+                        int* cols) {
+  const TensorRef& t = tensor_at(ts, i);
+  if (name) *name = t.name.c_str();
+  if (ptr_dev) *ptr_dev = t.ptr;
+  if (rows) *rows = t.rows;
+  if (cols) *cols = t.cols;
+}
+static void tensor_read(const std::vector<TensorRef>& ts, int i, float* out_host, cudaStream_t st) {
+  const TensorRef& t = tensor_at(ts, i);
+  RLREP_CHECK(out_host != nullptr, "null argument");
+  RLREP_CUDA(cudaMemcpy2DAsync(out_host, (size_t)t.cols * 4, t.ptr, (size_t)t.ld * 4, (size_t)t.cols * 4, t.rows,
+                               cudaMemcpyDeviceToHost, st));
+  RLREP_CUDA(cudaStreamSynchronize(st));
+}
+static void tensor_write(const std::vector<TensorRef>& ts, int i, const float* in_host, cudaStream_t st) {
+  const TensorRef& t = tensor_at(ts, i);
+  RLREP_CHECK(in_host != nullptr, "null argument");
+  RLREP_CUDA(cudaMemcpy2DAsync(t.ptr, (size_t)t.ld * 4, in_host, (size_t)t.cols * 4, (size_t)t.cols * 4, t.rows,
+                               cudaMemcpyHostToDevice, st));
+  RLREP_CUDA(cudaStreamSynchronize(st));
+}
+
 struct rlrep_agent {
   int device = current_device();
   std::unique_ptr<Agent> impl;
@@ -121,6 +150,118 @@ static void index_tensors(rlrep_agent* a) {
       }
     }
   }
+}
+
+// ------------------------------------------------------------------------------------------------ pixel agent handles
+struct PixelHandle {
+  int device = current_device();
+  std::unique_ptr<PixelAgent> impl;
+  std::vector<TensorRef> tensors;
+  cudaStream_t owned_stream = nullptr;  // created when the caller passed the (uncapturable) legacy default stream
+  virtual ~PixelHandle() {
+    if (impl) cudaStreamSynchronize(impl->stream());
+    impl.reset();
+    if (owned_stream) cudaStreamDestroy(owned_stream);
+  }
+};
+struct rlrep_drq : PixelHandle {
+  DrqV2& agent() { return static_cast<DrqV2&>(*impl); }
+};
+struct rlrep_mulv : PixelHandle {
+  MulvDrq& agent() { return static_cast<MulvDrq&>(*impl); }
+};
+struct rlrep_ldiff : PixelHandle {
+  LatentDiffSR& agent() { return static_cast<LatentDiffSR&>(*impl); }
+};
+
+// The agent runs on `stream`, or on a stream of its own when that is null.  Its tensors are indexed group by group under
+// the reference's names: the parameters, their gradients of the most recent update ("grad/<name>", for gradient-level
+// parity tests), then the target copies.
+template <class Handle, class Impl, class Config>
+static Handle* create_pixel(const Config& c, void* stream) {
+  std::unique_ptr<Handle> h(new Handle);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (st == nullptr) {
+    RLREP_CUDA(cudaStreamCreateWithFlags(&h->owned_stream, cudaStreamNonBlocking));
+    st = h->owned_stream;
+  }
+  h->impl.reset(new Impl(c, st));
+  for (ParamGroup* g : h->impl->groups()) {
+    auto add = [&](float* base, const std::string& from, const std::string& to) {
+      for (const ParamTensor& t : g->tensors) {
+        const std::string name = h->impl->tensor_name(*g, t.name);
+        RLREP_CHECK(name.compare(0, from.size(), from) == 0, name + " does not start with " + from);
+        h->tensors.push_back({to + name.substr(from.size()), base + t.offset, t.rows, t.cols, t.ld});
+      }
+    };
+    add(g->p, "", "");
+    if (g->g) add(g->g, "", "grad/");
+    if (g->target) add(g->target, g->target_prefix_from, g->target_prefix_to);
+  }
+  return h.release();
+}
+
+static int pixel_destroy(PixelHandle* h) {
+  RLREP_API_BEGIN_ON(h)
+  delete h;
+  RLREP_API_END
+}
+static int pixel_num_tensors(PixelHandle* h, int* n) {
+  RLREP_API_BEGIN_ON(h)
+  RLREP_CHECK(h && n, "null argument");
+  *n = (int)h->tensors.size();
+  RLREP_API_END
+}
+static int pixel_tensor_info(PixelHandle* h, int i, const char** name, float** ptr_dev, int* rows, int* cols) {
+  RLREP_API_BEGIN_ON(h)
+  RLREP_CHECK(h, "null argument");
+  tensor_info(h->tensors, i, name, ptr_dev, rows, cols);
+  RLREP_API_END
+}
+static int pixel_tensor_read(PixelHandle* h, int i, float* out_host) {
+  RLREP_API_BEGIN_ON(h)
+  RLREP_CHECK(h, "null argument");
+  tensor_read(h->tensors, i, out_host, h->impl->stream());
+  RLREP_API_END
+}
+static int pixel_tensor_write(PixelHandle* h, int i, const float* in_host) {
+  RLREP_API_BEGIN_ON(h)
+  RLREP_CHECK(h, "null argument");
+  tensor_write(h->tensors, i, in_host, h->impl->stream());
+  RLREP_API_END
+}
+static int pixel_sync_targets(PixelHandle* h) {
+  RLREP_API_BEGIN_ON(h)
+  RLREP_CHECK(h, "null argument");
+  h->impl->sync_targets_from_params();
+  RLREP_API_END
+}
+static int pixel_update_resident(PixelHandle* h, int n_steps, float stddev, float* total_ms) {
+  RLREP_API_BEGIN_ON(h)
+  RLREP_CHECK(h && total_ms, "null argument");
+  *total_ms = h->impl->update_resident(n_steps, stddev);
+  RLREP_API_END
+}
+static int pixel_profile_update(PixelHandle* h, float stddev, int max_entries, const char** names, float* ms,
+                                double* bytes, double* flops, int* n_entries) {
+  RLREP_API_BEGIN_ON(h)
+  RLREP_CHECK(h && n_entries && (max_entries == 0 || (names && ms)), "null argument");
+  std::vector<ProfileEntry> prof = h->impl->profile_update(stddev);
+  const int n = (int)std::min<size_t>(prof.size(), (size_t)max_entries);
+  for (int i = 0; i < n; ++i) {
+    names[i] = prof[i].name;  // string literals with static storage
+    ms[i] = prof[i].ms;
+    if (bytes) bytes[i] = prof[i].bytes;
+    if (flops) flops[i] = prof[i].flops;
+  }
+  *n_entries = (int)prof.size();
+  RLREP_API_END
+}
+static int pixel_last_launches(PixelHandle* h, int* launches) {
+  RLREP_API_BEGIN_ON(h)
+  RLREP_CHECK(h && launches, "null argument");
+  *launches = h->impl->last_launches;
+  RLREP_API_END
 }
 
 extern "C" {
@@ -566,14 +707,8 @@ int rlrep_conv_decoder_read_map(rlrep_conv_decoder* dec, int which, int i, float
   RLREP_API_END
 }
 
-// ------------------------------------------------------------------------------------------------ DrQ-v2 pixel agent
-struct rlrep_drq {
-  int device = current_device();
-  std::unique_ptr<DrqV2> impl;
-  std::vector<TensorRef> tensors;
-  cudaStream_t owned_stream = nullptr;
-};
-
+// ------------------------------------------------------------------------------------------------ pixel agents
+// rlrep_drq, rlrep_mulv and rlrep_ldiff are one handle over a PixelAgent: only create, update and act differ.
 int rlrep_drq_create(const rlrep_drq_config* c, void* stream, rlrep_drq** out) {
   RLREP_API_BEGIN
   RLREP_CHECK(c != nullptr && out != nullptr, "null argument");
@@ -582,83 +717,23 @@ int rlrep_drq_create(const rlrep_drq_config* c, void* stream, rlrep_drq** out) {
   d.bn_dim = c->bn_dim; d.hidden_dim = c->hidden_dim;
   d.encoder_lr = c->encoder_lr; d.actor_lr = c->actor_lr; d.critic_lr = c->critic_lr;
   d.tau = c->tau; d.stddev_clip = c->stddev_clip; d.precision = c->precision;
-  std::unique_ptr<rlrep_drq> h(new rlrep_drq);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (st == nullptr) {
-    RLREP_CUDA(cudaStreamCreateWithFlags(&h->owned_stream, cudaStreamNonBlocking));
-    st = h->owned_stream;
-  }
-  h->impl.reset(new DrqV2(d, st));
-  for (ParamGroup* g : h->impl->groups()) {
-    const std::string prefix = g->name == "encoder" ? "encoder." : "";
-    for (const ParamTensor& t : g->tensors) h->tensors.push_back({prefix + t.name, g->p + t.offset, t.rows, t.cols, t.ld});
-    // gradients of the most recent update, for gradient-level parity tests ("grad/<name>")
-    for (const ParamTensor& t : g->tensors)
-      h->tensors.push_back({"grad/" + prefix + t.name, g->g + t.offset, t.rows, t.cols, t.ld});
-    if (g->target)
-      for (const ParamTensor& t : g->tensors)
-        h->tensors.push_back({g->target_prefix_to + t.name.substr(g->target_prefix_from.size()), g->target + t.offset,
-                              t.rows, t.cols, t.ld});
-  }
-  *out = h.release();
+  *out = create_pixel<rlrep_drq, DrqV2>(d, stream);
   RLREP_API_END
 }
-int rlrep_drq_destroy(rlrep_drq* drq) {
-  RLREP_API_BEGIN_ON(drq)
-  if (drq) {
-    if (drq->impl) cudaStreamSynchronize(drq->impl->stream());
-    drq->impl.reset();
-    if (drq->owned_stream) cudaStreamDestroy(drq->owned_stream);
-  }
-  delete drq;
-  RLREP_API_END
-}
-int rlrep_drq_num_tensors(rlrep_drq* drq, int* n) {
-  RLREP_API_BEGIN_ON(drq)
-  *n = (int)drq->tensors.size();
-  RLREP_API_END
-}
+int rlrep_drq_destroy(rlrep_drq* drq) { return pixel_destroy(drq); }
+int rlrep_drq_num_tensors(rlrep_drq* drq, int* n) { return pixel_num_tensors(drq, n); }
 int rlrep_drq_tensor_info(rlrep_drq* drq, int i, const char** name, float** ptr_dev, int* rows, int* cols) {
-  RLREP_API_BEGIN_ON(drq)
-  RLREP_CHECK(i >= 0 && i < (int)drq->tensors.size(), "tensor index out of range");
-  const TensorRef& t = drq->tensors[i];
-  if (name) *name = t.name.c_str();
-  if (ptr_dev) *ptr_dev = t.ptr;
-  if (rows) *rows = t.rows;
-  if (cols) *cols = t.cols;
-  RLREP_API_END
+  return pixel_tensor_info(drq, i, name, ptr_dev, rows, cols);
 }
-int rlrep_drq_tensor_read(rlrep_drq* drq, int i, float* out_host) {
-  RLREP_API_BEGIN_ON(drq)
-  RLREP_CHECK(i >= 0 && i < (int)drq->tensors.size(), "tensor index out of range");
-  const TensorRef& t = drq->tensors[i];
-  cudaStream_t st = drq->impl->stream();
-  RLREP_CUDA(cudaMemcpy2DAsync(out_host, (size_t)t.cols * 4, t.ptr, (size_t)t.ld * 4, (size_t)t.cols * 4, t.rows,
-                               cudaMemcpyDeviceToHost, st));
-  RLREP_CUDA(cudaStreamSynchronize(st));
-  RLREP_API_END
-}
-int rlrep_drq_tensor_write(rlrep_drq* drq, int i, const float* in_host) {
-  RLREP_API_BEGIN_ON(drq)
-  RLREP_CHECK(i >= 0 && i < (int)drq->tensors.size(), "tensor index out of range");
-  const TensorRef& t = drq->tensors[i];
-  cudaStream_t st = drq->impl->stream();
-  RLREP_CUDA(cudaMemcpy2DAsync(t.ptr, (size_t)t.ld * 4, in_host, (size_t)t.cols * 4, (size_t)t.cols * 4, t.rows,
-                               cudaMemcpyHostToDevice, st));
-  RLREP_CUDA(cudaStreamSynchronize(st));
-  RLREP_API_END
-}
-int rlrep_drq_sync_targets(rlrep_drq* drq) {
-  RLREP_API_BEGIN_ON(drq)
-  drq->impl->sync_targets_from_params();
-  RLREP_API_END
-}
+int rlrep_drq_tensor_read(rlrep_drq* drq, int i, float* out_host) { return pixel_tensor_read(drq, i, out_host); }
+int rlrep_drq_tensor_write(rlrep_drq* drq, int i, const float* in_host) { return pixel_tensor_write(drq, i, in_host); }
+int rlrep_drq_sync_targets(rlrep_drq* drq) { return pixel_sync_targets(drq); }
 int rlrep_drq_update(rlrep_drq* drq, const unsigned char* img, const float* action, const float* reward,
                      const float* discount, const unsigned char* next_img, const int* shifts, const float* eps,
                      float stddev, float* metrics_host) {
   RLREP_API_BEGIN_ON(drq)
   RLREP_CHECK(drq && img && action && reward && discount && next_img && shifts && eps && metrics_host, "null argument");
-  drq->impl->update(img, action, reward, discount, next_img, shifts, eps, stddev, metrics_host);
+  drq->agent().update(img, action, reward, discount, next_img, shifts, eps, stddev, metrics_host);
   RLREP_API_END
 }
 int rlrep_drq_act(rlrep_drq* drq, const unsigned char* obs_host, const float* eps_host, float stddev, float* action_host) {
@@ -669,43 +744,17 @@ int rlrep_drq_act_batch(rlrep_drq* drq, const unsigned char* obs, const float* e
   RLREP_API_BEGIN_ON(drq)
   RLREP_CHECK(drq && obs && actions_host, "null argument");
   RLREP_CHECK(n > 0, "n must be positive");
-  drq->impl->act_batch(obs, eps_host, stddev, n, actions_host);
+  drq->agent().act_batch(obs, eps_host, stddev, n, actions_host);
   RLREP_API_END
 }
 int rlrep_drq_update_resident(rlrep_drq* drq, int n_steps, float stddev, float* total_ms) {
-  RLREP_API_BEGIN_ON(drq)
-  RLREP_CHECK(drq && total_ms, "null argument");
-  *total_ms = drq->impl->update_resident(n_steps, stddev);
-  RLREP_API_END
+  return pixel_update_resident(drq, n_steps, stddev, total_ms);
 }
 int rlrep_drq_profile_update(rlrep_drq* drq, float stddev, int max_entries, const char** names, float* ms, double* bytes,
                              double* flops, int* n_entries) {
-  RLREP_API_BEGIN_ON(drq)
-  RLREP_CHECK(drq && n_entries && (max_entries == 0 || (names && ms)), "null argument");
-  std::vector<ProfileEntry> prof = drq->impl->profile_update(stddev);
-  const int n = (int)std::min<size_t>(prof.size(), (size_t)max_entries);
-  for (int i = 0; i < n; ++i) {
-    names[i] = prof[i].name;
-    ms[i] = prof[i].ms;
-    if (bytes) bytes[i] = prof[i].bytes;
-    if (flops) flops[i] = prof[i].flops;
-  }
-  *n_entries = (int)prof.size();
-  RLREP_API_END
+  return pixel_profile_update(drq, stddev, max_entries, names, ms, bytes, flops, n_entries);
 }
-int rlrep_drq_last_launches(rlrep_drq* drq, int* launches) {
-  RLREP_API_BEGIN_ON(drq)
-  *launches = drq->impl->last_launches;
-  RLREP_API_END
-}
-
-// ------------------------------------------------------------------------------------------------ muLV-Rep DrQ-v2 pixel agent
-struct rlrep_mulv {
-  int device = current_device();
-  std::unique_ptr<MulvDrq> impl;
-  std::vector<TensorRef> tensors;
-  cudaStream_t owned_stream = nullptr;
-};
+int rlrep_drq_last_launches(rlrep_drq* drq, int* launches) { return pixel_last_launches(drq, launches); }
 
 int rlrep_mulv_create(const rlrep_mulv_config* c, void* stream, rlrep_mulv** out) {
   RLREP_API_BEGIN
@@ -715,80 +764,17 @@ int rlrep_mulv_create(const rlrep_mulv_config* c, void* stream, rlrep_mulv** out
   d.feat_dim = c->feat_dim; d.hidden_dim = c->hidden_dim; d.num_noise = c->num_noise;
   d.lr = c->lr; d.tau = c->tau; d.stddev_clip = c->stddev_clip; d.vae_w = c->vae_w; d.mse_w = c->mse_w;
   d.c_noise = c->c_noise; d.precision = c->precision;
-  std::unique_ptr<rlrep_mulv> h(new rlrep_mulv);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (st == nullptr) {
-    RLREP_CUDA(cudaStreamCreateWithFlags(&h->owned_stream, cudaStreamNonBlocking));
-    st = h->owned_stream;
-  }
-  h->impl.reset(new MulvDrq(d, st));
-  for (ParamGroup* g : h->impl->groups()) {
-    // the conv stacks name their tensors relative to the module ("convnet.0.weight"); the other groups carry full names
-    const bool rel = g->name == "encoder" || g->name == "predict_encoder" || g->name == "decoder";
-    const std::string prefix = rel ? g->name + "." : "";
-    for (const ParamTensor& t : g->tensors) h->tensors.push_back({prefix + t.name, g->p + t.offset, t.rows, t.cols, t.ld});
-    for (const ParamTensor& t : g->tensors)
-      h->tensors.push_back({"grad/" + prefix + t.name, g->g + t.offset, t.rows, t.cols, t.ld});
-    if (g->target)
-      for (const ParamTensor& t : g->tensors)
-        h->tensors.push_back({g->target_prefix_to + t.name.substr(g->target_prefix_from.size()), g->target + t.offset,
-                              t.rows, t.cols, t.ld});
-  }
-  *out = h.release();
+  *out = create_pixel<rlrep_mulv, MulvDrq>(d, stream);
   RLREP_API_END
 }
-int rlrep_mulv_destroy(rlrep_mulv* h) {
-  RLREP_API_BEGIN_ON(h)
-  if (h) {
-    if (h->impl) cudaStreamSynchronize(h->impl->stream());
-    h->impl.reset();
-    if (h->owned_stream) cudaStreamDestroy(h->owned_stream);
-  }
-  delete h;
-  RLREP_API_END
-}
-int rlrep_mulv_num_tensors(rlrep_mulv* h, int* n) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && n, "null argument");
-  *n = (int)h->tensors.size();
-  RLREP_API_END
-}
+int rlrep_mulv_destroy(rlrep_mulv* h) { return pixel_destroy(h); }
+int rlrep_mulv_num_tensors(rlrep_mulv* h, int* n) { return pixel_num_tensors(h, n); }
 int rlrep_mulv_tensor_info(rlrep_mulv* h, int i, const char** name, float** ptr_dev, int* rows, int* cols) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && i >= 0 && i < (int)h->tensors.size(), "tensor index out of range");
-  const TensorRef& t = h->tensors[i];
-  if (name) *name = t.name.c_str();
-  if (ptr_dev) *ptr_dev = t.ptr;
-  if (rows) *rows = t.rows;
-  if (cols) *cols = t.cols;
-  RLREP_API_END
+  return pixel_tensor_info(h, i, name, ptr_dev, rows, cols);
 }
-int rlrep_mulv_tensor_read(rlrep_mulv* h, int i, float* out_host) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && out_host && i >= 0 && i < (int)h->tensors.size(), "tensor index out of range");
-  const TensorRef& t = h->tensors[i];
-  cudaStream_t st = h->impl->stream();
-  RLREP_CUDA(cudaMemcpy2DAsync(out_host, (size_t)t.cols * 4, t.ptr, (size_t)t.ld * 4, (size_t)t.cols * 4, t.rows,
-                               cudaMemcpyDeviceToHost, st));
-  RLREP_CUDA(cudaStreamSynchronize(st));
-  RLREP_API_END
-}
-int rlrep_mulv_tensor_write(rlrep_mulv* h, int i, const float* in_host) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && in_host && i >= 0 && i < (int)h->tensors.size(), "tensor index out of range");
-  const TensorRef& t = h->tensors[i];
-  cudaStream_t st = h->impl->stream();
-  RLREP_CUDA(cudaMemcpy2DAsync(t.ptr, (size_t)t.ld * 4, in_host, (size_t)t.cols * 4, (size_t)t.cols * 4, t.rows,
-                               cudaMemcpyHostToDevice, st));
-  RLREP_CUDA(cudaStreamSynchronize(st));
-  RLREP_API_END
-}
-int rlrep_mulv_sync_targets(rlrep_mulv* h) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h, "null argument");
-  h->impl->sync_targets_from_params();
-  RLREP_API_END
-}
+int rlrep_mulv_tensor_read(rlrep_mulv* h, int i, float* out_host) { return pixel_tensor_read(h, i, out_host); }
+int rlrep_mulv_tensor_write(rlrep_mulv* h, int i, const float* in_host) { return pixel_tensor_write(h, i, in_host); }
+int rlrep_mulv_sync_targets(rlrep_mulv* h) { return pixel_sync_targets(h); }
 int rlrep_mulv_update(rlrep_mulv* h, const unsigned char* img, const float* action, const float* reward,
                       const float* discount, const unsigned char* next_img, const unsigned char* img_step1,
                       const int* shifts, const float* eps_z, const float* eps_act, const float* noise, float stddev,
@@ -796,7 +782,8 @@ int rlrep_mulv_update(rlrep_mulv* h, const unsigned char* img, const float* acti
   RLREP_API_BEGIN_ON(h)
   RLREP_CHECK(h && img && action && reward && discount && next_img && img_step1 && shifts && eps_z && eps_act && noise &&
                   metrics_host, "null argument");
-  h->impl->update(img, action, reward, discount, next_img, img_step1, shifts, eps_z, eps_act, noise, stddev, metrics_host);
+  h->agent().update(img, action, reward, discount, next_img, img_step1, shifts, eps_z, eps_act, noise, stddev,
+                    metrics_host);
   RLREP_API_END
 }
 int rlrep_mulv_act(rlrep_mulv* h, const unsigned char* obs_host, const float* eps_host, float stddev, float* action_host) {
@@ -807,44 +794,17 @@ int rlrep_mulv_act_batch(rlrep_mulv* h, const unsigned char* obs, const float* e
   RLREP_API_BEGIN_ON(h)
   RLREP_CHECK(h && obs && actions_host, "null argument");
   RLREP_CHECK(n > 0, "n must be positive");
-  h->impl->act_batch(obs, eps_host, stddev, n, actions_host);
+  h->agent().act_batch(obs, eps_host, stddev, n, actions_host);
   RLREP_API_END
 }
 int rlrep_mulv_update_resident(rlrep_mulv* h, int n_steps, float stddev, float* total_ms) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && total_ms, "null argument");
-  *total_ms = h->impl->update_resident(n_steps, stddev);
-  RLREP_API_END
+  return pixel_update_resident(h, n_steps, stddev, total_ms);
 }
 int rlrep_mulv_profile_update(rlrep_mulv* h, float stddev, int max_entries, const char** names, float* ms, double* bytes,
                               double* flops, int* n_entries) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && n_entries && (max_entries == 0 || (names && ms)), "null argument");
-  std::vector<ProfileEntry> prof = h->impl->profile_update(stddev);
-  const int n = (int)std::min<size_t>(prof.size(), (size_t)max_entries);
-  for (int i = 0; i < n; ++i) {
-    names[i] = prof[i].name;
-    ms[i] = prof[i].ms;
-    if (bytes) bytes[i] = prof[i].bytes;
-    if (flops) flops[i] = prof[i].flops;
-  }
-  *n_entries = (int)prof.size();
-  RLREP_API_END
+  return pixel_profile_update(h, stddev, max_entries, names, ms, bytes, flops, n_entries);
 }
-int rlrep_mulv_last_launches(rlrep_mulv* h, int* launches) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && launches, "null argument");
-  *launches = h->impl->last_launches;
-  RLREP_API_END
-}
-
-// ------------------------------------------------------------------------------------------------ latent Diff-SR DrQ-v2 (DRAFT)
-struct rlrep_ldiff {
-  int device = current_device();
-  std::unique_ptr<LatentDiffSR> impl;
-  std::vector<TensorRef> tensors;
-  cudaStream_t owned_stream = nullptr;
-};
+int rlrep_mulv_last_launches(rlrep_mulv* h, int* launches) { return pixel_last_launches(h, launches); }
 
 int rlrep_ldiff_create(const rlrep_ldiff_config* c, void* stream, rlrep_ldiff** out) {
   RLREP_API_BEGIN
@@ -855,87 +815,17 @@ int rlrep_ldiff_create(const rlrep_ldiff_config* c, void* stream, rlrep_ldiff** 
   d.hidden = c->hidden_dim; d.ae_lr = c->ae_lr; d.score_lr = c->score_lr; d.actor_lr = c->actor_lr; d.critic_lr = c->critic_lr;
   d.weight_decay = c->weight_decay; d.tau = c->tau; d.kl_coef = c->kl_coef; d.ae_coef = c->ae_coef;
   d.stddev_clip = c->stddev_clip; d.precision = c->precision;
-  std::unique_ptr<rlrep_ldiff> h(new rlrep_ldiff);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (st == nullptr) {
-    RLREP_CUDA(cudaStreamCreateWithFlags(&h->owned_stream, cudaStreamNonBlocking));
-    st = h->owned_stream;
-  }
-  h->impl.reset(new LatentDiffSR(d, st));
-  for (ParamGroup* g : h->impl->groups()) {
-    // the conv stacks name their tensors relative to the module ("convnet.0.weight" -> vae.encoder.convs.0.weight)
-    const bool enc = g->name == "vae.encoder", dec = g->name == "vae.decoder";
-    auto full = [&](const std::string& n, const std::string& prefix) {
-      if (enc) return prefix + "encoder.convs." + n.substr(std::string("convnet.").size());
-      if (dec) return prefix + "decoder.deconvs." + n.substr(std::string("deconvnet.").size());
-      return n;
-    };
-    for (const ParamTensor& t : g->tensors) h->tensors.push_back({full(t.name, "vae."), g->p + t.offset, t.rows, t.cols, t.ld});
-    if (g->g)
-      for (const ParamTensor& t : g->tensors)
-        h->tensors.push_back({"grad/" + full(t.name, "vae."), g->g + t.offset, t.rows, t.cols, t.ld});
-    if (g->target)
-      for (const ParamTensor& t : g->tensors) {
-        const std::string nm = (enc || dec) ? full(t.name, "vae_target.")
-                                            : g->target_prefix_to + t.name.substr(g->target_prefix_from.size());
-        h->tensors.push_back({nm, g->target + t.offset, t.rows, t.cols, t.ld});
-      }
-  }
-  *out = h.release();
+  *out = create_pixel<rlrep_ldiff, LatentDiffSR>(d, stream);
   RLREP_API_END
 }
-int rlrep_ldiff_destroy(rlrep_ldiff* h) {
-  RLREP_API_BEGIN_ON(h)
-  if (h) {
-    if (h->impl) cudaStreamSynchronize(h->impl->stream());
-    h->impl.reset();
-    if (h->owned_stream) cudaStreamDestroy(h->owned_stream);
-  }
-  delete h;
-  RLREP_API_END
-}
-int rlrep_ldiff_num_tensors(rlrep_ldiff* h, int* n) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && n, "null argument");
-  *n = (int)h->tensors.size();
-  RLREP_API_END
-}
+int rlrep_ldiff_destroy(rlrep_ldiff* h) { return pixel_destroy(h); }
+int rlrep_ldiff_num_tensors(rlrep_ldiff* h, int* n) { return pixel_num_tensors(h, n); }
 int rlrep_ldiff_tensor_info(rlrep_ldiff* h, int i, const char** name, float** ptr_dev, int* rows, int* cols) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && i >= 0 && i < (int)h->tensors.size(), "tensor index out of range");
-  const TensorRef& t = h->tensors[i];
-  if (name) *name = t.name.c_str();
-  if (ptr_dev) *ptr_dev = t.ptr;
-  if (rows) *rows = t.rows;
-  if (cols) *cols = t.cols;
-  RLREP_API_END
+  return pixel_tensor_info(h, i, name, ptr_dev, rows, cols);
 }
-int rlrep_ldiff_tensor_read(rlrep_ldiff* h, int i, float* out_host) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && out_host && i >= 0 && i < (int)h->tensors.size(), "tensor index out of range");
-  const TensorRef& t = h->tensors[i];
-  cudaStream_t st = h->impl->stream();
-  RLREP_CUDA(cudaMemcpy2DAsync(out_host, (size_t)t.cols * 4, t.ptr, (size_t)t.ld * 4, (size_t)t.cols * 4, t.rows,
-                               cudaMemcpyDeviceToHost, st));
-  RLREP_CUDA(cudaStreamSynchronize(st));
-  RLREP_API_END
-}
-int rlrep_ldiff_tensor_write(rlrep_ldiff* h, int i, const float* in_host) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && in_host && i >= 0 && i < (int)h->tensors.size(), "tensor index out of range");
-  const TensorRef& t = h->tensors[i];
-  cudaStream_t st = h->impl->stream();
-  RLREP_CUDA(cudaMemcpy2DAsync(t.ptr, (size_t)t.ld * 4, in_host, (size_t)t.cols * 4, (size_t)t.cols * 4, t.rows,
-                               cudaMemcpyHostToDevice, st));
-  RLREP_CUDA(cudaStreamSynchronize(st));
-  RLREP_API_END
-}
-int rlrep_ldiff_sync_targets(rlrep_ldiff* h) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h, "null argument");
-  h->impl->sync_targets_from_params();
-  RLREP_API_END
-}
+int rlrep_ldiff_tensor_read(rlrep_ldiff* h, int i, float* out_host) { return pixel_tensor_read(h, i, out_host); }
+int rlrep_ldiff_tensor_write(rlrep_ldiff* h, int i, const float* in_host) { return pixel_tensor_write(h, i, in_host); }
+int rlrep_ldiff_sync_targets(rlrep_ldiff* h) { return pixel_sync_targets(h); }
 int rlrep_ldiff_update(rlrep_ldiff* h, const rlrep_ldiff_inputs* in, float* metrics_host) {
   RLREP_API_BEGIN_ON(h)
   RLREP_CHECK(h && in && metrics_host, "null argument");
@@ -946,36 +836,17 @@ int rlrep_ldiff_update(rlrep_ldiff* h, const rlrep_ldiff_inputs* in, float* metr
   x.zeta_masks = in->zeta_masks; x.eps_act = in->eps_act; x.stddev = in->stddev;
   RLREP_CHECK(x.frames && x.next_frames && x.shifts && x.next_shifts && x.action && x.reward && x.discount && x.eps_post &&
                   x.alphabar && x.temb && x.noise && x.psi_masks && x.zeta_masks && x.eps_act, "null input pointer");
-  h->impl->update(x, metrics_host);
+  h->agent().update(x, metrics_host);
   RLREP_API_END
 }
 int rlrep_ldiff_update_resident(rlrep_ldiff* h, int n_steps, float stddev, float* total_ms) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && total_ms, "null argument");
-  *total_ms = h->impl->update_resident(n_steps, stddev);
-  RLREP_API_END
+  return pixel_update_resident(h, n_steps, stddev, total_ms);
 }
 int rlrep_ldiff_profile_update(rlrep_ldiff* h, float stddev, int max_entries, const char** names, float* ms, double* bytes,
                                double* flops, int* n_entries) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && n_entries && (max_entries == 0 || (names && ms)), "null argument");
-  std::vector<ProfileEntry> prof = h->impl->profile_update(stddev);
-  const int n = (int)std::min<size_t>(prof.size(), (size_t)max_entries);
-  for (int i = 0; i < n; ++i) {
-    names[i] = prof[i].name;
-    ms[i] = prof[i].ms;
-    if (bytes) bytes[i] = prof[i].bytes;
-    if (flops) flops[i] = prof[i].flops;
-  }
-  *n_entries = (int)prof.size();
-  RLREP_API_END
+  return pixel_profile_update(h, stddev, max_entries, names, ms, bytes, flops, n_entries);
 }
-int rlrep_ldiff_last_launches(rlrep_ldiff* h, int* launches) {
-  RLREP_API_BEGIN_ON(h)
-  RLREP_CHECK(h && launches, "null argument");
-  *launches = h->impl->last_launches;
-  RLREP_API_END
-}
+int rlrep_ldiff_last_launches(rlrep_ldiff* h, int* launches) { return pixel_last_launches(h, launches); }
 
 // ------------------------------------------------------------------------------------------------ communicator
 // ------------------------------------------------------------------------------------------------ pixel replay ring
@@ -1126,37 +997,26 @@ int rlrep_agent_destroy(rlrep_agent* agent) {
 }
 int rlrep_agent_num_tensors(rlrep_agent* agent, int* n) {
   RLREP_API_BEGIN_ON(agent)
+  RLREP_CHECK(agent && n, "null argument");
   *n = (int)agent->tensors.size();
   RLREP_API_END
 }
 int rlrep_agent_tensor_info(rlrep_agent* agent, int i, const char** name, float** ptr_dev, int* rows, int* cols) {
   RLREP_API_BEGIN_ON(agent)
-  RLREP_CHECK(i >= 0 && i < (int)agent->tensors.size(), "tensor index out of range");
-  const TensorRef& t = agent->tensors[i];
-  if (name) *name = t.name.c_str();
-  if (ptr_dev) *ptr_dev = t.ptr;
-  if (rows) *rows = t.rows;
-  if (cols) *cols = t.cols;
+  RLREP_CHECK(agent, "null argument");
+  tensor_info(agent->tensors, i, name, ptr_dev, rows, cols);
   RLREP_API_END
 }
 int rlrep_agent_tensor_read(rlrep_agent* agent, int i, float* out_host) {
   RLREP_API_BEGIN_ON(agent)
-  RLREP_CHECK(i >= 0 && i < (int)agent->tensors.size(), "tensor index out of range");
-  const TensorRef& t = agent->tensors[i];
-  cudaStream_t st = agent->impl->stream;
-  RLREP_CUDA(cudaMemcpy2DAsync(out_host, (size_t)t.cols * 4, t.ptr, (size_t)t.ld * 4, (size_t)t.cols * 4, t.rows,
-                               cudaMemcpyDeviceToHost, st));
-  RLREP_CUDA(cudaStreamSynchronize(st));
+  RLREP_CHECK(agent, "null argument");
+  tensor_read(agent->tensors, i, out_host, agent->impl->stream);
   RLREP_API_END
 }
 int rlrep_agent_tensor_write(rlrep_agent* agent, int i, const float* in_host) {
   RLREP_API_BEGIN_ON(agent)
-  RLREP_CHECK(i >= 0 && i < (int)agent->tensors.size(), "tensor index out of range");
-  const TensorRef& t = agent->tensors[i];
-  cudaStream_t st = agent->impl->stream;
-  RLREP_CUDA(cudaMemcpy2DAsync(t.ptr, (size_t)t.ld * 4, in_host, (size_t)t.cols * 4, (size_t)t.cols * 4, t.rows,
-                               cudaMemcpyHostToDevice, st));
-  RLREP_CUDA(cudaStreamSynchronize(st));
+  RLREP_CHECK(agent, "null argument");
+  tensor_write(agent->tensors, i, in_host, agent->impl->stream);
   RLREP_API_END
 }
 int rlrep_agent_get_log_alpha(rlrep_agent* agent, double* log_alpha) {

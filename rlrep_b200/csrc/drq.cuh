@@ -2,9 +2,7 @@
 #pragma once
 #include <memory>
 
-#include "agent.cuh"
-#include "conv.cuh"
-#include "pixel_act.cuh"
+#include "pixel_agent.cuh"
 
 namespace rlrep {
 
@@ -15,12 +13,9 @@ struct DrqConfig {
   int precision = PREC_TF32;
 };
 
-class DrqV2 {
+class DrqV2 : public PixelAgent {
  public:
   DrqV2(const DrqConfig& c, cudaStream_t s);
-  ~DrqV2();
-  DrqV2(const DrqV2&) = delete;
-  DrqV2& operator=(const DrqV2&) = delete;
 
   // One `train_step` that updates (the caller implements `update_every`).  Host buffers: img / next_img uint8
   // [B, C, H, H]; action [B, A]; reward, discount [B]; shifts int32 [2][B][2] (img then next_img; (x, y) in [0, 8]);
@@ -28,21 +23,17 @@ class DrqV2 {
   // metrics_out[5] = {critic_loss, mean(q_pred), mean(q_target), mean(reward), actor_loss}.
   void update(const unsigned char* img, const float* action, const float* reward, const float* discount,
               const unsigned char* next_img, const int* shifts, const float* eps, float stddev, float* metrics_out);
-  // Benchmark aids on the batch uploaded by the last update(): n_steps updates back to back, CUDA-event time of the loop
-  // in milliseconds; one update with an event behind every launch.
-  float update_resident(int n_steps, float stddev);
-  std::vector<ProfileEntry> profile_update(float stddev);
   // select_action on n observations (PixelPolicy::act): obs uint8 [n, C, H, H] host or device; eps [n, A] standard normal
   // or nullptr (deterministic: the mean); actions [n, A].  Reads the current weights and no update buffer.
   // The policy's buffers are allocated by the first call: a handle that never acts allocates nothing for it.
   void act_batch(const unsigned char* obs, const float* eps_host, float stddev, int n, float* actions_host);
-  void sync_targets_from_params();
-  std::vector<ParamGroup*> groups() { return {&enc_->group(), &actor_g_, &crit_g_}; }
-  cudaStream_t stream() const { return stream_; }
-  int last_launches = 0;
+  std::vector<ParamGroup*> groups() override { return {&enc_->group(), &actor_g_, &crit_g_}; }
+  std::string tensor_name(const ParamGroup& g, const std::string& t) const override {
+    return &g == &enc_->group() ? "encoder." + t : t;
+  }
 
  private:
-  void launch_update(float stddev);
+  void launch_update(float stddev) override;
   void trunk_forward(const LinearSlot& t, const ParamGroup& g, bool target, size_t ln_w, size_t ln_b, const float* x,
                      float* pre, float* out, int ld_out, float* xhat, float* rstd);
   void q_forward(bool target, int set);
@@ -50,7 +41,6 @@ class DrqV2 {
   void actor_forward(const float* latent, const float* eps, float stddev, int set, bool keep);
 
   DrqConfig cfg_;
-  cudaStream_t stream_;
   int B_, A_, bn_, H_, F_ = 0, LB_ = 0, LC_ = 0, LA_ = 0;
   std::unique_ptr<ConvEncoder> enc_;
   DeviceArena arena_;
@@ -59,8 +49,7 @@ class DrqV2 {
   LinearSlot ct_, q0_, q1a_, q1b_, q2a_, q2b_, at_, p0_, p1_, p2_;
   size_t cln_w_ = 0, cln_b_ = 0, aln_w_ = 0, aln_b_ = 0;
   Control* ctl_ = nullptr;
-  float* metrics_dev_ = nullptr;
-  unsigned char *img_dev_ = nullptr, *next_img_dev_ = nullptr, *stage_host_ = nullptr;
+  unsigned char *img_dev_ = nullptr, *next_img_dev_ = nullptr;
   int* shifts_dev_ = nullptr;
   float *eps_dev_ = nullptr, *action_dev_ = nullptr, *reward_dev_ = nullptr, *discount_dev_ = nullptr;
   float *latent_ = nullptr, *next_latent_ = nullptr, *dlatent_ = nullptr;
@@ -69,8 +58,7 @@ class DrqV2 {
   float *xhat_c_ = nullptr, *rstd_c_ = nullptr, *xhat_a_ = nullptr, *rstd_a_ = nullptr, *th_ = nullptr;
   float *ap1_ = nullptr, *ap2_ = nullptr, *raw_ = nullptr, *mu_ = nullptr, *dq_ = nullptr;
   float *dhid1_ = nullptr, *dhid0_ = nullptr, *dcat_ = nullptr, *dtpre_ = nullptr, *gb_ = nullptr, *gg_ = nullptr;
-  float *draw_ = nullptr, *dap2_ = nullptr, *dap1_ = nullptr, *dth_ = nullptr, *metrics_host_ = nullptr;
-  size_t stage_bytes_ = 0;
+  float *draw_ = nullptr, *dap2_ = nullptr, *dap1_ = nullptr, *dth_ = nullptr;
   std::unique_ptr<PixelPolicy> policy_;
 };
 

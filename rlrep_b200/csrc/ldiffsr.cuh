@@ -1,12 +1,10 @@
-// DRAFT (branch draft/ldiffsr-agent; not verified on hardware): latent Diff-SR DrQ-v2 pixel agent handle
-// (see agent_ldiffsr.cu).
+// Latent Diff-SR DrQ-v2 pixel agent handle (see agent_ldiffsr.cu).
 #pragma once
 #include <memory>
 
-#include "agent.cuh"
-#include "conv.cuh"
 #include "deconv.cuh"
 #include "nets.cuh"
+#include "pixel_agent.cuh"
 
 namespace rlrep {
 
@@ -41,12 +39,9 @@ struct BottleneckActs {
         *rstd_a = nullptr;
 };
 
-class LatentDiffSR {
+class LatentDiffSR : public PixelAgent {
  public:
   LatentDiffSR(const LdiffConfig& c, cudaStream_t s);
-  ~LatentDiffSR();
-  LatentDiffSR(const LatentDiffSR&) = delete;
-  LatentDiffSR& operator=(const LatentDiffSR&) = delete;
 
   struct Inputs {  // all host pointers; N = 4 * batch frames
     const unsigned char* frames;       // [N, 3, 84, 84]: the 3B frames of img_stack, then the B newest next frames
@@ -63,19 +58,19 @@ class LatentDiffSR {
   };
   // metrics_out[8] = {recon_loss, kl_loss, score_loss, critic_loss, mean(q_pred), mean(q_target), mean(reward), actor_loss}
   void update(const Inputs& in, float* metrics_out);
-  // n_steps updates on the inputs the last update() left in HBM (bench.py's device-timed figure) -> total ms; one eager
-  // update with an event behind every launch (per-kernel profile)
-  float update_resident(int n_steps, float stddev);
-  std::vector<ProfileEntry> profile_update(float stddev);
-  void sync_targets_from_params();
-  std::vector<ParamGroup*> groups() {
+  std::vector<ParamGroup*> groups() override {
     return {&enc_->group(), &vh_g_, &dec_->group(), &score_g_, &dead_g_, &actor_g_, &crit_g_};
   }
-  cudaStream_t stream() const { return stream_; }
-  int last_launches = 0;
+  // the conv stacks' "convnet.<i>.*" / "deconvnet.<i>.*" are the VAE's "vae.encoder.convs.<i>.*" /
+  // "vae.decoder.deconvs.<i>.*"
+  std::string tensor_name(const ParamGroup& g, const std::string& t) const override {
+    if (&g == &enc_->group()) return "vae.encoder.convs." + t.substr(std::string("convnet.").size());
+    if (&g == &dec_->group()) return "vae.decoder.deconvs." + t.substr(std::string("deconvnet.").size());
+    return t;
+  }
 
  private:
-  void launch_update(float stddev);
+  void launch_update(float stddev) override;
   ResNetSlots add_resnet(const std::string& prefix, int depth, int in, int out, int h);
   void resnet_forward(const ResNetSlots& n, bool target, int rows, Mat in, const float* masks, size_t mask_stride,
                       ResNetActs& a, float* out, int ld_out);
@@ -90,7 +85,6 @@ class LatentDiffSR {
   void actor_forward(Mat latent, const float* eps, float stddev, float* action_out, int ld_action, bool keep);
 
   LdiffConfig cfg_;
-  cudaStream_t stream_;
   int B_, N_, A_, L_, F_ = 0, feat_, bn_, H_, LA_ = 0, LZ_ = 0, T_ = 0;
   std::unique_ptr<ConvEncoder> enc_;
   std::unique_ptr<ConvDecoder> dec_;
@@ -103,8 +97,7 @@ class LatentDiffSR {
   ResNetSlots psi_, zeta_;
   RffCritic rff_;
   Control* ctl_ = nullptr;
-  float *metrics_dev_ = nullptr, *metrics_host_ = nullptr;
-  unsigned char *frames_dev_ = nullptr, *next_frames_dev_ = nullptr, *stage_host_ = nullptr;
+  unsigned char *frames_dev_ = nullptr, *next_frames_dev_ = nullptr;
   int *shifts_dev_ = nullptr, *next_shifts_dev_ = nullptr;
   float *action_dev_ = nullptr, *reward_dev_ = nullptr, *discount_dev_ = nullptr, *eps_post_dev_ = nullptr, *ab_dev_ = nullptr;
   float *temb_dev_ = nullptr, *noise_dev_ = nullptr, *psi_masks_dev_ = nullptr, *zeta_masks_dev_ = nullptr, *eps_act_dev_ = nullptr;
@@ -127,7 +120,6 @@ class LatentDiffSR {
   float *tpre_ = nullptr, *th_ = nullptr, *xhat_a_ = nullptr, *rstd_a_ = nullptr, *ap1_ = nullptr, *ap2_ = nullptr;
   float *raw_a_ = nullptr, *mu_ = nullptr, *draw_a_ = nullptr, *dap2_ = nullptr, *dap1_ = nullptr, *dth_ = nullptr;
   float* dtpre_ = nullptr;
-  size_t stage_bytes_ = 0;
   static constexpr int kKlBlocks = 64;
 };
 

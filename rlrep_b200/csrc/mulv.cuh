@@ -2,10 +2,8 @@
 #pragma once
 #include <memory>
 
-#include "agent.cuh"
-#include "conv.cuh"
 #include "deconv.cuh"
-#include "pixel_act.cuh"
+#include "pixel_agent.cuh"
 
 namespace rlrep {
 
@@ -28,12 +26,9 @@ struct GaussActs {
         *rstd_s = nullptr;
 };
 
-class MulvDrq {
+class MulvDrq : public PixelAgent {
  public:
   MulvDrq(const MulvConfig& c, cudaStream_t s);
-  ~MulvDrq();
-  MulvDrq(const MulvDrq&) = delete;
-  MulvDrq& operator=(const MulvDrq&) = delete;
 
   // One `update` that steps (the caller implements `up_every`).  Host buffers: img / next_img uint8 [B, C, H, H];
   // img_step1 uint8 [B, 3, H, H] (the last frame of the one-step-ahead observation); action [B, A]; reward, discount [B];
@@ -47,17 +42,16 @@ class MulvDrq {
   // standard normal or nullptr (eval_mode: the mean); actions [n, A].  Reads the current weights and no update buffer.
   // The policy's buffers are allocated by the first call: a handle that never acts allocates nothing for it.
   void act_batch(const unsigned char* obs, const float* eps_host, float stddev, int n, float* actions_host);
-  float update_resident(int n_steps, float stddev);
-  std::vector<ProfileEntry> profile_update(float stddev);
-  void sync_targets_from_params();
-  std::vector<ParamGroup*> groups() {
+  std::vector<ParamGroup*> groups() override {
     return {&enc_->group(), &penc_->group(), &dec_->group(), &actor_g_, &crit_g_, &fe_g_, &fd_g_, &ff_g_};
   }
-  cudaStream_t stream() const { return stream_; }
-  int last_launches = 0;
+  std::string tensor_name(const ParamGroup& g, const std::string& t) const override {
+    const bool conv_stack = &g == &enc_->group() || &g == &penc_->group() || &g == &dec_->group();
+    return conv_stack ? g.name + "." + t : t;
+  }
 
  private:
-  void launch_update(float stddev);
+  void launch_update(float stddev) override;
   void gauss_forward(const GaussHead& h, const ParamGroup& g, bool target, Mat x, GaussActs& a, bool keep);
   void gauss_backward(const GaussHead& h, ParamGroup& g, Mat x, const GaussActs& a, const float* dm, const float* draw,
                       bool wgrad);
@@ -67,7 +61,6 @@ class MulvDrq {
                      bool keep);
 
   MulvConfig cfg_;
-  cudaStream_t stream_;
   int B_, A_, D_, H_, NN_, F_ = 0, LF_ = 0, LA_ = 0, LDE_ = 0, LDS_ = 0;
   std::unique_ptr<ConvEncoder> enc_, penc_;
   std::unique_ptr<ConvDecoder> dec_;
@@ -78,11 +71,10 @@ class MulvDrq {
   LinearSlot at_, p0_, p1_, p2_, c14_, c2_, c5_, c3_, c6_, d1_, d2_, ds_, dr_;
   size_t aln_w_ = 0, aln_b_ = 0;
   Control* ctl_ = nullptr;
-  float* metrics_dev_ = nullptr;
-  unsigned char *img_dev_ = nullptr, *next_img_dev_ = nullptr, *step1_dev_ = nullptr, *stage_host_ = nullptr;
+  unsigned char *img_dev_ = nullptr, *next_img_dev_ = nullptr, *step1_dev_ = nullptr;
   int* shifts_dev_ = nullptr;
   float *eps_z_dev_ = nullptr, *eps_act_dev_ = nullptr, *noise_dev_ = nullptr, *action_dev_ = nullptr;
-  float *reward_dev_ = nullptr, *discount_dev_ = nullptr, *metrics_host_ = nullptr;
+  float *reward_dev_ = nullptr, *discount_dev_ = nullptr;
   float *enc_in_ = nullptr, *nsa_ = nullptr, *dstate_ = nullptr, *dstep1_ = nullptr;
   GaussActs ge_, gf_, gn_;
   float *z_ = nullptr, *dz_ = nullptr, *fh1_ = nullptr, *fh2_ = nullptr, *s_hat_ = nullptr, *ds_hat_ = nullptr;
@@ -95,7 +87,6 @@ class MulvDrq {
   float *tpre_ = nullptr, *th_ = nullptr, *xhat_a_ = nullptr, *rstd_a_ = nullptr, *ap1_ = nullptr, *ap2_ = nullptr;
   float *raw_a_ = nullptr, *mu_ = nullptr, *daction_ = nullptr, *draw_a_ = nullptr, *dap2_ = nullptr, *dap1_ = nullptr;
   float *dth_ = nullptr, *dtpre_ = nullptr;
-  size_t stage_bytes_ = 0;
   static constexpr int kKlBlocks = 64;
   std::unique_ptr<PixelPolicy> policy_;
 };

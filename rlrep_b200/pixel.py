@@ -297,6 +297,132 @@ class ConvDecoder:
         return out
 
 
+class _PixelAgent:
+    """What the pixel agents share: the device handle behind `rlrep_<_PREFIX>_*`, created by the first call that needs
+    it, its tensor index, and the weights and gradients under the reference's module names.  Subclasses set `_PREFIX`,
+    `_config(batch)` (the ctypes config of the handle) and `_kind(name)`, the layout class of a tensor name."""
+    _PREFIX = None
+    OUTCONV_SHAPE = None  # reference shape of the decoder's output convolution, if the agent has one
+
+    def __init__(self, precision):
+        # construction is lazy like the state-based agents: the device handle is created by the first call that needs
+        # it (and raises there without a CUDA device -- there is no CPU fallback)
+        self._precision = precision
+        self.lib = None
+        self._h = None
+        self._batch = None
+        self._pending = {}
+
+    def _fn(self, name):
+        return getattr(self.lib, f"rlrep_{self._PREFIX}_{name}")
+
+    # ---- handle ------------------------------------------------------------------------------------------------
+    def _ensure(self, batch):
+        if self._h is not None:
+            if batch != self._batch:
+                raise _lib.RlrepError(f"batch size is fixed per handle (was {self._batch}, got {batch})")
+            return
+        if not torch.cuda.is_available():
+            raise _lib.RlrepError(f"rlrep_b200.{type(self).__name__} needs a CUDA device (there is no CPU fallback)")
+        self.lib = _lib.load()
+        cfg = self._config(batch)
+        hd = C.c_void_p()
+        _lib.check(self._fn("create")(C.byref(cfg), None, C.byref(hd)))
+        self._h, self._batch = hd, batch
+        n = C.c_int()
+        _lib.check(self._fn("num_tensors")(hd, C.byref(n)))
+        self._index = {}
+        for i in range(n.value):
+            name, ptr, rows, cols = C.c_char_p(), C.c_void_p(), C.c_int(), C.c_int()
+            _lib.check(self._fn("tensor_info")(hd, i, C.byref(name), C.byref(ptr), C.byref(rows), C.byref(cols)))
+            self._index[name.value.decode()] = (i, rows.value, cols.value)
+        if self._pending:
+            sd, self._pending = self._pending, {}
+            self.load_state_dict(sd)
+
+    def prepare(self, batch_size):
+        """Create the device handle for `batch_size` ahead of the first update."""
+        self._ensure(int(batch_size))
+
+    def close(self):
+        h, self._h = self._h, None
+        if h and self.lib is not None:
+            self._fn("destroy")(h)
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    # ---- weights under the reference's module names ----------------------------------------------------------------
+    def _ref_shape(self, name, rows, cols):
+        return {"outconv": self.OUTCONV_SHAPE, "deconv": (32, 32, 3, 3), "conv0": (32, cols // 9, 3, 3),
+                "conv": (32, cols // 9, 3, 3), "vec": (rows,), "mat": (rows, cols)}[self._kind(name)]
+
+    def _read_all(self, keep):
+        sd = {}
+        for name, (i, rows, cols) in self._index.items():
+            if not keep(name):
+                continue
+            out = np.empty(rows * cols, dtype=np.float32)
+            _lib.check(self._fn("tensor_read")(self._h, i, out.ctypes.data))
+            t, kind = torch.from_numpy(out), self._kind(name)
+            if kind == "conv":      # stored [32, (ky, kx, c)] -> reference [32, c, ky, kx]
+                t = t.reshape(32, 3, 3, 32).permute(0, 3, 1, 2).contiguous()
+            elif kind == "deconv":  # stored [(ky, kx, c_out), c_in] -> reference [c_in, c_out, ky, kx]
+                t = t.reshape(3, 3, 32, 32).permute(3, 2, 0, 1).contiguous()
+            sd[name] = t.reshape(self._ref_shape(name, rows, cols))
+        return sd
+
+    def state_dict(self):
+        if self._h is None:
+            return dict(self._pending)
+        return self._read_all(lambda name: not name.startswith("grad/"))
+
+    def grads(self):
+        """Gradients left by the most recent update, under the reference's names."""
+        return {k[5:]: v for k, v in self._read_all(lambda name: name.startswith("grad/")).items()}
+
+    def load_state_dict(self, sd, sync_targets=None):
+        """Targets are copied from the loaded parameters unless `sd` carries them (or `sync_targets` says otherwise)."""
+        if self._h is None:
+            self._pending.update({k: torch.as_tensor(v).detach().clone() for k, v in sd.items()})
+            return
+        for k, v in sd.items():
+            i, rows, cols = self._index[k]
+            t = torch.as_tensor(v).detach().cpu().float()
+            if tuple(t.shape) != self._ref_shape(k, rows, cols):
+                raise ValueError(f"{k}: expected {self._ref_shape(k, rows, cols)}, got {tuple(t.shape)}")
+            kind = self._kind(k)
+            if kind == "conv":
+                t = t.permute(0, 2, 3, 1)
+            elif kind == "deconv":
+                t = t.permute(2, 3, 1, 0)
+            arr = np.ascontiguousarray(t.reshape(-1).numpy())
+            _lib.check(self._fn("tensor_write")(self._h, i, arr.ctypes.data))
+        if sync_targets or (sync_targets is None and not any("_target." in k for k in sd)):
+            _lib.check(self._fn("sync_targets")(self._h))
+
+    @property
+    def gpu_launches_last_update(self):
+        v = C.c_int()
+        _lib.check(self._fn("last_launches")(self._h, C.byref(v)))
+        return v.value
+
+    def _act_batch(self, obs, obs_shape, step, sample, explore=False):
+        """The handle's act_batch on uint8 observations [N, *obs_shape], with the noise N single acts would draw.
+        Returns (actions [N, A], the exploration phase's uniform draws [N, A] or None)."""
+        keep, ptr, n = _obs_batch(obs, obs_shape)
+        stddev = float(self.stddev_schedule(step))
+        eps, uni = _act_noise(n, self.action_dim, sample=sample, explore=explore)
+        out = np.empty((n, self.action_dim), dtype=np.float32)
+        _lib.check(self._fn("act_batch")(self._h, ptr, eps.ctypes.data if eps is not None else None, stddev, n,
+                                         out.ctypes.data))
+        del keep
+        return out, uni
+
+
 class DrqConfig(C.Structure):
     """Mirror of `rlrep_drq_config` (include/rlrep_b200.h)."""
     _fields_ = [("batch_size", C.c_int), ("channels", C.c_int), ("height", C.c_int), ("action_dim", C.c_int),
@@ -315,124 +441,43 @@ def _schedule(spec):
     return fn
 
 
-class DrQv2:
+class DrQv2(_PixelAgent):
     """Drop-in for the update path of agent.diffsrdrq.drqv2.DrQv2 (drqv2.py:12-148): same constructor
     (`obs_space`, `action_space`, `args` with tau / update_every / critic_loss / stddev_schedule / stddev_clip / bn_dim /
     actor_hidden_dim / critic_hidden_dim / encoder_lr / actor_lr / critic_lr) and `train_step(replay_iter, step)` with the
     reference's metric keys, plus `select_action(obs, step, deterministic)`.  The batch comes from the caller's replay
     iterator as in the reference (img_stack uint8 [B, 9, 84, 84], action, reward, discount, next_img_stack,
     next_img_step)."""
+    _PREFIX = "drq"
 
     def __init__(self, obs_space, action_space, args, *, precision="tf32"):
-        # construction is lazy like the state-based agents: the device handle is created by the first call that needs
-        # it (and raises there without a CUDA device -- there is no CPU fallback)
         if getattr(args, "critic_loss", "mse") != "mse":
             raise NotImplementedError("critic_loss='huber' (configs/drqv2.yaml ships 'mse')")
         if args.actor_hidden_dim != args.critic_hidden_dim:
             raise NotImplementedError("actor_hidden_dim != critic_hidden_dim")
+        super().__init__(precision)
         self.args = args
         self.obs_dim = tuple(int(x) for x in obs_space.shape)
         self.action_dim = int(action_space.shape[0])
         self.tau, self.update_every = float(args.tau), int(args.update_every)
         self.stddev_schedule, self.stddev_clip = _schedule(args.stddev_schedule), float(args.stddev_clip)
         self.bn_dim, self.hidden_dim = int(args.bn_dim), int(args.actor_hidden_dim)
-        self._precision = precision
         self._step = 1
-        self.lib = None
-        self._h = None
-        self._batch = None
-        self._pending = {}
 
-    # ---- handle ------------------------------------------------------------------------------------------------
-    def _ensure(self, batch):
-        if self._h is not None:
-            if batch != self._batch:
-                raise _lib.RlrepError(f"batch size is fixed per handle (was {self._batch}, got {batch})")
-            return
-        if not torch.cuda.is_available():
-            raise _lib.RlrepError("rlrep_b200.DrQv2 needs a CUDA device (there is no CPU fallback)")
-        self.lib = _lib.load()
+    def _config(self, batch):
         c, h, _ = self.obs_dim
-        cfg = DrqConfig(batch_size=batch, channels=c, height=h, action_dim=self.action_dim, bn_dim=self.bn_dim,
-                        hidden_dim=self.hidden_dim, encoder_lr=float(self.args.encoder_lr),
-                        actor_lr=float(self.args.actor_lr), critic_lr=float(self.args.critic_lr), tau=self.tau,
-                        stddev_clip=self.stddev_clip, precision=_lib.PRECISION[self._precision])
-        hd = C.c_void_p()
-        _lib.check(self.lib.rlrep_drq_create(C.byref(cfg), None, C.byref(hd)))
-        self._h, self._batch = hd, batch
-        n = C.c_int()
-        _lib.check(self.lib.rlrep_drq_num_tensors(hd, C.byref(n)))
-        self._index = {}
-        for i in range(n.value):
-            name, ptr, rows, cols = C.c_char_p(), C.c_void_p(), C.c_int(), C.c_int()
-            _lib.check(self.lib.rlrep_drq_tensor_info(hd, i, C.byref(name), C.byref(ptr), C.byref(rows), C.byref(cols)))
-            self._index[name.value.decode()] = (i, rows.value, cols.value)
-        if self._pending:
-            sd, self._pending = self._pending, {}
-            self.load_state_dict(sd)
+        return DrqConfig(batch_size=batch, channels=c, height=h, action_dim=self.action_dim, bn_dim=self.bn_dim,
+                         hidden_dim=self.hidden_dim, encoder_lr=float(self.args.encoder_lr),
+                         actor_lr=float(self.args.actor_lr), critic_lr=float(self.args.critic_lr), tau=self.tau,
+                         stddev_clip=self.stddev_clip, precision=_lib.PRECISION[self._precision])
 
-    def close(self):
-        h, self._h = self._h, None
-        if h and self.lib is not None:
-            self.lib.rlrep_drq_destroy(h)
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    # ---- weights under the reference's module names ----------------------------------------------------------------
-    def _ref_shape(self, name, rows, cols):
+    @staticmethod
+    def _kind(name):
         if ".convnet." in name and name.endswith("weight"):
-            return (32, cols // 9, 3, 3)
+            return "conv0" if name.endswith("convnet.0.weight") else "conv"
         if name.endswith("bias") or ".trunk.1." in name:
-            return (rows,)
-        return (rows, cols)
-
-    def state_dict(self):
-        if self._h is None:
-            return dict(self._pending)
-        return self._read_all(lambda name: not name.startswith("grad/"))
-
-    def grads(self):
-        """Gradients left by the most recent update (critic / encoder: critic step; actor: actor step), reference names."""
-        return {k[5:]: v for k, v in self._read_all(lambda name: name.startswith("grad/")).items()}
-
-    def _read_all(self, keep):
-        sd = {}
-        for name, (i, rows, cols) in self._index.items():
-            if not keep(name):
-                continue
-            out = np.empty(rows * cols, dtype=np.float32)
-            _lib.check(self.lib.rlrep_drq_tensor_read(self._h, i, out.ctypes.data))
-            t = torch.from_numpy(out)
-            if ".convnet." in name and name.endswith("weight") and not name.endswith("convnet.0.weight"):
-                t = t.reshape(32, 3, 3, 32).permute(0, 3, 1, 2).contiguous()  # stored (ky, kx, c) -> reference (c, ky, kx)
-            sd[name] = t.reshape(self._ref_shape(name, rows, cols))
-        return sd
-
-    def load_state_dict(self, sd, sync_targets=None):
-        if self._h is None:
-            self._pending.update({k: torch.as_tensor(v).detach().clone() for k, v in sd.items()})
-            return
-        for k, v in sd.items():
-            i, rows, cols = self._index[k]
-            t = torch.as_tensor(v).detach().cpu().float()
-            if tuple(t.shape) != self._ref_shape(k, rows, cols):
-                raise ValueError(f"{k}: expected {self._ref_shape(k, rows, cols)}, got {tuple(t.shape)}")
-            if ".convnet." in k and k.endswith("weight") and not k.endswith("convnet.0.weight"):
-                t = t.permute(0, 2, 3, 1)
-            arr = np.ascontiguousarray(t.reshape(-1).numpy())
-            _lib.check(self.lib.rlrep_drq_tensor_write(self._h, i, arr.ctypes.data))
-        if sync_targets or (sync_targets is None and not any(k.startswith("critic_target.") for k in sd)):
-            _lib.check(self.lib.rlrep_drq_sync_targets(self._h))
-
-    @property
-    def gpu_launches_last_update(self):
-        v = C.c_int()
-        _lib.check(self.lib.rlrep_drq_last_launches(self._h, C.byref(v)))
-        return v.value
+            return "vec"
+        return "mat"
 
     # ---- reference surface ---------------------------------------------------------------------------------------
     def _draw(self, n):
@@ -455,18 +500,7 @@ class DrQv2:
         select_action calls advance it."""
         if self._h is None:
             raise _lib.RlrepError("call prepare(batch_size) or train_step once before select_action")
-        keep, ptr, n = _obs_batch(obs, self.obs_dim)
-        stddev = float(self.stddev_schedule(step))
-        eps, _ = _act_noise(n, self.action_dim, sample=not deterministic)
-        out = np.empty((n, self.action_dim), dtype=np.float32)
-        _lib.check(self.lib.rlrep_drq_act_batch(self._h, ptr, eps.ctypes.data if eps is not None else None, stddev, n,
-                                                out.ctypes.data))
-        del keep
-        return out
-
-    def prepare(self, batch_size):
-        """Create the device handle for `batch_size` ahead of the first train_step."""
-        self._ensure(int(batch_size))
+        return self._act_batch(obs, self.obs_dim, step, sample=not deterministic)[0]
 
     def train_step(self, replay_iter, step):
         self._step += 1
@@ -504,7 +538,7 @@ def _cfg_get(cfg, key, default=None):
     return getattr(cfg, key, default)
 
 
-class MuLVDrQv2:
+class MuLVDrQv2(_PixelAgent):
     """Drop-in for the update path of agent.mulvdrq.drqv2.DrQV2Agent (drqv2.py:198-461): same constructor
     (`obs_shape`, `action_shape`, `cfg` -- the attribute dict of mulv_config.py) and `update(replay_iter, step)`.  Only
     the shipped configuration path is built (aug, no pre_aug, back_q2feat, tanh heads, ReLU critic, Huber loss,
@@ -512,6 +546,8 @@ class MuLVDrQv2:
     as in the reference: (img uint8 [B, 9, 84, 84], action, reward, discount, next_img, img_step1)."""
 
     METRICS = ("critic_loss", "critic_q1", "critic_q2", "critic_target_q", "s_loss", "r_loss", "kl_loss", "actor_loss")
+    _PREFIX = "mulv"
+    OUTCONV_SHAPE = (3, 32, 2, 2)
 
     def __init__(self, obs_shape, action_shape, cfg, *, precision="tf32"):
         get = lambda k, d=None: _cfg_get(cfg, k, d)
@@ -520,60 +556,22 @@ class MuLVDrQv2:
                                          ("l2_norm", 0.0)) if get(k, want) != want]
         if unsupported or not float(get("c_targ_tau", 0.01)) < 1.0:
             raise NotImplementedError(f"only mulv_config.py's default path is built (differs in: {unsupported})")
+        super().__init__(precision)
         self.cfg = cfg
         self.obs_shape = tuple(int(x) for x in obs_shape)
         self.action_dim = int(action_shape[0])
         self.up_every = int(get("up_every", 2))
         self.stddev_schedule = _schedule(get("stddev_schedule", "linear(1.0,0.1,500000)"))
         self.feat_dim, self.hidden_dim, self.num_noise = int(get("feat_dim", 100)), int(get("hid_dim", 1024)), 20
-        self._precision = precision
-        self.lib = None
-        self._h = None
-        self._batch = None
-        self._pending = {}
 
-    def _ensure(self, batch):
-        if self._h is not None:
-            if batch != self._batch:
-                raise _lib.RlrepError(f"batch size is fixed per handle (was {self._batch}, got {batch})")
-            return
-        if not torch.cuda.is_available():
-            raise _lib.RlrepError("rlrep_b200.MuLVDrQv2 needs a CUDA device (there is no CPU fallback)")
-        self.lib = _lib.load()
+    def _config(self, batch):
         get = lambda k, d: _cfg_get(self.cfg, k, d)
         c, h, _ = self.obs_shape
-        cfg = MulvConfig(batch_size=batch, channels=c, height=h, action_dim=self.action_dim, feat_dim=self.feat_dim,
-                         hidden_dim=self.hidden_dim, num_noise=self.num_noise, lr=float(get("lr", 1e-4)),
-                         tau=float(get("c_targ_tau", 0.01)), stddev_clip=float(get("stddev_clip", 0.3)),
-                         vae_w=float(get("vae_w", 0.5)), mse_w=float(get("mse_w", 1.0)), c_noise=float(get("c_noise", 0.1)),
-                         precision=_lib.PRECISION[self._precision])
-        hd = C.c_void_p()
-        _lib.check(self.lib.rlrep_mulv_create(C.byref(cfg), None, C.byref(hd)))
-        self._h, self._batch = hd, batch
-        n = C.c_int()
-        _lib.check(self.lib.rlrep_mulv_num_tensors(hd, C.byref(n)))
-        self._index = {}
-        for i in range(n.value):
-            name, ptr, rows, cols = C.c_char_p(), C.c_void_p(), C.c_int(), C.c_int()
-            _lib.check(self.lib.rlrep_mulv_tensor_info(hd, i, C.byref(name), C.byref(ptr), C.byref(rows), C.byref(cols)))
-            self._index[name.value.decode()] = (i, rows.value, cols.value)
-        if self._pending:
-            sd, self._pending = self._pending, {}
-            self.load_state_dict(sd)
-
-    def prepare(self, batch_size):
-        self._ensure(int(batch_size))
-
-    def close(self):
-        h, self._h = self._h, None
-        if h and self.lib is not None:
-            self.lib.rlrep_mulv_destroy(h)
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
+        return MulvConfig(batch_size=batch, channels=c, height=h, action_dim=self.action_dim, feat_dim=self.feat_dim,
+                          hidden_dim=self.hidden_dim, num_noise=self.num_noise, lr=float(get("lr", 1e-4)),
+                          tau=float(get("c_targ_tau", 0.01)), stddev_clip=float(get("stddev_clip", 0.3)),
+                          vae_w=float(get("vae_w", 0.5)), mse_w=float(get("mse_w", 1.0)),
+                          c_noise=float(get("c_noise", 0.1)), precision=_lib.PRECISION[self._precision])
 
     # ---- weights under the reference's module names ----------------------------------------------------------------
     @staticmethod
@@ -589,59 +587,6 @@ class MuLVDrQv2:
                 return "vec"
             return "mat"
         return "vec"
-
-    def _ref_shape(self, name, rows, cols):
-        return {"outconv": (3, 32, 2, 2), "deconv": (32, 32, 3, 3), "conv0": (32, cols // 9, 3, 3),
-                "conv": (32, cols // 9, 3, 3), "vec": (rows,), "mat": (rows, cols)}[self._kind(name)]
-
-    def _read_all(self, keep):
-        sd = {}
-        for name, (i, rows, cols) in self._index.items():
-            if not keep(name):
-                continue
-            out = np.empty(rows * cols, dtype=np.float32)
-            _lib.check(self.lib.rlrep_mulv_tensor_read(self._h, i, out.ctypes.data))
-            t, kind = torch.from_numpy(out), self._kind(name)
-            if kind == "conv":      # stored [32, (ky, kx, c)] -> reference [32, c, ky, kx]
-                t = t.reshape(32, 3, 3, 32).permute(0, 3, 1, 2).contiguous()
-            elif kind == "deconv":  # stored [(ky, kx, c_out), c_in] -> reference [c_in, c_out, ky, kx]
-                t = t.reshape(3, 3, 32, 32).permute(3, 2, 0, 1).contiguous()
-            sd[name] = t.reshape(self._ref_shape(name, rows, cols))
-        return sd
-
-    def state_dict(self):
-        if self._h is None:
-            return dict(self._pending)
-        return self._read_all(lambda name: not name.startswith("grad/"))
-
-    def grads(self):
-        """Gradients left by the most recent update (actor: actor step; everything else: the model/critic step)."""
-        return {k[5:]: v for k, v in self._read_all(lambda name: name.startswith("grad/")).items()}
-
-    def load_state_dict(self, sd, sync_targets=None):
-        if self._h is None:
-            self._pending.update({k: torch.as_tensor(v).detach().clone() for k, v in sd.items()})
-            return
-        for k, v in sd.items():
-            i, rows, cols = self._index[k]
-            t = torch.as_tensor(v).detach().cpu().float()
-            if tuple(t.shape) != self._ref_shape(k, rows, cols):
-                raise ValueError(f"{k}: expected {self._ref_shape(k, rows, cols)}, got {tuple(t.shape)}")
-            kind = self._kind(k)
-            if kind == "conv":
-                t = t.permute(0, 2, 3, 1)
-            elif kind == "deconv":
-                t = t.permute(2, 3, 1, 0)
-            arr = np.ascontiguousarray(t.reshape(-1).numpy())
-            _lib.check(self.lib.rlrep_mulv_tensor_write(self._h, i, arr.ctypes.data))
-        if sync_targets or (sync_targets is None and not any("_target." in k for k in sd)):
-            _lib.check(self.lib.rlrep_mulv_sync_targets(self._h))
-
-    @property
-    def gpu_launches_last_update(self):
-        v = C.c_int()
-        _lib.check(self.lib.rlrep_mulv_last_launches(self._h, C.byref(v)))
-        return v.value
 
     # ---- reference surface ---------------------------------------------------------------------------------------
     def _draw(self, n):
@@ -671,14 +616,8 @@ class MuLVDrQv2:
         is bit-identical to `act(obs[i])`, and the generator advances exactly as N consecutive act calls advance it."""
         if self._h is None:
             raise _lib.RlrepError("call prepare(batch_size) or update once before act")
-        keep, ptr, n = _obs_batch(obs, self.obs_shape)
-        stddev = float(self.stddev_schedule(step))
         explore = not eval_mode and step < int(_cfg_get(self.cfg, "num_expl_steps", 2000))
-        eps, uni = _act_noise(n, self.action_dim, sample=not eval_mode, explore=explore)
-        out = np.empty((n, self.action_dim), dtype=np.float32)
-        _lib.check(self.lib.rlrep_mulv_act_batch(self._h, ptr, eps.ctypes.data if eps is not None else None, stddev, n,
-                                                 out.ctypes.data))
-        del keep
+        out, uni = self._act_batch(obs, self.obs_shape, step, sample=not eval_mode, explore=explore)
         return uni if explore else out
 
     def update(self, replay_iter, step):
@@ -701,10 +640,6 @@ class MuLVDrQv2:
         return {k: float(v) for k, v in zip(self.METRICS, m)}
 
 
-# ======================================================================================================================
-# DRAFT (branch draft/ldiffsr-agent): host mirror of agent/diffsrdrq/latent_diff_sr.py:LatentDiffSRDrQv2.  The device path
-# behind it (csrc/agent_ldiffsr.cu) compiles but has NOT been run on hardware yet; the RNG bookkeeping below is checked on
-# the CPU against the oracle (tests/test_host_logic.py).
 class LdiffConfig(C.Structure):
     """Mirror of `rlrep_ldiff_config` (include/rlrep_b200.h)."""
     _fields_ = [("batch_size", C.c_int), ("action_dim", C.c_int), ("latent_dim", C.c_int), ("feature_dim", C.c_int),
@@ -721,11 +656,13 @@ class LdiffInputs(C.Structure):
                [("stddev", C.c_float)]
 
 
-class LatentDiffSRDrQv2:
+class LatentDiffSRDrQv2(_PixelAgent):
     """Drop-in for the update path of agent.diffsrdrq.latent_diff_sr.LatentDiffSRDrQv2: same constructor
     (`obs_space`, `action_space`, `args`) and `train_step(replay_iter, step)` with the reference's metric keys.  Only
     configs/latent_diff_sr.yaml's path is built (use_repr_target, back_critic_grad, critic_loss mse, reg_coef 0,
     grad_norm null, extra_repr_step 1, do_scale false, repr_coef 1, ae_lr == score_lr)."""
+    _PREFIX = "ldiff"
+    OUTCONV_SHAPE = (3, 32, 3, 3)
 
     def __init__(self, obs_space, action_space, args, *, precision="tf32"):
         a = args
@@ -735,6 +672,7 @@ class LatentDiffSRDrQv2:
                                  ("noise_schedule", "linear")) if getattr(a, k, want) != want]
         if bad or float(a.ae_lr) != float(a.score_lr) or a.bn_dim is None:
             raise NotImplementedError(f"only configs/latent_diff_sr.yaml's path is built (differs in: {bad})")
+        super().__init__(precision)
         self.args = a
         self.obs_dim = tuple(int(x) for x in obs_space.shape)
         if self.obs_dim != (9, 84, 84):
@@ -748,18 +686,7 @@ class LatentDiffSRDrQv2:
         betas = np.linspace(float(a.noise_param1), float(a.noise_param2), int(a.num_noises))  # util.py:118-134
         self.alphabars = torch.as_tensor(np.cumprod(1 - betas, axis=0), dtype=torch.float32)
         self.num_noises = int(a.num_noises)
-        self._precision = precision
         self._step = 1
-        self.lib = None
-        self._h = None
-        self._batch = None
-        self._pending = {}
-
-    @property
-    def gpu_launches_last_update(self):
-        v = C.c_int()
-        _lib.check(self.lib.rlrep_ldiff_last_launches(self._h, C.byref(v)))
-        return v.value
 
     def _draw(self, n):
         """RNG consumption of one updating train_step in the reference's order (oracle/ldiffsr_oracle.py header)."""
@@ -783,34 +710,15 @@ class LatentDiffSRDrQv2:
                     psi_masks=torch.stack([torch.cat([s, c]) for s, c in zip(psi_score, psi_critic)]).numpy(),
                     zeta_masks=torch.stack(zeta).numpy(), eps_act=torch.stack(eps_act).numpy())
 
-    def _ensure(self, batch):
-        if self._h is not None:
-            if batch != self._batch:
-                raise _lib.RlrepError(f"batch size is fixed per handle (was {self._batch}, got {batch})")
-            return
-        if not torch.cuda.is_available():
-            raise _lib.RlrepError("rlrep_b200.LatentDiffSRDrQv2 needs a CUDA device (there is no CPU fallback)")
-        self.lib = _lib.load()
+    def _config(self, batch):
         a = self.args
-        cfg = LdiffConfig(batch_size=batch, action_dim=self.action_dim, latent_dim=self.L, feature_dim=self.feat,
-                          bn_dim=int(a.bn_dim), psi_hidden_dim=self.psi[0], psi_hidden_depth=self.psi[1],
-                          zeta_hidden_dim=self.zeta[0], zeta_hidden_depth=self.zeta[1], hidden_dim=int(a.actor_hidden_dim),
-                          ae_lr=float(a.ae_lr), score_lr=float(a.score_lr), actor_lr=float(a.actor_lr),
-                          critic_lr=float(a.critic_lr), weight_decay=0.01, tau=float(a.tau), kl_coef=float(a.kl_coef),
-                          ae_coef=float(a.ae_coef), stddev_clip=float(a.stddev_clip), precision=_lib.PRECISION[self._precision])
-        hd = C.c_void_p()
-        _lib.check(self.lib.rlrep_ldiff_create(C.byref(cfg), None, C.byref(hd)))
-        self._h, self._batch = hd, batch
-        n = C.c_int()
-        _lib.check(self.lib.rlrep_ldiff_num_tensors(hd, C.byref(n)))
-        self._index = {}
-        for i in range(n.value):
-            name, ptr, rows, cols = C.c_char_p(), C.c_void_p(), C.c_int(), C.c_int()
-            _lib.check(self.lib.rlrep_ldiff_tensor_info(hd, i, C.byref(name), C.byref(ptr), C.byref(rows), C.byref(cols)))
-            self._index[name.value.decode()] = (i, rows.value, cols.value)
-        if self._pending:
-            sd, self._pending = self._pending, {}
-            self.load_state_dict(sd)
+        return LdiffConfig(batch_size=batch, action_dim=self.action_dim, latent_dim=self.L, feature_dim=self.feat,
+                           bn_dim=int(a.bn_dim), psi_hidden_dim=self.psi[0], psi_hidden_depth=self.psi[1],
+                           zeta_hidden_dim=self.zeta[0], zeta_hidden_depth=self.zeta[1],
+                           hidden_dim=int(a.actor_hidden_dim), ae_lr=float(a.ae_lr), score_lr=float(a.score_lr),
+                           actor_lr=float(a.actor_lr), critic_lr=float(a.critic_lr), weight_decay=0.01, tau=float(a.tau),
+                           kl_coef=float(a.kl_coef), ae_coef=float(a.ae_coef), stddev_clip=float(a.stddev_clip),
+                           precision=_lib.PRECISION[self._precision])
 
     @staticmethod
     def _kind(name):
@@ -825,44 +733,6 @@ class LatentDiffSRDrQv2:
                 return "vec"
             return "mat"
         return "vec"
-
-    def _ref_shape(self, name, rows, cols):
-        return {"outconv": (3, 32, 3, 3), "deconv": (32, 32, 3, 3), "conv0": (32, cols // 9, 3, 3), "conv": (32, cols // 9, 3, 3),
-                "vec": (rows,), "mat": (rows, cols)}[self._kind(name)]
-
-    def state_dict(self):
-        if self._h is None:
-            return dict(self._pending)
-        sd = {}
-        for name, (i, rows, cols) in self._index.items():
-            if name.startswith("grad/"):
-                continue
-            out = np.empty(rows * cols, dtype=np.float32)
-            _lib.check(self.lib.rlrep_ldiff_tensor_read(self._h, i, out.ctypes.data))
-            t, kind = torch.from_numpy(out), self._kind(name)
-            if kind == "conv":
-                t = t.reshape(32, 3, 3, 32).permute(0, 3, 1, 2).contiguous()
-            elif kind == "deconv":
-                t = t.reshape(3, 3, 32, 32).permute(3, 2, 0, 1).contiguous()
-            sd[name] = t.reshape(self._ref_shape(name, rows, cols))
-        return sd
-
-    def load_state_dict(self, sd, sync_targets=None):
-        if self._h is None:
-            self._pending.update({k: torch.as_tensor(v).detach().clone() for k, v in sd.items()})
-            return
-        for k, v in sd.items():
-            i, rows, cols = self._index[k]
-            t = torch.as_tensor(v).detach().cpu().float()
-            kind = self._kind(k)
-            if kind == "conv":
-                t = t.permute(0, 2, 3, 1)
-            elif kind == "deconv":
-                t = t.permute(2, 3, 1, 0)
-            arr = np.ascontiguousarray(t.reshape(-1).numpy())
-            _lib.check(self.lib.rlrep_ldiff_tensor_write(self._h, i, arr.ctypes.data))
-        if sync_targets or (sync_targets is None and not any("_target." in k for k in sd)):
-            _lib.check(self.lib.rlrep_ldiff_sync_targets(self._h))
 
     def train_step(self, replay_iter, step):
         self._step += 1

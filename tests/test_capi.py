@@ -52,3 +52,25 @@ def test_no_cpu_fallback(lib):
     agent = SACAgent(17, 6, Sp(), hidden_dim=32)  # construction is lazy; the first call that needs the device raises
     with pytest.raises(RlrepError):
         agent.select_action(np.zeros(17))
+
+
+def _handle_entry_points():
+    pixel = [n for n in declared_symbols() if re.match(r"rlrep_(drq|mulv|ldiff)_", n) and not n.endswith("_create")]
+    return pixel + ["rlrep_agent_num_tensors", "rlrep_agent_tensor_info", "rlrep_agent_tensor_read",
+                    "rlrep_agent_tensor_write"]
+
+
+@pytest.mark.parametrize("name", _handle_entry_points())
+def test_null_handle_is_an_error_not_a_crash(lib, name):
+    """Every entry point that takes a pixel-agent handle, and the state agents' tensor accessors, reject a NULL handle
+    with an error code and message before touching the device; destroying NULL is a no-op."""
+    from rlrep_b200 import _lib
+    fn = getattr(_lib.load(), name)
+    args = [0.0 if t in (C.c_float, C.c_double) else 0 if t in (C.c_int, C.c_longlong) else None for t in fn.argtypes]
+    # leave a different message behind first, so the one checked below is this call's
+    assert lib.rlrep_agent_create_sharded(None, None, None, None) != 0
+    if name.endswith("_destroy"):
+        assert fn(*args) == 0
+    else:
+        assert fn(*args) != 0
+        assert b"null argument" in lib.rlrep_last_error()

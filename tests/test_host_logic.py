@@ -215,7 +215,7 @@ def test_implicit_convolution_algebra():
 
 
 def test_latent_diffsr_draw_consumes_the_generator_like_the_reference():
-    """DRAFT shim (branch draft/ldiffsr-agent): the host-side randomness of one updating train_step -- shifts, posterior
+    """Latent Diff-SR DrQ-v2 shim: the host-side randomness of one updating train_step -- shifts, posterior
     noise, diffusion levels / noise, the dropout masks of the online score network (drawn as Bernoulli(0.9) tensors, which
     is what F.dropout consumes), the action normals -- leaves the CPU generator exactly where the oracle (bit-identical
     to the reference class, tests/golden/ldiffsr_b4.npz) leaves it, and the masks are the ones the oracle applied."""
