@@ -351,6 +351,14 @@ RLREP_EXPORT int rlrep_drq_update_resident(rlrep_drq* drq, int n_steps, float st
 RLREP_EXPORT int rlrep_drq_profile_update(rlrep_drq* drq, float stddev, int max_entries, const char** names, float* ms,
                                           double* bytes, double* flops, int* n_entries);
 RLREP_EXPORT int rlrep_drq_last_launches(rlrep_drq* drq, int* launches);
+/* Optimiser state that is not a tensor, for checkpoints.  The handle's tensor index also lists the Adam moments of every
+ * parameter as "optim.m/<name>" / "optim.v/<name>" (same shape and layout as the parameter; torch.optim.Adam's exp_avg /
+ * exp_avg_sq), and with these counters they let a resumed handle continue bit-identically.  The pixel agents' counters are
+ * the Adam step counts: here t_feature counts the encoder's optimiser, t_critic the critic's, t_actor the actor's.  They
+ * have no `steps` gate and no temperature: steps, t_alpha and log_alpha* read as 0, and set refuses non-zero values in
+ * them.  Set takes effect at the next update (the Adam bias corrections are recomputed from the counters every update). */
+RLREP_EXPORT int rlrep_drq_get_optim_state(rlrep_drq* drq, rlrep_optim_state* out);
+RLREP_EXPORT int rlrep_drq_set_optim_state(rlrep_drq* drq, const rlrep_optim_state* in);
 
 /* ------------------------------------------------------------------------------------------------
  * muLV-Rep DrQ-v2 pixel agent -- replaces `DrQV2Agent(obs_shape, action_shape, cfg)` and the updating half of
@@ -398,6 +406,11 @@ RLREP_EXPORT int rlrep_mulv_update_resident(rlrep_mulv* h, int n_steps, float st
 RLREP_EXPORT int rlrep_mulv_profile_update(rlrep_mulv* h, float stddev, int max_entries, const char** names, float* ms,
                                            double* bytes, double* flops, int* n_entries);
 RLREP_EXPORT int rlrep_mulv_last_launches(rlrep_mulv* h, int* launches);
+/* Checkpoint counters with the contract of rlrep_drq_get_optim_state: t_critic is the Adam step count that every
+ * representation and critic group shares (encoder, predict_encoder, decoder, feat_encoder, feat_decoder, feat_f, critic),
+ * t_actor the actor's; t_feature advances with every update and drives no optimiser. */
+RLREP_EXPORT int rlrep_mulv_get_optim_state(rlrep_mulv* h, rlrep_optim_state* out);
+RLREP_EXPORT int rlrep_mulv_set_optim_state(rlrep_mulv* h, const rlrep_optim_state* in);
 
 /* ------------------------------------------------------------------------------------------------
  * Latent Diff-SR DrQ-v2 pixel agent -- replaces
@@ -444,6 +457,11 @@ RLREP_EXPORT int rlrep_ldiff_update_resident(rlrep_ldiff* h, int n_steps, float 
 RLREP_EXPORT int rlrep_ldiff_profile_update(rlrep_ldiff* h, float stddev, int max_entries, const char** names, float* ms,
                                             double* bytes, double* flops, int* n_entries);
 RLREP_EXPORT int rlrep_ldiff_last_launches(rlrep_ldiff* h, int* launches);
+/* Checkpoint counters with the contract of rlrep_drq_get_optim_state: t_feature counts the VAE's and the score network's
+ * optimisers (one step count, like their one learning rate), t_critic the critic's, t_actor the actor's.  The score
+ * blocks' unused `residual` layers have no optimiser state and no "optim.*" entries. */
+RLREP_EXPORT int rlrep_ldiff_get_optim_state(rlrep_ldiff* h, rlrep_optim_state* out);
+RLREP_EXPORT int rlrep_ldiff_set_optim_state(rlrep_ldiff* h, const rlrep_optim_state* in);
 
 /* Kernels launched by the most recent train() (a graph replay counts the kernels it contains). */
 /* Batched policy evaluation (utils/util.py:40-57 `eval_policy` over vectorised environments, or any caller that has many

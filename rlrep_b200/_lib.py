@@ -167,6 +167,8 @@ def _declare(lib: C.CDLL) -> None:
             f"rlrep_{prefix}_profile_update": [vp, C.c_float, i, C.POINTER(C.c_char_p), C.POINTER(C.c_float),
                                                C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(i)],
             f"rlrep_{prefix}_last_launches": [vp, C.POINTER(i)],
+            f"rlrep_{prefix}_get_optim_state": [vp, C.POINTER(OptimState)],
+            f"rlrep_{prefix}_set_optim_state": [vp, C.POINTER(OptimState)],
         })
     lib.rlrep_agent_metric_name.argtypes = [vp, i]
     lib.rlrep_agent_metric_name.restype = C.c_char_p

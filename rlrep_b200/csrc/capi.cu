@@ -176,7 +176,8 @@ struct rlrep_ldiff : PixelHandle {
 
 // The agent runs on `stream`, or on a stream of its own when that is null.  Its tensors are indexed group by group under
 // the reference's names: the parameters, their gradients of the most recent update ("grad/<name>", for gradient-level
-// parity tests), then the target copies.
+// parity tests), the Adam moments of groups that have an optimiser ("optim.m/<name>", "optim.v/<name>": with
+// rlrep_<agent>_get/set_optim_state they make a checkpoint resume bit-identically), then the target copies.
 template <class Handle, class Impl, class Config>
 static Handle* create_pixel(const Config& c, void* stream) {
   std::unique_ptr<Handle> h(new Handle);
@@ -196,6 +197,10 @@ static Handle* create_pixel(const Config& c, void* stream) {
     };
     add(g->p, "", "");
     if (g->g) add(g->g, "", "grad/");
+    if (g->m && g->v) {
+      add(g->m, "", "optim.m/");
+      add(g->v, "", "optim.v/");
+    }
     if (g->target) add(g->target, g->target_prefix_from, g->target_prefix_to);
   }
   return h.release();
@@ -261,6 +266,35 @@ static int pixel_last_launches(PixelHandle* h, int* launches) {
   RLREP_API_BEGIN_ON(h)
   RLREP_CHECK(h && launches, "null argument");
   *launches = h->impl->last_launches;
+  RLREP_API_END
+}
+// The pixel agents' optimiser counters are the three Adam step counters of the control block; they have no `steps`
+// gate and no temperature, so those fields read as 0 and a non-zero value for them is refused.
+static int pixel_get_optim_state(PixelHandle* h, rlrep_optim_state* out) {
+  RLREP_API_BEGIN_ON(h)
+  RLREP_CHECK(h && out, "null argument");
+  Control c;
+  cudaStream_t st = h->impl->stream();
+  RLREP_CUDA(cudaMemcpyAsync(&c, h->impl->control(), sizeof(c), cudaMemcpyDeviceToHost, st));
+  RLREP_CUDA(cudaStreamSynchronize(st));
+  *out = rlrep_optim_state{};
+  out->t_feature = c.t_feat; out->t_critic = c.t_critic; out->t_actor = c.t_actor;
+  RLREP_API_END
+}
+static int pixel_set_optim_state(PixelHandle* h, const rlrep_optim_state* in) {
+  RLREP_API_BEGIN_ON(h)
+  RLREP_CHECK(h && in, "null argument");
+  RLREP_CHECK(in->steps == 0 && in->t_alpha == 0 && in->log_alpha == 0.0 && in->log_alpha_m == 0.0 &&
+                  in->log_alpha_v == 0.0,
+              "pixel agents have no steps gate and no temperature: steps, t_alpha and log_alpha* must be 0");
+  RLREP_CHECK(in->t_feature >= 0 && in->t_critic >= 0 && in->t_actor >= 0, "Adam step counters must be non-negative");
+  Control c;
+  cudaStream_t st = h->impl->stream();
+  RLREP_CUDA(cudaMemcpyAsync(&c, h->impl->control(), sizeof(c), cudaMemcpyDeviceToHost, st));
+  RLREP_CUDA(cudaStreamSynchronize(st));
+  c.t_feat = in->t_feature; c.t_critic = in->t_critic; c.t_actor = in->t_actor;
+  RLREP_CUDA(cudaMemcpyAsync(h->impl->control(), &c, sizeof(c), cudaMemcpyHostToDevice, st));
+  RLREP_CUDA(cudaStreamSynchronize(st));
   RLREP_API_END
 }
 
@@ -755,6 +789,10 @@ int rlrep_drq_profile_update(rlrep_drq* drq, float stddev, int max_entries, cons
   return pixel_profile_update(drq, stddev, max_entries, names, ms, bytes, flops, n_entries);
 }
 int rlrep_drq_last_launches(rlrep_drq* drq, int* launches) { return pixel_last_launches(drq, launches); }
+int rlrep_drq_get_optim_state(rlrep_drq* drq, rlrep_optim_state* out) { return pixel_get_optim_state(drq, out); }
+int rlrep_drq_set_optim_state(rlrep_drq* drq, const rlrep_optim_state* in) {
+  return pixel_set_optim_state(drq, in);
+}
 
 int rlrep_mulv_create(const rlrep_mulv_config* c, void* stream, rlrep_mulv** out) {
   RLREP_API_BEGIN
@@ -805,6 +843,10 @@ int rlrep_mulv_profile_update(rlrep_mulv* h, float stddev, int max_entries, cons
   return pixel_profile_update(h, stddev, max_entries, names, ms, bytes, flops, n_entries);
 }
 int rlrep_mulv_last_launches(rlrep_mulv* h, int* launches) { return pixel_last_launches(h, launches); }
+int rlrep_mulv_get_optim_state(rlrep_mulv* h, rlrep_optim_state* out) { return pixel_get_optim_state(h, out); }
+int rlrep_mulv_set_optim_state(rlrep_mulv* h, const rlrep_optim_state* in) {
+  return pixel_set_optim_state(h, in);
+}
 
 int rlrep_ldiff_create(const rlrep_ldiff_config* c, void* stream, rlrep_ldiff** out) {
   RLREP_API_BEGIN
@@ -847,6 +889,10 @@ int rlrep_ldiff_profile_update(rlrep_ldiff* h, float stddev, int max_entries, co
   return pixel_profile_update(h, stddev, max_entries, names, ms, bytes, flops, n_entries);
 }
 int rlrep_ldiff_last_launches(rlrep_ldiff* h, int* launches) { return pixel_last_launches(h, launches); }
+int rlrep_ldiff_get_optim_state(rlrep_ldiff* h, rlrep_optim_state* out) { return pixel_get_optim_state(h, out); }
+int rlrep_ldiff_set_optim_state(rlrep_ldiff* h, const rlrep_optim_state* in) {
+  return pixel_set_optim_state(h, in);
+}
 
 // ------------------------------------------------------------------------------------------------ communicator
 // ------------------------------------------------------------------------------------------------ pixel replay ring

@@ -48,7 +48,6 @@ class DrqV2 : public PixelAgent {
   ParamGroup crit_g_, actor_g_;
   LinearSlot ct_, q0_, q1a_, q1b_, q2a_, q2b_, at_, p0_, p1_, p2_;
   size_t cln_w_ = 0, cln_b_ = 0, aln_w_ = 0, aln_b_ = 0;
-  Control* ctl_ = nullptr;
   unsigned char *img_dev_ = nullptr, *next_img_dev_ = nullptr;
   int* shifts_dev_ = nullptr;
   float *eps_dev_ = nullptr, *action_dev_ = nullptr, *reward_dev_ = nullptr, *discount_dev_ = nullptr;

@@ -96,7 +96,6 @@ class LatentDiffSR : public PixelAgent {
   BottleneckSlots bneck_;
   ResNetSlots psi_, zeta_;
   RffCritic rff_;
-  Control* ctl_ = nullptr;
   unsigned char *frames_dev_ = nullptr, *next_frames_dev_ = nullptr;
   int *shifts_dev_ = nullptr, *next_shifts_dev_ = nullptr;
   float *action_dev_ = nullptr, *reward_dev_ = nullptr, *discount_dev_ = nullptr, *eps_post_dev_ = nullptr, *ab_dev_ = nullptr;

@@ -70,7 +70,6 @@ class MulvDrq : public PixelAgent {
   GaussHead fe_, ff_;
   LinearSlot at_, p0_, p1_, p2_, c14_, c2_, c5_, c3_, c6_, d1_, d2_, ds_, dr_;
   size_t aln_w_ = 0, aln_b_ = 0;
-  Control* ctl_ = nullptr;
   unsigned char *img_dev_ = nullptr, *next_img_dev_ = nullptr, *step1_dev_ = nullptr;
   int* shifts_dev_ = nullptr;
   float *eps_z_dev_ = nullptr, *eps_act_dev_ = nullptr, *noise_dev_ = nullptr, *action_dev_ = nullptr;

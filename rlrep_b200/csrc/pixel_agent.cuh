@@ -33,6 +33,9 @@ class PixelAgent {
   // target <- params of every group that has a Polyak target (after loading weights)
   void sync_targets_from_params();
   cudaStream_t stream() const { return stream_; }
+  // The Adam step counters (t_feat, t_critic, t_actor) are the optimiser state that is not a tensor: the tick at the head
+  // of every update derives that update's bias corrections from them, so writing them is all a resume needs.
+  Control* control() const { return ctl_; }
   int last_launches = 0;
 
  protected:
@@ -46,6 +49,7 @@ class PixelAgent {
   void finish_update(float stddev, float* metrics_out, int n_metrics);
 
   cudaStream_t stream_;
+  Control* ctl_ = nullptr;        // in the agent's arena
   float* metrics_dev_ = nullptr;  // [kMetrics], in the agent's arena
   unsigned char* stage_host_ = nullptr;
   float* metrics_host_ = nullptr;

@@ -299,9 +299,12 @@ class ConvDecoder:
 
 class _PixelAgent:
     """What the pixel agents share: the device handle behind `rlrep_<_PREFIX>_*`, created by the first call that needs
-    it, its tensor index, and the weights and gradients under the reference's module names.  Subclasses set `_PREFIX`,
-    `_config(batch)` (the ctypes config of the handle) and `_kind(name)`, the layout class of a tensor name."""
+    it, its tensor index, the weights and gradients under the reference's module names, and checkpoints.  Subclasses set
+    `_PREFIX`, `_ALG` (the checkpoint's `alg`), `_config(batch)` (the ctypes config of the handle), `_kind(name)`, the
+    layout class of a tensor name, and `_step` when they keep the reference's host step counter."""
     _PREFIX = None
+    _ALG = None
+    _step = None
     OUTCONV_SHAPE = None  # reference shape of the decoder's output convolution, if the agent has one
 
     def __init__(self, precision):
@@ -378,11 +381,24 @@ class _PixelAgent:
     def state_dict(self):
         if self._h is None:
             return dict(self._pending)
-        return self._read_all(lambda name: not name.startswith("grad/"))
+        return self._read_all(lambda name: not name.startswith(("grad/", "optim.")))
 
     def grads(self):
         """Gradients left by the most recent update, under the reference's names."""
         return {k[5:]: v for k, v in self._read_all(lambda name: name.startswith("grad/")).items()}
+
+    def _write(self, k, v):
+        i, rows, cols = self._index[k]
+        t = torch.as_tensor(v).detach().cpu().float()
+        if tuple(t.shape) != self._ref_shape(k, rows, cols):
+            raise ValueError(f"{k}: expected {self._ref_shape(k, rows, cols)}, got {tuple(t.shape)}")
+        kind = self._kind(k)
+        if kind == "conv":
+            t = t.permute(0, 2, 3, 1)
+        elif kind == "deconv":
+            t = t.permute(2, 3, 1, 0)
+        arr = np.ascontiguousarray(t.reshape(-1).numpy())
+        _lib.check(self._fn("tensor_write")(self._h, i, arr.ctypes.data))
 
     def load_state_dict(self, sd, sync_targets=None):
         """Targets are copied from the loaded parameters unless `sd` carries them (or `sync_targets` says otherwise)."""
@@ -390,19 +406,73 @@ class _PixelAgent:
             self._pending.update({k: torch.as_tensor(v).detach().clone() for k, v in sd.items()})
             return
         for k, v in sd.items():
-            i, rows, cols = self._index[k]
-            t = torch.as_tensor(v).detach().cpu().float()
-            if tuple(t.shape) != self._ref_shape(k, rows, cols):
-                raise ValueError(f"{k}: expected {self._ref_shape(k, rows, cols)}, got {tuple(t.shape)}")
-            kind = self._kind(k)
-            if kind == "conv":
-                t = t.permute(0, 2, 3, 1)
-            elif kind == "deconv":
-                t = t.permute(2, 3, 1, 0)
-            arr = np.ascontiguousarray(t.reshape(-1).numpy())
-            _lib.check(self._fn("tensor_write")(self._h, i, arr.ctypes.data))
+            self._write(k, v)
         if sync_targets or (sync_targets is None and not any("_target." in k for k in sd)):
             _lib.check(self._fn("sync_targets")(self._h))
+
+    # ---- checkpoints ---------------------------------------------------------------------------------------------
+    def _need_handle(self, what):
+        if self._h is None:
+            raise _lib.RlrepError(f"{what} needs the device handle: call prepare(batch_size) or run an update first")
+
+    def optimizer_state_dict(self, step=None):
+        """Adam moments of every optimised parameter (`optim.m/<name>`, `optim.v/<name>`: torch.optim.Adam's -- for the
+        score network AdamW's -- exp_avg / exp_avg_sq of that parameter, in its reference shape and layout) plus `control`:
+        the three Adam step counters and `agent_step`, the host step counter that gates `update_every`.  `step` is only
+        used by μLV-Rep, which keeps no such counter (its caller owns the step): it becomes `agent_step`, None when not
+        given.  DrQ-v2 and latent Diff-SR save their own `_step` and ignore `step`."""
+        self._need_handle("optimizer_state_dict")
+        sd = self._read_all(lambda name: name.startswith("optim."))
+        st = _lib.OptimState()
+        _lib.check(self._fn("get_optim_state")(self._h, C.byref(st)))
+        sd["control"] = {"t_feature": st.t_feature, "t_critic": st.t_critic, "t_actor": st.t_actor,
+                         "agent_step": self._step if self._step is not None else step}
+        return sd
+
+    def load_optimizer_state_dict(self, sd):
+        """The inverse of optimizer_state_dict: moments are shape-checked like load_state_dict's weights."""
+        self._need_handle("load_optimizer_state_dict")
+        for k, v in sd.items():
+            if k == "control":
+                continue
+            if not k.startswith("optim.") or k not in self._index:
+                raise ValueError(f"{k}: not an optimiser tensor of this agent")
+            self._write(k, v)
+        ctl = sd["control"]
+        st = _lib.OptimState(t_feature=int(ctl["t_feature"]), t_critic=int(ctl["t_critic"]), t_actor=int(ctl["t_actor"]))
+        _lib.check(self._fn("set_optim_state")(self._h, C.byref(st)))
+        if self._step is not None:
+            self._step = int(ctl["agent_step"])
+
+    def save(self, path, step=None):
+        """Checkpoint in the state agents' format (rlrep_b200.agents): a torch.save'd dict with the parameters and Polyak
+        targets under the reference's state_dict names and the optimiser state that makes a resumed run continue
+        bit-identically.  `step` is saved as μLV-Rep's `agent_step` and ignored by the other agents (see
+        optimizer_state_dict)."""
+        self._need_handle("save")
+        torch.save({"format": "rlrep_b200/1", "alg": self._ALG, "obs_shape": self._observation_shape(),
+                    "action_dim": self.action_dim, "batch_size": self._batch, "precision": self._precision,
+                    "state_dict": self.state_dict(), "optimizer": self.optimizer_state_dict(step)}, path)
+
+    def load(self, path, load_optimizer=True):
+        """Restore a checkpoint written by `save`.  An agent without a handle gets one at the checkpoint's batch size; a
+        handle of another batch size is refused (the batch size is fixed per handle).  The precision may differ from the
+        saved one, but then the run does not continue bit-identically.  With load_optimizer=False only the parameters and
+        their saved targets are written: the handle's moments, step counters and host step counter are left as they are
+        (zero on a handle that has not updated yet)."""
+        ck = torch.load(path, map_location="cpu", weights_only=True)
+        if ck.get("format") != "rlrep_b200/1" or ck.get("alg") != self._ALG:
+            raise _lib.RlrepError(f"{path}: not a rlrep_b200 checkpoint of a {self._ALG} agent")
+        if (tuple(ck["obs_shape"]), ck["action_dim"]) != (self._observation_shape(), self.action_dim):
+            raise _lib.RlrepError(f"{path}: saved for observation shape {tuple(ck['obs_shape'])} and action dimension "
+                                  f"{ck['action_dim']}, this agent has {self._observation_shape()} and {self.action_dim}")
+        self._ensure(int(ck["batch_size"]))
+        self.load_state_dict(ck["state_dict"], sync_targets=False)
+        if load_optimizer:
+            self.load_optimizer_state_dict(ck["optimizer"])
+
+    def _observation_shape(self):
+        return self.obs_dim
 
     @property
     def gpu_launches_last_update(self):
@@ -449,6 +519,7 @@ class DrQv2(_PixelAgent):
     iterator as in the reference (img_stack uint8 [B, 9, 84, 84], action, reward, discount, next_img_stack,
     next_img_step)."""
     _PREFIX = "drq"
+    _ALG = "drqv2"
 
     def __init__(self, obs_space, action_space, args, *, precision="tf32"):
         if getattr(args, "critic_loss", "mse") != "mse":
@@ -547,6 +618,7 @@ class MuLVDrQv2(_PixelAgent):
 
     METRICS = ("critic_loss", "critic_q1", "critic_q2", "critic_target_q", "s_loss", "r_loss", "kl_loss", "actor_loss")
     _PREFIX = "mulv"
+    _ALG = "mulvdrq"
     OUTCONV_SHAPE = (3, 32, 2, 2)
 
     def __init__(self, obs_shape, action_shape, cfg, *, precision="tf32"):
@@ -572,6 +644,9 @@ class MuLVDrQv2(_PixelAgent):
                           tau=float(get("c_targ_tau", 0.01)), stddev_clip=float(get("stddev_clip", 0.3)),
                           vae_w=float(get("vae_w", 0.5)), mse_w=float(get("mse_w", 1.0)),
                           c_noise=float(get("c_noise", 0.1)), precision=_lib.PRECISION[self._precision])
+
+    def _observation_shape(self):
+        return self.obs_shape
 
     # ---- weights under the reference's module names ----------------------------------------------------------------
     @staticmethod
@@ -662,6 +737,7 @@ class LatentDiffSRDrQv2(_PixelAgent):
     configs/latent_diff_sr.yaml's path is built (use_repr_target, back_critic_grad, critic_loss mse, reg_coef 0,
     grad_norm null, extra_repr_step 1, do_scale false, repr_coef 1, ae_lr == score_lr)."""
     _PREFIX = "ldiff"
+    _ALG = "ldiffsr"
     OUTCONV_SHAPE = (3, 32, 3, 3)
 
     def __init__(self, obs_space, action_space, args, *, precision="tf32"):
