@@ -73,6 +73,9 @@ typedef struct rlrep_epilogue {
  * phi(s,a) . mu(s')^T (ctrlsac_agent.py:229).
  *   path = 0: tcgen05 TF32 tensor-core kernel (TMA operands: 16-byte aligned bases, ld % 4 == 0)
  *   path = 1: CUDA-core exact-FP32 kernel (any alignment; optional second K segment A2 for cat() inputs)
+ *   path = 2: dispatched as an agent's TF32 GEMM runner does: tensor cores or CUDA cores by shape, and a deep and skinny
+ *             GEMM (K in the tens of thousands, a handful of tiles) cut into K groups whose sum a finishing pass turns
+ *             into C with the epilogue applied; no A2, and bn = split_k = 0
  * bn / split_k = 0 lets the library choose; ws_dev (split-K partials, ws_floats floats) may be NULL.
  */
 RLREP_EXPORT int rlrep_gemm(void* stream, int path, int M, int N, int K, const float* A_dev, int lda, int a_mn,

@@ -205,11 +205,15 @@ def make_epilogue(bias=None, r1=None, aux=None, pre_out=None, act="none", dact="
     return e
 
 
+_GEMM_PATH = {"tc": 0, "simt": 1, "runner": 2}
+
+
 def gemm(A, B, C_out, *, a_mn=False, b_mn=False, path="tc", epi: Epilogue | None = None, A2=None, bn=0, split_k=0,
          ws=None):
     """C = epilogue(sum_k A(m,k) B(n,k)) on torch CUDA tensors (kernel-level entry, used by tests).
 
-    K-major operand: tensor [rows, K]; MN-major operand: tensor [K, rows]."""
+    K-major operand: tensor [rows, K]; MN-major operand: tensor [K, rows].  path = "tc" (tensor cores), "simt" (CUDA
+    cores) or "runner" (dispatched as an agent's TF32 GEMM runner does, K groups for deep and skinny GEMMs included)."""
     lib = load()
     M = A.shape[1] if a_mn else A.shape[0]
     K = A.shape[0] if a_mn else A.shape[1]
@@ -219,7 +223,7 @@ def gemm(A, B, C_out, *, a_mn=False, b_mn=False, path="tc", epi: Epilogue | None
         K += A2.shape[1]
     assert (B.shape[0] if b_mn else B.shape[1]) == K
     epi = epi or make_epilogue()
-    rc = lib.rlrep_gemm(current_stream_ptr(), 0 if path == "tc" else 1, M, N, K, A.data_ptr(), A.stride(0), int(a_mn),
+    rc = lib.rlrep_gemm(current_stream_ptr(), _GEMM_PATH[path], M, N, K, A.data_ptr(), A.stride(0), int(a_mn),
                         A2.data_ptr() if A2 is not None else None, A2.stride(0) if A2 is not None else 0, K1,
                         B.data_ptr(), B.stride(0), int(b_mn), C_out.data_ptr(), C_out.stride(0), C.byref(epi), bn,
                         split_k, ws.data_ptr() if ws is not None else None, ws.numel() if ws is not None else 0)

@@ -46,6 +46,18 @@ Epilogue to_epilogue(const rlrep_epilogue* e) {
 
 using namespace rlrep;
 
+// The TF32 GemmRunner behind rlrep_gemm's path 2 (one per thread, like the chain recorder below): it dispatches exactly as an
+// agent's runner does -- tensor cores or CUDA cores by shape, K groups plus their finishing pass for deep and skinny GEMMs --
+// and keeps its plans and K-group workspace between calls.
+static GemmRunner& gemm_runner() {
+  thread_local std::unique_ptr<GemmRunner> r;
+  if (!r) {
+    r.reset(new GemmRunner());
+    r->init(PREC_TF32, 0);
+  }
+  return *r;
+}
+
 // Calibration kernels for rlrep_gemm_bench (path 2 / 3): an empty kernel, plain and with programmatic dependent
 // launch, to measure the per-launch floor of a dependent kernel chain on this GPU.
 __global__ void null_kernel(float* p) {
@@ -318,6 +330,9 @@ int rlrep_gemm(void* stream, int path, int M, int N, int K, const float* A, int 
   if (path == 0) {
     TcGemmPlan p = make_tc_plan(g, bn, split_k, ws, ws_floats);
     launch_tc(p, st);
+  } else if (path == 2) {
+    RLREP_CHECK(A2 == nullptr && bn == 0 && split_k == 0, "path 2 plans the GEMM itself: no A2, bn or split_k");
+    gemm_runner().run(g, st);
   } else {
     launch_simt(g, st);
   }

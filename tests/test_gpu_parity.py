@@ -17,70 +17,6 @@ pytestmark = pytest.mark.gpu
 HC = dict(S=17, A=6)
 
 
-# ------------------------------------------------------------------------------------------------ GEMM
-@pytest.mark.parametrize("a_mn,b_mn", [(0, 0), (0, 1), (1, 0), (1, 1)])
-@pytest.mark.parametrize("shape", [(256, 2048, 1024), (256, 256, 2048), (2048, 1024, 256), (200, 136, 100),
-                                   (128, 128, 32), (64, 32, 64)])
-def test_gemm_tf32_all_majors(lib, a_mn, b_mn, shape):
-    from rlrep_b200 import _lib
-    M, N, K = shape
-    if a_mn and M % 32:
-        M = (M + 31) // 32 * 32  # MN-major operands are fetched through a (mn % 32, k, mn / 32) TMA view
-    if b_mn and N % 32:
-        N = (N + 31) // 32 * 32
-    torch.manual_seed(0)
-    A = torch.randn((K, M) if a_mn else (M, K), device="cuda")
-    B = torch.randn((K, N) if b_mn else (N, K), device="cuda")
-    bias = torch.randn(N, device="cuda")
-    ws = torch.empty(16 * M * N, device="cuda")
-    ref = torch.nn.functional.elu((A.t() if a_mn else A).double() @ (B.t() if b_mn else B).double().t() + bias.double())
-    for bn, sk in ((0, 0), (32, 1), (64, 2), (128, 1), (256, 1)):
-        C = torch.full((M, N), float("nan"), device="cuda")
-        _lib.gemm(A, B, C, a_mn=bool(a_mn), b_mn=bool(b_mn), path="tc", epi=_lib.make_epilogue(bias=bias, act="elu"),
-                  bn=bn, split_k=sk, ws=ws)
-        err = ((C.double() - ref).norm() / ref.norm()).item()
-        assert err < 1e-3, (bn, sk, err)  # TF32: 10-bit mantissa operands, fp32 accumulate
-
-
-@pytest.mark.parametrize("a_mn,b_mn", [(0, 0), (0, 1), (1, 1)])
-def test_gemm_fp32_cuda_cores(lib, a_mn, b_mn):
-    from rlrep_b200 import _lib
-    torch.manual_seed(1)
-    M, N, K = 100, 23, 300
-    A = torch.randn((K, M) if a_mn else (M, K), device="cuda")
-    B = torch.randn((K, N) if b_mn else (N, K), device="cuda")
-    C = torch.empty((M, N), device="cuda")
-    _lib.gemm(A, B, C, a_mn=bool(a_mn), b_mn=bool(b_mn), path="simt")
-    ref = (A.t() if a_mn else A).double() @ (B.t() if b_mn else B).double().t()
-    assert ((C.double() - ref).norm() / ref.norm()).item() < 1e-5
-
-
-def test_gemm_tf32_rejects_unfetchable_operands(lib):
-    from rlrep_b200 import _lib
-    A, B, C = torch.randn(64, 100, device="cuda"), torch.randn(64, 72, device="cuda"), torch.empty(100, 72, device="cuda")
-    with pytest.raises(_lib.RlrepError):  # MN-major with mn % 32 != 0 must be refused loudly (CUDA-core path handles it)
-        _lib.gemm(A, B, C, a_mn=True, b_mn=True, path="tc")
-    _lib.gemm(A, B, C, a_mn=True, b_mn=True, path="simt")
-    assert ((C.double() - A.double().t() @ B.double()).norm() / C.double().norm()).item() < 1e-5
-
-
-def test_gemm_two_segment_input_and_derivative_epilogue(lib):
-    """cat(s, a) read from two buffers (first layers) and the fused activation-derivative epilogue (dgrad)."""
-    from rlrep_b200 import _lib
-    torch.manual_seed(2)
-    X1, X2 = torch.randn(64, 17, device="cuda"), torch.randn(64, 6, device="cuda")
-    W = torch.randn(40, 23, device="cuda")
-    C = torch.empty(64, 40, device="cuda")
-    _lib.gemm(X1, W, C, path="simt", A2=X2, epi=_lib.make_epilogue(act="tanh"))
-    ref = torch.tanh(torch.cat([X1, X2], 1).double() @ W.double().t())
-    assert (C.double() - ref).abs().max().item() < 1e-5
-    H = torch.randn(64, 23, device="cuda")
-    dX = torch.empty(64, 23, device="cuda")
-    _lib.gemm(C, W, dX, b_mn=True, path="simt", epi=_lib.make_epilogue(aux=H, dact="elu_out"))
-    ref = (C.double() @ W.double()) * torch.where(H > 0, torch.ones_like(H), H + 1).double()
-    assert ((dX.double() - ref).norm() / ref.norm()).item() < 1e-5
-
-
 # ------------------------------------------------------------------------------------------------ replay ring
 def test_gather_is_bit_exact_vs_reference_semantics():
     """buffer.sample == fp32 cast of the fp64 rows at the drawn indices (utils/buffer.py:39-48), bit for bit."""
