@@ -249,6 +249,46 @@ RLREP_EXPORT int rlrep_agent_profile_train(rlrep_agent* agent, rlrep_ring* ring,
                                            const float* eps_host, int max_entries, const char** names, float* ms,
                                            double* bytes, double* flops, int* n_entries);
 /* ------------------------------------------------------------------------------------------------
+ * SAC seed populations: `members` SAC agents of ONE configuration (cfg->alg must be RLREP_ALG_SAC; typically one per seed)
+ * in one handle.  The members' parameters, gradients, Adam moments, Polyak targets, activations and control blocks are
+ * identical layouts at a fixed stride in one allocation, and every kernel of the update takes the member from a grid
+ * dimension: rlrep_sacpop_train runs the update of all members as ONE launch sequence -- as many launches as one lone SAC
+ * agent's update, replayed as one CUDA graph from the third call on -- and member m computes bit for bit what a lone
+ * rlrep_agent_train computes with member m's weights, ring, indices and noise (the GEMMs run the lone agent's plan).
+ * Per-member arrays are member-major: idx [members * n_idx], eps [members * n_eps], metrics [members * n_metrics], with
+ * the per-member counts of rlrep_sacpop_train_counts and the metric names of a lone SAC agent.  `eps` may be a host or a
+ * device pointer (as for rlrep_agent_train); an out-of-range replay index is refused with an error naming the member.
+ * Tensors are indexed like a lone SAC agent's (names, shapes, "optim.m/<name>", "optim.v/<name>", targets) and accessed
+ * per member.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct rlrep_sacpop rlrep_sacpop;
+RLREP_EXPORT int rlrep_sacpop_create(const rlrep_agent_config* cfg, int members, void* stream, rlrep_sacpop** out);
+RLREP_EXPORT int rlrep_sacpop_destroy(rlrep_sacpop* pop);
+RLREP_EXPORT int rlrep_sacpop_members(rlrep_sacpop* pop, int* members);
+RLREP_EXPORT int rlrep_sacpop_num_tensors(rlrep_sacpop* pop, int* n);
+RLREP_EXPORT int rlrep_sacpop_tensor_info(rlrep_sacpop* pop, int member, int i, const char** name, float** ptr_dev,
+                                          int* rows, int* cols);
+RLREP_EXPORT int rlrep_sacpop_tensor_read(rlrep_sacpop* pop, int member, int i, float* out_host);
+RLREP_EXPORT int rlrep_sacpop_tensor_write(rlrep_sacpop* pop, int member, int i, const float* in_host);
+/* target <- parameter copies for every member (use after writing parameters). */
+RLREP_EXPORT int rlrep_sacpop_sync_targets(rlrep_sacpop* pop);
+RLREP_EXPORT int rlrep_sacpop_get_optim_state(rlrep_sacpop* pop, int member, rlrep_optim_state* out);
+RLREP_EXPORT int rlrep_sacpop_set_optim_state(rlrep_sacpop* pop, int member, const rlrep_optim_state* in);
+RLREP_EXPORT int rlrep_sacpop_train_counts(rlrep_sacpop* pop, int* n_idx, int* n_eps, int* n_metrics);
+RLREP_EXPORT const char* rlrep_sacpop_metric_name(rlrep_sacpop* pop, int i);
+/* rings [n_rings == members]: member m samples rings[m]; every ring has the configuration's state and action dims. */
+RLREP_EXPORT int rlrep_sacpop_train(rlrep_sacpop* pop, rlrep_ring* const* rings, int n_rings, const int64_t* idx_host,
+                                    int n_idx, const float* eps, int n_eps, float* metrics_host, int n_metrics);
+/* select_action of every member in one launch: states [members * state_dim], eps NULL (mean action) or
+ * [members * action_dim] -> actions [members * action_dim], unclamped like rlrep_agent_act. */
+RLREP_EXPORT int rlrep_sacpop_act(rlrep_sacpop* pop, const float* states_host, const float* eps_host, float* actions_host);
+/* rlrep_agent_train_resident for the population: idx [n_steps * members * n_idx], eps [n_steps * members * n_eps]. */
+RLREP_EXPORT int rlrep_sacpop_train_resident(rlrep_sacpop* pop, rlrep_ring* const* rings, int n_rings,
+                                             const int64_t* idx_host, const float* eps_host, int n_steps, float* total_ms);
+/* kernel launches of the most recent rlrep_sacpop_train (the same count as a lone SAC agent's update) */
+RLREP_EXPORT int rlrep_sacpop_last_launches(rlrep_sacpop* pop, int* launches);
+
+/* ------------------------------------------------------------------------------------------------
  * DrQ-v2 pixel encoder -- replaces `Encoder.forward` / its autograd backward and `RandomShiftsAug`
  * (agent/diffsrdrq/network_arch/drqv2.py:21-57,138-167; agent/mulvdrq/drqv2.py:19-96).  First building block of the
  * pixel agents; the agents themselves are not assembled yet (DESIGN.md section 0).

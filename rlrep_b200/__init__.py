@@ -21,6 +21,9 @@ def __getattr__(name):  # lazy: importing the package must not require torch.cud
     if name == "PixelReplayBuffer":
         from . import pixel_replay
         return pixel_replay.PixelReplayBuffer
+    if name == "SACPopulation":
+        from . import sac_population
+        return sac_population.SACPopulation
     if name == "Population":
         from . import population
         return population.Population

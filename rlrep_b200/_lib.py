@@ -170,8 +170,27 @@ def _declare(lib: C.CDLL) -> None:
             f"rlrep_{prefix}_get_optim_state": [vp, C.POINTER(OptimState)],
             f"rlrep_{prefix}_set_optim_state": [vp, C.POINTER(OptimState)],
         })
+    sigs.update({
+        "rlrep_sacpop_create": [C.POINTER(AgentConfig), i, vp, C.POINTER(vp)],
+        "rlrep_sacpop_destroy": [vp],
+        "rlrep_sacpop_members": [vp, C.POINTER(i)],
+        "rlrep_sacpop_num_tensors": [vp, C.POINTER(i)],
+        "rlrep_sacpop_tensor_info": [vp, i, i, C.POINTER(C.c_char_p), C.POINTER(vp), C.POINTER(i), C.POINTER(i)],
+        "rlrep_sacpop_tensor_read": [vp, i, i, vp],
+        "rlrep_sacpop_tensor_write": [vp, i, i, vp],
+        "rlrep_sacpop_sync_targets": [vp],
+        "rlrep_sacpop_get_optim_state": [vp, i, C.POINTER(OptimState)],
+        "rlrep_sacpop_set_optim_state": [vp, i, C.POINTER(OptimState)],
+        "rlrep_sacpop_train_counts": [vp, C.POINTER(i), C.POINTER(i), C.POINTER(i)],
+        "rlrep_sacpop_train": [vp, vp, i, vp, i, vp, i, vp, i],
+        "rlrep_sacpop_act": [vp, vp, vp, vp],
+        "rlrep_sacpop_train_resident": [vp, vp, i, vp, vp, i, C.POINTER(C.c_float)],
+        "rlrep_sacpop_last_launches": [vp, C.POINTER(i)],
+    })
     lib.rlrep_agent_metric_name.argtypes = [vp, i]
     lib.rlrep_agent_metric_name.restype = C.c_char_p
+    lib.rlrep_sacpop_metric_name.argtypes = [vp, i]
+    lib.rlrep_sacpop_metric_name.restype = C.c_char_p
     for name, argtypes in sigs.items():
         fn = getattr(lib, name)
         fn.argtypes = argtypes

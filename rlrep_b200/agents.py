@@ -20,16 +20,17 @@ import torch
 from . import _lib
 
 
-def _orthogonal(out_f, in_f):
+def _orthogonal(out_f, in_f, generator=None):
     w = torch.empty(out_f, in_f)
-    torch.nn.init.orthogonal_(w)  # utils/util.py:61-66 (weight_init)
+    torch.nn.init.orthogonal_(w, generator=generator)  # utils/util.py:61-66 (weight_init)
     return w
 
 
-def _default_linear(out_f, in_f):
+def _default_linear(out_f, in_f, generator=None):
     """nn.Linear's default init (kaiming_uniform(a=sqrt(5)) == U(+-1/sqrt(fan_in)) for weight and bias)."""
     bound = 1.0 / math.sqrt(in_f)
-    return (torch.rand(out_f, in_f) * 2 - 1) * bound, (torch.rand(out_f) * 2 - 1) * bound
+    return ((torch.rand(out_f, in_f, generator=generator) * 2 - 1) * bound,
+            (torch.rand(out_f, generator=generator) * 2 - 1) * bound)
 
 
 class _Handle:
@@ -160,12 +161,14 @@ class SACAgent:
 
     def __init__(self, state_dim, action_dim, action_space, lr=3e-4, discount=0.99, target_update_period=2, tau=0.005,
                  alpha=0.1, auto_entropy_tuning=True, hidden_dim=1024, *, precision="tf32", use_cuda_graph=True,
-                 noise_device="cpu", **extra):
+                 noise_device="cpu", generator=None, **extra):
         """`noise_device`: where train() draws its Gaussian noise.  "cpu" (default) uses torch's global CPU generator -- the
         stream the reference consumes when it runs on the CPU, and the one the oracle / golden fixtures are pinned to.
         "cuda" draws the same tensors, in the same order and shapes, with torch's CUDA generator -- the stream the
         reference consumes when it runs with device = cuda (torch.randn_like on CUDA tensors) -- so the noise never exists
-        on the host: no host RNG time and no PCIe transfer (4 MB per update for LV-Rep at B = 1024)."""
+        on the host: no host RNG time and no PCIe transfer (4 MB per update for LV-Rep at B = 1024).
+        `generator`: a CPU torch.Generator the initial weights are drawn from instead of the global generator (same draws,
+        same order)."""
         if noise_device not in ("cpu", "cuda"):
             raise ValueError("noise_device must be 'cpu' or 'cuda'")
         self.noise_device = noise_device
@@ -182,7 +185,7 @@ class SACAgent:
         self._extra = extra
         self._h: _Handle | None = None
         self._batch = None
-        self._pending_state = self._initial_state()  # host copy until the handle exists
+        self._pending_state = self._initial_state(generator)  # host copy until the handle exists
 
     # ---- configuration of the C handle (overridden per algorithm) -------------------------------------------
     def _config(self, batch_size) -> _lib.AgentConfig:
@@ -212,13 +215,13 @@ class SACAgent:
         S, A = self.state_dim, self.action_dim
         return [("actor.trunk.0", H, S, "orth"), ("actor.trunk.2", H, H, "orth"), ("actor.trunk.4", 2 * A, H, "orth")]
 
-    def _initial_state(self):
+    def _initial_state(self, generator=None):
         sd = {}
         for name, out, inp, kind in self._layers():
             if kind == "orth":  # modules that call self.apply(util.weight_init): orthogonal weight, zero bias
-                sd[name + ".weight"], sd[name + ".bias"] = _orthogonal(out, inp), torch.zeros(out)
+                sd[name + ".weight"], sd[name + ".bias"] = _orthogonal(out, inp, generator), torch.zeros(out)
             else:
-                sd[name + ".weight"], sd[name + ".bias"] = _default_linear(out, inp)
+                sd[name + ".weight"], sd[name + ".bias"] = _default_linear(out, inp, generator)
         return sd
 
     # ---- handle management --------------------------------------------------------------------------------------
@@ -388,7 +391,10 @@ class SACAgent:
         return idx, self._pack(eps)
 
     def _info(self, m):
-        d = dict(zip(self._h.metric_names, (float(x) for x in m)))
+        return self._sac_info(dict(zip(self._h.metric_names, (float(x) for x in m))))
+
+    @staticmethod
+    def _sac_info(d):
         # sac_agent.py:131-135: q_loss = mse1 + mse2; 'q2' reports mean(Q1)
         return {"q_loss": float(np.float32(d["q1_loss"]) + np.float32(d["q2_loss"])), "q1": d["q1"], "q2": d["q1"],
                 "actor_loss": d["actor_loss"], "alpha_loss": d["alpha_loss"], "alpha": d["alpha"]}

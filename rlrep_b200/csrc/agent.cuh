@@ -35,10 +35,13 @@ class DeviceArena {
     reqs_.push_back(r);
     total_ += (count * sizeof(T) + 255) & ~size_t(255);
   }
-  void commit() {
+  // copies > 1: that many identical layouts back to back (a population's members, members.cuh), bytes() apart; the
+  // registered pointers are the first copy's.
+  void commit(int copies = 1) {
     RLREP_CHECK(base_ == nullptr, "arena already committed");
-    RLREP_CUDA(cudaMalloc(&base_, total_ ? total_ : 256));
-    RLREP_CUDA(cudaMemset(base_, 0, total_ ? total_ : 256));
+    if (total_ == 0) total_ = 256;
+    RLREP_CUDA(cudaMalloc(&base_, total_ * copies));
+    RLREP_CUDA(cudaMemset(base_, 0, total_ * copies));
     // The memset runs on the legacy default stream and is asynchronous with respect to the agents' NON-BLOCKING
     // streams: without this wait it can still be zeroing the arena when the first copies into it (control block,
     // weights) have already landed.
@@ -229,6 +232,9 @@ class GemmRunner {
   // Share of the GPU the next GEMMs should plan for: 0.5 inside fork()/join() sections where two independent kernel
   // chains run on two streams, 1.0 elsewhere.  Part of the plan-cache key.
   void set_sm_share(double share) { sm_share_ = share; }
+  // Population handles (members.cuh): the linear-layer passes below run every GEMM for all members at once.
+  void set_members(const Members& mb) { mb_ = mb; }
+  const Members& members() const { return mb_; }
 
   // GEMM chains (gemm_chain.cuh): between begin_chain(s) and end_chain() every run() is RECORDED instead of launched --
   // whatever stream it names -- and end_chain() executes the recorded DAG as one persistent kernel on `s` (dependencies are
@@ -248,6 +254,7 @@ class GemmRunner {
   std::vector<std::unique_ptr<GemmChain>> chains_;
   Precision prec_ = PREC_TF32;
   double sm_share_ = 1.0;
+  Members mb_;
   float* ws_ = nullptr;
   size_t ws_floats_ = 0;
   // K-group partial outputs of GEMMs with a huge K and a handful of tiles (run(): "deep and skinny"); grown on first use of a
@@ -323,6 +330,12 @@ class Agent {
   // all steps uploaded before the timed region, staged per step by device-to-device copies); returns the CUDA-event
   // time of the whole loop in milliseconds.  State advances exactly as n_steps train() calls would.
   virtual float train_resident(Ring& ring, const long long* idx_host, const float* eps_host, int n_steps) = 0;
+  // Population agents (members.cuh; SacBase): train / train_resident / act over one ring and one row of inputs per member.
+  virtual void train_members(Ring* const* rings, const long long* idx_host, int n_idx, const float* eps_host, int n_eps,
+                             float* metrics_host, int n_metrics) = 0;
+  virtual float train_resident_members(Ring* const* rings, const long long* idx_host, const float* eps_host,
+                                       int n_steps) = 0;
+  virtual void act_members(const float* states_host, const float* eps_host, float* actions_host) = 0;
   // One eager (non-graph) train() with an event behind every launch -> per-launch (kernel name, ms).
   virtual std::vector<ProfileEntry> profile_train(Ring& ring, const long long* idx_host, const float* eps_host) = 0;
   virtual int idx_per_train() const = 0;  // replay indices consumed per train()
@@ -338,11 +351,14 @@ class Agent {
 
   AgentConfig cfg;
   cudaStream_t stream = nullptr;
-  Control* ctl = nullptr;
+  Control* ctl = nullptr;  // member 0's control block; member m's is mb.stride * m bytes on
   int last_launches = 0;
+  Members mb;  // n = 1, stride = 0 for a lone agent
 };
 
 std::unique_ptr<Agent> make_sac_agent(const AgentConfig& cfg, cudaStream_t s);
+// `members` SAC agents of one configuration trained as one batched update (members.cuh)
+std::unique_ptr<Agent> make_sac_population(const AgentConfig& cfg, cudaStream_t s, int members);
 std::unique_ptr<Agent> make_ctrlsac_agent(const AgentConfig& cfg, cudaStream_t s);
 std::unique_ptr<Agent> make_vlsac_agent(const AgentConfig& cfg, cudaStream_t s);
 std::unique_ptr<Agent> make_spedersac_agent(const AgentConfig& cfg, cudaStream_t s);

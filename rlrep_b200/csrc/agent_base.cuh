@@ -1,6 +1,8 @@
 // SacBase: what every SAC-family agent shares (reference: agent/sac/sac_agent.py) -- the tanh-Gaussian actor with
 // its forward/backward, the control block with the float64 temperature, staging of the host-drawn indices and
 // noise, metrics read-back, and the eager -> capture -> replay protocol of train().
+// An agent built with members > 1 is a population (members.cuh): that many agents of this configuration, each with its
+// own arena copy, trained by the one launch sequence every train() call runs.
 #pragma once
 #include "staging.cuh"
 
@@ -10,14 +12,16 @@ namespace rlrep {
 
 class SacBase : public Agent {
  public:
-  SacBase(const AgentConfig& c, cudaStream_t s) {
+  SacBase(const AgentConfig& c, cudaStream_t s, int members = 1) {
     cfg = c;
     stream = s;
     S_ = c.state_dim;
     A_ = c.action_dim;
     B_ = c.batch;
     AH_ = c.actor_hidden_dim;
+    members_ = members;
     RLREP_CHECK(S_ > 0 && A_ > 0 && B_ > 0, "bad agent dimensions");
+    RLREP_CHECK(members_ >= 1 && members_ <= kActRows, "a population has 1 to 1024 members");
   }
   ~SacBase() override {
     for (cudaEvent_t e : events_) cudaEventDestroy(e);
@@ -33,53 +37,72 @@ class SacBase : public Agent {
 
   void train(Ring& ring, const long long* idx_host, int n_idx, const float* eps_host, int n_eps, float* metrics_host,
              int n_metrics) override {
-    RLREP_CHECK(ring.S == S_ && ring.A == A_, "ring shape does not match the agent");
-    RLREP_CHECK(n_idx == idx_per_train() && n_eps == eps_per_train(), "wrong number of indices / noise values");
-    RLREP_CHECK(n_metrics >= (int)metric_names().size(), "metrics buffer too small");
-    for (int i = 0; i < n_idx; ++i)
-      RLREP_CHECK(!is_replay_index(i) || (idx_host[i] >= 0 && idx_host[i] < ring.size), "replay index out of range");
-    bind_ring(ring);
+    Ring* rings[1] = {&ring};
+    train_members(rings, idx_host, n_idx, eps_host, n_eps, metrics_host, n_metrics);
+  }
+  // rings[m], idx_host [members, idx_per_train()], eps_host [members, eps_per_train()] and metrics_host
+  // [members, metric_names().size()] belong to member m.
+  void train_members(Ring* const* rings, const long long* idx_host, int n_idx, const float* eps_host, int n_eps,
+                     float* metrics_host, int n_metrics) override {
+    const int ni = idx_per_train(), ne = eps_per_train(), nm = (int)metric_names().size();
+    for (int m = 0; m < members_; ++m)
+      RLREP_CHECK(rings[m]->S == S_ && rings[m]->A == A_, "ring shape does not match the agent" + member_note(m));
+    RLREP_CHECK(n_idx == members_ * ni && n_eps == members_ * ne, "wrong number of indices / noise values");
+    RLREP_CHECK(n_metrics >= members_ * nm, "metrics buffer too small");
+    for (int m = 0; m < members_; ++m)
+      for (int i = 0; i < ni; ++i) {
+        const long long j = idx_host[(size_t)m * ni + i];
+        RLREP_CHECK(!is_replay_index(i) || (j >= 0 && j < rings[m]->size), "replay index out of range" + member_note(m));
+      }
+    bind_rings(rings);
     RLREP_CUDA(cudaStreamSynchronize(stream));  // pinned staging is reused across calls
     std::memcpy(idx_host_, idx_host, (size_t)n_idx * sizeof(long long));
-    RLREP_CUDA(cudaMemcpyAsync(idx_dev_, idx_host_, (size_t)n_idx * sizeof(long long), cudaMemcpyHostToDevice, stream));
+    to_members(idx_dev_, idx_host_, (size_t)ni * sizeof(long long), cudaMemcpyHostToDevice);
     if (is_device_pointer(eps_host)) {
       // noise drawn on the device by the caller (agents.py noise_device = "cuda"): it never touches the host
-      RLREP_CUDA(cudaMemcpyAsync(eps_dev_, eps_host, (size_t)n_eps * sizeof(float), cudaMemcpyDeviceToDevice, stream));
+      to_members(eps_dev_, eps_host, (size_t)ne * sizeof(float), cudaMemcpyDeviceToDevice);
     } else {
       std::memcpy(eps_host_, eps_host, (size_t)n_eps * sizeof(float));
-      RLREP_CUDA(cudaMemcpyAsync(eps_dev_, eps_host_, (size_t)n_eps * sizeof(float), cudaMemcpyHostToDevice, stream));
+      to_members(eps_dev_, eps_host_, (size_t)ne * sizeof(float), cudaMemcpyHostToDevice);
     }
     const long long before = launch_count();
     const bool was_captured = graph_.captured();
-    graph_.run(stream, cfg.use_graph != 0, [&] { update(ring); });
+    graph_.run(stream, cfg.use_graph != 0, [&] { update(*rings[0]); });
     if (!was_captured) launches_per_train_ = (int)(launch_count() - before);
     last_launches = launches_per_train_;
-    RLREP_CUDA(cudaMemcpyAsync(metrics_host_, metrics_dev_, kNumMetrics * sizeof(float), cudaMemcpyDeviceToHost, stream));
+    // one device-to-host copy of every member's kNumMetrics-float block
+    copy_members(metrics_host_, kNumMetrics * sizeof(float), metrics_dev_, (size_t)mb.stride, kNumMetrics * sizeof(float),
+                 cudaMemcpyDeviceToHost);
     RLREP_CUDA(cudaStreamSynchronize(stream));
-    std::memcpy(metrics_host, metrics_host_, metric_names().size() * sizeof(float));
+    for (int m = 0; m < members_; ++m)
+      std::memcpy(metrics_host + (size_t)m * nm, metrics_host_ + (size_t)m * kNumMetrics, nm * sizeof(float));
   }
 
   float train_resident(Ring& ring, const long long* idx_host, const float* eps_host, int n_steps) override {
-    const int ni = idx_per_train(), ne = eps_per_train();
-    RLREP_CHECK(ring.S == S_ && ring.A == A_ && n_steps > 0, "bad arguments");
-    bind_ring(ring);
+    Ring* rings[1] = {&ring};
+    return train_resident_members(rings, idx_host, eps_host, n_steps);
+  }
+  // idx_host [n_steps, members, idx_per_train()], eps_host [n_steps, members, eps_per_train()]
+  float train_resident_members(Ring* const* rings, const long long* idx_host, const float* eps_host, int n_steps) override {
+    const int ni = idx_per_train(), ne = eps_per_train(), N = members_;
+    RLREP_CHECK(n_steps > 0, "bad arguments");
+    for (int m = 0; m < N; ++m) RLREP_CHECK(rings[m]->S == S_ && rings[m]->A == A_, "bad arguments");
+    bind_rings(rings);
     long long* idx_all = nullptr;
     float* eps_all = nullptr;
-    RLREP_CUDA(cudaMalloc(&idx_all, (size_t)n_steps * ni * sizeof(long long)));
-    RLREP_CUDA(cudaMalloc(&eps_all, (size_t)n_steps * ne * sizeof(float)));
-    RLREP_CUDA(cudaMemcpy(idx_all, idx_host, (size_t)n_steps * ni * sizeof(long long), cudaMemcpyHostToDevice));
-    RLREP_CUDA(cudaMemcpy(eps_all, eps_host, (size_t)n_steps * ne * sizeof(float), cudaMemcpyHostToDevice));
+    RLREP_CUDA(cudaMalloc(&idx_all, (size_t)n_steps * N * ni * sizeof(long long)));
+    RLREP_CUDA(cudaMalloc(&eps_all, (size_t)n_steps * N * ne * sizeof(float)));
+    RLREP_CUDA(cudaMemcpy(idx_all, idx_host, (size_t)n_steps * N * ni * sizeof(long long), cudaMemcpyHostToDevice));
+    RLREP_CUDA(cudaMemcpy(eps_all, eps_host, (size_t)n_steps * N * ne * sizeof(float), cudaMemcpyHostToDevice));
     cudaEvent_t e0, e1;
     RLREP_CUDA(cudaEventCreate(&e0));
     RLREP_CUDA(cudaEventCreate(&e1));
     RLREP_CUDA(cudaStreamSynchronize(stream));
     RLREP_CUDA(cudaEventRecord(e0, stream));
     for (int i = 0; i < n_steps; ++i) {
-      RLREP_CUDA(cudaMemcpyAsync(idx_dev_, idx_all + (size_t)i * ni, (size_t)ni * sizeof(long long),
-                                 cudaMemcpyDeviceToDevice, stream));
-      RLREP_CUDA(cudaMemcpyAsync(eps_dev_, eps_all + (size_t)i * ne, (size_t)ne * sizeof(float),
-                                 cudaMemcpyDeviceToDevice, stream));
-      graph_.run(stream, cfg.use_graph != 0, [&] { update(ring); });
+      to_members(idx_dev_, idx_all + (size_t)i * N * ni, (size_t)ni * sizeof(long long), cudaMemcpyDeviceToDevice);
+      to_members(eps_dev_, eps_all + (size_t)i * N * ne, (size_t)ne * sizeof(float), cudaMemcpyDeviceToDevice);
+      graph_.run(stream, cfg.use_graph != 0, [&] { update(*rings[0]); });
     }
     RLREP_CUDA(cudaEventRecord(e1, stream));
     RLREP_CUDA(cudaEventSynchronize(e1));
@@ -122,6 +145,24 @@ class SacBase : public Agent {
   void act(const float* state_host, const float* eps_host, float* action_host) override {
     act_batch(state_host, eps_host, 1, action_host);
   }
+  // One observation per member: states_host [members, S], eps_host [members, A] or nullptr -> actions_host [members, A],
+  // one launch.
+  void act_members(const float* states_host, const float* eps_host, float* actions_host) override {
+    RLREP_CHECK(states_host && actions_host, "bad arguments");
+    if (members_ == 1) return act_batch(states_host, eps_host, 1, actions_host);
+    const Linear l0 = a0_.view(actor_g_), l1 = a1_.view(actor_g_), l2 = a2_.view(actor_g_);
+    const int W = S_ + A_;
+    RLREP_CUDA(cudaStreamSynchronize(stream));  // the staging buffers are reused
+    for (int m = 0; m < members_; ++m) {
+      float* dst = act_in_host_ + (size_t)m * W;
+      std::memcpy(dst, states_host + (size_t)m * S_, S_ * sizeof(float));
+      if (eps_host) std::memcpy(dst + S_, eps_host + (size_t)m * A_, A_ * sizeof(float));
+    }
+    launch_actor_act(act_in_dev_, 1, S_, A_, AH_, l0.W, l0.ld, l0.b, l1.W, l1.ld, l1.b, l2.W, l2.ld, l2.b,
+                     eps_host != nullptr, act_out_dev_, stream, mb);
+    RLREP_CUDA(cudaStreamSynchronize(stream));
+    std::memcpy(actions_host, act_out_host_, (size_t)members_ * A_ * sizeof(float));
+  }
   void act_batch(const float* states_host, const float* eps_host, int rows, float* actions_host) override {
     RLREP_CHECK(rows >= 0 && states_host && actions_host, "bad arguments");
     const Linear l0 = a0_.view(actor_g_), l1 = a1_.view(actor_g_), l2 = a2_.view(actor_g_);
@@ -143,12 +184,31 @@ class SacBase : public Agent {
 
  protected:
   // Captured graphs bake ring.data into their gather nodes: a different ring (also one that happens to live at a freed
-  // ring's address) invalidates the graph.
-  void bind_ring(const Ring& ring) {
-    if (ring_bound_ != ring.generation) {
-      graph_.reset();
-      ring_bound_ = ring.generation;
+  // ring's address) invalidates the graph.  A population's members read their ring from a word in their arena
+  // (ring_slot_), rewritten here whenever the set of rings changes.
+  void bind_rings(Ring* const* rings) {
+    bool same = true;
+    for (int m = 0; m < members_; ++m) same = same && rings_bound_[m] == rings[m]->generation;
+    if (same) return;
+    graph_.reset();
+    for (int m = 0; m < members_; ++m) rings_bound_[m] = rings[m]->generation;
+    if (members_ > 1) {
+      std::vector<const float*> data(members_);
+      for (int m = 0; m < members_; ++m) data[m] = rings[m]->data;
+      RLREP_CUDA(cudaStreamSynchronize(stream));
+      to_members(ring_slot_, data.data(), sizeof(const float*), cudaMemcpyHostToDevice);
+      RLREP_CUDA(cudaStreamSynchronize(stream));
     }
+  }
+  std::string member_note(int m) const { return members_ > 1 ? " (member " + std::to_string(m) + ")" : ""; }
+  // dst_dev / src each hold `members_` blocks of `bytes`, one per member, at member pitch dpitch / spitch.
+  void copy_members(void* dst, size_t dpitch, const void* src, size_t spitch, size_t bytes, cudaMemcpyKind kind) {
+    if (members_ == 1) RLREP_CUDA(cudaMemcpyAsync(dst, src, bytes, kind, stream));
+    else RLREP_CUDA(cudaMemcpy2DAsync(dst, dpitch, src, spitch, bytes, members_, kind, stream));
+  }
+  // members_ dense blocks of `bytes` at src -> the same buffer of every member's arena
+  void to_members(void* dst_dev, const void* src, size_t bytes, cudaMemcpyKind kind) {
+    copy_members(dst_dev, (size_t)mb.stride, src, bytes, bytes, kind);
   }
   // One full train() worth of launches on `stream`, reading idx_dev_ / eps_dev_ and writing metrics_dev_.
   virtual void update(Ring& ring) = 0;
@@ -240,9 +300,11 @@ class SacBase : public Agent {
     arena_.want(&cat_next_, (size_t)B_ * LDSA_);  // cat(s', a')   (critic step)
     arena_.want(&cat_pi_, (size_t)B_ * LDSA_);    // cat(s, a_pi)  (actor step)
     arena_.want(&dlogp_, 4);
-    RLREP_CUDA(cudaMallocHost(&metrics_host_, kNumMetrics * sizeof(float)));
-    RLREP_CUDA(cudaMallocHost(&idx_host_, (size_t)(n_idx > 0 ? n_idx : 1) * sizeof(long long)));
-    RLREP_CUDA(cudaMallocHost(&eps_host_, (size_t)(n_eps > 0 ? n_eps : 1) * sizeof(float)));
+    if (members_ > 1) arena_.want(&ring_slot_, 1);
+    rings_bound_.assign(members_, 0);
+    RLREP_CUDA(cudaMallocHost(&metrics_host_, (size_t)members_ * kNumMetrics * sizeof(float)));
+    RLREP_CUDA(cudaMallocHost(&idx_host_, (size_t)members_ * (n_idx > 0 ? n_idx : 1) * sizeof(long long)));
+    RLREP_CUDA(cudaMallocHost(&eps_host_, (size_t)members_ * (n_eps > 0 ? n_eps : 1) * sizeof(float)));
     // select_action staging: mapped pinned memory the policy kernel reads / writes directly
     RLREP_CUDA(cudaHostAlloc(&act_in_host_, (size_t)kActRows * (S_ + A_) * sizeof(float), cudaHostAllocMapped));
     RLREP_CUDA(cudaHostAlloc(&act_out_host_, (size_t)kActRows * A_ * sizeof(float), cudaHostAllocMapped));
@@ -252,13 +314,16 @@ class SacBase : public Agent {
   }
 
   void finish_setup(size_t gemm_ws_floats) {
-    arena_.commit();
+    arena_.commit(members_);
+    if (members_ > 1) mb = Members{members_, (long long)arena_.bytes()};
     gemm_.init(static_cast<Precision>(cfg.precision), gemm_ws_floats);
+    gemm_.set_members(mb);
     Control h;
     std::memset(&h, 0, sizeof(h));
     h.log_alpha = std::log(cfg.alpha0);  // torch.tensor(np.log(alpha)), float64
     h.alpha = (float)cfg.alpha0;
-    RLREP_CUDA(cudaMemcpyAsync(ctl, &h, sizeof(h), cudaMemcpyHostToDevice, stream));
+    for (int m = 0; m < members_; ++m)
+      RLREP_CUDA(cudaMemcpyAsync(member_ptr(ctl, m * mb.stride), &h, sizeof(h), cudaMemcpyHostToDevice, stream));
     RLREP_CUDA(cudaStreamSynchronize(stream));
   }
 
@@ -276,7 +341,7 @@ class SacBase : public Agent {
     linear_fwd(gemm_, s, B_, obs, l0, ACT_ELU, h1, AH_);
     linear_fwd(gemm_, s, B_, Mat{h1, AH_}, l1, ACT_ELU, h2, AH_);
     linear_fwd(gemm_, s, B_, Mat{h2, AH_}, l2, ACT_NONE, hd, LDH_);
-    launch_actor_sample(hd, LDH_, B_, A_, eps, cat_buf + S_, LDSA_, logp_out, s, obs.p, obs.ld, S_);
+    launch_actor_sample(hd, LDH_, B_, A_, eps, cat_buf + S_, LDSA_, logp_out, s, obs.p, obs.ld, S_, mb);
     return Mat{cat_buf, LDSA_};
   }
   // The two halves of actor_forward_cat for callers that run the trunk GEMMs of several networks as one GEMM chain.
@@ -332,7 +397,7 @@ class SacBase : public Agent {
     const Linear l0 = a0_.view(actor_g_), l1 = a1_.view(actor_g_), l2 = a2_.view(actor_g_);
     // dgrad chain on the main stream; weight / bias gradients trail it on an aux branch
     cudaStream_t w = aux(1);
-    launch_actor_sample_bwd(head_, LDH_, B_, A_, eps, dsa_ + S_, LDSA_, dlogp_, dhead_, LDH_, stream);
+    launch_actor_sample_bwd(head_, LDH_, B_, A_, eps, dsa_ + S_, LDSA_, dlogp_, dhead_, LDH_, stream, mb);
     wait_for(w, mark(stream));
     linear_wgrad(gemm_, w, B_, Mat{dhead_, LDH_}, Mat{ah2_, AH_}, l2, Mat(), 0, false);
     linear_dgrad(gemm_, stream, B_, Mat{dhead_, LDH_}, l2, DACT_ELU_OUT, Mat{ah2_, AH_}, dah2_, AH_);
@@ -344,13 +409,13 @@ class SacBase : public Agent {
     {
       const ColJob jobs[3] = {bias_job(B_, Mat{dhead_, LDH_}, l2), bias_job(B_, Mat{dah2_, AH_}, l1),
                               bias_job(B_, Mat{dah1_, AH_}, l0)};
-      launch_colreduce_multi(jobs, 3, w);
+      launch_colreduce_multi(jobs, 3, w, mb);
     }
     join_aux(1, stream);
   }
   void actor_adam() {
     launch_adam_polyak(actor_g_.p, actor_g_.g, actor_g_.m, actor_g_.v, actor_g_.n, &ctl->actor, nullptr, 0, 0.f,
-                       nullptr, stream);
+                       nullptr, stream, mb);
   }
   TickParams base_tick() const {
     TickParams t;
@@ -379,7 +444,9 @@ class SacBase : public Agent {
   DeviceArena arena_;
   GemmRunner gemm_;
   GraphReplay graph_;
-  unsigned long long ring_bound_ = 0;  // Ring::generation the captured graph was built against
+  std::vector<unsigned long long> rings_bound_;  // Ring::generation of each member's ring the captured graph was built against
+  int members_ = 1;
+  const float** ring_slot_ = nullptr;  // population: the member's ring (Ring::data), read by the gather
   int launches_per_train_ = 0;
   ParamGroup actor_g_;
   LinearSlot a0_, a1_, a2_;

@@ -9,7 +9,7 @@ namespace {
 
 class SacAgent final : public SacBase {
  public:
-  SacAgent(const AgentConfig& c, cudaStream_t s) : SacBase(c, s) {
+  SacAgent(const AgentConfig& c, cudaStream_t s, int members) : SacBase(c, s, members) {
     H_ = c.hidden_dim;
     RLREP_CHECK(H_ % 32 == 0, "hidden_dim must be a multiple of 32");
     const RecordLayout lay = RecordLayout::of(S_, A_);
@@ -61,7 +61,8 @@ class SacAgent final : public SacBase {
   const std::vector<std::string>& metric_names() const override { return names_; }
   std::vector<ParamGroup*> groups() override { return {&crit_g_, &actor_g_}; }
   void sync_targets_from_params() override {
-    RLREP_CUDA(cudaMemcpyAsync(crit_g_.target, crit_g_.p, crit_g_.n_target * 4, cudaMemcpyDeviceToDevice, stream));
+    copy_members(crit_g_.target, (size_t)mb.stride, crit_g_.p, (size_t)mb.stride, crit_g_.n_target * 4,
+                 cudaMemcpyDeviceToDevice);
     RLREP_CUDA(cudaStreamSynchronize(stream));
   }
 
@@ -70,8 +71,8 @@ class SacAgent final : public SacBase {
     begin_update();
     TickParams t = base_tick();
     t.k_feat = 0;
-    launch_tick(ctl, t, stream);
-    launch_gather(ring.data, R_ / 4, idx_dev_, B_, batch_, stream);
+    launch_tick(ctl, t, stream, mb);
+    launch_gather(ring.data, R_ / 4, idx_dev_, B_, batch_, stream, mb, ring_slot_);
     critic_step();
     actor_step();
   }
@@ -84,19 +85,19 @@ class SacAgent final : public SacBase {
     linear_fwd(gemm_, stream, B_, x, l0, ACT_ELU, hid0_, 2 * H_, x2, k1);
     linear_fwd(gemm_, stream, B_, Mat{hid0_, 2 * H_}, l1a, ACT_ELU, hid1a_, H_);
     linear_fwd(gemm_, stream, B_, Mat{hid0_ + H_, 2 * H_}, l1b, ACT_ELU, hid1b_, H_);
-    launch_rowdot(hid1a_, H_, B_, H_, l2a.W, l2a.b, q1, stream);
-    launch_rowdot(hid1b_, H_, B_, H_, l2b.W, l2b.b, q2, stream);
+    launch_rowdot(hid1a_, H_, B_, H_, l2a.W, l2a.b, q1, stream, mb);
+    launch_rowdot(hid1b_, H_, B_, H_, l2b.W, l2b.b, q2, stream, mb);
   }
   // (dq1, dq2) -> d hid1 -> d hid0 (activations of the matching critic_forward must be live)
   void critic_backward_to_hid0(bool with_wgrad) {
     const Linear l1a = c1a_.view(crit_g_), l1b = c1b_.view(crit_g_), l2a = c2a_.view(crit_g_), l2b = c2b_.view(crit_g_);
-    launch_outer_dact(dq1_, l2a.W, B_, H_, hid1a_, H_, DACT_ELU_OUT, dhid1a_, H_, stream);
-    launch_outer_dact(dq2_, l2b.W, B_, H_, hid1b_, H_, DACT_ELU_OUT, dhid1b_, H_, stream);
+    launch_outer_dact(dq1_, l2a.W, B_, H_, hid1a_, H_, DACT_ELU_OUT, dhid1a_, H_, stream, mb);
+    launch_outer_dact(dq2_, l2b.W, B_, H_, hid1b_, H_, DACT_ELU_OUT, dhid1b_, H_, stream, mb);
     if (with_wgrad) {
-      launch_colreduce(hid1a_, H_, B_, H_, dq1_, l2a.dW, 0, stream);
-      launch_colreduce(dq1_, 1, B_, 1, nullptr, l2a.db, 0, stream);
-      launch_colreduce(hid1b_, H_, B_, H_, dq2_, l2b.dW, 0, stream);
-      launch_colreduce(dq2_, 1, B_, 1, nullptr, l2b.db, 0, stream);
+      launch_colreduce(hid1a_, H_, B_, H_, dq1_, l2a.dW, 0, stream, mb);
+      launch_colreduce(dq1_, 1, B_, 1, nullptr, l2a.db, 0, stream, mb);
+      launch_colreduce(hid1b_, H_, B_, H_, dq2_, l2b.dW, 0, stream, mb);
+      launch_colreduce(dq2_, 1, B_, 1, nullptr, l2b.db, 0, stream, mb);
       linear_wgrad(gemm_, stream, B_, Mat{dhid1a_, H_}, Mat{hid0_, 2 * H_}, l1a);
       linear_wgrad(gemm_, stream, B_, Mat{dhid1b_, H_}, Mat{hid0_ + H_, 2 * H_}, l1b);
     }
@@ -110,11 +111,11 @@ class SacAgent final : public SacBase {
     critic_forward(s2a, Mat(), 0, /*target=*/true, nq1_, nq2_);
     critic_forward(sa, Mat(), 0, false, q1_, q2_);
     launch_td_critic_loss(batch_ + off_r_, batch_ + off_d_, R_, nq1_, nq2_, logp2_, q1_, q2_, B_, cfg.discount, ctl,
-                          dq1_, dq2_, metrics_dev_ + 0, stream);
+                          dq1_, dq2_, metrics_dev_ + 0, stream, 0, mb);
     critic_backward_to_hid0(true);
     linear_wgrad(gemm_, stream, B_, Mat{dhid0_, 2 * H_}, sa, c0_.view(crit_g_));
     launch_adam_polyak(crit_g_.p, crit_g_.g, crit_g_.m, crit_g_.v, crit_g_.n, &ctl->critic, crit_g_.target,
-                       crit_g_.n_target, cfg.tau, &ctl->polyak_critic, stream);
+                       crit_g_.n_target, cfg.tau, &ctl->polyak_critic, stream, mb);
   }
 
   void actor_step() {  // sac_agent.py:138-166
@@ -123,7 +124,7 @@ class SacAgent final : public SacBase {
     const Mat spi = actor_forward_cat(s, eps, cat_pi_, logp_);
     critic_forward(spi, Mat(), 0, false, q1_, q2_);
     launch_actor_alpha_loss(q1_, q2_, logp_, B_, (float)(-A_), cfg.learn_alpha, ctl, dq1_, dq2_, dlogp_,
-                            metrics_dev_ + 4, stream);
+                            metrics_dev_ + 4, stream, mb);
     critic_backward_to_hid0(false);
     dgrad_to_action(Mat{dhid0_, 2 * H_}, c0_.view(crit_g_));
     actor_backward(s, eps);
@@ -143,7 +144,10 @@ class SacAgent final : public SacBase {
 }  // namespace
 
 std::unique_ptr<Agent> make_sac_agent(const AgentConfig& cfg, cudaStream_t s) {
-  return std::unique_ptr<Agent>(new SacAgent(cfg, s));
+  return std::unique_ptr<Agent>(new SacAgent(cfg, s, 1));
+}
+std::unique_ptr<Agent> make_sac_population(const AgentConfig& cfg, cudaStream_t s, int members) {
+  return std::unique_ptr<Agent>(new SacAgent(cfg, s, members));
 }
 
 }  // namespace rlrep

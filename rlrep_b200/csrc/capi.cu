@@ -120,19 +120,23 @@ static void tensor_info(const std::vector<TensorRef>& ts, int i, const char** na
   if (rows) *rows = t.rows;
   if (cols) *cols = t.cols;
 }
-static void tensor_read(const std::vector<TensorRef>& ts, int i, float* out_host, cudaStream_t st) {
-  const TensorRef& t = tensor_at(ts, i);
+static void tensor_read(const TensorRef& t, float* out_host, cudaStream_t st) {
   RLREP_CHECK(out_host != nullptr, "null argument");
   RLREP_CUDA(cudaMemcpy2DAsync(out_host, (size_t)t.cols * 4, t.ptr, (size_t)t.ld * 4, (size_t)t.cols * 4, t.rows,
                                cudaMemcpyDeviceToHost, st));
   RLREP_CUDA(cudaStreamSynchronize(st));
 }
-static void tensor_write(const std::vector<TensorRef>& ts, int i, const float* in_host, cudaStream_t st) {
-  const TensorRef& t = tensor_at(ts, i);
+static void tensor_read(const std::vector<TensorRef>& ts, int i, float* out_host, cudaStream_t st) {
+  tensor_read(tensor_at(ts, i), out_host, st);
+}
+static void tensor_write(const TensorRef& t, const float* in_host, cudaStream_t st) {
   RLREP_CHECK(in_host != nullptr, "null argument");
   RLREP_CUDA(cudaMemcpy2DAsync(t.ptr, (size_t)t.ld * 4, in_host, (size_t)t.cols * 4, (size_t)t.cols * 4, t.rows,
                                cudaMemcpyHostToDevice, st));
   RLREP_CUDA(cudaStreamSynchronize(st));
+}
+static void tensor_write(const std::vector<TensorRef>& ts, int i, const float* in_host, cudaStream_t st) {
+  tensor_write(tensor_at(ts, i), in_host, st);
 }
 
 struct rlrep_agent {
@@ -1001,9 +1005,7 @@ int rlrep_agent_create_sharded(const rlrep_agent_config* c, rlrep_comm* comm, vo
   return create_agent(c, comm, stream, out);
 }
 
-static int create_agent(const rlrep_agent_config* c, rlrep_comm* comm, void* stream, rlrep_agent** out) {
-  RLREP_API_BEGIN
-  RLREP_CHECK(c != nullptr && out != nullptr, "null argument");
+static AgentConfig agent_config(const rlrep_agent_config* c) {
   AgentConfig a;
   a.alg = c->alg;
   a.state_dim = c->state_dim; a.action_dim = c->action_dim; a.batch = c->batch_size;
@@ -1023,14 +1025,27 @@ static int create_agent(const rlrep_agent_config* c, rlrep_comm* comm, void* str
   a.num_noise = c->num_noise; a.num_noises = c->num_noises;
   a.sigma_scale = c->sigma_scale_factor;
   RLREP_CHECK(a.target_update_period > 0, "target_update_period must be positive");
-  std::unique_ptr<rlrep_agent> h(new rlrep_agent);
+  return a;
+}
+
+// The handle runs on `stream`; the legacy default stream cannot be captured into a CUDA graph, so for a null `stream` the
+// handle gets a private one.  Every entry point that hands results back to the host synchronises it, so callers never
+// observe the difference.
+static cudaStream_t handle_stream(rlrep_agent* h, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (st == nullptr) {
-    // The legacy default stream cannot be captured into a CUDA graph: give the handle a private stream.  Every
-    // entry point that hands results back to the host synchronises it, so callers never observe the difference.
     RLREP_CUDA(cudaStreamCreateWithFlags(&h->owned_stream, cudaStreamNonBlocking));
     st = h->owned_stream;
   }
+  return st;
+}
+
+static int create_agent(const rlrep_agent_config* c, rlrep_comm* comm, void* stream, rlrep_agent** out) {
+  RLREP_API_BEGIN
+  RLREP_CHECK(c != nullptr && out != nullptr, "null argument");
+  const AgentConfig a = agent_config(c);
+  std::unique_ptr<rlrep_agent> h(new rlrep_agent);
+  cudaStream_t st = handle_stream(h.get(), stream);
   if (comm != nullptr) {
     RLREP_CHECK(a.alg == RLREP_ALG_CTRLSAC, "batch sharding is implemented for ctrlsac (the path with a B x B exchange)");
     h->impl = make_ctrlsac_sharded_agent(a, st, comm->impl.get());
@@ -1205,6 +1220,164 @@ int rlrep_agent_profile_train(rlrep_agent* agent, rlrep_ring* ring, const int64_
 int rlrep_agent_sync_targets(rlrep_agent* agent) {
   RLREP_API_BEGIN_ON(agent)
   agent->impl->sync_targets_from_params();
+  RLREP_API_END
+}
+
+// ------------------------------------------------------------------------------------------------ SAC populations
+struct rlrep_sacpop : rlrep_agent {};
+
+static Members pop_members(rlrep_sacpop* p) { return p->impl->mb; }
+static void check_member(rlrep_sacpop* p, int member) {
+  RLREP_CHECK(member >= 0 && member < pop_members(p).n, "member index out of range");
+}
+static TensorRef member_tensor(rlrep_sacpop* p, int member, int i) {
+  check_member(p, member);
+  TensorRef t = tensor_at(p->tensors, i);
+  t.ptr = member_ptr(t.ptr, member * pop_members(p).stride);
+  return t;
+}
+static Control* member_control(rlrep_sacpop* p, int member) {
+  check_member(p, member);
+  return member_ptr(p->impl->ctl, member * pop_members(p).stride);
+}
+static std::vector<Ring*> member_rings(rlrep_sacpop* p, rlrep_ring* const* rings, int n_rings) {
+  RLREP_CHECK(n_rings == pop_members(p).n, "one ring per member");
+  std::vector<Ring*> out(n_rings);
+  for (int m = 0; m < n_rings; ++m) {
+    RLREP_CHECK(rings[m] != nullptr, "null argument");
+    out[m] = rings[m]->impl.get();
+  }
+  return out;
+}
+
+int rlrep_sacpop_create(const rlrep_agent_config* c, int members, void* stream, rlrep_sacpop** out) {
+  RLREP_API_BEGIN
+  RLREP_CHECK(c != nullptr && out != nullptr, "null argument");
+  RLREP_CHECK(c->alg == RLREP_ALG_SAC, "populations are implemented for sac");
+  RLREP_CHECK(members >= 1, "a population needs at least one member");
+  const AgentConfig a = agent_config(c);
+  std::unique_ptr<rlrep_sacpop> h(new rlrep_sacpop);
+  cudaStream_t st = handle_stream(h.get(), stream);
+  h->impl = make_sac_population(a, st, members);
+  index_tensors(h.get());
+  *out = h.release();
+  RLREP_API_END
+}
+int rlrep_sacpop_destroy(rlrep_sacpop* pop) {
+  RLREP_API_BEGIN_ON(pop)
+  if (pop && pop->impl) cudaStreamSynchronize(pop->impl->stream);
+  if (pop) {
+    pop->impl.reset();
+    if (pop->owned_stream) cudaStreamDestroy(pop->owned_stream);
+  }
+  delete pop;
+  RLREP_API_END
+}
+int rlrep_sacpop_members(rlrep_sacpop* pop, int* members) {
+  RLREP_API_BEGIN_ON(pop)
+  RLREP_CHECK(pop && members, "null argument");
+  *members = pop_members(pop).n;
+  RLREP_API_END
+}
+int rlrep_sacpop_num_tensors(rlrep_sacpop* pop, int* n) { return rlrep_agent_num_tensors(pop, n); }
+int rlrep_sacpop_tensor_info(rlrep_sacpop* pop, int member, int i, const char** name, float** ptr_dev, int* rows,
+                             int* cols) {
+  RLREP_API_BEGIN_ON(pop)
+  RLREP_CHECK(pop, "null argument");
+  const TensorRef t = member_tensor(pop, member, i);
+  if (name) *name = tensor_at(pop->tensors, i).name.c_str();
+  if (ptr_dev) *ptr_dev = t.ptr;
+  if (rows) *rows = t.rows;
+  if (cols) *cols = t.cols;
+  RLREP_API_END
+}
+int rlrep_sacpop_tensor_read(rlrep_sacpop* pop, int member, int i, float* out_host) {
+  RLREP_API_BEGIN_ON(pop)
+  RLREP_CHECK(pop && out_host, "null argument");
+  tensor_read(member_tensor(pop, member, i), out_host, pop->impl->stream);
+  RLREP_API_END
+}
+int rlrep_sacpop_tensor_write(rlrep_sacpop* pop, int member, int i, const float* in_host) {
+  RLREP_API_BEGIN_ON(pop)
+  RLREP_CHECK(pop && in_host, "null argument");
+  tensor_write(member_tensor(pop, member, i), in_host, pop->impl->stream);
+  RLREP_API_END
+}
+int rlrep_sacpop_sync_targets(rlrep_sacpop* pop) {
+  RLREP_API_BEGIN_ON(pop)
+  RLREP_CHECK(pop, "null argument");
+  pop->impl->sync_targets_from_params();
+  RLREP_API_END
+}
+int rlrep_sacpop_get_optim_state(rlrep_sacpop* pop, int member, rlrep_optim_state* out) {
+  RLREP_API_BEGIN_ON(pop)
+  RLREP_CHECK(pop && out, "null argument");
+  Control h;
+  RLREP_CUDA(cudaMemcpyAsync(&h, member_control(pop, member), sizeof(h), cudaMemcpyDeviceToHost, pop->impl->stream));
+  RLREP_CUDA(cudaStreamSynchronize(pop->impl->stream));
+  out->steps = h.steps;
+  out->t_feature = h.t_feat; out->t_critic = h.t_critic; out->t_actor = h.t_actor; out->t_alpha = h.t_alpha;
+  out->log_alpha = h.log_alpha; out->log_alpha_m = h.la_m; out->log_alpha_v = h.la_v;
+  RLREP_API_END
+}
+int rlrep_sacpop_set_optim_state(rlrep_sacpop* pop, int member, const rlrep_optim_state* in) {
+  RLREP_API_BEGIN_ON(pop)
+  RLREP_CHECK(pop && in, "null argument");
+  Control* c = member_control(pop, member);
+  cudaStream_t st = pop->impl->stream;
+  Control h;
+  RLREP_CUDA(cudaMemcpyAsync(&h, c, sizeof(h), cudaMemcpyDeviceToHost, st));
+  RLREP_CUDA(cudaStreamSynchronize(st));
+  h.steps = in->steps;
+  h.t_feat = in->t_feature; h.t_critic = in->t_critic; h.t_actor = in->t_actor; h.t_alpha = in->t_alpha;
+  h.log_alpha = in->log_alpha; h.la_m = in->log_alpha_m; h.la_v = in->log_alpha_v;
+  h.alpha = (float)std::exp(in->log_alpha);
+  RLREP_CUDA(cudaMemcpyAsync(c, &h, sizeof(h), cudaMemcpyHostToDevice, st));
+  RLREP_CUDA(cudaStreamSynchronize(st));
+  RLREP_API_END
+}
+int rlrep_sacpop_train_counts(rlrep_sacpop* pop, int* n_idx, int* n_eps, int* n_metrics) {
+  RLREP_API_BEGIN_ON(pop)
+  RLREP_CHECK(pop && n_idx && n_eps && n_metrics, "null argument");
+  *n_idx = pop->impl->idx_per_train();
+  *n_eps = pop->impl->eps_per_train();
+  *n_metrics = (int)pop->impl->metric_names().size();
+  RLREP_API_END
+}
+const char* rlrep_sacpop_metric_name(rlrep_sacpop* pop, int i) {
+  if (pop == nullptr) {
+    set_last_error("null argument");
+    return nullptr;
+  }
+  return rlrep_agent_metric_name(pop, i);
+}
+int rlrep_sacpop_train(rlrep_sacpop* pop, rlrep_ring* const* rings, int n_rings, const int64_t* idx_host, int n_idx,
+                       const float* eps, int n_eps, float* metrics_host, int n_metrics) {
+  RLREP_API_BEGIN_ON(pop)
+  RLREP_CHECK(pop && rings && idx_host && eps && metrics_host, "null argument");
+  const std::vector<Ring*> r = member_rings(pop, rings, n_rings);
+  pop->impl->train_members(r.data(), reinterpret_cast<const long long*>(idx_host), n_idx, eps, n_eps, metrics_host,
+                           n_metrics);
+  RLREP_API_END
+}
+int rlrep_sacpop_act(rlrep_sacpop* pop, const float* states_host, const float* eps_host, float* actions_host) {
+  RLREP_API_BEGIN_ON(pop)
+  RLREP_CHECK(pop && states_host && actions_host, "null argument");
+  pop->impl->act_members(states_host, eps_host, actions_host);
+  RLREP_API_END
+}
+int rlrep_sacpop_train_resident(rlrep_sacpop* pop, rlrep_ring* const* rings, int n_rings, const int64_t* idx_host,
+                                const float* eps_host, int n_steps, float* total_ms) {
+  RLREP_API_BEGIN_ON(pop)
+  RLREP_CHECK(pop && rings && idx_host && eps_host && total_ms, "null argument");
+  const std::vector<Ring*> r = member_rings(pop, rings, n_rings);
+  *total_ms = pop->impl->train_resident_members(r.data(), reinterpret_cast<const long long*>(idx_host), eps_host, n_steps);
+  RLREP_API_END
+}
+int rlrep_sacpop_last_launches(rlrep_sacpop* pop, int* launches) {
+  RLREP_API_BEGIN_ON(pop)
+  RLREP_CHECK(pop && launches, "null argument");
+  *launches = pop->impl->last_launches;
   RLREP_API_END
 }
 

@@ -11,6 +11,8 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include "members.cuh"
+
 namespace rlrep {
 
 enum Act : int { ACT_NONE = 0, ACT_ELU = 1, ACT_RELU = 2, ACT_TANH = 3, ACT_SIN = 4 };
@@ -31,6 +33,16 @@ struct Epilogue {
   int accumulate = 0;
   float scale = 1.0f;
 };
+
+// The epilogue of a population member: every operand pointer moved by `off` bytes (members.cuh).
+__host__ __device__ __forceinline__ Epilogue member_epilogue(Epilogue e, long long off) {
+  e.bias = member_ptr(e.bias, off);
+  e.r1_u = member_ptr(e.r1_u, off);
+  e.r1_v = member_ptr(e.r1_v, off);
+  e.aux = member_ptr(e.aux, off);
+  e.pre_out = member_ptr(e.pre_out, off);
+  return e;
+}
 
 __device__ __forceinline__ float apply_act(float v, int act) {
   switch (act) {

@@ -62,6 +62,9 @@ struct GemmArgs {
   float* C = nullptr;
   int ldc = 0;
   Epilogue epi;
+  // Population GEMM (members.cuh): mb.n independent GEMMs of this shape in one launch, member m's operands, output and
+  // epilogue operands at mb.stride * m bytes from the ones given here.  Plain one-tile-per-CTA GEMMs only.
+  Members mb;
 };
 
 // ---- tcgen05 path (TF32 inputs, FP32 accumulate in TMEM, TMA-fed) ----

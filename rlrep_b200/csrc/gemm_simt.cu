@@ -32,7 +32,19 @@ struct SimtParams {
   long long sbn, sbk;  // B(n,k) = B[n*sbn + k*sbk]
   float* C;
   long long scm, scn;  // C(m,n) = C[m*scm + n*scn]
+  long long mstride;   // population GEMM (members.cuh): bytes between consecutive members' operands
 };
+// The operands of member blockIdx.z (members.cuh).
+template <bool MEMBERS>
+__device__ __forceinline__ SimtParams member_params(SimtParams p, Epilogue& epi) {
+  const long long off = member_offset<MEMBERS>(p.mstride);
+  p.A = member_ptr(p.A, off);
+  p.A2 = member_ptr(p.A2, off);
+  p.B = member_ptr(p.B, off);
+  p.C = member_ptr(p.C, off);
+  epi = member_epilogue(epi, off);
+  return p;
+}
 
 template <int ACT, int DACT>
 __device__ __forceinline__ void store_micro_tile(const SimtParams& p, const Epilogue& epi, const float (&acc)[4][4], int m0,
@@ -56,7 +68,10 @@ __device__ __forceinline__ void store_one(const Epilogue& epi, float v, int m, i
 }
 
 // ------------------------------------------------------------------------------------------------ tiled
-__global__ void __launch_bounds__(256) gemm_tiled_kernel(const SimtParams p, const Epilogue epi) {
+template <bool MEMBERS>
+__device__ __forceinline__ void gemm_tiled(const SimtParams& pm, const Epilogue& epi_in) {
+  Epilogue epi = epi_in;
+  const SimtParams p = member_params<MEMBERS>(pm, epi);
   __shared__ __align__(16) float As[TBK][TBM + 4];
   __shared__ __align__(16) float Bs[TBK][TBN + 4];
   const int tid = threadIdx.x;
@@ -128,7 +143,10 @@ __global__ void __launch_bounds__(256) gemm_tiled_kernel(const SimtParams p, con
 
 // ------------------------------------------------------------------------------------------------ skinny: warp per row
 // One output at a time: both operand streams advance by a constant stride, so the inner loop is two loads and an FMA.
-__global__ void __launch_bounds__(256) skinny_rowwarp_kernel(const SimtParams p, const Epilogue epi) {
+template <bool MEMBERS>
+__device__ __forceinline__ void skinny_rowwarp(const SimtParams& pm, const Epilogue& epi_in) {
+  Epilogue epi = epi_in;
+  const SimtParams p = member_params<MEMBERS>(pm, epi);
   const int m = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (m >= p.M) return;
   const float* arow = p.A + (long long)m * p.sam;
@@ -157,8 +175,10 @@ __global__ void __launch_bounds__(256) skinny_rowwarp_kernel(const SimtParams p,
 
 // ------------------------------------------------------------------------------------------------ skinny: thread per row
 // B must be contiguous in n (sbn == 1): the N loads of a k-step then use immediate offsets from one base pointer.
-template <int NT>
-__global__ void __launch_bounds__(256) skinny_rowthread_kernel(const SimtParams p, const Epilogue epi, int swapped) {
+template <int NT, bool MEMBERS>
+__device__ __forceinline__ void skinny_rowthread(const SimtParams& pm, const Epilogue& epi_in, int swapped) {
+  Epilogue epi = epi_in;
+  const SimtParams p = member_params<MEMBERS>(pm, epi);
   __shared__ float red[8][32][NT + 1];
   const int lane = threadIdx.x & 31, slice = threadIdx.x >> 5;
   const int m = blockIdx.x * 32 + lane;
@@ -198,13 +218,36 @@ __global__ void __launch_bounds__(256) skinny_rowthread_kernel(const SimtParams 
   }
 }
 
-void launch_rowwarp(const SimtParams& p, const Epilogue& e, cudaStream_t s) {
-  skinny_rowwarp_kernel<<<ceil_div(p.M * 32, 256), 256, 0, s>>>(p, e);
+// The kernels: the lone form, and the population form (SimtParams::mstride, member = blockIdx.z).
+__global__ void __launch_bounds__(256) gemm_tiled_kernel(const SimtParams p, const Epilogue epi) {
+  gemm_tiled<false>(p, epi);
+}
+__global__ void __launch_bounds__(256) gemm_tiled_members_kernel(const SimtParams p, const Epilogue epi) {
+  gemm_tiled<true>(p, epi);
+}
+__global__ void __launch_bounds__(256) skinny_rowwarp_kernel(const SimtParams p, const Epilogue epi) {
+  skinny_rowwarp<false>(p, epi);
+}
+__global__ void __launch_bounds__(256) skinny_rowwarp_members_kernel(const SimtParams p, const Epilogue epi) {
+  skinny_rowwarp<true>(p, epi);
+}
+template <int NT>
+__global__ void __launch_bounds__(256) skinny_rowthread_kernel(const SimtParams p, const Epilogue epi, int swapped) {
+  skinny_rowthread<NT, false>(p, epi, swapped);
+}
+template <int NT>
+__global__ void __launch_bounds__(256) skinny_rowthread_members_kernel(const SimtParams p, const Epilogue epi, int swapped) {
+  skinny_rowthread<NT, true>(p, epi, swapped);
+}
+
+void launch_rowwarp(const SimtParams& p, const Epilogue& e, int members, cudaStream_t s) {
+  (members > 1 ? skinny_rowwarp_members_kernel : skinny_rowwarp_kernel)<<<dim3(ceil_div(p.M * 32, 256), 1, members), 256, 0, s>>>(p, e);
   RLREP_LAUNCHED_W("skinny_rowwarp", s, 4.0 * ((double)p.M * p.K + (double)p.N * p.K + (double)p.M * p.N), 2.0 * p.M * p.N * p.K);
 }
 template <int NT>
-void launch_rowthread(const SimtParams& p, const Epilogue& e, int swapped, cudaStream_t s) {
-  skinny_rowthread_kernel<NT><<<ceil_div(p.M, 32), 256, 0, s>>>(p, e, swapped);
+void launch_rowthread(const SimtParams& p, const Epilogue& e, int swapped, int members, cudaStream_t s) {
+  (members > 1 ? skinny_rowthread_members_kernel<NT> : skinny_rowthread_kernel<NT>)<<<dim3(ceil_div(p.M, 32), 1, members), 256, 0, s>>>(
+      p, e, swapped);
   RLREP_LAUNCHED_W("skinny_rowthread", s, 4.0 * ((double)p.M * p.K + (double)p.N * p.K + (double)p.M * p.N), 2.0 * p.M * p.N * p.K);
 }
 
@@ -229,15 +272,17 @@ void launch_simt(const GemmArgs& a, cudaStream_t stream) {
   p.C = a.C;
   p.scm = a.ldc;
   p.scn = 1;
+  p.mstride = a.mb.stride;
+  const int nm = a.mb.n;
   const bool plain_epi = a.epi.pre_out == nullptr;  // pre_out uses (m, n) addressing the skinny kernels do not remap
   if (a.A2 == nullptr && plain_epi && a.N <= 32 && !a.a_mn && a.K >= 64 && a.conv_w == 0) {
-    launch_rowwarp(p, a.epi, stream);
+    launch_rowwarp(p, a.epi, nm, stream);
     return;
   }
   if (a.A2 == nullptr && plain_epi && a.N <= 32 && a.a_mn && a.b_mn && a.M >= 64) {
-    if (a.N <= 8) launch_rowthread<8>(p, a.epi, 0, stream);
-    else if (a.N <= 16) launch_rowthread<16>(p, a.epi, 0, stream);
-    else launch_rowthread<32>(p, a.epi, 0, stream);
+    if (a.N <= 8) launch_rowthread<8>(p, a.epi, 0, nm, stream);
+    else if (a.N <= 16) launch_rowthread<16>(p, a.epi, 0, nm, stream);
+    else launch_rowthread<32>(p, a.epi, 0, nm, stream);
     return;
   }
   if (a.A2 == nullptr && plain_epi && a.M <= 32 && a.a_mn && a.b_mn && a.N >= 64) {
@@ -247,13 +292,13 @@ void launch_simt(const GemmArgs& a, cudaStream_t stream) {
     q.A = a.B; q.sam = 1; q.sak = a.ldb;
     q.B = a.A; q.sbn = 1; q.sbk = a.lda;
     q.scm = 1; q.scn = a.ldc;
-    if (q.N <= 8) launch_rowthread<8>(q, a.epi, 1, stream);
-    else if (q.N <= 16) launch_rowthread<16>(q, a.epi, 1, stream);
-    else launch_rowthread<32>(q, a.epi, 1, stream);
+    if (q.N <= 8) launch_rowthread<8>(q, a.epi, 1, nm, stream);
+    else if (q.N <= 16) launch_rowthread<16>(q, a.epi, 1, nm, stream);
+    else launch_rowthread<32>(q, a.epi, 1, nm, stream);
     return;
   }
-  dim3 grid(ceil_div(a.N, TBN), ceil_div(a.M, TBM));
-  gemm_tiled_kernel<<<grid, 256, 0, stream>>>(p, a.epi);
+  dim3 grid(ceil_div(a.N, TBN), ceil_div(a.M, TBM), nm);
+  (nm > 1 ? gemm_tiled_members_kernel : gemm_tiled_kernel)<<<grid, 256, 0, stream>>>(p, a.epi);
   RLREP_LAUNCHED_W("gemm_simt", stream, 4.0 * ((double)p.M * p.K + (double)p.N * p.K + (double)p.M * p.N), 2.0 * p.M * p.N * p.K);
 }
 

@@ -42,13 +42,14 @@ EncodeTiledFn get_encode_fn() {
 }
 
 // K-major operand: tensor map over a row-major fp32 matrix [rows, K] with leading dimension ld; box = box_rows x 32.
-CUtensorMap make_map_kmajor(const float* base, int rows, int cols, int ld, int box_rows) {
+// A population's operand (mb.n > 1) gets the member as a third, outermost dimension of stride mb.stride bytes.
+CUtensorMap make_map_kmajor(const float* base, int rows, int cols, int ld, int box_rows, const Members& mb = Members()) {
   CUtensorMap m;
-  cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t gstride[1] = {(cuuint64_t)ld * 4};
-  cuuint32_t box[2] = {32u, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1u, 1u};
-  CUresult r = get_encode_fn()(&m, CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, 2, const_cast<float*>(base), gdim, gstride, box,
+  cuuint64_t gdim[3] = {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)mb.n};
+  cuuint64_t gstride[2] = {(cuuint64_t)ld * 4, (cuuint64_t)mb.stride};
+  cuuint32_t box[3] = {32u, (cuuint32_t)box_rows, 1u};
+  cuuint32_t estr[3] = {1u, 1u, 1u};
+  CUresult r = get_encode_fn()(&m, CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, mb.n > 1 ? 3 : 2, const_cast<float*>(base), gdim, gstride, box,
                                estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                                CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   RLREP_CHECK(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed with CUresult " + std::to_string((int)r));
@@ -59,13 +60,13 @@ CUtensorMap make_map_kmajor(const float* base, int rows, int cols, int ld, int b
 // instruction fetches all the 32-wide boxes of a tile: box = {32, 32, tile_mn / 32}.  Elements with mn >= the real
 // extent alias the next k-row (never out of the allocation as long as K*ld floats are readable plus the arena's
 // padding); they only feed output rows / columns that are never stored.
-CUtensorMap make_map_mnmajor(const float* base, int K, int mn, int ld, int tile_mn) {
+CUtensorMap make_map_mnmajor(const float* base, int K, int mn, int ld, int tile_mn, const Members& mb = Members()) {
   CUtensorMap m;
-  cuuint64_t gdim[3] = {32u, (cuuint64_t)K, (cuuint64_t)((mn + 31) / 32)};
-  cuuint64_t gstride[2] = {(cuuint64_t)ld * 4, 128u};
-  cuuint32_t box[3] = {32u, 32u, (cuuint32_t)(tile_mn / 32)};
-  cuuint32_t estr[3] = {1u, 1u, 1u};
-  CUresult r = get_encode_fn()(&m, CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, 3, const_cast<float*>(base), gdim, gstride, box,
+  cuuint64_t gdim[4] = {32u, (cuuint64_t)K, (cuuint64_t)((mn + 31) / 32), (cuuint64_t)mb.n};
+  cuuint64_t gstride[3] = {(cuuint64_t)ld * 4, 128u, (cuuint64_t)mb.stride};
+  cuuint32_t box[4] = {32u, 32u, (cuuint32_t)(tile_mn / 32), 1u};
+  cuuint32_t estr[4] = {1u, 1u, 1u, 1u};
+  CUresult r = get_encode_fn()(&m, CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, mb.n > 1 ? 4 : 3, const_cast<float*>(base), gdim, gstride, box,
                                estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B,
                                CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   RLREP_CHECK(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled (3-D) failed with CUresult " + std::to_string((int)r));
@@ -232,6 +233,16 @@ TcGemmPlan make_tc_plan(const GemmArgs& a, int bn, int split_k, float* /*ws*/, s
     if (plain && a.conv_w > 0 && p.persistent && p.bn == 32 && a.N <= 32 && rows <= 256) p.halo_rows = rows;
   }
   // (a compacting GEMM whose plan has no halo is refused by GemmRunner::run_compact before anything is launched)
+  // A population GEMM runs the plan a lone agent gets for this shape -- member m then computes exactly what that agent
+  // computes -- on the one-tile-per-CTA kernel, with the member as the outermost dimension of both tensor maps.
+  RLREP_CHECK(a.mb.n == 1 || (a.mb.n > 1 && a.mb.stride > 0 && a.mb.stride % 16 == 0 && !p.persistent && p.halo_rows == 0 &&
+                              p.k_groups == 1 && a.conv_w == 0 && a.conv_wgrad_hi == 0),
+              "population GEMMs: plain one-tile-per-CTA GEMMs with a 16-byte member stride only");
+  if (a.mb.n > 1) {
+    p.tmA = a.a_mn ? make_map_mnmajor(a.A, a.K, a.M, a.lda, BM, a.mb) : make_map_kmajor(a.A, a.M, a.K, a.lda, BM, a.mb);
+    p.tmB = a.b_mn ? make_map_mnmajor(a.B, a.K, a.N, a.ldb, p.bn, a.mb) : make_map_kmajor(a.B, a.N, a.K, a.ldb, p.bn, a.mb);
+    return p;
+  }
   p.tmA = a.a_mn ? make_map_mnmajor(a.A, a.K, a.M, a.lda, BM)
                  : make_map_kmajor(a.A, a.M, a.conv_w > 0 ? 32 : a.K, a.lda, p.halo_rows > 0 ? p.halo_rows : BM);
   {

@@ -292,11 +292,11 @@ __device__ __forceinline__ bool store_tile(const TileStore& t, const Epilogue* e
   return arrived;
 }
 
-template <int BN, bool A_MN, bool B_MN>
-__global__ void __launch_bounds__(kThreads, 1)
-gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                 float* __restrict__ C, int ldc, int M, int N, int K, int kb_per_split, int stages, int push, int conv_w,
-                 const Epilogue epi) {
+// Body of gemm_tf32_kernel and of its population form gemm_tf32_members_kernel (MEMBERS, GemmArgs::mb).
+template <int BN, bool A_MN, bool B_MN, bool MEMBERS>
+__device__ __forceinline__ void gemm_tf32_body(const CUtensorMap& tmA, const CUtensorMap& tmB, float* __restrict__ C,
+                                               int ldc, int M, int N, int K, int kb_per_split, int stages, int push,
+                                               int conv_w, const Epilogue& epi, long long mstride) {
   // `stages` is a launch parameter: short K-slices run with a shallow ring so that two CTAs (of this or of a
   // concurrent GEMM on another stream) fit on one SM; long ones get the deepest ring that fits.
   const int STAGES = stages;
@@ -329,7 +329,11 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   const int lane = threadIdx.x & 31;
   if (threadIdx.x == 0) trace(0);
   const int n0 = blockIdx.x * BN;
-  const int m0 = blockIdx.y * BM;
+  // population GEMM (MEMBERS): gridDim.y = members x M-tiles, and the tensor maps have the member as their outermost
+  // dimension (GemmArgs::mb)
+  const int member = MEMBERS ? blockIdx.y / ((M + BM - 1) / BM) : 0;
+  const int m0 = (blockIdx.y - member * ((M + BM - 1) / BM)) * BM;
+  if constexpr (MEMBERS) C = member_ptr(C, member * mstride);
   const int splits = gridDim.z / groups;
   if (groups > 1) C += (size_t)(blockIdx.z / splits) * (size_t)(((M + BM - 1) / BM) * BM) * ldc;
   const int nkb_total = (K + BK - 1) / BK;
@@ -346,6 +350,13 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     uint8_t* b_dst = sB + s * B_BYTES;
     // MN-major operands: one 3-D box {32 (m % 32), 32 (k), rows / 32 (m / 32)} lands as consecutive 4 KB sub-boxes
     // implicit convolution (conv_w > 0): k-block t is tap (t / 3, t % 3) -- the same 32 channels, rows shifted on the grid
+    if constexpr (MEMBERS) {
+      if (!A_MN) ptx::tma_load_3d(a_dst, &tmA, &full_bar[s], k0, m0, member);
+      else ptx::tma_load_4d(a_dst, &tmA, &full_bar[s], 0, k0, m0 / 32, member);
+      if (!B_MN) ptx::tma_load_3d(b_dst, &tmB, &full_bar[s], k0, n0, member);
+      else ptx::tma_load_4d(b_dst, &tmB, &full_bar[s], 0, k0, n0 / 32, member);
+      return;
+    }
     if (!A_MN) {
       const int t = kb_begin + it;
       if (conv_w > 0) ptx::tma_load_2d(a_dst, &tmA, &full_bar[s], 0, m0 + (t / 3) * conv_w + (t % 3));
@@ -480,7 +491,13 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     t.row_bias = push ? 0 : t.row0;
     t.m0 = m0; t.n0 = n0; t.M = M; t.N = N;
     t.C = C; t.ldc = ldc;
-    const bool arrived = store_tile(t, &epi);
+    bool arrived;
+    if constexpr (MEMBERS) {
+      const Epilogue em = member_epilogue(epi, member * mstride);
+      arrived = store_tile(t, &em);
+    } else {
+      arrived = store_tile(t, &epi);
+    }
     if (threadIdx.x == 0) trace(7);
     if (splits > 1 && !push) {  // peers may still be reading this CTA's staging tile: do not exit before they are done
       if (!arrived) ptx::cluster_arrive_relaxed();
@@ -489,6 +506,22 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   }
 
   if (threadIdx.x == 64) trace(8);
+}
+
+template <int BN, bool A_MN, bool B_MN>
+__global__ void __launch_bounds__(kThreads, 1)
+gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
+                 float* __restrict__ C, int ldc, int M, int N, int K, int kb_per_split, int stages, int push, int conv_w,
+                 const Epilogue epi) {
+  gemm_tf32_body<BN, A_MN, B_MN, false>(tmA, tmB, C, ldc, M, N, K, kb_per_split, stages, push, conv_w, epi, 0);
+}
+// mstride bytes between consecutive members' operands, output and epilogue operands; gridDim.y = members x M-tiles
+template <int BN, bool A_MN, bool B_MN>
+__global__ void __launch_bounds__(kThreads, 1)
+gemm_tf32_members_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
+                         float* __restrict__ C, int ldc, int M, int N, int K, int kb_per_split, int stages, int push,
+                         int conv_w, const Epilogue epi, long long mstride) {
+  gemm_tf32_body<BN, A_MN, B_MN, true>(tmA, tmB, C, ldc, M, N, K, kb_per_split, stages, push, conv_w, epi, mstride);
 }
 
 // 32 x 32 chunk of the persistent kernel's epilogue: rows come out of the warp's transpose buffer, lanes cover four rows x
@@ -991,10 +1024,11 @@ void launch_variant_persistent(const TcGemmPlan& p, cudaStream_t stream) {
 template <int BN, bool A_MN, bool B_MN>
 void fill_launch_config(cudaLaunchConfig_t& cfg, cudaLaunchAttribute* attr, dim3 grid, int split_k, int stages,
                         bool push, cudaStream_t stream) {
-  auto kern = gemm_tf32_kernel<BN, A_MN, B_MN>;
   static bool attr_set = false;  // per template instantiation
   if (!attr_set) {
-    RLREP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem));
+    RLREP_CUDA(cudaFuncSetAttribute(gemm_tf32_kernel<BN, A_MN, B_MN>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem));
+    RLREP_CUDA(cudaFuncSetAttribute(gemm_tf32_members_kernel<BN, A_MN, B_MN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    kMaxSmem));
     attr_set = true;
   }
   cfg = {};
@@ -1018,20 +1052,23 @@ void launch_variant(const TcGemmPlan& p, cudaStream_t stream) {
   RLREP_CHECK(!p.push || (p.split_k > 1 && smem_bytes(BN, p.stages, true) <= kMaxSmem), "bad push-mode plan");
   cudaLaunchConfig_t cfg;
   cudaLaunchAttribute attr[2];
-  fill_launch_config<BN, A_MN, B_MN>(cfg, attr, dim3(ceil_div(a.N, BN), ceil_div(a.M, BM), p.split_k * p.k_groups),
+  fill_launch_config<BN, A_MN, B_MN>(cfg, attr, dim3(ceil_div(a.N, BN), ceil_div(a.M, BM) * a.mb.n, p.split_k * p.k_groups),
                                      p.split_k, p.stages, p.push, stream);
   attr[1] = pdl_attribute();
   cfg.numAttrs = 2;
-  RLREP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tf32_kernel<BN, A_MN, B_MN>, p.tmA, p.tmB, a.C, a.ldc, a.M, a.N, a.K,
-                                p.kb_per_split, p.stages,
-                                (p.push ? 1 : 0) | ((p.k_groups - 1) << 8),
-                                a.conv_wgrad_hi > 0 ? -1 : a.conv_w, a.epi));
+  const int push = (p.push ? 1 : 0) | ((p.k_groups - 1) << 8);
+  if (a.mb.n > 1)
+    RLREP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tf32_members_kernel<BN, A_MN, B_MN>, p.tmA, p.tmB, a.C, a.ldc, a.M, a.N, a.K,
+                                  p.kb_per_split, p.stages, push, a.conv_w, a.epi, a.mb.stride));
+  else
+    RLREP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tf32_kernel<BN, A_MN, B_MN>, p.tmA, p.tmB, a.C, a.ldc, a.M, a.N, a.K,
+                                  p.kb_per_split, p.stages, push, a.conv_wgrad_hi > 0 ? -1 : a.conv_w, a.epi));
   g_trace_reader = &read_trace_here;
   // implicit convolution: A is the [M, 32] pixel matrix, read once from HBM (the nine shifted re-reads hit L2)
   RLREP_LAUNCHED_W("gemm_tf32", stream,
-                   4.0 * ((double)a.M * (a.conv_w > 0 ? 32 : a.K) + (double)(a.conv_wgrad_hi > 0 ? 128 : a.N) * a.K +
-                          (double)a.M * a.N),
-                   2.0 * a.M * a.N * a.K);
+                   4.0 * a.mb.n * ((double)a.M * (a.conv_w > 0 ? 32 : a.K) + (double)(a.conv_wgrad_hi > 0 ? 128 : a.N) * a.K +
+                                   (double)a.M * a.N),
+                   2.0 * a.M * a.N * a.K * a.mb.n);
 }
 
 // How many clusters of `split_k` CTAs of this variant the GPU can hold at once (occupancy API; clusters must fit in

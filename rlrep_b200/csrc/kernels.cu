@@ -22,13 +22,15 @@ __device__ __forceinline__ AdamHyper adam_hyper(double lr, long long t) {
   return h;
 }
 
-__global__ void tick_kernel(Control* c, const TickParams p) {
+template <bool MEMBERS>
+__global__ void tick_kernel(Control* c, const TickParams p, long long mstride) {
   // One warp: every lane reads the counters, then each of the (k_feat + 5) independent results -- two double-precision
   // pow() each -- is computed by its own lane instead of one after the other (7.5 us -> ~2 us at the head of every update).
   ptx::pdl_wait();
   ptx::pdl_launch_dependents();
   const int lane = threadIdx.x;
   if (blockIdx.x != 0 || lane >= 32) return;
+  c = member_ptr(c, member_offset<MEMBERS>(mstride));
   const long long t_feat = c->t_feat, t_critic = c->t_critic, t_actor = c->t_actor, t_alpha = c->t_alpha;
   const int steps = c->steps + 1;
   const double log_alpha = c->log_alpha;
@@ -51,10 +53,15 @@ __global__ void tick_kernel(Control* c, const TickParams p) {
 }
 
 // ------------------------------------------------------------------------------------------- ring
+template <bool MEMBERS>
 __global__ void gather_kernel(const float4* __restrict__ ring, int rec4, const long long* __restrict__ idx, int B,
-                              float4* __restrict__ out) {
+                              float4* __restrict__ out, const float* const* ring_slot, long long mstride) {
   ptx::pdl_wait();
   ptx::pdl_launch_dependents();
+  const long long off = member_offset<MEMBERS>(mstride);
+  if constexpr (MEMBERS) ring = reinterpret_cast<const float4*>(*member_ptr(ring_slot, off));
+  idx = member_ptr(idx, off);
+  out = member_ptr(out, off);
   const int total = B * rec4;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
     const int b = i / rec4, c = i - b * rec4;
@@ -99,15 +106,18 @@ __global__ void __launch_bounds__(256) ce_rows_kernel(float* __restrict__ logits
 struct RowDotJobs {
   RowDotJob j[2];
 };
-__global__ void __launch_bounds__(128) rowdot_kernel(const RowDotJobs jobs, int rows) {
+template <bool MEMBERS>
+__global__ void __launch_bounds__(128) rowdot_kernel(const RowDotJobs jobs, int rows, long long mstride) {
   __shared__ float scratch[33];
+  const long long off = member_offset<MEMBERS>(mstride);
   const RowDotJob& jb = jobs.j[blockIdx.y];
+  const float* X = member_ptr(jb.X, off);
   const int row = blockIdx.x;
-  const float* x = jb.X + (size_t)row * jb.ld;
-  const float* w = jb.w;
+  const float* x = X + (size_t)row * jb.ld;
+  const float* w = member_ptr(jb.w, off);
   const int D = jb.D;
   float acc = 0.f;
-  if (((jb.ld | D) & 3) == 0 && ((reinterpret_cast<uintptr_t>(jb.X) | reinterpret_cast<uintptr_t>(w)) & 15) == 0) {
+  if (((jb.ld | D) & 3) == 0 && ((reinterpret_cast<uintptr_t>(X) | reinterpret_cast<uintptr_t>(w)) & 15) == 0) {
     const float4* x4 = reinterpret_cast<const float4*>(x);
     const float4* w4 = reinterpret_cast<const float4*>(w);
     float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
@@ -122,14 +132,17 @@ __global__ void __launch_bounds__(128) rowdot_kernel(const RowDotJobs jobs, int 
     for (int j = threadIdx.x; j < D; j += 128) acc = fmaf(x[j], __ldg(w + j), acc);
   }
   acc = block_sum<128>(acc, scratch);
-  if (threadIdx.x == 0) jb.y[row] = acc + (jb.b ? __ldg(jb.b) : 0.f);
+  if (threadIdx.x == 0) member_ptr(jb.y, off)[row] = acc + (jb.b ? __ldg(member_ptr(jb.b, off)) : 0.f);
 }
 
 // 32 columns x 8 row-slices per CTA; fixed-order smem reduction across the slices.
+template <bool MEMBERS>
 __global__ void __launch_bounds__(256) colreduce_kernel(const float* __restrict__ X, int ld, int rows, int cols,
                                                         const float* __restrict__ u, float* __restrict__ out,
-                                                        int accumulate) {
+                                                        int accumulate, long long mstride) {
   __shared__ float part[8][33];
+  const long long off = member_offset<MEMBERS>(mstride);
+  X = member_ptr(X, off); u = member_ptr(u, off); out = member_ptr(out, off);
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
   const int j = blockIdx.x * 32 + tx;
   float acc = 0.f;
@@ -238,17 +251,19 @@ struct ColJobs {
 };
 // 32 columns x 32 row-slices per 1024-thread CTA: at B = 256 every thread issues its 8 loads back to back (one
 // memory round trip for the whole reduction instead of 32 dependent-latency steps), then a fixed-order smem tree.
-__global__ void __launch_bounds__(1024) colreduce_multi_kernel(const ColJobs jobs) {
+template <bool MEMBERS>
+__global__ void __launch_bounds__(1024) colreduce_multi_kernel(const ColJobs jobs, long long mstride) {
   __shared__ float part[32][33];
   ptx::pdl_wait();
   ptx::pdl_launch_dependents();
+  const long long off = member_offset<MEMBERS>(mstride);
   const ColJob& jb = jobs.j[blockIdx.y];
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
   const int j = blockIdx.x * 32 + tx;
   if (blockIdx.x * 32 >= jb.cols) return;
   float acc = 0.f;
   if (j < jb.cols) {
-    const float* x = jb.X + j;
+    const float* x = member_ptr(jb.X, off) + j;
     int i = ty;
     for (; i + 7 * 32 < jb.rows; i += 8 * 32) {
       float v[8], w[8];
@@ -256,7 +271,7 @@ __global__ void __launch_bounds__(1024) colreduce_multi_kernel(const ColJobs job
       for (int q = 0; q < 8; ++q) v[q] = x[(size_t)(i + q * 32) * jb.ld];
       if (jb.u) {
 #pragma unroll
-        for (int q = 0; q < 8; ++q) w[q] = __ldg(jb.u + i + q * 32);
+        for (int q = 0; q < 8; ++q) w[q] = __ldg(member_ptr(jb.u, off) + i + q * 32);
 #pragma unroll
         for (int q = 0; q < 8; ++q) acc = fmaf(w[q], v[q], acc);
       } else {
@@ -266,7 +281,7 @@ __global__ void __launch_bounds__(1024) colreduce_multi_kernel(const ColJobs job
     }
     for (; i < jb.rows; i += 32) {
       const float v = x[(size_t)i * jb.ld];
-      acc = jb.u ? fmaf(__ldg(jb.u + i), v, acc) : acc + v;
+      acc = jb.u ? fmaf(__ldg(member_ptr(jb.u, off) + i), v, acc) : acc + v;
     }
   }
   part[ty][tx] = acc;
@@ -275,13 +290,16 @@ __global__ void __launch_bounds__(1024) colreduce_multi_kernel(const ColJobs job
     float t = 0.f;
 #pragma unroll
     for (int k = 0; k < 32; ++k) t += part[k][tx];
-    jb.out[j] = t;
+    member_ptr(jb.out, off)[j] = t;
   }
 }
 
+template <bool MEMBERS>
 __global__ void outer_dact_kernel(const float* __restrict__ u, const float* __restrict__ w, int rows, int cols,
                                   const float* __restrict__ aux, int ld_aux, int dact, float* __restrict__ out,
-                                  int ld_out) {
+                                  int ld_out, long long mstride) {
+  const long long off = member_offset<MEMBERS>(mstride);
+  u = member_ptr(u, off); w = member_ptr(w, off); aux = member_ptr(aux, off); out = member_ptr(out, off);
   const size_t total = (size_t)rows * cols;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
     const int r = (int)(i / cols), c = (int)(i - (size_t)r * cols);
@@ -402,15 +420,18 @@ constexpr float kLogStdMin = -5.f, kLogStdMax = 2.f;  // sac_agent.py:64
 struct ActorSampleJobs {
   ActorSampleJob j[2];
 };
-__global__ void actor_sample_kernel(const ActorSampleJobs jobs, int ld_head, int B, int A, int lda, int S) {
+template <bool MEMBERS>
+__global__ void actor_sample_kernel(const ActorSampleJobs jobs, int ld_head, int B, int A, int lda, int S,
+                                    long long mstride) {
   ptx::pdl_wait();
   ptx::pdl_launch_dependents();
   const ActorSampleJob& jb = jobs.j[blockIdx.y];
-  const float* __restrict__ head = jb.head;
-  const float* __restrict__ eps = jb.eps;
-  float* __restrict__ action = jb.action;
-  float* __restrict__ logp = jb.logp;
-  const float* __restrict__ obs = jb.obs;
+  const long long off = member_offset<MEMBERS>(mstride);
+  const float* __restrict__ head = member_ptr(jb.head, off);
+  const float* __restrict__ eps = member_ptr(jb.eps, off);
+  float* __restrict__ action = member_ptr(jb.action, off);
+  float* __restrict__ logp = member_ptr(jb.logp, off);
+  const float* __restrict__ obs = member_ptr(jb.obs, off);
   const int ld_obs = jb.ld_obs;
   const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (b >= B) return;
@@ -446,17 +467,21 @@ __global__ void actor_sample_kernel(const ActorSampleJobs jobs, int ld_head, int
 // with the lanes striding over the inputs -- and writes tanh(mu) (explore = 0) or tanh(mu + std * eps).  `in` and `out` may
 // be mapped pinned host memory: the kernel then reads the observation and writes the action over PCIe itself and the host
 // only synchronises, no copy calls (the path main.py takes once per environment step).
+template <bool MEMBERS>
 __global__ void __launch_bounds__(256) actor_act_kernel(const float* __restrict__ in, int S, int A, int H,
                                                         const float* __restrict__ W0, int ld0, const float* __restrict__ b0,
                                                         const float* __restrict__ W1, int ld1, const float* __restrict__ b1,
                                                         const float* __restrict__ W2, int ld2, const float* __restrict__ b2,
-                                                        int explore, float* __restrict__ out) {
+                                                        int explore, float* __restrict__ out, long long mstride) {
   extern __shared__ float sm[];
+  const long long off = member_offset<MEMBERS>(mstride);
+  W0 = member_ptr(W0, off); b0 = member_ptr(b0, off); W1 = member_ptr(W1, off); b1 = member_ptr(b1, off);
+  W2 = member_ptr(W2, off); b2 = member_ptr(b2, off);
   float* x = sm;                 // [S]
   float* h1 = x + ((S + 3) & ~3);  // [H]
   float* h2 = h1 + H;            // [H]
   float* hd = h2 + H;            // [2A]
-  const int row = blockIdx.x, warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
+  const int row = (MEMBERS ? blockIdx.z * gridDim.x : 0) + blockIdx.x, warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
   const float* r = in + (size_t)row * (S + A);
   for (int j = threadIdx.x; j < S; j += blockDim.x) x[j] = r[j];
   __syncthreads();
@@ -487,11 +512,16 @@ __global__ void __launch_bounds__(256) actor_act_kernel(const float* __restrict_
   }
 }
 
+template <bool MEMBERS>
 __global__ void actor_sample_bwd_kernel(const float* __restrict__ head, int ld_head, int B, int A,
                                         const float* __restrict__ eps, const float* __restrict__ d_action, int ldd,
-                                        const float* __restrict__ dlogp_scalar, float* __restrict__ dhead, int ld_dh) {
+                                        const float* __restrict__ dlogp_scalar, float* __restrict__ dhead, int ld_dh,
+                                        long long mstride) {
   ptx::pdl_wait();
   ptx::pdl_launch_dependents();
+  const long long off = member_offset<MEMBERS>(mstride);
+  head = member_ptr(head, off); eps = member_ptr(eps, off); d_action = member_ptr(d_action, off);
+  dlogp_scalar = member_ptr(dlogp_scalar, off); dhead = member_ptr(dhead, off);
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B * A) return;
   const int b = i / A, j = i - b * A;
@@ -511,6 +541,7 @@ __global__ void actor_sample_bwd_kernel(const float* __restrict__ head, int ld_h
 }
 
 // ------------------------------------------------------------------------------------------- critic loss
+template <bool MEMBERS>
 __global__ void __launch_bounds__(256) td_critic_loss_kernel(const float* __restrict__ reward,
                                                              const float* __restrict__ done, int ld_rd,
                                                              const float* __restrict__ nq1,
@@ -519,8 +550,13 @@ __global__ void __launch_bounds__(256) td_critic_loss_kernel(const float* __rest
                                                              const float* __restrict__ q1, const float* __restrict__ q2,
                                                              int B, int norm_B, float gamma,
                                                              const Control* __restrict__ c, float* __restrict__ dq1,
-                                                             float* __restrict__ dq2, float* __restrict__ metrics) {
+                                                             float* __restrict__ dq2, float* __restrict__ metrics,
+                                                             long long mstride) {
   __shared__ float scratch[33];
+  const long long off = member_offset<MEMBERS>(mstride);
+  reward = member_ptr(reward, off); done = member_ptr(done, off); nq1 = member_ptr(nq1, off); nq2 = member_ptr(nq2, off);
+  logp2 = member_ptr(logp2, off); q1 = member_ptr(q1, off); q2 = member_ptr(q2, off); c = member_ptr(c, off);
+  dq1 = member_ptr(dq1, off); dq2 = member_ptr(dq2, off); metrics = member_ptr(metrics, off);
   const float alpha = c->alpha;
   const float inv_b = 1.f / (float)norm_B;
   float l1 = 0.f, l2 = 0.f, s1 = 0.f, s2 = 0.f;
@@ -547,14 +583,19 @@ __global__ void __launch_bounds__(256) td_critic_loss_kernel(const float* __rest
   }
 }
 
+template <bool MEMBERS>
 __global__ void __launch_bounds__(256) actor_alpha_loss_kernel(const float* __restrict__ q1,
                                                                const float* __restrict__ q2,
                                                                const float* __restrict__ logp, int B,
                                                                float target_entropy, int learn_alpha, Control* c,
                                                                float* __restrict__ dq1, float* __restrict__ dq2,
                                                                float* __restrict__ dlogp_scalar,
-                                                               float* __restrict__ metrics) {
+                                                               float* __restrict__ metrics, long long mstride) {
   __shared__ float scratch[33];
+  const long long off = member_offset<MEMBERS>(mstride);
+  q1 = member_ptr(q1, off); q2 = member_ptr(q2, off); logp = member_ptr(logp, off); c = member_ptr(c, off);
+  dq1 = member_ptr(dq1, off); dq2 = member_ptr(dq2, off); dlogp_scalar = member_ptr(dlogp_scalar, off);
+  metrics = member_ptr(metrics, off);
   const float alpha = c->alpha;
   const float inv_b = 1.f / (float)B;
   float la = 0.f, ent = 0.f, raw = 0.f;
@@ -800,13 +841,17 @@ __device__ __forceinline__ float adam_elem(float& p, float g, float& m, float& v
   return p;
 }
 
+template <bool MEMBERS>
 __global__ void __launch_bounds__(256) adam_polyak_kernel(float4* __restrict__ p, const float4* __restrict__ g,
                                                           float4* __restrict__ m, float4* __restrict__ v, size_t n4,
                                                           const AdamHyper* __restrict__ hyper,
                                                           float4* __restrict__ target, size_t n4_polyak, float tau,
-                                                          const int* __restrict__ polyak_flag) {
+                                                          const int* __restrict__ polyak_flag, long long mstride) {
   ptx::pdl_wait();
   ptx::pdl_launch_dependents();
+  const long long off = member_offset<MEMBERS>(mstride);
+  p = member_ptr(p, off); g = member_ptr(g, off); m = member_ptr(m, off); v = member_ptr(v, off);
+  hyper = member_ptr(hyper, off); target = member_ptr(target, off); polyak_flag = member_ptr(polyak_flag, off);
   const float ss = hyper->step_size, bc2s = hyper->bc2_sqrt;
   const bool do_polyak = target != nullptr && (polyak_flag == nullptr || *polyak_flag != 0);
   const float omt = 1.f - tau;
@@ -1071,16 +1116,17 @@ int grid_for(size_t work_items, int threads, int per_sm = 8) {
 
 }  // namespace
 
-void launch_tick(Control* c, const TickParams& p, cudaStream_t s) {
+void launch_tick(Control* c, const TickParams& p, cudaStream_t s, Members mb) {
   RLREP_CHECK(p.k_feat <= kMaxFeatureSteps, "too many feature steps per update");
-  launch_pdl(tick_kernel, 1, 32, 0, s, c, p);
+  launch_pdl((mb.n > 1 ? tick_kernel<true> : tick_kernel<false>), dim3(1, 1, mb.n), 32, 0, s, c, p, mb.stride);
   RLREP_LAUNCHED("tick", s);
 }
 
-void launch_gather(const float* ring, int rec4, const long long* idx, int B, float* out, cudaStream_t s) {
-  launch_pdl(gather_kernel, grid_for((size_t)B * rec4, 256), 256, 0, s, reinterpret_cast<const float4*>(ring), rec4, idx, B,
-             reinterpret_cast<float4*>(out));
-  RLREP_LAUNCHED_W("gather", s, 2.0 * 16.0 * (double)B * rec4, 0.0);
+void launch_gather(const float* ring, int rec4, const long long* idx, int B, float* out, cudaStream_t s, Members mb,
+                   const float* const* ring_slot) {
+  launch_pdl((mb.n > 1 ? gather_kernel<true> : gather_kernel<false>), dim3(grid_for((size_t)B * rec4, 256), 1, mb.n), 256, 0, s, reinterpret_cast<const float4*>(ring),
+             rec4, idx, B, reinterpret_cast<float4*>(out), ring_slot, mb.stride);
+  RLREP_LAUNCHED_W("gather", s, 2.0 * 16.0 * (double)B * rec4 * mb.n, 0.0);
 }
 
 void launch_ring_write(float* ring, int rec4, long long capacity, long long start, const float* rows, int n,
@@ -1097,24 +1143,25 @@ void launch_ce_rows(float* logits, int ld, int rows, int cols, int diag_off, flo
   RLREP_LAUNCHED_W("ce_rows", s, 3.0 * 4.0 * (double)rows * cols, 0.0);
 }
 
-void launch_rowdot(const float* X, int ld, int rows, int D, const float* w, const float* b, float* y, cudaStream_t s) {
+void launch_rowdot(const float* X, int ld, int rows, int D, const float* w, const float* b, float* y, cudaStream_t s,
+                   Members mb) {
   RowDotJobs js;
   js.j[0] = RowDotJob{X, w, b, y, ld, D};
   js.j[1] = js.j[0];
-  rowdot_kernel<<<dim3(rows, 1), 128, 0, s>>>(js, rows);
+  (mb.n > 1 ? rowdot_kernel<true> : rowdot_kernel<false>)<<<dim3(rows, 1, mb.n), 128, 0, s>>>(js, rows, mb.stride);
   RLREP_LAUNCHED("rowdot", s);
 }
 void launch_rowdot_pair(const RowDotJob& a, const RowDotJob& b, int rows, cudaStream_t s) {
   RowDotJobs js;
   js.j[0] = a;
   js.j[1] = b;
-  rowdot_kernel<<<dim3(rows, 2), 128, 0, s>>>(js, rows);
+  rowdot_kernel<false><<<dim3(rows, 2), 128, 0, s>>>(js, rows, 0LL);
   RLREP_LAUNCHED("rowdot", s);
 }
 
 void launch_colreduce(const float* X, int ld, int rows, int cols, const float* u, float* out, int accumulate,
-                      cudaStream_t s) {
-  colreduce_kernel<<<ceil_div(cols, 32), 256, 0, s>>>(X, ld, rows, cols, u, out, accumulate);
+                      cudaStream_t s, Members mb) {
+  (mb.n > 1 ? colreduce_kernel<true> : colreduce_kernel<false>)<<<dim3(ceil_div(cols, 32), 1, mb.n), 256, 0, s>>>(X, ld, rows, cols, u, out, accumulate, mb.stride);
   RLREP_LAUNCHED("colreduce", s);
 }
 
@@ -1142,7 +1189,7 @@ void launch_colsum_finish(const float* partial, int chunks, int cols, float* out
   RLREP_LAUNCHED("colsum_tall_final", s);
 }
 
-void launch_colreduce_multi(const ColJob* jobs, int n_jobs, cudaStream_t s) {
+void launch_colreduce_multi(const ColJob* jobs, int n_jobs, cudaStream_t s, Members mb) {
   RLREP_CHECK(n_jobs >= 1 && n_jobs <= kMaxColJobs, "too many column-reduction jobs for one launch");
   ColJobs js;
   int max_cols = 0;
@@ -1150,14 +1197,14 @@ void launch_colreduce_multi(const ColJob* jobs, int n_jobs, cudaStream_t s) {
     js.j[i] = jobs[i];
     if (jobs[i].cols > max_cols) max_cols = jobs[i].cols;
   }
-  launch_pdl(colreduce_multi_kernel, dim3(ceil_div(max_cols, 32), n_jobs), 1024, 0, s, js);
+  launch_pdl((mb.n > 1 ? colreduce_multi_kernel<true> : colreduce_multi_kernel<false>), dim3(ceil_div(max_cols, 32), n_jobs, mb.n), 1024, 0, s, js, mb.stride);
   RLREP_LAUNCHED("colreduce_multi", s);
 }
 
 void launch_outer_dact(const float* u, const float* w, int rows, int cols, const float* aux, int ld_aux, int dact,
-                       float* out, int ld_out, cudaStream_t s) {
-  outer_dact_kernel<<<grid_for((size_t)rows * cols, 256), 256, 0, s>>>(u, w, rows, cols, aux, ld_aux, dact, out,
-                                                                      ld_out);
+                       float* out, int ld_out, cudaStream_t s, Members mb) {
+  (mb.n > 1 ? outer_dact_kernel<true> : outer_dact_kernel<false>)<<<dim3(grid_for((size_t)rows * cols, 256), 1, mb.n), 256, 0, s>>>(u, w, rows, cols, aux, ld_aux, dact,
+                                                                                      out, ld_out, mb.stride);
   RLREP_LAUNCHED("outer_dact", s);
 }
 
@@ -1186,11 +1233,11 @@ void launch_actor_head(const ActorHeadArgs& a, cudaStream_t s) {
 }
 
 void launch_actor_sample(const float* head, int ld_head, int B, int A, const float* eps, float* action, int lda,
-                         float* logp, cudaStream_t s, const float* obs, int ld_obs, int S) {
+                         float* logp, cudaStream_t s, const float* obs, int ld_obs, int S, Members mb) {
   ActorSampleJobs js;
   js.j[0] = ActorSampleJob{head, eps, action, logp, obs, ld_obs};
   js.j[1] = js.j[0];
-  launch_pdl(actor_sample_kernel, dim3(ceil_div(B * 32, 128), 1), 128, 0, s, js, ld_head, B, A, lda, S);
+  launch_pdl((mb.n > 1 ? actor_sample_kernel<true> : actor_sample_kernel<false>), dim3(ceil_div(B * 32, 128), 1, mb.n), 128, 0, s, js, ld_head, B, A, lda, S, mb.stride);
   RLREP_LAUNCHED("actor_sample", s);
 }
 void launch_actor_sample_pair(const ActorSampleJob& j0, const ActorSampleJob& j1, int ld_head, int B, int A, int lda, int S,
@@ -1198,39 +1245,40 @@ void launch_actor_sample_pair(const ActorSampleJob& j0, const ActorSampleJob& j1
   ActorSampleJobs js;
   js.j[0] = j0;
   js.j[1] = j1;
-  launch_pdl(actor_sample_kernel, dim3(ceil_div(B * 32, 128), 2), 128, 0, s, js, ld_head, B, A, lda, S);
+  launch_pdl(actor_sample_kernel<false>, dim3(ceil_div(B * 32, 128), 2), 128, 0, s, js, ld_head, B, A, lda, S, 0LL);
   RLREP_LAUNCHED("actor_sample", s);
 }
 
 void launch_actor_act(const float* in, int rows, int S, int A, int H, const float* W0, int ld0, const float* b0,
                       const float* W1, int ld1, const float* b1, const float* W2, int ld2, const float* b2, int explore,
-                      float* out, cudaStream_t s) {
+                      float* out, cudaStream_t s, Members mb) {
   const size_t smem = (size_t)(((S + 3) & ~3) + 2 * H + 2 * A) * sizeof(float);
   RLREP_CHECK(smem <= 48 * 1024, "actor too wide for the one-launch select_action kernel");
-  actor_act_kernel<<<rows, 256, smem, s>>>(in, S, A, H, W0, ld0, b0, W1, ld1, b1, W2, ld2, b2, explore, out);
+  (mb.n > 1 ? actor_act_kernel<true> : actor_act_kernel<false>)<<<dim3(rows, 1, mb.n), 256, smem, s>>>(in, S, A, H, W0, ld0, b0, W1, ld1, b1, W2, ld2, b2, explore, out,
+                                                         mb.stride);
   RLREP_LAUNCHED("actor_act", s);
 }
 
 void launch_actor_sample_bwd(const float* head, int ld_head, int B, int A, const float* eps, const float* d_action,
-                             int ldd, const float* dlogp_scalar, float* dhead, int ld_dhead, cudaStream_t s) {
-  launch_pdl(actor_sample_bwd_kernel, ceil_div(B * A, 128), 128, 0, s, head, ld_head, B, A, eps, d_action, ldd, dlogp_scalar,
-             dhead, ld_dhead);
+                             int ldd, const float* dlogp_scalar, float* dhead, int ld_dhead, cudaStream_t s, Members mb) {
+  launch_pdl((mb.n > 1 ? actor_sample_bwd_kernel<true> : actor_sample_bwd_kernel<false>), dim3(ceil_div(B * A, 128), 1, mb.n), 128, 0, s, head, ld_head, B, A, eps, d_action, ldd,
+             dlogp_scalar, dhead, ld_dhead, mb.stride);
   RLREP_LAUNCHED("actor_sample_bwd", s);
 }
 
 void launch_td_critic_loss(const float* reward, const float* done, int ld_rd, const float* nq1, const float* nq2,
                            const float* logp2, const float* q1, const float* q2, int B, float gamma, const Control* c,
-                           float* dq1, float* dq2, float* metrics, cudaStream_t s, int norm_B) {
-  td_critic_loss_kernel<<<1, 256, 0, s>>>(reward, done, ld_rd, nq1, nq2, logp2, q1, q2, B, norm_B > 0 ? norm_B : B, gamma,
-                                          c, dq1, dq2, metrics);
+                           float* dq1, float* dq2, float* metrics, cudaStream_t s, int norm_B, Members mb) {
+  (mb.n > 1 ? td_critic_loss_kernel<true> : td_critic_loss_kernel<false>)<<<dim3(1, 1, mb.n), 256, 0, s>>>(reward, done, ld_rd, nq1, nq2, logp2, q1, q2, B,
+                                                         norm_B > 0 ? norm_B : B, gamma, c, dq1, dq2, metrics, mb.stride);
   RLREP_LAUNCHED("td_critic_loss", s);
 }
 
 void launch_actor_alpha_loss(const float* q1, const float* q2, const float* logp, int B, float target_entropy,
                              int learn_alpha, Control* c, float* dq1, float* dq2, float* dlogp_scalar, float* metrics,
-                             cudaStream_t s) {
-  actor_alpha_loss_kernel<<<1, 256, 0, s>>>(q1, q2, logp, B, target_entropy, learn_alpha, c, dq1, dq2, dlogp_scalar,
-                                            metrics);
+                             cudaStream_t s, Members mb) {
+  (mb.n > 1 ? actor_alpha_loss_kernel<true> : actor_alpha_loss_kernel<false>)<<<dim3(1, 1, mb.n), 256, 0, s>>>(q1, q2, logp, B, target_entropy, learn_alpha, c, dq1, dq2,
+                                                           dlogp_scalar, metrics, mb.stride);
   RLREP_LAUNCHED("actor_alpha_loss", s);
 }
 
@@ -1305,12 +1353,12 @@ void launch_group_mean_bwd(const float* dmean, const float* hid, int ld, int B, 
 }
 
 void launch_adam_polyak(float* p, const float* g, float* m, float* v, size_t n, const AdamHyper* hyper, float* target,
-                        size_t n_polyak, float tau, const int* polyak_flag, cudaStream_t s) {
+                        size_t n_polyak, float tau, const int* polyak_flag, cudaStream_t s, Members mb) {
   RLREP_CHECK(n % 4 == 0 && n_polyak % 4 == 0, "optimizer arenas are padded to float4");
   const size_t n4 = n / 4;
-  launch_pdl(adam_polyak_kernel, grid_for(n4, 256, 16), 256, 0, s, reinterpret_cast<float4*>(p),
+  launch_pdl((mb.n > 1 ? adam_polyak_kernel<true> : adam_polyak_kernel<false>), dim3(grid_for(n4, 256, 16), 1, mb.n), 256, 0, s, reinterpret_cast<float4*>(p),
              reinterpret_cast<const float4*>(g), reinterpret_cast<float4*>(m), reinterpret_cast<float4*>(v), n4, hyper,
-             reinterpret_cast<float4*>(target), n_polyak / 4, tau, polyak_flag);
+             reinterpret_cast<float4*>(target), n_polyak / 4, tau, polyak_flag, mb.stride);
   // 28 B/param (p, g, m, v read; p, m, v written) + 12 B/param of Polyak (p is already in registers: target read +
   // written = 8 B; counted as 12 like SURVEY.md 8d counts a stand-alone Polyak) -- a gated Polyak fires every 2nd step
   const double polyak = target ? 12.0 * (double)n_polyak * (polyak_flag ? 0.5 : 1.0) : 0.0;

@@ -2,12 +2,15 @@
 // replay gather, contrastive log-sum-exp / cross-entropy, reward head, N=1 critic heads, TD target and
 // critic loss, tanh-Gaussian actor sample / log-prob (forward + backward), actor / temperature loss,
 // the fused multi-tensor Adam + Polyak kernel and the per-update control-block "tick".
+// The launchers that take `Members mb` also run for a population (members.cuh): one launch covers all mb.n members, every
+// pointer argument is member 0's and member m works on its own copies, in exactly the order a lone launch does.
 #pragma once
 #include <cuda_runtime.h>
 
 #include <cstdint>
 
 #include "epilogue.cuh"
+#include "members.cuh"
 
 namespace rlrep {
 
@@ -39,10 +42,12 @@ struct TickParams {
   int critic_steps;        // 1 if the critic optimiser steps this agent (0 for diffsrsac, SURVEY A.6 #1)
 };
 
-void launch_tick(Control* c, const TickParams& p, cudaStream_t s);
+void launch_tick(Control* c, const TickParams& p, cudaStream_t s, Members mb = Members());
 
-// Replay gather: out[b, :] = ring[idx[b], :], rows are rec4 float4 wide (128-bit loads/stores).
-void launch_gather(const float* ring, int rec4, const long long* idx, int B, float* out, cudaStream_t s);
+// Replay gather: out[b, :] = ring[idx[b], :], rows are rec4 float4 wide (128-bit loads/stores).  ring_slot != nullptr: the
+// ring is *ring_slot, a device word in the (member's) arena -- a population's members each sample their own ring.
+void launch_gather(const float* ring, int rec4, const long long* idx, int B, float* out, cudaStream_t s,
+                   Members mb = Members(), const float* const* ring_slot = nullptr);
 // Scatter of freshly added rows into the ring at slots (start + i) % capacity.
 void launch_ring_write(float* ring, int rec4, long long capacity, long long start, const float* rows, int n,
                        cudaStream_t s);
@@ -53,7 +58,8 @@ void launch_ce_rows(float* logits, int ld, int rows, int cols, int diag_off, flo
                     cudaStream_t s);
 
 // y[i] = sum_j X[i,j] w[j] + b[0]  (N = 1 linear heads; one CTA per row)
-void launch_rowdot(const float* X, int ld, int rows, int D, const float* w, const float* b, float* y, cudaStream_t s);
+void launch_rowdot(const float* X, int ld, int rows, int D, const float* w, const float* b, float* y, cudaStream_t s,
+                   Members mb = Members());
 // Two such heads over the same rows in one launch (the twin Q heads).
 struct RowDotJob {
   const float* X;
@@ -65,7 +71,7 @@ struct RowDotJob {
 void launch_rowdot_pair(const RowDotJob& a, const RowDotJob& b, int rows, cudaStream_t s);
 // out[j] (+)= sum_i u[i] * X[i,j]   (u == nullptr: plain column sum).  Deterministic.
 void launch_colreduce(const float* X, int ld, int rows, int cols, const float* u, float* out, int accumulate,
-                      cudaStream_t s);
+                      cudaStream_t s, Members mb = Members());
 // out[j] = sum_i X[i, j] for very tall X (rows ~ 1e5..1e6): `chunks` CTAs per 32 columns, partial is [chunks, cols].
 // C[m, n] = epilogue(sum_g ws[g * group_stride + m * ldw + n]): the finish of a K-grouped GEMM (GemmArgs::k_groups), groups
 // added in order.
@@ -84,10 +90,10 @@ struct ColJob {
   int ld, rows, cols;
 };
 constexpr int kMaxColJobs = 8;
-void launch_colreduce_multi(const ColJob* jobs, int n_jobs, cudaStream_t s);
+void launch_colreduce_multi(const ColJob* jobs, int n_jobs, cudaStream_t s, Members mb = Members());
 // out[i,j] = u[i] * w[j] * dact(aux[i,j])   (backward of an N = 1 head into its hidden layer)
 void launch_outer_dact(const float* u, const float* w, int rows, int cols, const float* aux, int ld_aux, int dact,
-                       float* out, int ld_out, cudaStream_t s);
+                       float* out, int ld_out, cudaStream_t s, Members mb = Members());
 
 // Reward head loss (ctrlsac_agent.py:233): r_loss = 0.5 * mean((pred - r)^2); dpred = (pred - r) * inv_batch.
 // Also finishes the feature metrics: model_loss = sum(loss_rows) * inv_batch, total = model + r.
@@ -98,7 +104,8 @@ void launch_feature_loss_finalize(const float* loss_rows, int rows, const float*
 //   head [B, ld_head >= 2A] = (mu | raw log-std); eps [B, A];  out action [B, lda] (tanh(u)), logp [B]
 // obs != nullptr: also copy obs[b, 0:S] to action[b, -S:0], i.e. build the contiguous cat(obs, action) row.
 void launch_actor_sample(const float* head, int ld_head, int B, int A, const float* eps, float* action, int lda,
-                         float* logp, cudaStream_t s, const float* obs = nullptr, int ld_obs = 0, int S = 0);
+                         float* logp, cudaStream_t s, const float* obs = nullptr, int ld_obs = 0, int S = 0,
+                         Members mb = Members());
 // Two independent launch_actor_sample calls with the same shapes (ld_head, B, A, lda, S) as one launch.
 struct ActorSampleJob {
   const float* head;
@@ -118,19 +125,21 @@ void launch_contrastive_head(float* logits, int ld, int rows, int cols, int diag
                              float* loss_rows, float* pred, float* dpred, float* metrics, unsigned* counter,
                              cudaStream_t s);
 // select_action / batched policy evaluation in one launch: out[r, :] = tanh(mu(in[r, :S]) (+ std * in[r, S:S+A] if explore));
-// `in` / `out` may be mapped pinned host memory (see actor_act_kernel).
+// `in` / `out` may be mapped pinned host memory (see actor_act_kernel).  A population evaluates `rows` rows per member:
+// member m's rows follow member m - 1's in `in` and `out`, and its weights are at mb.stride * m bytes from W0 ... b2.
 void launch_actor_act(const float* in, int rows, int S, int A, int H, const float* W0, int ld0, const float* b0,
                       const float* W1, int ld1, const float* b1, const float* W2, int ld2, const float* b2, int explore,
-                      float* out, cudaStream_t s);
+                      float* out, cudaStream_t s, Members mb = Members());
 void launch_actor_sample_bwd(const float* head, int ld_head, int B, int A, const float* eps, const float* d_action,
-                             int ldd, const float* dlogp_scalar, float* dhead, int ld_dhead, cudaStream_t s);
+                             int ldd, const float* dlogp_scalar, float* dhead, int ld_dhead, cudaStream_t s,
+                             Members mb = Members());
 
 // TD target + twin-critic MSE (ctrlsac_agent.py:263-286; sac_agent.py:112-123):
 //   y = r + (1 - d) * gamma * (min(nq1, nq2) - alpha * logp2)
 //   dq1 = 2 (q1 - y) / B, dq2 likewise;  metrics[0..3] = q1_loss, q2_loss, mean(q1), mean(q2)
 void launch_td_critic_loss(const float* reward, const float* done, int ld_rd, const float* nq1, const float* nq2,
                            const float* logp2, const float* q1, const float* q2, int B, float gamma, const Control* c,
-                           float* dq1, float* dq2, float* metrics, cudaStream_t s, int norm_B = 0);
+                           float* dq1, float* dq2, float* metrics, cudaStream_t s, int norm_B = 0, Members mb = Members());
 
 // Fused heads of the chained CTRL critic / actor steps (kernels.cu "fused SAC heads"): hid_t / hid are [B, 2H] hidden
 // activations of the twin critic (target / live), w2 / w5 the two N = 1 heads; outputs as the kernels they replace.
@@ -171,7 +180,7 @@ void launch_actor_head(const ActorHeadArgs& a, cudaStream_t s);
 //   metrics[0..2] = actor_loss, alpha_loss, alpha (after the step, like `info['alpha'] = self.alpha`).
 void launch_actor_alpha_loss(const float* q1, const float* q2, const float* logp, int B, float target_entropy,
                              int learn_alpha, Control* c, float* dq1, float* dq2, float* dlogp_scalar, float* metrics,
-                             cudaStream_t s);
+                             cudaStream_t s, Members mb = Members());
 
 // Batch-sharded pieces (agent_ctrlsac_dp.cu).  norm_B = GLOBAL batch: every mean is a partial sum / norm_B that the
 // caller all-reduces.  partial = {share of actor_loss, share of mean(-logp - target_entropy)}; alpha_step consumes the
@@ -336,7 +345,7 @@ void launch_scale_inplace(float* p, size_t n, float scale, cudaStream_t s);  // 
 //   torch.optim.Adam defaults: beta = (0.9, 0.999), eps = 1e-8, no weight decay / amsgrad.
 //   target[0:n_polyak] = tau * p_new + (1 - tau) * target   when *polyak_flag != 0 (or flag == nullptr).
 void launch_adam_polyak(float* p, const float* g, float* m, float* v, size_t n, const AdamHyper* hyper, float* target,
-                        size_t n_polyak, float tau, const int* polyak_flag, cudaStream_t s);
+                        size_t n_polyak, float tau, const int* polyak_flag, cudaStream_t s, Members mb = Members());
 // Polyak only (critic_target of agents whose critic optimiser never steps).
 void launch_polyak(const float* p, float* target, size_t n, float tau, const int* polyak_flag, cudaStream_t s);
 

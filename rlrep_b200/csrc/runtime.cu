@@ -219,6 +219,7 @@ bool GemmRunner::run_compact(GemmArgs a, int wp, int ho, cudaStream_t s) {
 }
 
 void GemmRunner::run(const GemmArgs& a, cudaStream_t s) {
+  RLREP_CHECK(a.mb.n == 1 || !recording_, "population GEMMs do not join GEMM chains");
   if (recording_) {
     if (chain_eligible(a)) {
       pending_.push_back(a);
@@ -238,7 +239,7 @@ void GemmRunner::run(const GemmArgs& a, cudaStream_t s) {
   // Deep and skinny (the pixel agents' 39,200-wide linears at batch 256: K = 39,200 and 2 x 1..4 tiles): a split-K cluster
   // holds 8 CTAs, so such a GEMM runs on 16-64 CTAs that stream ~5 MB each.  Cut K into groups (GemmArgs::k_groups: own
   // cluster and raw partial output each), then one elementwise pass adds the groups and applies the epilogue.
-  if (a.k_groups == 1 && a.conv_w == 0 && a.conv_wgrad_hi == 0 && !recording_) {
+  if (a.k_groups == 1 && a.conv_w == 0 && a.conv_wgrad_hi == 0 && !recording_ && a.mb.n == 1) {
     const int tiles = ceil_div(a.M, 128) * ceil_div(a.N, 128), nkb = ceil_div(a.K, 32);
     int groups = 1;
     constexpr int kCtaCap = 296;  // up to two waves of CTAs (measured on the muLV update: 148 -> 5.82 ms, 296 -> 5.77 ms)
@@ -280,6 +281,7 @@ void GemmRunner::run(const GemmArgs& a, cudaStream_t s) {
     k->epi.pre_out = a.epi.pre_out; k->epi.ld_aux = a.epi.ld_aux; k->epi.ld_pre = a.epi.ld_pre;
     k->epi.act = a.epi.act; k->epi.dact = a.epi.dact; k->epi.accumulate = a.epi.accumulate;
     k->epi.scale = a.epi.scale;
+    k->mb.n = a.mb.n; k->mb.stride = a.mb.stride;
     k->K1 = sm_share_ < 0.75 ? 1 : 0;  // (K1 is unused on this path) plans differ with the share of the GPU
   }
   auto it = plans_.find(key);
@@ -302,6 +304,7 @@ void linear_fwd(GemmRunner& g, cudaStream_t s, int rows, Mat x, const Linear& l,
   a.epi.bias = l.b;
   a.epi.act = act;
   if (pre_out) { a.epi.pre_out = pre_out; a.epi.ld_pre = ldy; }
+  a.mb = g.members();
   g.run(a, s);
 }
 
@@ -314,6 +317,7 @@ void linear_dgrad(GemmRunner& g, cudaStream_t s, int rows, Mat dy, const Linear&
   a.C = dx; a.ldc = lddx;
   a.epi.dact = dact;
   a.epi.aux = aux.p; a.epi.ld_aux = aux.ld;
+  a.mb = g.members();
   g.run(a, s);
 }
 
@@ -331,6 +335,7 @@ void linear_wgrad(GemmRunner& g, cudaStream_t s, int rows, Mat dy, Mat x, const 
     a.A = dy.p; a.lda = dy.ld; a.a_mn = true;
     a.B = x.p; a.ldb = x.ld; a.b_mn = true;
     a.C = l.dW; a.ldc = l.ld;
+    a.mb = g.members();
     g.run(a, s);
   } else {
     // two input segments -> two column blocks of dW
@@ -339,6 +344,7 @@ void linear_wgrad(GemmRunner& g, cudaStream_t s, int rows, Mat dy, Mat x, const 
     a.A = dy.p; a.lda = dy.ld; a.a_mn = true;
     a.B = x.p; a.ldb = x.ld; a.b_mn = true;
     a.C = l.dW; a.ldc = l.ld;
+    a.mb = g.members();
     g.run(a, s);
     GemmArgs b = a;
     b.N = l.in - k1;
@@ -346,7 +352,7 @@ void linear_wgrad(GemmRunner& g, cudaStream_t s, int rows, Mat dy, Mat x, const 
     b.C = l.dW + k1;
     g.run(b, s);
   }
-  if (bias_grad) launch_colreduce(dy.p, dy.ld, rows, l.out, nullptr, l.db, 0, s);
+  if (bias_grad) launch_colreduce(dy.p, dy.ld, rows, l.out, nullptr, l.db, 0, s, g.members());
 }
 
 // ================================================================================================ GraphReplay
